@@ -16,6 +16,9 @@ Default workload: N=1 -> c2 = configs[1] (20 x 8192 SIFT-128, the configuration 
 `value`  : ordered descriptor pairs / device time of the step, inputs resident in HBM (max over ranks).
 `e2e`    : same metric through the public call with pinned HOST buffers (H2D + D2H inside the timed region).
 Prints ONE JSON line on rank 0.
+--dump-outputs DIR: the match lists of the last timed step as DIR/<name>.npy (float64), for comparing two builds output
+                    for output: pair_ptr [n*n + 1] (rows of cell (i, j) are pair_ptr[i + j*n] : pair_ptr[i + j*n + 1]),
+                    matches [M x 2] (1-based feature indices, as in the `matches` cell) and, pairwise, metric [M].
 """
 from __future__ import annotations
 
@@ -51,6 +54,7 @@ CONFIGS = {   # name -> (synth config id, kind, workload label)
     "c5": (5, "pairwise", "C5: 300 images x 4096 KAZE-64 f32 keypoints, pairwise exhaustive 2-NN, ratio 0.7, threshold 1.5"),
 }
 C5_INPUT = {"Matchingmethod": "Exhaustive", "Matchingthreshold": 1.5, "Ratiothreshold": 0.7, "useMATLABFeatureMatch": 0}
+DUMP_LIMIT = 64 << 20   # bytes --dump-outputs may write; the largest, c5 (0.65 M match rows and their metric), needs about 16 MB
 
 
 def default_config(n_gpus):
@@ -195,6 +199,30 @@ def blas_exhaustive_rate(X, nq):
     return {"engine": "numpy sgemm + argpartition (nearest2SSDExhaustive's blocked GEMM form, k = %d)" % KNN,
             "value": nq * float(F) / dt, "unit": UNIT, "cores": os.cpu_count(),
             "sample": f"{nq} query rows x all {F} train rows in blocks of {block} rows ({dt:.1f} s), scaled linearly"}
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy in float64 (exact for every index, offset and distance here)."""
+    arrays = {name: np.ascontiguousarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: the outputs take {total} bytes, more than --dump-outputs writes ({DUMP_LIMIT})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def pairwise_csr_of_shares(counts, rows_all, met_all):
+    """One CSR (pair_ptr, rows, metric) of the whole pair list from the per-rank shares in the layout of
+    multigpu.exchange_pairwise_lists (counts [world x cells], rows [world x Mmax x 2], metric [world x Mmax]); every cell
+    was computed by exactly one rank."""
+    starts = np.cumsum(counts, axis=1) - counts          # offset of each cell in its rank's buffer
+    total = counts.sum(axis=0)
+    owner = counts.argmax(axis=0)
+    spans = [(owner[c], starts[owner[c], c], starts[owner[c], c] + total[c]) for c in np.flatnonzero(total)]
+    rows = np.concatenate([rows_all[r, a:b] for r, a, b in spans] or [np.zeros((0, 2), rows_all.dtype)])
+    met = np.concatenate([met_all[r, a:b] for r, a, b in spans] or [np.zeros(0, met_all.dtype)])
+    return np.concatenate([[0], np.cumsum(total)]), rows, met
 
 
 def base_config(cfg, desc, ratio):
@@ -367,6 +395,8 @@ def run_ours(args, rank, world, local_rank):
     ms_per_step = total_ms / args.steps
     value = pairs_total / (ms_per_step / 1e3)
     multi_csr = plan.download() if rank == 0 else None     # the lists of the last timed step (all ranks' records)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pair_ptr": multi_csr[2], "matches": multi_csr[3]})
 
     # ---- end to end: pinned host buffers in, host match lists out -------------------------------
     def step_e2e():
@@ -474,7 +504,7 @@ def run_ours(args, rank, world, local_rank):
             same = np.array_equal(gi, oi) and np.array_equal(gd.view(np.uint32), od.view(np.uint32))
             line["parity_check"] = ("ok" if same else "MISMATCH") + f": kNN rows [0,{nq}) == oracle (indices and float bits)"
         if world == 1 and cfg == "c2" and not args.no_extra:
-            line["config6_real_valued_ms"] = real_valued_step_ms(pkg, ctx, torch, stream, flush)
+            line["config6_real_valued_ms"] = real_valued_step_ms(pkg, ctx, torch, stream, flush, args.steps)
         print(json.dumps(line), flush=True)
     plan.close()
     for p in host_ptrs:
@@ -483,7 +513,7 @@ def run_ours(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
-def real_valued_step_ms(pkg, ctx, torch, stream, flush, steps=5):
+def real_valued_step_ms(pkg, ctx, torch, stream, flush, steps):
     """The C2-sized set with REAL-valued SIFT-like descriptors (synth config 6: not exactly representable in bf16, what
     MATLAB's single SIFT / KAZE deliver): device ms per step of the same pipeline, beside the integer-SIFT headline."""
     desc, c = pkg.synth.make_config(6)
@@ -564,6 +594,12 @@ def run_ours_pairwise(args, rank, world, local_rank, pkg, ctx, stream, cfg, torc
     launches = L.aps_launch_count() - launches0
     tc_ms, tc_launches = ctx.tc_time()
     stats = ctx.last_stats()
+    if args.dump_outputs:   # every rank's share of the last timed step, merged on rank 0
+        shares = ((np.diff(mine[0])[None], mine[1][None], mine[2][None]) if world == 1 else
+                  pkg.multigpu.exchange_pairwise_lists(*mine, world, dist, torch, "cuda"))
+        if rank == 0:
+            pp, rows, met = pairwise_csr_of_shares(*shares)
+            dump_outputs(args.dump_outputs, {"pair_ptr": pp, "matches": rows, "metric": met})
     total_ms = sum(times)
     if world > 1:
         t = torch.tensor([total_ms, tc_ms], dtype=torch.float64, device="cuda")
@@ -659,13 +695,17 @@ def run_ours_pairwise(args, rank, world, local_rank, pkg, ctx, stream, cfg, torc
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every timed loop (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default=None, choices=sorted(CONFIGS), help="default: c2 on one GPU, c3 on several")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the real-valued (config 6) side measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the match lists of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)   # timing rule: at least 3 untimed warm-up steps
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

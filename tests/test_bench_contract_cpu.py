@@ -44,6 +44,39 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+
+
+def test_pairwise_shares_merge_into_one_csr():
+    """--dump-outputs on several ranks: the block-cyclic shares of the pair list (as multigpu.exchange_pairwise_lists
+    returns them) merge into the CSR one rank computes."""
+    import numpy as np
+
+    import bench
+
+    n, world = 6, 4
+    rng = np.random.default_rng(1)
+    counts = np.zeros(n * n, np.int64)
+    pairs = [i + j * n for j in range(n) for i in range(j)]          # column-major pair list
+    counts[pairs] = rng.integers(0, 4, len(pairs))
+    pp = np.concatenate([[0], np.cumsum(counts)])
+    rows = rng.integers(1, 1000, (pp[-1], 2)).astype(np.uint32)
+    met = rng.random(pp[-1])
+    share_counts = np.zeros((world, n * n), np.int64)
+    for o, c in enumerate(pairs):
+        share_counts[o % world, c] = counts[c]
+    m_max = int(share_counts.sum(1).max())
+    rows_all, met_all = np.zeros((world, m_max, 2), np.uint32), np.zeros((world, m_max))
+    for r in range(world):
+        mine = np.concatenate([np.arange(pp[c], pp[c + 1]) for c in range(n * n) if share_counts[r, c]] or [[]]).astype(int)
+        rows_all[r, :len(mine)], met_all[r, :len(mine)] = rows[mine], met[mine]
+    got_pp, got_rows, got_met = bench.pairwise_csr_of_shares(share_counts, rows_all, met_all)
+    assert np.array_equal(got_pp, pp) and np.array_equal(got_rows, rows) and np.array_equal(got_met, met)
+
+
 def test_product_arm_needs_a_gpu():
     import torch
 
