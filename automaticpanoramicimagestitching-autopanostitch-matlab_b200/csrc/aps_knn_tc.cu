@@ -12,31 +12,34 @@
 // per-pair sweeps of <= 48 tiles, the branch-free SEGMENT epilogue (KCT == 3, CS == 2; see top2_of_32 below):
 // 16 epilogue warps, two sorted lists of three per row, no data-dependent branch.
 //
-// CTA = 352 threads, persistent over work units.  A unit = TWO 128-row query blocks (256 rows, both A
+// CTA = 384 threads (three warpgroups), persistent over work units.  A unit = TWO 128-row query blocks (256 rows, both A
 // tiles resident in shared memory) x a range of 128-column train tiles; every B tile feeds two MMA
 // groups (one per row block), which halves the operand traffic per output and lets each query row be
 // owned by exactly ONE epilogue thread -- one top-K' list per row, half the insertions of a
 // column-split epilogue.
-//   warp 0   : TMA producer  (two A tiles per unit; per step one B tile + per-column (scale,bias))
+//   warp 0   : TMA producer  (two A tiles per unit; per step one B tile, + per-column (scale,bias) on short sweeps)
 //   warps 1-2: one single-thread tcgen05.mma issuer per row block (warp 1 also owns the TMEM allocation);
 //              independent issuers remove head-of-line blocking between the two epilogue groups
-//   warps 3-6: epilogue group 0 = row block 0, warps 7-10: group 1 = row block 1 (thread == query row,
+//   warp 3   : idle (warpgroup 0 = the control warps: setmaxnreg.dec to 48 registers, setmaxnreg.inc to 224 for the
+//              epilogue warpgroups, which no longer spill; 20 warps, 64 / 104 for the KCT == 3 variant)
+//   warps 4-7: epilogue group 0 = row block 0, warps 8-11: group 1 = row block 1 (thread == query row,
 //              tcgen05.ld 32x32b from the warp's TMEM lane quadrant).  Long sweeps (PRE), per 128-column tile:
-//              (1) straight-line scan: all four tcgen05.ld .x32 in flight, 16 FMNMX3 trees = the maxima of the 16
+//              (1) straight-line scan: tcgen05.ld .x32 double-buffered, 16 FMNMX3 trees = the maxima of the 16
 //                  8-column groups of RAW accumulators, against a per-tile threshold derived from the row's K'-th
 //                  best (theta) and the tile's (min,max) column scale / bias (aps_k_tile_bounds; the train view
 //                  is sorted by scale so the bounds are tight) -- no per-column constant, no multiply;
 //              (2) ONE warp vote; no lane flagged a group -> next tile (~270 instructions per tile and warp);
 //              (3) otherwise the union of the flagged groups is RE-READ from TMEM (tcgen05.ld .x8, rounds of four)
 //                  by the converged warp, the slot is handed back to the tensor pipe, and the flagged lanes scale
-//                  (broadcast LDS.128 of the constants), search and replace-min: scores in registers as packed
+//                  (the groups' constants read from L2 with LDG.128, issued before the re-read; no per-tile wait on a
+//                  constants ring), search and replace-min: scores in registers as packed
 //                  keys (value bits & ~7 | slot), train-row indices in shared memory.  One run-time-indexed copy
 //                  of the insertion code.
 //              Short sweeps (!PRE: the lists never leave their filling phase) keep the per-chunk loop: scale every
 //              32-column chunk, group maxima, branch-free replace-min for the groups that hold a candidate.
 // TMEM: 4 accumulator slots of 128 columns = slot(tile parity, row block): the tensor pipe fills the
 // slots of tile t+1 while both groups drain tile t.  Pipelines (all mbarrier based): B ring (4 x 32 KB),
-// A pair (single buffered per unit), accumulator slots, (scale,bias) ring.
+// A pair (single buffered per unit), accumulator slots, (scale,bias) ring (short sweeps only).
 // Scheduling: units that fill whole rounds of the grid span all train tiles; the last, partial round is
 // balanced either by cutting its units into <= 4 equal column segments or by cutting its tile steps into
 // one equal share per CTA (make_schedule), each piece filling its own candidate list of the row.
@@ -44,8 +47,9 @@
 // What bounds it (C2 = 163840^2 pairs, D = 128; profiles/r2_ncu_history.txt, profiles/r2_ncu_k_knn_tc.txt):
 //   * accumulators never read (-DAPS_TC_NOEPI): TMA + MMA alone 3.39 ms = 2027 TFLOP/s -- the floor of this tiling
 //     (85 % of nominal; the same with the A operand in TMEM: shared-memory bandwidth is not the limiter);
-//   * full kernel 4.71-4.87 ms = 1410-1460 TFLOP/s = 0.88-0.90 of the measured cuBLAS bf16 burst figure (round 1:
-//     5.79 ms; per-chunk group-gated version: 5.32 ms); C3 (F = 1e6, long sweeps) 1635 TFLOP/s = 1.01 of it.
+//   * full kernel 4.60 ms = 1493 TFLOP/s = 0.92 of the measured cuBLAS bf16 burst figure (B200, 1000 W, 1965 MHz;
+//     round 2: 4.71-4.87 ms, before the register split and the removal of the constants ring on long sweeps; round 1:
+//     5.79 ms; per-chunk group-gated version: 5.32 ms); C3 (F = 1e6, long sweeps) 1635 TFLOP/s = 1.01 of it (round 2).
 //     What is left at C2 is the VARIANCE of the epilogue: a tile with insertions (39 % of them) takes ~4x the cycles
 //     of one without, and two accumulator slots per row block cannot average that out: the epilogue warps wait for
 //     acc_full 22 % of their time while the issuers spin on acc_empty.  K'(1 + ln(F/K')) ~ 67 insertions per row are
@@ -77,7 +81,10 @@ constexpr int KC = 8;          // candidates per (row, segment)
 constexpr int CSPLIT = 1;      // epilogue groups per row block (each scans TN/CSPLIT columns of every tile, own list)
 constexpr int MAX_SEG = 4 / CSPLIT;  // column segments of a tail unit; a row has MAX_SEG*CSPLIT <= 4 candidate lists
 constexpr int NUM_EPI_WARPS = 4 * RB * CSPLIT;
-constexpr int FIRST_EPI_WARP = 1 + RB;  // warp 0 producer, warps 1..RB MMA issuers (one per row block)
+// warpgroup 0: warp 0 producer, warps 1..RB MMA issuers (one per row block), warp 3 idle; the epilogue groups start
+// at warpgroup 1, so that setmaxnreg (per warpgroup) can move registers from the control warps to the epilogue
+constexpr int FIRST_EPI_WARP = 4;
+static_assert(1 + RB <= FIRST_EPI_WARP, "producer and issuers fit in warpgroup 0");
 constexpr int NUM_THREADS = 32 * (FIRST_EPI_WARP + NUM_EPI_WARPS);
 static_assert(NUM_ACC_SLOTS * TN == 512, "TMEM budget");
 
@@ -89,6 +96,9 @@ struct Barriers {
   uint32_t tmem_base;
   uint32_t pad;
 };
+// byte distance from a full barrier to its empty partner: one base register per ring, the partner is an immediate offset
+constexpr uint32_t kAccEmptyOff = offsetof(Barriers, acc_empty) - offsetof(Barriers, acc_full);
+constexpr uint32_t kCsEmptyOff = offsetof(Barriers, cs_empty) - offsetof(Barriers, cs_full);
 
 // The row's top-KC list lives in shared memory, slot-major ([slot][row], conflict-free), descending
 // by score; addressed by 32-bit shared-window addresses (ld/st.shared, not generic).  Out of line
@@ -224,13 +234,26 @@ __device__ __forceinline__ void insert3(float x, uint32_t px, float& l1, float& 
   p1 = c1 ? px : p1;
 }
 constexpr uint32_t kKeyFloorBits = 0xff7fff80u;  // finite, below every real score: masked columns / empty entries
-constexpr int threads_for(int cs) { return 32 * (1 + RB + 4 * RB * cs); }
+__host__ __device__ constexpr int threads_for(int cs) { return 32 * (FIRST_EPI_WARP + 4 * RB * cs); }
+// Register split.  __launch_bounds__(threads, 1) makes ptxas allocate 65536 / threads registers per thread (rounded
+// down to 8) at launch: 168 for 384 threads, 96 for 640.  Warpgroup 0 (mbarrier waits and address arithmetic) drops to
+// kCtlRegs with setmaxnreg.dec; the epilogue warpgroups take what that frees with setmaxnreg.inc (224 and 104), so the
+// per-tile scan and the insertion code no longer spill.  The launcher checks the allocation: setmaxnreg.inc would wait
+// for ever if warpgroup 0 freed fewer registers than the epilogue asks for.
+__host__ __device__ constexpr int ctl_regs(int cs) { return cs == 1 ? 48 : 64; }
+__host__ __device__ constexpr int launch_regs(int cs) { return (65536 / threads_for(cs)) & ~7; }
+__host__ __device__ constexpr int epi_regs(int cs) {
+  return ((launch_regs(cs) * threads_for(cs) - 128 * ctl_regs(cs)) / (threads_for(cs) - 128)) & ~7;
+}
+static_assert(epi_regs(1) == 224 && epi_regs(2) == 104, "register split");
 
 // KCT = candidates kept per list: 8, or 4 for the per-pair searches (k = 2: fewer insertions on short sweeps)
 // CS = epilogue groups per row block (each scans TN/CS columns of every tile and keeps its own list)
 template <bool BIAS, bool DUMP, bool PRE, int KCT, int CS = CSPLIT>
 __global__ void __launch_bounds__(threads_for(CS), 1)
 k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_t, const KParams Pin) {
+  // PRE runs only the long-sweep scan below, which reads the per-column constants from global memory: no ring stage
+  static_assert(!PRE || (CS == 1 && !DUMP), "PRE has no (scale, bias) ring");
   // two launches cover one search when the list size depends on a device-side flag: the other one exits here
   if (Pin.variant_flag && ((*Pin.variant_flag != 0) != (Pin.variant_want != 0))) return;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -274,70 +297,83 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
   tc_fence_after();
   const uint32_t tmem_base = bars->tmem_base;
 
-  if (warp == 0) {
-    // ===================================== TMA producer =====================================
-    if (elect_one()) {
-      uint32_t bs = 0, bph = 0, aph = 0, cs = 0, cph = 0;
-      for (int64_t u = blockIdx.x; u < num_units; u += gridDim.x) {
-        const Unit x = get_unit(P, u);
-        if (x.tl >= x.th) continue;
-        mbar_wait_backoff(&bars->a_empty, aph ^ 1);   // every MMA of the previous unit has read its A tiles
-        mbar_arrive_expect_tx(&bars->a_full, (uint32_t)(RB * a_bytes));
-        for (int r = 0; r < RB; ++r)
-          for (int s = 0; s < ksl; ++s)
-            tma_load_2d(smem_a + r * a_bytes + s * (TM * 128), &map_q, s * KSLAB,
-                        (int)(x.qrow0 + r * TM), &bars->a_full);
-        aph ^= 1;
-        for (int64_t t = x.tl; t < x.th; ++t) {
-          mbar_wait_backoff(&bars->cs_empty[cs], cph ^ 1);
-          mbar_arrive_expect_tx(&bars->cs_full[cs], (BIAS ? 2u : 1u) * TN * (uint32_t)sizeof(float));
-          bulk_load_1d(smem_cs + cs * 2 * TN, P.colscale + t * TN, TN * (uint32_t)sizeof(float), &bars->cs_full[cs]);
-          if (BIAS)
-            bulk_load_1d(smem_cs + cs * 2 * TN + TN, P.colbias + t * TN, TN * (uint32_t)sizeof(float), &bars->cs_full[cs]);
-          if (++cs == NUM_CS_STAGES) { cs = 0; cph ^= 1; }
-          mbar_wait_backoff(&bars->b_empty[bs], bph ^ 1);
-          mbar_arrive_expect_tx(&bars->b_full[bs], (uint32_t)b_bytes);
-          for (int s = 0; s < ksl; ++s)
-            tma_load_2d(smem_b + bs * b_bytes + s * (TN * 128), &map_t, s * KSLAB, (int)(t * TN), &bars->b_full[bs]);
-          if (++bs == NUM_B_STAGES) { bs = 0; bph ^= 1; }
-        }
-      }
-    }
-  } else if (warp <= RB) {
-    // ===================================== MMA issuers =======================================
-    // One issuing thread per row block: each waits only for ITS epilogue group's accumulator slot, so a
-    // slow group (insertion-heavy tile) does not stall the other group's MMAs (no head-of-line blocking).
-    if (elect_one()) {
-      const int r = warp - 1;
-      const uint32_t idesc = P.idesc;
-      const uint32_t a_addr = smem_u32(smem_a + r * a_bytes);
-      uint32_t bs = 0, bph = 0, aph = 0, tcount = 0;
-      for (int64_t u = blockIdx.x; u < num_units; u += gridDim.x) {
-        const Unit x = get_unit(P, u);
-        if (x.tl >= x.th) continue;
-        mbar_wait(&bars->a_full, aph);
-        aph ^= 1;
-        for (int64_t t = x.tl; t < x.th; ++t, ++tcount) {
-          const uint32_t slot = (tcount & 1) * RB + r, acph = (tcount >> 1) & 1;
-          mbar_wait(&bars->acc_empty[slot], acph ^ 1);
-          mbar_wait(&bars->b_full[bs], bph);
-          tc_fence_after();
-          const uint32_t b_addr = smem_u32(smem_b + bs * b_bytes);
-          const uint32_t d_tmem = tmem_base + slot * TN;
-          for (int k = 0; k < kst; ++k) {
-            const int slab = k >> 2, kin = k & 3;  // 4 K steps (32 B each) per 128-byte swizzle row
-            const uint64_t adesc = make_kmajor_sw128_desc(a_addr + slab * (TM * 128) + kin * 32);
-            const uint64_t bdesc = make_kmajor_sw128_desc(b_addr + slab * (TN * 128) + kin * 32);
-            umma_bf16(d_tmem, adesc, bdesc, idesc, k > 0 ? 1u : 0u);
+  // ptxas gives each role the register budget of the setmaxnreg that dominates it: the split sits inside the
+  // role branches (a block reached from both sides gets the smaller budget), once per warpgroup
+  if (warp < FIRST_EPI_WARP) {
+    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(ctl_regs(CS)));
+    if (warp == 0) {
+      // ===================================== TMA producer =====================================
+      if (elect_one()) {
+        uint32_t bs = 0, bph = 0, aph = 0, cs = 0, cph = 0;
+        for (int64_t u = blockIdx.x; u < num_units; u += gridDim.x) {
+          const Unit x = get_unit(P, u);
+          if (x.tl >= x.th) continue;
+          mbar_wait_backoff(&bars->a_empty, aph ^ 1);   // every MMA of the previous unit has read its A tiles
+          mbar_arrive_expect_tx(&bars->a_full, (uint32_t)(RB * a_bytes));
+          for (int r = 0; r < RB; ++r)
+            for (int s = 0; s < ksl; ++s)
+              tma_load_2d(smem_a + r * a_bytes + s * (TM * 128), &map_q, s * KSLAB,
+                          (int)(x.qrow0 + r * TM), &bars->a_full);
+          aph ^= 1;
+          for (int64_t t = x.tl; t < x.th; ++t) {
+            if constexpr (!PRE) {  // long sweeps read the per-column constants of the few candidate groups from L2
+              mbar_wait_backoff(&bars->cs_empty[cs], cph ^ 1);
+              mbar_arrive_expect_tx(&bars->cs_full[cs], (BIAS ? 2u : 1u) * TN * (uint32_t)sizeof(float));
+              bulk_load_1d(smem_cs + cs * 2 * TN, P.colscale + t * TN, TN * (uint32_t)sizeof(float), &bars->cs_full[cs]);
+              if (BIAS)
+                bulk_load_1d(smem_cs + cs * 2 * TN + TN, P.colbias + t * TN, TN * (uint32_t)sizeof(float), &bars->cs_full[cs]);
+              if (++cs == NUM_CS_STAGES) { cs = 0; cph ^= 1; }
+            }
+            mbar_wait_backoff(&bars->b_empty[bs], bph ^ 1);
+            mbar_arrive_expect_tx(&bars->b_full[bs], (uint32_t)b_bytes);
+            for (int s = 0; s < ksl; ++s)
+              tma_load_2d(smem_b + bs * b_bytes + s * (TN * 128), &map_t, s * KSLAB, (int)(t * TN), &bars->b_full[bs]);
+            if (++bs == NUM_B_STAGES) { bs = 0; bph ^= 1; }
           }
-          tc_commit(&bars->acc_full[slot]);  // this row block's accumulator is ready for its epilogue group
-          tc_commit(&bars->b_empty[bs]);     // B stage reusable once BOTH issuers' MMAs have read it (count RB)
-          if (++bs == NUM_B_STAGES) { bs = 0; bph ^= 1; }
         }
-        tc_commit(&bars->a_empty);
       }
-    }
+    } else if (warp <= RB) {
+      // ===================================== MMA issuers =======================================
+      // One issuing thread per row block: each waits only for ITS epilogue group's accumulator slot, so a
+      // slow group (insertion-heavy tile) does not stall the other group's MMAs (no head-of-line blocking).
+      if (elect_one()) {
+        const int r = warp - 1;
+        const uint32_t idesc = P.idesc;
+        const uint32_t a_addr = smem_u32(smem_a + r * a_bytes);
+        const uint32_t b_addr0 = smem_u32(smem_b);
+        const uint32_t b_full0 = smem_u32(&bars->b_full[0]), b_empty0 = smem_u32(&bars->b_empty[0]);
+        // this row block's accumulator slots are r (even tiles) and RB + r (odd tiles)
+        const uint32_t acc_bar = smem_u32(&bars->acc_full[r]);
+        uint32_t bs = 0, bph = 0, aph = 0, par = 0, acph = 0;  // par = tile parity, acph = its slot's phase
+        for (int64_t u = blockIdx.x; u < num_units; u += gridDim.x) {
+          const Unit x = get_unit(P, u);
+          if (x.tl >= x.th) continue;
+          mbar_wait(&bars->a_full, aph);
+          aph ^= 1;
+          for (uint32_t i = 0, n = (uint32_t)(x.th - x.tl); i < n; ++i) {
+            mbar_wait(acc_bar + kAccEmptyOff + par * (RB * 8), acph ^ 1);
+            mbar_wait(b_full0 + bs * 8, bph);
+            tc_fence_after();
+            const uint32_t b_addr = b_addr0 + bs * b_bytes;
+            const uint32_t d_tmem = tmem_base + (par * RB + r) * TN;
+            for (int k = 0; k < kst; ++k) {
+              const int slab = k >> 2, kin = k & 3;  // 4 K steps (32 B each) per 128-byte swizzle row
+              const uint64_t adesc = make_kmajor_sw128_desc(a_addr + slab * (TM * 128) + kin * 32);
+              const uint64_t bdesc = make_kmajor_sw128_desc(b_addr + slab * (TN * 128) + kin * 32);
+              umma_bf16(d_tmem, adesc, bdesc, idesc, k > 0 ? 1u : 0u);
+            }
+            tc_commit(acc_bar + par * (RB * 8));  // this row block's accumulator is ready for its epilogue group
+            tc_commit(b_empty0 + bs * 8);           // B stage reusable once BOTH issuers' MMAs have read it (count RB)
+            if (++bs == NUM_B_STAGES) { bs = 0; bph ^= 1; }
+            par ^= 1;
+            acph ^= par ^ 1;  // back to the even slot: next phase
+          }
+          tc_commit(&bars->a_empty);
+        }
+      }
+    }  // warp 3: idle
   } else {
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(epi_regs(CS)));
     // ===================================== epilogue =========================================
     // Group g (4 warps, one per TMEM lane quadrant) owns row block g of the unit: thread == query row.
     const int quad = warp & 3;        // TMEM lane quadrant this warp may access
@@ -347,25 +383,36 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
     constexpr int CG = TN / CS;
     const int row_in_tile = quad * 32 + lane;
     const uint32_t si = smem_u32(smem_topi + (egrp * KC) * TM + row_in_tile);  // this row's index slots
-    uint32_t tcount = 0;  // tiles consumed so far (same sequence as the MMA warp's)
+    // Position in the tile sequence (the MMA issuer's): accumulator slot (tile parity) * RB + grp and its phase, and
+    // the (scale, bias) ring stage of short sweeps.  Barrier and TMEM addresses are 32-bit, computed once.
+    const uint32_t acc_bar = smem_u32(&bars->acc_full[grp]), cs_bar = smem_u32(&bars->cs_full[0]);
+    const uint32_t cs_smem0 = smem_u32(smem_cs + ch * CG);
+    const uint32_t tmem_row = tmem_base + ((uint32_t)(quad * 32) << 16) + grp * TN + ch * CG;
+    uint32_t par = 0, acph = 0, cs = 0, cph = 0;
+    auto next_tile = [&]() {
+      par ^= 1;
+      acph ^= par ^ 1;
+      if (!PRE && ++cs == NUM_CS_STAGES) { cs = 0; cph ^= 1; }
+    };
     for (int64_t u = blockIdx.x; u < num_units; u += gridDim.x) {
       const Unit x = get_unit(P, u);
       if (x.skip) continue;  // balanced tail: this CTA's share has no second piece
       const int64_t qrow = x.qrow0 + grp * TM + row_in_tile;
+      // train columns are 32-bit (cand_idx): tile loops count and compare in 32 bits.  A column segment can start past
+      // the last tile (tl > th: e.g. 5 tiles in 4 segments of 2): no tiles, but its lists are still written empty.
+      const uint32_t nt = x.th > x.tl ? (uint32_t)(x.th - x.tl) : 0u, ct0 = (uint32_t)x.t0, ct1 = (uint32_t)x.t1;
       if constexpr (KCT == 3) {
         // ---- short sweeps: branch-free two-best per segment, merged into the group's sorted top-3 of the row ----
         float l1 = __uint_as_float(kKeyFloorBits), l2 = l1, l3 = l1;
         uint32_t p1 = 0xffffffffu, p2 = 0xffffffffu, p3 = 0xffffffffu;
-        for (int64_t t = x.tl; t < x.th; ++t, ++tcount) {
-          const uint32_t slot = (tcount & 1) * RB + grp, acph = (tcount >> 1) & 1;
-          const uint32_t cs = tcount % NUM_CS_STAGES, cph = (tcount / NUM_CS_STAGES) & 1;
-          mbar_wait(&bars->acc_full[slot], acph);
-          mbar_wait(&bars->cs_full[cs], cph);
+        uint32_t col0 = (uint32_t)(x.tl * TN) + ch * CG;
+        for (uint32_t i = 0; i < nt; ++i, col0 += TN, next_tile()) {
+          mbar_wait(acc_bar + par * (RB * 8), acph);
+          mbar_wait(cs_bar + cs * 8, cph);
           tc_fence_after();
-          const uint32_t cscale = smem_u32(smem_cs + cs * 2 * TN + ch * CG);
-          const int64_t col0 = t * TN + ch * CG;
-          const bool partial = (col0 < x.t0) || (col0 + CG > x.t1);
-          const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + slot * TN + ch * CG;
+          const uint32_t cscale = cs_smem0 + cs * (2 * TN * 4);
+          const bool partial = (col0 < ct0) || (col0 + CG > ct1);
+          const uint32_t taddr = tmem_row + par * (RB * TN);
           float m1 = __uint_as_float(kKeyFloorBits), m2 = m1;
 #pragma unroll 1
           for (int c = 0; c < CG / 32; ++c) {
@@ -393,7 +440,7 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
             for (int j = 0; j < 32; ++j)  // key = score with the column-in-tile in the 7 low mantissa bits
               cur[j] = __uint_as_float((__float_as_uint(cur[j]) & ~127u) | (cbase + (uint32_t)j));
             if (partial) {  // first / last tile of the train image: foreign columns can never be selected
-              const int lo = (int)max(x.t0 - col0, (int64_t)0) - c * 32, hi = (int)min(x.t1 - col0, (int64_t)CG) - c * 32;
+              const int lo = max((int)(ct0 - col0), 0) - c * 32, hi = min((int)(ct1 - col0), CG) - c * 32;
 #pragma unroll
               for (int j = 0; j < 32; ++j)
                 if (j < lo || j >= hi) cur[j] = __uint_as_float(kKeyFloorBits | (cbase + (uint32_t)j));
@@ -404,10 +451,10 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
           tc_fence_before();
           __syncwarp();
           if (lane == 0) {
-            mbar_arrive(&bars->acc_empty[slot]);
-            mbar_arrive(&bars->cs_empty[cs]);
+            mbar_arrive(acc_bar + kAccEmptyOff + par * (RB * 8));
+            mbar_arrive(cs_bar + kCsEmptyOff + cs * 8);
           }
-          const uint32_t base = (uint32_t)(t * TN);
+          const uint32_t base = col0 - ch * CG;
           insert3(m1, base + (__float_as_uint(m1) & 127u), l1, l2, l3, p1, p2, p3);
           insert3(m2, base + (__float_as_uint(m2) & 127u), l1, l2, l3, p1, p2, p3);
         }
@@ -429,23 +476,23 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
       }
       float theta = bv[KCT - 1];    // min of bv == the row's K'-th best score so far (empty slots: -FLT_MAX)
       int minpos = KCT - 1;         // slot holding it
-      float4 tb_next = (PRE && x.tl < x.th) ? __ldg(P.tile_bounds + x.tl) : make_float4(0.f, 0.f, 0.f, 0.f);
-      for (int64_t t = x.tl; t < x.th; ++t, ++tcount) {
-        const uint32_t slot = (tcount & 1) * RB + grp, acph = (tcount >> 1) & 1;
-        const uint32_t cs = tcount % NUM_CS_STAGES, cph = (tcount / NUM_CS_STAGES) & 1;
-        mbar_wait(&bars->acc_full[slot], acph);
-        mbar_wait(&bars->cs_full[cs], cph);
+      const float4* tbp = P.tile_bounds + x.tl;
+      float4 tb_next = (PRE && nt > 0) ? __ldg(tbp) : make_float4(0.f, 0.f, 0.f, 0.f);
+      uint32_t col0 = (uint32_t)(x.tl * TN) + ch * CG;
+      for (uint32_t i = 0; i < nt; ++i, col0 += TN, next_tile()) {
+        const uint32_t acc_off = par * (RB * 8);
+        mbar_wait(acc_bar + acc_off, acph);
+        if (!PRE) mbar_wait(cs_bar + cs * 8, cph);
         tc_fence_after();
-        const uint32_t cscale = smem_u32(smem_cs + cs * 2 * TN + ch * CG);
-        const int64_t col0 = t * TN + ch * CG;
-        const bool partial = (col0 < x.t0) || (col0 + CG > x.t1);
-        const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + slot * TN + ch * CG;
+        const uint32_t cscale = cs_smem0 + cs * (2 * TN * 4);
+        const bool partial = (col0 < ct0) || (col0 + CG > ct1);
+        const uint32_t taddr = tmem_row + par * (RB * TN);
         // Conservative pre-filter on the RAW accumulators: a column can only beat theta if
         //   acc > (theta - bias_max(tile)) / scale_max(tile)     (1/scale_min when the numerator is negative);
         // train rows are sorted by scale (aps_prep.cu), so the bound is tight and the common path needs
         // neither the per-column constants nor a multiply.
         const float4 tb = tb_next;  // fetched one tile ahead: the global-load latency stays off the critical path
-        if (PRE && t + 1 < x.th) tb_next = __ldg(P.tile_bounds + t + 1);
+        if (PRE && i + 1 < nt) tb_next = __ldg(tbp + i + 1);
         auto pre_threshold = [&](float th) {
           const float num = th - tb.z - 1.0e-6f * (fabsf(th) + fabsf(tb.z));
           return num * (num >= 0.f ? tb.x : tb.y);
@@ -493,12 +540,10 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
             if (partial) pend = 0xffffu;
             uint32_t uni = __reduce_or_sync(0xffffffffu, pend);
             // one flagged group of this lane: scale, mask, insert (inlined once per stash position below)
-            auto search_group = [&](float(&v)[8], const int g) {
-              const float4 s0 = lds_f32x4(cscale + (8 * g) * 4);
-              const float4 s1 = lds_f32x4(cscale + (8 * g + 4) * 4);
+            auto search_group = [&](float(&v)[8], const int g, const float4 (&s)[2], const float4 (&b)[2]) {
+              const float4 s0 = s[0], s1 = s[1];
               if (BIAS) {
-                const float4 b0 = lds_f32x4(cscale + (TN + 8 * g) * 4);
-                const float4 b1 = lds_f32x4(cscale + (TN + 8 * g + 4) * 4);
+                const float4 b0 = b[0], b1 = b[1];
                 v[0] = fmaf(v[0], s0.x, b0.x); v[1] = fmaf(v[1], s0.y, b0.y);
                 v[2] = fmaf(v[2], s0.z, b0.z); v[3] = fmaf(v[3], s0.w, b0.w);
                 v[4] = fmaf(v[4], s1.x, b1.x); v[5] = fmaf(v[5], s1.y, b1.y);
@@ -510,8 +555,8 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
               if (partial) {  // first / last tile of the searched range: foreign columns can never be selected
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
-                  const int64_t col = col0 + 8 * g + j;
-                  if (col < x.t0 || col >= x.t1) v[j] = -CUDART_INF_F;
+                  const uint32_t col = col0 + 8 * g + j;
+                  if (col < ct0 || col >= ct1) v[j] = -CUDART_INF_F;
                 }
               }
               float gm = fmaxf(fmaxf(v[0], v[1]), v[2]);
@@ -522,10 +567,10 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
                 int js = 7;
 #pragma unroll
                 for (int j = 6; j >= 0; --j) js = (v[j] == gm) ? j : js;
-                sts_u32(si + minpos * SLOT_STRIDE, (uint32_t)(col0 + 8 * g + js));
+                sts_u32(si + minpos * SLOT_STRIDE, col0 + 8 * g + js);
                 const float key = __uint_as_float((__float_as_uint(gm) & ~7u) | (uint32_t)minpos);
 #pragma unroll
-                for (int i = 0; i < KCT; ++i) bv[i] = (i == minpos) ? key : bv[i];
+                for (int k = 0; k < KCT; ++k) bv[k] = (k == minpos) ? key : bv[k];
                 if constexpr (KCT == 8) {
                   float m01 = fminf(fminf(bv[0], bv[1]), bv[2]);
                   float m23 = fminf(fminf(bv[3], bv[4]), bv[5]);
@@ -554,6 +599,20 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
                 gq[q] = uni ? __ffs((int)uni) - 1 : 31;  // 31: no group (bit 31 of pend is never set)
                 uni &= uni - 1;
               }
+              // the groups' scales (and biases) straight from L2, in flight together with the TMEM re-read (same
+              // address in every lane: one request per load); no (scale, bias) ring stage to wait for on any tile
+              float4 gs[4][2], gb[4][2];
+#pragma unroll
+              for (int q = 0; q < 4; ++q) {
+                const float4* s4 = reinterpret_cast<const float4*>(P.colscale + col0 + 8 * (gq[q] & 15));
+                gs[q][0] = __ldg(s4);
+                gs[q][1] = __ldg(s4 + 1);
+                if (BIAS) {
+                  const float4* b4 = reinterpret_cast<const float4*>(P.colbias + col0 + 8 * (gq[q] & 15));
+                  gb[q][0] = __ldg(b4);
+                  gb[q][1] = __ldg(b4 + 1);
+                }
+              }
               float vs[32];
               __syncwarp();
 #pragma unroll
@@ -562,12 +621,12 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
               if (uni == 0u) {
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive(&bars->acc_empty[slot]);
+                if (lane == 0) mbar_arrive(acc_bar + kAccEmptyOff + acc_off);
                 slot_released = true;
               }
 #pragma unroll
               for (int q = 0; q < 4; ++q)
-                if ((pend >> gq[q]) & 1u) search_group(*reinterpret_cast<float(*)[8]>(vs + 8 * q), gq[q]);
+                if ((pend >> gq[q]) & 1u) search_group(*reinterpret_cast<float(*)[8]>(vs + 8 * q), gq[q], gs[q], gb[q]);
             }
           }
 #endif
@@ -678,8 +737,8 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
         tc_fence_before();
         __syncwarp();
         if (lane == 0) {
-          if (!slot_released) mbar_arrive(&bars->acc_empty[slot]);
-          mbar_arrive(&bars->cs_empty[cs]);
+          if (!slot_released) mbar_arrive(acc_bar + kAccEmptyOff + acc_off);
+          if (!PRE) mbar_arrive(cs_bar + kCsEmptyOff + cs * 8);
         }
       }
       if (qrow < x.qend) {
@@ -712,6 +771,21 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
 }
 
 }  // namespace
+
+// Sets the shared-memory size and checks the register allocation the setmaxnreg split was computed for (a smaller one
+// would leave the epilogue's setmaxnreg.inc waiting for registers that warpgroup 0 never frees).
+template <typename Kern>
+static int prepare_launch(Kern kern, int cs, size_t smem) {
+  APS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cudaFuncAttributes fa;
+  APS_CUDA(cudaFuncGetAttributes(&fa, kern));
+  if (fa.numRegs != launch_regs(cs)) {
+    aps_set_error(APS_ERR_CUDA, "", "k_knn_tc allocates %d registers per thread, the register split assumes %d",
+                  fa.numRegs, launch_regs(cs));
+    return APS_ERR_CUDA;
+  }
+  return APS_OK;
+}
 
 int aps_k_knn_tc_supported(int Dp) { return Dp == 64 || Dp == 128; }
 int aps_k_knn_tc_tile_rows() { return TN; }
@@ -857,7 +931,7 @@ int aps_k_knn_tc(cudaStream_t s, int sm_count, const aps_tc_problem& p, cudaEven
   const unsigned grid = (unsigned)(units < sm_count ? units : sm_count);  // upper bound in second-pass mode
   if (ev0) APS_CUDA(cudaEventRecord(ev0, s));
   auto launch = [&](auto kern) -> int {
-    APS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    APS_TRY(prepare_launch(kern, CSPLIT, smem));
     kern<<<grid, NUM_THREADS, smem, s>>>(map_q, map_t, P);
     return APS_OK;
   };
@@ -941,14 +1015,13 @@ int aps_k_knn_tc_units(cudaStream_t s, int sm_count, const aps_tc_problem& p, co
   const size_t smem = 1024 + (size_t)RB * TM * p.Dp * 2 + (size_t)NUM_B_STAGES * TN * p.Dp * 2 +
                       (size_t)NUM_CS_STAGES * 2 * TN * sizeof(float) + (size_t)RB * cs_groups * KC * TM * 4 + sizeof(Barriers);
   const unsigned grid = (unsigned)(n_units < sm_count ? n_units : sm_count);
-  int threads = NUM_THREADS;
+  const int threads = threads_for(cs_groups);
   auto launch = [&](auto kern) -> int {
-    APS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    APS_TRY(prepare_launch(kern, cs_groups, smem));
     kern<<<grid, threads, smem, s>>>(map_q, map_t, P);
     return APS_OK;
   };
   if (p.kcand == 3) {  // short sweeps: branch-free two-best per segment, two epilogue groups (lists) per row block
-    threads = threads_for(2);
     P.cand_stride = aps_k_knn_tc_tile_mode_stride();
     APS_TRY(p.bias ? launch(k_knn_tc<true, false, false, 3, 2>) : launch(k_knn_tc<false, false, false, 3, 2>));
   } else if (p.kcand == 4)

@@ -30,9 +30,11 @@ static __device__ __forceinline__ bool elect_one() {
 static __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
 }
-static __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+// The uint32_t overloads take the barrier's 32-bit shared-window address: per-tile loops compute it once.
+static __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
+static __device__ __forceinline__ void mbar_arrive(uint64_t* bar) { mbar_arrive(smem_u32(bar)); }
 static __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
@@ -40,8 +42,7 @@ static __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint
 // polling loops of the producer / MMA lanes then cost almost no issue slots (they were 21 % of all
 // executed instructions with the default time limit -- profiles/r1_ncu_history.txt)
 constexpr uint32_t kSuspendHintNs = 20000;
-static __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
+static __device__ __forceinline__ void mbar_wait(uint32_t addr, uint32_t parity) {
   uint32_t done;
 #ifdef APS_TC_WATCHDOG
   uint32_t spins = 0;
@@ -62,6 +63,7 @@ static __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity)
 #endif
   } while (!done);
 }
+static __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) { mbar_wait(smem_u32(bar), parity); }
 // producer / MMA-issuer flavour: back off between probes so the spinning lane does not steal issue
 // slots from the epilogue warp that shares its SM sub-partition
 static __device__ __forceinline__ void mbar_wait_backoff(uint64_t* bar, uint32_t parity) {
@@ -92,10 +94,10 @@ static __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, 
 }
 static __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 static __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-static __device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
+static __device__ __forceinline__ void tc_commit(uint32_t bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
+static __device__ __forceinline__ void tc_commit(uint64_t* bar) { tc_commit(smem_u32(bar)); }
 // D[tmem] (+)= A[smem] * B[smem]^T ; kind::f16 (bf16 inputs, fp32 accumulate)
 static __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
                                           uint32_t accumulate) {
