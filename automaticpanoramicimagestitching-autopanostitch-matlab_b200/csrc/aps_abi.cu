@@ -1028,6 +1028,109 @@ extern "C" int aps_debug_tc_scores(aps_ctx* c, const float* Q, int64_t nq, const
   return APS_OK;
 }
 
+// diagnostics: the candidate lists of one tcgen05 launch, with the operands, constants and schedule it ran on.  The
+// preparation and the launch are the ones of float_knn: prep 0 = the global plan (APS_NORM_GLOBAL, fp16 operands,
+// scale-only scores), prep 1 = flann_knn_win (raw rows, bf16, bias -|t|^2/2); rows != NULL = its second pass.
+extern "C" int aps_debug_tc_candidates(aps_ctx* c, const float* Q, int64_t nq, const float* T, int64_t nt, int D,
+                                       int prep, int natural_order, int64_t q0, int64_t q1, int64_t t0, int64_t t1,
+                                       const int32_t* rows, int64_t nrows, uint32_t* cand_idx, float* cand_score,
+                                       int32_t* perm, uint16_t* q_bits, uint16_t* t_bits, float* colscale,
+                                       float* colbias, int64_t* info) {
+  APS_CTX(c);
+  if (!Q || !T || nq <= 0 || nt <= 0 || D <= 0 || (prep != 0 && prep != 1) || !cand_idx || !cand_score || !perm ||
+      !q_bits || !t_bits || !colscale || !colbias || !info)
+    APS_FAIL(APS_ERR_ARGS, "", "bad arguments");
+  if (q0 < 0 || q1 > nq || q0 >= q1 || t0 < 0 || t1 > nt || t0 >= t1) APS_FAIL(APS_ERR_ARGS, "", "range out of bounds");
+  if (rows && (nrows < 0 || nrows > q1 - q0)) APS_FAIL(APS_ERR_ARGS, "", "more listed rows than the query range holds");
+  const int Dp = (D + 63) / 64 * 64;
+  if (!aps_k_knn_tc_supported(Dp)) APS_FAIL(APS_ERR_DIM, "", "unsupported descriptor length %d", D);
+  if (rows)
+    for (int64_t i = 0; i < nrows; ++i)
+      if (rows[i] < q0 || rows[i] >= q1) APS_FAIL(APS_ERR_ARGS, "", "listed row %lld outside the query range", (long long)rows[i]);
+  cudaStream_t s = c->stream;
+  const bool self = (Q == T && nq == nt), global = prep == 0;
+  const int norm_mode = global ? APS_NORM_GLOBAL : APS_NORM_NONE, bias_mode = global ? 0 : 1;
+  FloatSet ts, qs;
+  DevBuf<uint8_t> tmp;
+  ts.fp16 = qs.fp16 = global;  // as aps_gplan_create
+  APS_TRY(floatset_alloc(c, ts, nt, D));
+  APS_TRY(floatset_reset_flags(c, ts));
+  APS_TRY(stage_matrix(c, T, nt, D, 4, APS_ROW_MAJOR, ts.raw.p, tmp));
+  if (!self) {
+    APS_TRY(floatset_alloc(c, qs, nq, D));
+    APS_TRY(stage_matrix(c, Q, nq, D, 4, APS_ROW_MAJOR, qs.raw.p, tmp));
+  }
+  // both flag passes (shared flag words) before the operands of either side, as flann_knn_win
+  FloatSet* sides[2] = {&ts, self ? nullptr : &qs};
+  for (FloatSet* f : sides) {
+    if (!f) continue;
+    if (norm_mode != APS_NORM_NONE) APS_TRY(f->xn.alloc((size_t)f->N * D, s));
+    APS_TRY(aps_k_prepare_norm(s, f->raw.p, f->N, D, norm_mode, f->xn.p ? f->xn.p : f->raw.p, f->sq.p, f->invn.p,
+                               ts.flags.p, f->fp16));
+  }
+  for (FloatSet* f : sides) {
+    if (!f) continue;
+    APS_TRY(f->xb.alloc((size_t)f->N * Dp, s));
+    APS_TRY(f->colscale.alloc((size_t)f->N + 256, s));
+    APS_TRY(f->colbias.alloc((size_t)f->N + 256, s));
+    APS_TRY(aps_k_prepare_operands(s, f->raw.p, f->xn.p ? f->xn.p : f->raw.p, f->sq.p, f->invn.p, f->N, D, Dp, ts.flags.p,
+                                   bias_mode, f->xb.p, f->colscale.p, f->colbias.p, f->fp16));
+  }
+  APS_TRY(floatset_finish_train(c, ts, !natural_order));
+  const FloatSide qv = self ? ts.side() : qs.side(), tv = ts.side();
+  aps_tc_problem p;
+  p.Qb = qv.xb; p.Tb = tv.xb_t; p.colscale = tv.colscale_t; p.colbias = tv.colbias_t; p.tile_bounds = tv.tile_bounds;
+  p.bias = bias_mode;
+  p.Fq_total = nq; p.Ft_total = nt; p.Dp = Dp;
+  p.q0 = q0; p.q1 = q1; p.t0 = t0; p.t1 = t1;
+  p.kcand = 8;
+  p.dump = nullptr;
+  p.operand_fp16 = global ? 2 : 0;
+  p.exact_flag = ts.flags.p;
+  const int64_t nr = q1 - q0;
+  DevBuf<int32_t> drows;
+  DevBuf<__nv_bfloat16> qb2;
+  if (rows) {  // float_knn's second pass: the listed rows gathered into a compact query matrix, count on the device
+    const int32_t cnt = (int32_t)nrows;
+    APS_TRY(drows.alloc((size_t)nr + 1, s));
+    APS_TRY(qb2.alloc((size_t)nr * Dp, s));
+    if (nrows > 0) APS_CUDA(cudaMemcpyAsync(drows.p, rows, (size_t)nrows * 4, cudaMemcpyHostToDevice, s));
+    APS_CUDA(cudaMemcpyAsync(drows.p + nr, &cnt, 4, cudaMemcpyHostToDevice, s));
+    APS_TRY(aps_k_gather_rows(s, qv.xb, Dp, drows.p, drows.p + nr, nr, qb2.p));
+    p.Qb = qb2.p; p.Fq_total = nr; p.q0 = 0; p.q1 = nr;
+    p.nrows_dev = drows.p + nr;
+  }
+  p.nslot = aps_k_knn_tc_slots(c->sm_count, nr, t0, t1, rows ? 1 : 0);
+  int d[7];
+  APS_TRY(aps_k_knn_tc_describe(c->sm_count, p, d));
+  DevBuf<uint32_t> cidx;
+  DevBuf<float> cscore;
+  const size_t ncand = (size_t)nr * p.nslot * 8;
+  APS_TRY(cidx.alloc(ncand, s));
+  APS_TRY(cscore.alloc(ncand, s));
+  APS_CUDA(cudaMemsetAsync(cidx.p, 0xA5, ncand * 4, s));    // 0xA5A5A5A5: never a train position of these sizes
+  APS_CUDA(cudaMemsetAsync(cscore.p, 0xFF, ncand * 4, s));  // NaN
+  p.cand_idx = cidx.p; p.cand_score = cscore.p;
+  APS_TRY(aps_k_knn_tc(s, c->sm_count, p));
+  int32_t exact = 0;
+  APS_CUDA(cudaMemcpyAsync(&exact, ts.flags.p, 4, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(cand_idx, cidx.p, ncand * 4, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(cand_score, cscore.p, ncand * 4, cudaMemcpyDeviceToHost, s));
+  if (tv.perm) APS_CUDA(cudaMemcpyAsync(perm, tv.perm, (size_t)nt * 4, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpy2DAsync(q_bits, (size_t)D * 2, qv.xb, (size_t)Dp * 2, (size_t)D * 2, (size_t)nq, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpy2DAsync(t_bits, (size_t)D * 2, ts.xb.p, (size_t)Dp * 2, (size_t)D * 2, (size_t)nt, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(colscale, ts.colscale.p, (size_t)nt * 4, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(colbias, ts.colbias.p, (size_t)nt * 4, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaStreamSynchronize(s));
+  if (!tv.perm)
+    for (int64_t i = 0; i < nt; ++i) perm[i] = (int32_t)i;
+  // float_knn: rows of full-width units are re-ranked from list 0 alone (first pass only)
+  const int64_t rows_full = (!rows && p.nslot > 1) ? aps_k_knn_tc_full_rows(c->sm_count, nr, t0, t1) : 0;
+  const int64_t v[11] = {c->sm_count, d[0], rows_full, exact, p.operand_fp16, d[1], d[2], d[3], d[4], d[5], d[6]};
+  memcpy(info, v, sizeof v);
+  return APS_OK;
+}
+
 // diagnostics: the fp16 screen of ONE (query set, train set) pair, with the raw accumulator registers
 extern "C" int aps_debug_pair_screen(aps_ctx* c, const float* A, int64_t N1, const float* B, int64_t N2, int D,
                                      float* b1b2, uint32_t* dump, int dump_tiles) {

@@ -182,6 +182,9 @@ int aps_k_knn_tc_tile_mode_segment();  // ... and the columns per segment (two b
 int aps_k_knn_tc_units(cudaStream_t s, int sm_count, const aps_tc_problem& p, const aps_tc_unit* d_units,
                        int64_t n_units);
 int aps_k_knn_tc_slots(int sm_count, int64_t nq, int64_t t0, int64_t t1, int all_segmented = 0);  // lists per row
+// the schedule aps_k_knn_tc launches for p: out[0..6] = nslot, pre-filtered long sweep (0/1), units_full, tail_units,
+// tail_seg, tail_balanced, tiles_per_seg
+int aps_k_knn_tc_describe(int sm_count, const aps_tc_problem& p, int* out);
 int64_t aps_k_knn_tc_full_rows(int sm_count, int64_t nq, int64_t t0, int64_t t1);  // leading query rows that only fill list 0
 int aps_k_gather_rows(cudaStream_t s, const __nv_bfloat16* src, int Dp, const int32_t* rows, const int32_t* nrows_dev,
                       int64_t max_rows, __nv_bfloat16* dst);
@@ -209,7 +212,7 @@ struct aps_pair_tables {
   // grows by the 7 key bits.
   int tile_mode;
   // != 0: the tensor pass ran on fp16 operands (10-bit mantissa): the operand-rounding term of eps is 2.0e-3 instead of
-  // 7.9e-3.  1 = never exact (pairwise: normalised rows are rounded), 2 = flags[0] tells (global path, set by K1)
+  // 1.57e-2.  1 = never exact (pairwise: normalised rows are rounded), 2 = flags[0] tells (global path, set by K1)
   int operand_fp16;
   // 'subsetpdist2' with images above the subset size: the train rows of such an image are a random subset stored as a
   // "virtual image" at rows >= vfirst of the train view; vmap[row - vfirst] = 0-based local index in the original image

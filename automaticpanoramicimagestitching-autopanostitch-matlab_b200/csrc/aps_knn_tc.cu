@@ -873,6 +873,24 @@ int aps_k_knn_tc_slots(int sm_count, int64_t nq, int64_t t0, int64_t t1, int all
   return make_schedule(sm_count, nq, t0, t1, all_segmented != 0).nslot;
 }
 
+// the raw pre-filter pays once a unit sweeps >= ~100 tiles (insert probability per chunk ~ 64 / tiles seen)
+static bool use_prefilter(const TcSchedule& sc, const aps_tc_problem& p) {
+  const int64_t sweep = (sc.tile_hi - sc.tile_lo) / ((sc.units_full && !p.nrows_dev) ? 1 : (sc.tail_seg > 0 ? sc.tail_seg : 1));
+  return sweep >= 96 && p.tile_bounds != nullptr;
+}
+
+int aps_k_knn_tc_describe(int sm_count, const aps_tc_problem& p, int* out) {
+  const TcSchedule sc = make_schedule(sm_count, p.q1 - p.q0, p.t0, p.t1, p.nrows_dev != nullptr);
+  out[0] = sc.nslot;
+  out[1] = use_prefilter(sc, p) ? 1 : 0;
+  out[2] = sc.units_full;
+  out[3] = sc.tail_units;
+  out[4] = sc.tail_seg;
+  out[5] = sc.tail_balanced;
+  out[6] = sc.tiles_per_seg;
+  return APS_OK;
+}
+
 int aps_k_knn_tc(cudaStream_t s, int sm_count, const aps_tc_problem& p, cudaEvent_t ev0, cudaEvent_t ev1) {
   if (!aps_k_knn_tc_supported(p.Dp)) {
     aps_set_error(APS_ERR_DIM, "", "tcgen05 path supports padded descriptor lengths 64 and 128 (got %d)", p.Dp);
@@ -935,9 +953,7 @@ int aps_k_knn_tc(cudaStream_t s, int sm_count, const aps_tc_problem& p, cudaEven
     kern<<<grid, NUM_THREADS, smem, s>>>(map_q, map_t, P);
     return APS_OK;
   };
-  // the raw pre-filter pays once a unit sweeps >= ~100 tiles (insert probability per chunk ~ 64 / tiles seen)
-  const int64_t sweep = (sc.tile_hi - sc.tile_lo) / ((sc.units_full && !p.nrows_dev) ? 1 : (sc.tail_seg > 0 ? sc.tail_seg : 1));
-  const bool pre = sweep >= 96 && p.tile_bounds != nullptr;
+  const bool pre = use_prefilter(sc, p);
   if (p.dump)
     APS_TRY(p.bias ? launch(k_knn_tc<true, true, false, KC>) : launch(k_knn_tc<false, true, false, KC>));
   else if (p.exact_flag && !p.nrows_dev) {

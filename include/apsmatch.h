@@ -317,6 +317,22 @@ int aps_debug_pair_screen(aps_ctx* ctx, const float* A, int64_t N1, const float*
                           uint32_t* dump, int dump_tiles);
 int aps_debug_tc_scores(aps_ctx* ctx, const float* Q, int64_t nq, const float* T, int64_t nt, int D, int nseg,
                         float* scores, uint32_t* cand_idx, float* cand_score);
+/* The candidate lists of one tcgen05 launch, prepared and scheduled as the float searches run it.  Q [nq x D], T [nt x D]
+ * ROW-major float; Q == T (and nq == nt) is a self-search.  prep 0: the global plan's preparation (rows normalised as
+ * featureMatchingGlobal, fp16 operands, score = dot * scale); prep 1: flann_knn_win's (rows as given, bf16 operands,
+ * score = dot - |t|^2/2).  The train view is sorted by scale unless natural_order.  Query rows [q0,q1) are searched
+ * against train positions [t0,t1) of that view; rows != NULL runs the second pass of the search instead: the nrows
+ * listed query rows (each inside [q0,q1)), gathered, every unit cut into column segments.
+ * Outputs: cand_idx / cand_score with room for (q1-q0) x 32 entries, of which [(q1-q0) x nslot x 8] are written (row i
+ * of the second pass = rows[i]): train-view positions (0xFFFFFFFF = empty) and packed scores, filled with 0xA5A5A5A5 /
+ * NaN before the launch; perm [nt] train-view position -> row of T; q_bits [nq x D] and t_bits [nt x D]: the 16-bit
+ * operands (fp16 or bf16) in the rows' original order; colscale / colbias [nt] per row of T.  info [11]: sm_count,
+ * nslot, rows_full (leading rows whose candidates are all in list 0), operands-exact flag, operand kind (2 fp16, 0 bf16),
+ * pre-filtered long sweep, units_full, tail_units, tail_seg, tail_balanced, tiles_per_seg. */
+int aps_debug_tc_candidates(aps_ctx* ctx, const float* Q, int64_t nq, const float* T, int64_t nt, int D, int prep,
+                            int natural_order, int64_t q0, int64_t q1, int64_t t0, int64_t t1, const int32_t* rows,
+                            int64_t nrows, uint32_t* cand_idx, float* cand_score, int32_t* perm, uint16_t* q_bits,
+                            uint16_t* t_bits, float* colscale, float* colbias, int64_t* info);
 
 #ifdef __cplusplus
 }

@@ -44,7 +44,7 @@ def run(A, B, label):
     sqA, sqB = (A * A).sum(1), (B * B).sum(1)
     score = bf16(A) @ bf16(B).T - 0.5 * sqB[None, :]
     maxsq = max(1.0, float(max(sqA.max(), sqB.max())))
-    eps0 = (1e-4 + 7.9e-3) * maxsq
+    eps0 = (1e-4 + 1.57e-2) * maxsq
     r2 = ratio * ratio
     # streaming top-4
     o4 = np.argsort(-score, axis=1)[:, :4]
