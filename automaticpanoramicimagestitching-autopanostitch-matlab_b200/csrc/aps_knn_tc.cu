@@ -30,11 +30,14 @@
 //                  is sorted by scale so the bounds are tight) -- no per-column constant, no multiply;
 //              (2) ONE warp vote; no lane flagged a group -> next tile (~270 instructions per tile and warp);
 //              (3) otherwise the union of the flagged groups is RE-READ from TMEM (tcgen05.ld .x8, rounds of four)
-//                  by the converged warp, the slot is handed back to the tensor pipe, and the flagged lanes scale
-//                  (the groups' constants read from L2 with LDG.128, issued before the re-read; no per-tile wait on a
-//                  constants ring), search and replace-min: scores in registers as packed
-//                  keys (value bits & ~7 | slot), train-row indices in shared memory.  One run-time-indexed copy
-//                  of the insertion code.
+//                  by the converged warp, the slot is handed back to the tensor pipe, and the flagged lanes scale,
+//                  search and replace-min: scores in registers as packed keys (value bits & ~7 | slot), train-row
+//                  indices in shared memory.  One run-time-indexed copy of the insertion code.  The column constants
+//                  never cost an L2 round trip in the walk: every tile, each lane prefetches the NEXT tile's 4 scales
+//                  (and biases) with one LDG.128 next to the tile-bounds prefetch; a flagged tile writes them once to
+//                  the warp's 1 KB staging area (STS.128 per lane, in the (scale, bias) ring region that long sweeps do
+//                  not use), and each round reads its groups' values with broadcast LDS.128 issued before the re-read.
+//                  No per-tile wait on a constants ring either.
 //              Short sweeps (!PRE: the lists never leave their filling phase) keep the per-chunk loop: scale every
 //              32-column chunk, group maxima, branch-free replace-min for the groups that hold a candidate.
 // TMEM: 4 accumulator slots of 128 columns = slot(tile parity, row block): the tensor pipe fills the
@@ -47,13 +50,14 @@
 // What bounds it (C2 = 163840^2 pairs, D = 128; profiles/r2_ncu_history.txt, profiles/r2_ncu_k_knn_tc.txt):
 //   * accumulators never read (-DAPS_TC_NOEPI): TMA + MMA alone 3.39 ms = 2027 TFLOP/s -- the floor of this tiling
 //     (85 % of nominal; the same with the A operand in TMEM: shared-memory bandwidth is not the limiter);
-//   * full kernel 4.60 ms = 1493 TFLOP/s = 0.92 of the measured cuBLAS bf16 burst figure (B200, 1000 W, 1965 MHz;
-//     round 2: 4.71-4.87 ms, before the register split and the removal of the constants ring on long sweeps; round 1:
-//     5.79 ms; per-chunk group-gated version: 5.32 ms); C3 (F = 1e6, long sweeps) 1635 TFLOP/s = 1.01 of it (round 2).
-//     What is left at C2 is the VARIANCE of the epilogue: a tile with insertions (39 % of them) takes ~4x the cycles
-//     of one without, and two accumulator slots per row block cannot average that out: the epilogue warps wait for
-//     acc_full 22 % of their time while the issuers spin on acc_empty.  K'(1 + ln(F/K')) ~ 67 insertions per row are
-//     inherent to a streaming top-K';
+//   * full kernel 4.35 ms = 1580 TFLOP/s = 0.98 of the measured cuBLAS bf16 burst figure (B200, 1000 W, 1965 MHz;
+//     round 3: 4.60 ms, with the flagged groups' constants loaded from L2 in every round of the walk; round 2:
+//     4.71-4.87 ms, before the register split; round 1: 5.79 ms; per-chunk group-gated version: 5.32 ms); C3 (F = 1e6,
+//     long sweeps) 1635 TFLOP/s = 1.01 of it (round 2).
+//     What is left at C2 is the epilogue's own work (per-tile clocks, -DAPS_TC_TILE_CLOCKS, profiles/tile_clocks.py):
+//     1262 busy cycles per tile and warp on average against ~1200 for the MMAs; a tile with insertions (39 % of them)
+//     takes ~2100 (of which ~910 insertions), one without ~730, and the epilogue warps still wait for acc_full 14 % of
+//     their cycles.  K'(1 + ln(F/K')) ~ 67 insertions per row are inherent to a streaming top-K';
 //   * not kept: A operand in TMEM with three slots (5.34 ms); separate scan / insert warps with setmaxnreg
 //     (5.13 ms: the per-tile hand-off costs more than it frees); two lists per row on column halves with 16
 //     epilogue warps (twice the insertions); fp16 accumulators (rounding breaks the completeness proof on
@@ -108,9 +112,27 @@ __device__ __forceinline__ float4 lds_f32x4(uint32_t a) {
   asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
   return v;
 }
+__device__ __forceinline__ void sts_f32x4(uint32_t a, float4 v) {
+  asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+}
 __device__ __forceinline__ uint32_t lds_u32(uint32_t a) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
 __device__ __forceinline__ void sts_u32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 constexpr uint32_t SLOT_STRIDE = TM * 4;                  // bytes between consecutive slots of one row
+
+#ifdef APS_TC_TILE_CLOCKS
+// Measurement aid (-DAPS_TC_TILE_CLOCKS, profiles/tile_clocks.py): lane 0 of every epilogue warp of a long-sweep launch
+// writes one record of kClkWords words per tile: clock() cycles of (0) the acc_full wait, (1) the scan and vote, (2) the
+// walk of the flagged groups without its insertions (per-tile staging, TMEM re-reads, waits for the column constants),
+// (3) the insertions (search_group), (4) the whole tile; (5) the union of flagged groups, (6) the rounds, (7) flags
+// (1: flagged, 2: partial tile, 4: first tile of the unit).  Records beyond kClkCap per warp are dropped; second-pass
+// (nrows_dev) launches record nothing, so the buffer holds the last first-pass launch.
+constexpr int kClkWords = 8, kClkCap = 8192, kClkCtas = 160;
+__device__ uint32_t* g_tile_clk;    // [kClkCtas][8 epilogue warps][kClkCap][kClkWords]
+__device__ uint32_t* g_tile_clk_n;  // [kClkCtas][8 epilogue warps] records of the last recorded launch
+#define APS_CLK(...) __VA_ARGS__
+#else
+#define APS_CLK(...)
+#endif
 
 struct KParams {
   int64_t q0, q1, t0, t1;
@@ -387,8 +409,13 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
     // the (scale, bias) ring stage of short sweeps.  Barrier and TMEM addresses are 32-bit, computed once.
     const uint32_t acc_bar = smem_u32(&bars->acc_full[grp]), cs_bar = smem_u32(&bars->cs_full[0]);
     const uint32_t cs_smem0 = smem_u32(smem_cs + ch * CG);
+    // long sweeps: the ring region holds one staging area per epilogue warp for the column constants of a flagged
+    // tile (TN scales, TN biases: 8 warps x 1 KB = the ring's 8 KB)
+    static_assert(NUM_EPI_WARPS * 2 * TN <= NUM_CS_STAGES * 2 * TN, "staging fits in the (scale, bias) ring");
+    const uint32_t stage = smem_u32(smem_cs) + (warp - FIRST_EPI_WARP) * (2 * TN * 4);
     const uint32_t tmem_row = tmem_base + ((uint32_t)(quad * 32) << 16) + grp * TN + ch * CG;
     uint32_t par = 0, acph = 0, cs = 0, cph = 0;
+    APS_CLK(uint32_t clk_n = 0;)
     auto next_tile = [&]() {
       par ^= 1;
       acph ^= par ^ 1;
@@ -479,11 +506,21 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
       const float4* tbp = P.tile_bounds + x.tl;
       float4 tb_next = (PRE && nt > 0) ? __ldg(tbp) : make_float4(0.f, 0.f, 0.f, 0.f);
       uint32_t col0 = (uint32_t)(x.tl * TN) + ch * CG;
+      // long sweeps: the tile's column constants, lane l holding columns 4l .. 4l+3, loaded one tile ahead
+      float4 cs_next = make_float4(0.f, 0.f, 0.f, 0.f), cb_next = cs_next;
+      if (PRE && nt > 0) {
+        cs_next = __ldg(reinterpret_cast<const float4*>(P.colscale + col0) + lane);
+        if (BIAS) cb_next = __ldg(reinterpret_cast<const float4*>(P.colbias + col0) + lane);
+      }
       for (uint32_t i = 0; i < nt; ++i, col0 += TN, next_tile()) {
         const uint32_t acc_off = par * (RB * 8);
+        // (clk_meta: flags | union << 8 | rounds << 16)
+        APS_CLK(const uint32_t ck0 = (uint32_t)clock(); uint32_t ck_vote = 0, ck_walk = 0, ck_ins = 0,
+                clk_meta = i == 0 ? 4u : 0u;)
         mbar_wait(acc_bar + acc_off, acph);
         if (!PRE) mbar_wait(cs_bar + cs * 8, cph);
         tc_fence_after();
+        APS_CLK(const uint32_t ck1 = (uint32_t)clock();)
         const uint32_t cscale = cs_smem0 + cs * (2 * TN * 4);
         const bool partial = (col0 < ct0) || (col0 + CG > ct1);
         const uint32_t taddr = tmem_row + par * (RB * TN);
@@ -492,7 +529,12 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
         // train rows are sorted by scale (aps_prep.cu), so the bound is tight and the common path needs
         // neither the per-column constants nor a multiply.
         const float4 tb = tb_next;  // fetched one tile ahead: the global-load latency stays off the critical path
-        if (PRE && i + 1 < nt) tb_next = __ldg(tbp + i + 1);
+        const float4 cs_cur = cs_next, cb_cur = cb_next;  // (same)
+        if (PRE && i + 1 < nt) {
+          tb_next = __ldg(tbp + i + 1);
+          cs_next = __ldg(reinterpret_cast<const float4*>(P.colscale + col0 + TN) + lane);
+          if (BIAS) cb_next = __ldg(reinterpret_cast<const float4*>(P.colbias + col0 + TN) + lane);
+        }
         auto pre_threshold = [&](float th) {
           const float num = th - tb.z - 1.0e-6f * (fabsf(th) + fabsf(tb.z));
           return num * (num >= 0.f ? tb.x : tb.y);
@@ -533,12 +575,20 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
 #pragma unroll
           for (int g = 3; g < 15; g += 2) tmax = fmaxf(fmaxf(tmax, rm[g]), rm[g + 1]);
           tmax = fmaxf(tmax, rm[15]);
-          if (__any_sync(0xffffffffu, partial || tmax > thr_pre)) {
+          const bool flagged = __any_sync(0xffffffffu, partial || tmax > thr_pre);
+          APS_CLK(ck_vote = (uint32_t)clock(); clk_meta |= (flagged ? 1u : 0u) | (__any_sync(~0u, partial) ? 2u : 0u);)
+          if (flagged) {
             uint32_t pend = 0;
 #pragma unroll
             for (int g = 0; g < 16; ++g) pend |= (rm[g] > thr_pre) ? (1u << g) : 0u;
             if (partial) pend = 0xffffu;
             uint32_t uni = __reduce_or_sync(0xffffffffu, pend);
+            // the tile's constants, prefetched a tile ahead, go to this warp's staging area once (one STS.128 per
+            // lane); every round then reads its groups' 8 values with broadcast LDS.128: no L2 round trip in the walk
+            sts_f32x4(stage + 16 * lane, cs_cur);
+            if (BIAS) sts_f32x4(stage + TN * 4 + 16 * lane, cb_cur);
+            __syncwarp();
+            APS_CLK(clk_meta |= (uint32_t)__popc(uni) << 8;)
             // one flagged group of this lane: scale, mask, insert (inlined once per stash position below)
             auto search_group = [&](float(&v)[8], const int g, const float4 (&s)[2], const float4 (&b)[2]) {
               const float4 s0 = s[0], s1 = s[1];
@@ -599,18 +649,17 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
                 gq[q] = uni ? __ffs((int)uni) - 1 : 31;  // 31: no group (bit 31 of pend is never set)
                 uni &= uni - 1;
               }
-              // the groups' scales (and biases) straight from L2, in flight together with the TMEM re-read (same
-              // address in every lane: one request per load); no (scale, bias) ring stage to wait for on any tile
+              // the groups' scales (and biases) from the staging area, in flight together with the TMEM re-read (same
+              // address in every lane: a broadcast)
               float4 gs[4][2], gb[4][2];
 #pragma unroll
               for (int q = 0; q < 4; ++q) {
-                const float4* s4 = reinterpret_cast<const float4*>(P.colscale + col0 + 8 * (gq[q] & 15));
-                gs[q][0] = __ldg(s4);
-                gs[q][1] = __ldg(s4 + 1);
+                const uint32_t s4 = stage + 32 * (gq[q] & 15);
+                gs[q][0] = lds_f32x4(s4);
+                gs[q][1] = lds_f32x4(s4 + 16);
                 if (BIAS) {
-                  const float4* b4 = reinterpret_cast<const float4*>(P.colbias + col0 + 8 * (gq[q] & 15));
-                  gb[q][0] = __ldg(b4);
-                  gb[q][1] = __ldg(b4 + 1);
+                  gb[q][0] = lds_f32x4(s4 + TN * 4);
+                  gb[q][1] = lds_f32x4(s4 + TN * 4 + 16);
                 }
               }
               float vs[32];
@@ -618,16 +667,34 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
 #pragma unroll
               for (int q = 0; q < 4; ++q) tmem_ld8(taddr + 8 * (gq[q] & 15), *reinterpret_cast<float(*)[8]>(vs + 8 * q));
               tmem_wait_ld(vs);
+#ifdef APS_TC_TILE_CLOCKS
+              {  // consume every constant here, so that the wait for them is counted in the walk, not the insertions
+                float w = 0.f;
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                  asm volatile("add.f32 %0, %0, %1;" : "+f"(w) : "f"(gs[q][0].x + gs[q][0].y + gs[q][0].z + gs[q][0].w));
+                  asm volatile("add.f32 %0, %0, %1;" : "+f"(w) : "f"(gs[q][1].x + gs[q][1].y + gs[q][1].z + gs[q][1].w));
+                  if (BIAS) {
+                    asm volatile("add.f32 %0, %0, %1;" : "+f"(w) : "f"(gb[q][0].x + gb[q][0].y + gb[q][0].z + gb[q][0].w));
+                    asm volatile("add.f32 %0, %0, %1;" : "+f"(w) : "f"(gb[q][1].x + gb[q][1].y + gb[q][1].z + gb[q][1].w));
+                  }
+                }
+                clk_meta |= (__float_as_uint(w) == 0x7fc00001u) ? 8u : 0u;
+              }
+#endif
               if (uni == 0u) {
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(acc_bar + kAccEmptyOff + acc_off);
                 slot_released = true;
               }
+              APS_CLK(clk_meta += 1u << 16; const uint32_t cr = (uint32_t)clock();)
 #pragma unroll
               for (int q = 0; q < 4; ++q)
                 if ((pend >> gq[q]) & 1u) search_group(*reinterpret_cast<float(*)[8]>(vs + 8 * q), gq[q], gs[q], gb[q]);
+              APS_CLK(__syncwarp(); ck_ins += (uint32_t)clock() - cr;)
             }
+            APS_CLK(ck_walk = (uint32_t)clock() - ck_vote - ck_ins;)
           }
 #endif
         } else {
@@ -740,6 +807,17 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
           if (!slot_released) mbar_arrive(acc_bar + kAccEmptyOff + acc_off);
           if (!PRE) mbar_arrive(cs_bar + kCsEmptyOff + cs * 8);
         }
+#ifdef APS_TC_TILE_CLOCKS
+        if (PRE && g_tile_clk && !P.nrows_dev && blockIdx.x < kClkCtas && lane == 0) {
+          const uint32_t ck2 = (uint32_t)clock(), w = blockIdx.x * NUM_EPI_WARPS + (warp - FIRST_EPI_WARP);
+          if (clk_n < (uint32_t)kClkCap) {
+            uint4* r = reinterpret_cast<uint4*>(g_tile_clk + ((size_t)w * kClkCap + clk_n) * kClkWords);
+            r[0] = make_uint4(ck1 - ck0, ck_vote - ck1, ck_walk, ck_ins);
+            r[1] = make_uint4(ck2 - ck0, (clk_meta >> 8) & 0xffu, clk_meta >> 16, clk_meta & 0xffu);
+          }
+          g_tile_clk_n[w] = min(++clk_n, (uint32_t)kClkCap);
+        }
+#endif
       }
       if (qrow < x.qend) {
         const int cstr = P.cand_stride;
@@ -771,6 +849,37 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
 }
 
 }  // namespace
+
+#ifdef APS_TC_TILE_CLOCKS
+// op 0: allocate (once) and zero the record buffer and point the kernel at it; op 1: copy the counts
+// ([kClkCtas * 8] uint32) and the records ([kClkCtas * 8 * kClkCap * kClkWords] uint32) to host memory;
+// op 2: write (kClkCtas, epilogue warps, kClkCap, kClkWords) to counts.  Not part of apsmatch.h.
+extern "C" __attribute__((visibility("default"))) int aps_debug_tile_clocks(int op, uint32_t* counts, uint32_t* records) {
+  static uint32_t *d_rec = nullptr, *d_n = nullptr;
+  const size_t nw = (size_t)kClkCtas * NUM_EPI_WARPS, nrec = nw * kClkCap * kClkWords;
+  if (op == 2) {
+    counts[0] = kClkCtas; counts[1] = NUM_EPI_WARPS; counts[2] = kClkCap; counts[3] = kClkWords;
+    return APS_OK;
+  }
+  if (op == 0) {
+    if (!d_rec) {
+      APS_CUDA(cudaMalloc((void**)&d_rec, nrec * 4));
+      APS_CUDA(cudaMalloc((void**)&d_n, nw * 4));
+      APS_CUDA(cudaMemcpyToSymbol(g_tile_clk, &d_rec, sizeof d_rec));
+      APS_CUDA(cudaMemcpyToSymbol(g_tile_clk_n, &d_n, sizeof d_n));
+    }
+    APS_CUDA(cudaMemset(d_rec, 0, nrec * 4));
+    APS_CUDA(cudaMemset(d_n, 0, nw * 4));
+    APS_CUDA(cudaDeviceSynchronize());
+    return APS_OK;
+  }
+  if (!d_rec) return APS_ERR_ARGS;
+  APS_CUDA(cudaDeviceSynchronize());
+  APS_CUDA(cudaMemcpy(counts, d_n, nw * 4, cudaMemcpyDeviceToHost));
+  APS_CUDA(cudaMemcpy(records, d_rec, nrec * 4, cudaMemcpyDeviceToHost));
+  return APS_OK;
+}
+#endif
 
 // Sets the shared-memory size and checks the register allocation the setmaxnreg split was computed for (a smaller one
 // would leave the epilogue's setmaxnreg.inc waiting for registers that warpgroup 0 never frees).
