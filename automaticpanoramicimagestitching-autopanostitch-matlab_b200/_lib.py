@@ -148,6 +148,8 @@ def lib():
         "aps_debug_tc_scores": (i32, [vp, vp, i64, vp, i64, i32, i32, vp, vp, vp]),
         "aps_debug_tc_candidates": (i32, [vp, vp, i64, vp, i64, i32, i32, i32, i64, i64, i64, i64, vp, i64, vp, vp, vp,
                                           vp, vp, vp, vp, vp]),
+        "aps_debug_tc_candidates_k": (i32, [vp, vp, i64, vp, i64, i32, i32, i32, i64, i64, i64, i64, vp, i64, vp, vp, vp,
+                                            vp, vp, vp, vp, vp, i32]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)  # AttributeError here == the library does not export a declared symbol

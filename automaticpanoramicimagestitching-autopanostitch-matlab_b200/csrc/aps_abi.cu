@@ -223,10 +223,15 @@ int copy_out_matrix(aps_ctx* c, const uint32_t* idx_rm, const float* dist_rm, in
 // ------------------------------------------------------------------------------------------------
 // float search driver: tcgen05 candidates + exact re-rank (+ exact fallback rows), or exact only.
 
+// The completeness proof needs the K'-th candidate strictly beyond the k-th neighbour.  Candidates per list of the tensor
+// pass: 8 for k <= 5 (6 when the operands are exact), 16 for 6 <= k <= kTcMaxK -- at least 3 ranks between the k-th
+// neighbour and the list's floor.  Larger k stays on the exact engine.
+constexpr int kTcMaxK = 12;
+static int tc_list_length(int k) { return k <= 5 ? 8 : 16; }
+
 bool tc_wanted(const aps_ctx* c, int D, int64_t nq, int64_t nt, int k) {
   if (c->float_engine == 1) return false;
-  // the completeness proof needs the K'-th candidate (K' = 8) strictly beyond the k-th neighbour
-  if (k > 5) return false;
+  if (k > kTcMaxK) return false;
   int Dp = (D + 63) / 64 * 64;
   if (!aps_k_knn_tc_supported(Dp)) return false;
   if (c->float_engine == 2) return true;
@@ -235,7 +240,7 @@ bool tc_wanted(const aps_ctx* c, int D, int64_t nq, int64_t nt, int k) {
 
 // Rows the first proof left open: a SHORT list goes straight to the exact engine (its train range is split over 32
 // CTAs per 8 rows, aps_knn_exact.cu) -- a second tensor pass over a handful of rows keeps only 4 CTAs busy for a whole
-// sweep; a LONG list (real-valued descriptors with tightly packed neighbours) takes the 32-candidate tensor pass.
+// sweep; a LONG list (real-valued descriptors with tightly packed neighbours) takes the 4-segment tensor pass.
 __global__ void k_route_unproven(int32_t* __restrict__ fb, int32_t* __restrict__ n1, int32_t* __restrict__ fb2,
                                  int32_t* __restrict__ n2, int short_list, int32_t* __restrict__ report) {
   __shared__ int n;
@@ -267,7 +272,8 @@ int float_knn(aps_ctx* c, const FloatSide& Q, int64_t q0, int64_t q1, const Floa
   }
   c->stats[2] = 2;
   const int Dp = (D + 63) / 64 * 64;
-  const int kcand = 8;
+  const int kcand = tc_list_length(k);
+  const int kcap_exact = kcand == 8 ? 6 : 0;  // K' = 16 has no exact-operand variant
   const int nslot = aps_k_knn_tc_slots(c->sm_count, nq, t0, t1);  // candidate lists per row (tail balancing)
   DevBuf<uint32_t> cidx;
   DevBuf<float> cscore;
@@ -299,7 +305,7 @@ int float_knn(aps_ctx* c, const FloatSide& Q, int64_t q0, int64_t q1, const Floa
   aps_pair_tables gpt;       // global searches: only the operand kind travels in here (eoff == nullptr)
   memset(&gpt, 0, sizeof gpt);
   gpt.operand_fp16 = p.operand_fp16;
-  p.exact_flag = flags_dev;  // exact operands (integer SIFT): 6 candidates per list are enough to prove a top-5
+  p.exact_flag = flags_dev;  // exact operands (integer SIFT): 6 candidates per list are enough to prove a top-5 (K' = 8)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   if (c->timing) {
     APS_CUDA(cudaEventCreate(&ev0));
@@ -310,20 +316,20 @@ int float_knn(aps_ctx* c, const FloatSide& Q, int64_t q0, int64_t q1, const Floa
     c->tc_events.push_back(ev0);
     c->tc_events.push_back(ev1);
   }
-  // rows of full-width units keep all their candidates in list 0: 8 lanes per row instead of 32
+  // rows of full-width units keep all their candidates in list 0: kcand lanes per row instead of nslot * kcand
   const int64_t rows_full = nslot > 1 ? aps_k_knn_tc_full_rows(c->sm_count, nq, t0, t1) : 0;
   if (rows_full > 0)
     APS_TRY(aps_k_rerank(c->stream, Q.xn, Q.sq, Q.invn, T.xn, T.sq, D, metric, q0, rows_full, t0, 1, kcand, cidx.p,
                          cscore.p, flags_dev, bias_mode, flags_dev, k, out_row0, idx, dist, fb.p, fb.p + nq, &gpt,
-                         nullptr, nullptr, T.perm, nslot * kcand, /*kcap_exact*/ 6));
+                         nullptr, nullptr, T.perm, nslot * kcand, kcap_exact));
   if (nq > rows_full)
     APS_TRY(aps_k_rerank(c->stream, Q.xn, Q.sq, Q.invn, T.xn, T.sq, D, metric, q0 + rows_full, nq - rows_full, t0, nslot,
                          kcand, cidx.p + (size_t)rows_full * nslot * kcand, cscore.p + (size_t)rows_full * nslot * kcand,
                          flags_dev, bias_mode, flags_dev, k, out_row0, idx, dist, fb.p, fb.p + nq, &gpt, nullptr,
-                         nullptr, T.perm, 0, /*kcap_exact*/ 6));
+                         nullptr, T.perm, 0, kcap_exact));
   // Rows that could not be proven complete (device-side list, no host round trip) get a SECOND tensor pass with
-  // 4 column segments = 32 candidates per row: with inexact (non bf16-representable) operands the error bound
-  // is ~0.016 in squared distance and 8 candidates often do not reach beyond it; 32 usually do.
+  // 4 column segments = 4 * kcand (32 or 64) candidates per row: with inexact (non bf16-representable) operands the error
+  // bound is ~0.016 in squared distance and 8 candidates often do not reach beyond it; 32 usually do.
   const int nslot2 = aps_k_knn_tc_slots(c->sm_count, nq, t0, t1, /*all_segmented*/ 1);
   DevBuf<int32_t> fb2;
   APS_TRY(fb2.alloc((size_t)nq + 1, c->stream));
@@ -1029,17 +1035,19 @@ extern "C" int aps_debug_tc_scores(aps_ctx* c, const float* Q, int64_t nq, const
 }
 
 // diagnostics: the candidate lists of one tcgen05 launch, with the operands, constants and schedule it ran on.  The
-// preparation and the launch are the ones of float_knn: prep 0 = the global plan (APS_NORM_GLOBAL, fp16 operands,
-// scale-only scores), prep 1 = flann_knn_win (raw rows, bf16, bias -|t|^2/2); rows != NULL = its second pass.
-extern "C" int aps_debug_tc_candidates(aps_ctx* c, const float* Q, int64_t nq, const float* T, int64_t nt, int D,
-                                       int prep, int natural_order, int64_t q0, int64_t q1, int64_t t0, int64_t t1,
-                                       const int32_t* rows, int64_t nrows, uint32_t* cand_idx, float* cand_score,
-                                       int32_t* perm, uint16_t* q_bits, uint16_t* t_bits, float* colscale,
-                                       float* colbias, int64_t* info) {
+// preparation and the launch are the ones of float_knn for a search of k neighbours: prep 0 = the global plan
+// (APS_NORM_GLOBAL, fp16 operands, scale-only scores), prep 1 = flann_knn_win (raw rows, bf16, bias -|t|^2/2);
+// rows != NULL = its second pass.
+extern "C" int aps_debug_tc_candidates_k(aps_ctx* c, const float* Q, int64_t nq, const float* T, int64_t nt, int D,
+                                         int prep, int natural_order, int64_t q0, int64_t q1, int64_t t0, int64_t t1,
+                                         const int32_t* rows, int64_t nrows, uint32_t* cand_idx, float* cand_score,
+                                         int32_t* perm, uint16_t* q_bits, uint16_t* t_bits, float* colscale,
+                                         float* colbias, int64_t* info, int k) {
   APS_CTX(c);
   if (!Q || !T || nq <= 0 || nt <= 0 || D <= 0 || (prep != 0 && prep != 1) || !cand_idx || !cand_score || !perm ||
       !q_bits || !t_bits || !colscale || !colbias || !info)
     APS_FAIL(APS_ERR_ARGS, "", "bad arguments");
+  if (k < 1 || k > kTcMaxK) APS_FAIL(APS_ERR_K, "", "the tensor path serves 1 <= k <= %d (got %d)", kTcMaxK, k);
   if (q0 < 0 || q1 > nq || q0 >= q1 || t0 < 0 || t1 > nt || t0 >= t1) APS_FAIL(APS_ERR_ARGS, "", "range out of bounds");
   if (rows && (nrows < 0 || nrows > q1 - q0)) APS_FAIL(APS_ERR_ARGS, "", "more listed rows than the query range holds");
   const int Dp = (D + 63) / 64 * 64;
@@ -1083,7 +1091,7 @@ extern "C" int aps_debug_tc_candidates(aps_ctx* c, const float* Q, int64_t nq, c
   p.bias = bias_mode;
   p.Fq_total = nq; p.Ft_total = nt; p.Dp = Dp;
   p.q0 = q0; p.q1 = q1; p.t0 = t0; p.t1 = t1;
-  p.kcand = 8;
+  p.kcand = tc_list_length(k);
   p.dump = nullptr;
   p.operand_fp16 = global ? 2 : 0;
   p.exact_flag = ts.flags.p;
@@ -1105,7 +1113,7 @@ extern "C" int aps_debug_tc_candidates(aps_ctx* c, const float* Q, int64_t nq, c
   APS_TRY(aps_k_knn_tc_describe(c->sm_count, p, d));
   DevBuf<uint32_t> cidx;
   DevBuf<float> cscore;
-  const size_t ncand = (size_t)nr * p.nslot * 8;
+  const size_t ncand = (size_t)nr * p.nslot * p.kcand;
   APS_TRY(cidx.alloc(ncand, s));
   APS_TRY(cscore.alloc(ncand, s));
   APS_CUDA(cudaMemsetAsync(cidx.p, 0xA5, ncand * 4, s));    // 0xA5A5A5A5: never a train position of these sizes
@@ -1126,8 +1134,21 @@ extern "C" int aps_debug_tc_candidates(aps_ctx* c, const float* Q, int64_t nq, c
     for (int64_t i = 0; i < nt; ++i) perm[i] = (int32_t)i;
   // float_knn: rows of full-width units are re-ranked from list 0 alone (first pass only)
   const int64_t rows_full = (!rows && p.nslot > 1) ? aps_k_knn_tc_full_rows(c->sm_count, nr, t0, t1) : 0;
-  const int64_t v[11] = {c->sm_count, d[0], rows_full, exact, p.operand_fp16, d[1], d[2], d[3], d[4], d[5], d[6]};
+  const int64_t v[12] = {c->sm_count, d[0], rows_full, exact, p.operand_fp16, d[1], d[2], d[3], d[4], d[5], d[6],
+                         p.kcand};
   memcpy(info, v, sizeof v);
+  return APS_OK;
+}
+
+extern "C" int aps_debug_tc_candidates(aps_ctx* c, const float* Q, int64_t nq, const float* T, int64_t nt, int D,
+                                       int prep, int natural_order, int64_t q0, int64_t q1, int64_t t0, int64_t t1,
+                                       const int32_t* rows, int64_t nrows, uint32_t* cand_idx, float* cand_score,
+                                       int32_t* perm, uint16_t* q_bits, uint16_t* t_bits, float* colscale,
+                                       float* colbias, int64_t* info) {
+  int64_t v[12];
+  APS_TRY(aps_debug_tc_candidates_k(c, Q, nq, T, nt, D, prep, natural_order, q0, q1, t0, t1, rows, nrows, cand_idx,
+                                    cand_score, perm, q_bits, t_bits, colscale, colbias, info ? v : nullptr, 4));
+  memcpy(info, v, 11 * sizeof(int64_t));
   return APS_OK;
 }
 

@@ -164,7 +164,7 @@ struct aps_tc_problem {
   int64_t q0, q1;  // query rows to search
   int64_t t0, t1;  // train rows searched
   int nslot;       // candidate lists per row: aps_k_knn_tc_slots(...) for this problem
-  int kcand;       // candidates kept per (row, segment): 8
+  int kcand;       // candidates kept per (row, segment): 8 (k <= 5) or 16 (6 <= k <= 12)
   uint32_t* cand_idx;   // [ (q1-q0) x nslot x kcand ] global train row (0-based) or 0xFFFFFFFF
   float* cand_score;    // same shape: score (dot*scale+bias), -inf for empty slots
   float* dump;          // optional [ (q1-q0) x (t1-t0) ] raw scores (tests only), else nullptr
@@ -173,7 +173,8 @@ struct aps_tc_problem {
                                        // F32 accumulate.  1 = operands never treated as exact, 2 = flags[0] says whether they are
   const int32_t* exact_flag = nullptr; // device flag "operands are exact in bf16" (K1): when given, the first pass keeps 6
                                        // candidates per list instead of 8 for exact operands (lists stay 8 wide, two
-                                       // entries empty): eps is ~1e-4 then, and 6 still prove a top-5
+                                       // entries empty): eps is ~1e-4 then, and 6 still prove a top-5.  Not read
+                                       // with kcand 16
 };
 int aps_k_knn_tc_supported(int Dp);
 int aps_k_knn_tc_tile_rows();  // rows per train tile (for aps_k_tile_bounds)

@@ -7,8 +7,10 @@
 // instruction) with the accumulator in TMEM, operands staged in shared memory by TMA
 // (SWIZZLE_128B, K-major), and a fused top-K' selection in the epilogue: the distance matrix is
 // never written.  The K' best train rows per (query row, column segment) go to aps_rerank.cu, which
-// recomputes them exactly in FP32 and proves the top-k complete.  K' = 8; 6 when the operands are exact in
-// bf16 (device flag, both variants launched, one exits at once); 4 in the per-pair searches (k = 2) -- or, for
+// recomputes them exactly in FP32 and proves the top-k complete.  K' = 8 for k <= 5; 6 when the operands are exact in
+// bf16 (device flag, both variants launched, one exits at once); 16 for 6 <= k <= 12 (one variant, no exact-operand
+// sub-variant: the proof keeps >= 4 ranks between the k-th neighbour and the list's floor, as K' = 8 keeps 3 for
+// k = 5); 4 in the per-pair searches (k = 2) -- or, for
 // per-pair sweeps of <= 48 tiles, the branch-free SEGMENT epilogue (KCT == 3, CS == 2; see top2_of_32 below):
 // 16 epilogue warps, two sorted lists of three per row, no data-dependent branch.
 //
@@ -81,7 +83,8 @@ constexpr int TN = 128;        // train rows per step (UMMA N)
 constexpr int NUM_B_STAGES = 4;
 constexpr int NUM_ACC_SLOTS = 2 * RB;  // slot = (tile parity) * RB + row block ; 4 x 128 columns = all of TMEM
 constexpr int NUM_CS_STAGES = 8;
-constexpr int KC = 8;          // candidates per (row, segment)
+constexpr int KC = 8;          // candidates per (row, segment) for k <= 5
+constexpr int KC_LARGE = 16;   // ... for 6 <= k <= 12
 constexpr int CSPLIT = 1;      // epilogue groups per row block (each scans TN/CSPLIT columns of every tile, own list)
 constexpr int MAX_SEG = 4 / CSPLIT;  // column segments of a tail unit; a row has MAX_SEG*CSPLIT <= 4 candidate lists
 constexpr int NUM_EPI_WARPS = 4 * RB * CSPLIT;
@@ -91,6 +94,8 @@ constexpr int FIRST_EPI_WARP = 4;
 static_assert(1 + RB <= FIRST_EPI_WARP, "producer and issuers fit in warpgroup 0");
 constexpr int NUM_THREADS = 32 * (FIRST_EPI_WARP + NUM_EPI_WARPS);
 static_assert(NUM_ACC_SLOTS * TN == 512, "TMEM budget");
+// train-row slots per list in shared memory: KC for every list of up to KC candidates, one layout for all of them
+__host__ __device__ constexpr int list_slots(int kct) { return kct > KC ? kct : KC; }
 
 struct Barriers {
   uint64_t b_full[NUM_B_STAGES], b_empty[NUM_B_STAGES];
@@ -103,6 +108,12 @@ struct Barriers {
 // byte distance from a full barrier to its empty partner: one base register per ring, the partner is an immediate offset
 constexpr uint32_t kAccEmptyOff = offsetof(Barriers, acc_empty) - offsetof(Barriers, acc_full);
 constexpr uint32_t kCsEmptyOff = offsetof(Barriers, cs_empty) - offsetof(Barriers, cs_full);
+// dynamic shared memory of a launch: A pair, B ring, (scale, bias) ring, the lists' train rows, barriers
+constexpr size_t smem_bytes(int dp, int cs, int kct) {
+  return 1024 + (size_t)RB * TM * dp * 2 + (size_t)NUM_B_STAGES * TN * dp * 2 + (size_t)NUM_CS_STAGES * 2 * TN * 4 +
+         (size_t)RB * cs * list_slots(kct) * TM * 4 + sizeof(Barriers);
+}
+static_assert(smem_bytes(128, CSPLIT, KC_LARGE) <= 232448, "K' = 16 lists fit the 227 KB of a block at Dp = 128");
 
 // The row's top-KC list lives in shared memory, slot-major ([slot][row], conflict-free), descending
 // by score; addressed by 32-bit shared-window addresses (ld/st.shared, not generic).  Out of line
@@ -255,6 +266,13 @@ __device__ __forceinline__ void insert3(float x, uint32_t px, float& l1, float& 
   l1 = c1 ? x : l1;
   p1 = c1 ? px : p1;
 }
+// minimum of a K' = 16 list (FMNMX3 tree)
+__device__ __forceinline__ float list_min16(const float (&bv)[16]) {
+  const float m0 = fminf(fminf(bv[0], bv[1]), bv[2]), m1 = fminf(fminf(bv[3], bv[4]), bv[5]);
+  const float m2 = fminf(fminf(bv[6], bv[7]), bv[8]), m3 = fminf(fminf(bv[9], bv[10]), bv[11]);
+  const float m4 = fminf(fminf(bv[12], bv[13]), bv[14]);
+  return fminf(fminf(fminf(m0, m1), fminf(m2, m3)), fminf(m4, bv[15]));
+}
 constexpr uint32_t kKeyFloorBits = 0xff7fff80u;  // finite, below every real score: masked columns / empty entries
 __host__ __device__ constexpr int threads_for(int cs) { return 32 * (FIRST_EPI_WARP + 4 * RB * cs); }
 // Register split.  __launch_bounds__(threads, 1) makes ptxas allocate 65536 / threads registers per thread (rounded
@@ -285,8 +303,9 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
   uint8_t* smem_a = smem;                                      // RB x a_bytes (both row blocks of the unit)
   uint8_t* smem_b = smem_a + RB * a_bytes;                     // NUM_B_STAGES x b_bytes
   float* smem_cs = (float*)(smem_b + NUM_B_STAGES * b_bytes);  // NUM_CS_STAGES x {TN scales, TN biases}
-  uint32_t* smem_topi = (uint32_t*)(smem_cs + NUM_CS_STAGES * 2 * TN);  // [RB*CS][KC][TM] train rows of the top-K'
-  Barriers* bars = (Barriers*)(smem_topi + RB * CS * KC * TM);
+  constexpr int KL = list_slots(KCT);
+  uint32_t* smem_topi = (uint32_t*)(smem_cs + NUM_CS_STAGES * 2 * TN);  // [RB*CS][KL][TM] train rows of the top-K'
+  Barriers* bars = (Barriers*)(smem_topi + RB * CS * KL * TM);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int ksl = Pin.dp / KSLAB;   // 128-byte K slabs per operand row
@@ -404,7 +423,7 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
     const int ch = egrp % CS;   // column part of every tile this warp scans
     constexpr int CG = TN / CS;
     const int row_in_tile = quad * 32 + lane;
-    const uint32_t si = smem_u32(smem_topi + (egrp * KC) * TM + row_in_tile);  // this row's index slots
+    const uint32_t si = smem_u32(smem_topi + (egrp * KL) * TM + row_in_tile);  // this row's index slots
     // Position in the tile sequence (the MMA issuer's): accumulator slot (tile parity) * RB + grp and its phase, and
     // the (scale, bias) ring stage of short sweeps.  Barrier and TMEM addresses are 32-bit, computed once.
     const uint32_t acc_bar = smem_u32(&bars->acc_full[grp]), cs_bar = smem_u32(&bars->cs_full[0]);
@@ -494,11 +513,13 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
         }
         continue;
       }
-      // row-private top-KC (unsorted; aps_rerank.cu orders exactly): scores in registers, train rows in smem
+      // row-private top-KC (unsorted; aps_rerank.cu orders exactly): scores in registers, train rows in smem.  The low
+      // mantissa bits of a retained score hold its slot number: 3 bits, 4 for K' = 16
+      constexpr uint32_t kSlot = KCT > 8 ? 15u : 7u;
       float bv[KCT];
 #pragma unroll
       for (int i = 0; i < KCT; ++i) {
-        bv[i] = __uint_as_float(0xff7ffff8u | (uint32_t)i);  // ~ -FLT_MAX with the slot number in the low bits
+        bv[i] = __uint_as_float((0xff7fffffu & ~kSlot) | (uint32_t)i);  // ~ -FLT_MAX with the slot number in the low bits
         sts_u32(si + i * SLOT_STRIDE, 0xffffffffu);
       }
       float theta = bv[KCT - 1];    // min of bv == the row's K'-th best score so far (empty slots: -FLT_MAX)
@@ -618,10 +639,12 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
 #pragma unroll
                 for (int j = 6; j >= 0; --j) js = (v[j] == gm) ? j : js;
                 sts_u32(si + minpos * SLOT_STRIDE, col0 + 8 * g + js);
-                const float key = __uint_as_float((__float_as_uint(gm) & ~7u) | (uint32_t)minpos);
+                const float key = __uint_as_float((__float_as_uint(gm) & ~kSlot) | (uint32_t)minpos);
 #pragma unroll
                 for (int k = 0; k < KCT; ++k) bv[k] = (k == minpos) ? key : bv[k];
-                if constexpr (KCT == 8) {
+                if constexpr (KCT == 16) {
+                  theta = list_min16(bv);
+                } else if constexpr (KCT == 8) {
                   float m01 = fminf(fminf(bv[0], bv[1]), bv[2]);
                   float m23 = fminf(fminf(bv[3], bv[4]), bv[5]);
                   theta = fminf(fminf(m01, m23), fminf(bv[6], bv[7]));
@@ -630,7 +653,7 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
                 } else {
                   theta = fminf(fminf(bv[0], bv[1]), fminf(bv[2], bv[3]));
                 }
-                minpos = (int)(__float_as_uint(theta) & 7u);
+                minpos = (int)(__float_as_uint(theta) & kSlot);
 #pragma unroll
                 for (int j = 0; j < 8; ++j) v[j] = (j == js) ? -CUDART_INF_F : v[j];
                 gm = fmaxf(fmaxf(v[0], v[1]), v[2]);
@@ -769,12 +792,14 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
 #pragma unroll
                     for (int j = 6; j >= 0; --j) js = (cur[8 * g + j] == gm) ? j : js;
                     sts_u32(si + minpos * SLOT_STRIDE, (uint32_t)(col0 + c * 32 + 8 * g + js));
-                    // the 3 low mantissa bits of a retained score hold its slot number: one FMNMX tree yields the
-                    // new minimum AND its slot (the 7-ulp truncation is covered by the re-rank's eps)
-                    const float key = __uint_as_float((__float_as_uint(gm) & ~7u) | (uint32_t)minpos);
+                    // the 3 (K' = 16: 4) low mantissa bits of a retained score hold its slot number: one FMNMX tree
+                    // yields the new minimum AND its slot (the 7- or 15-ulp truncation is covered by the re-rank's eps)
+                    const float key = __uint_as_float((__float_as_uint(gm) & ~kSlot) | (uint32_t)minpos);
 #pragma unroll
                     for (int i = 0; i < KCT; ++i) bv[i] = (i == minpos) ? key : bv[i];
-                    if constexpr (KCT == 8) {
+                    if constexpr (KCT == 16) {
+                      theta = list_min16(bv);
+                    } else if constexpr (KCT == 8) {
                       float m01 = fminf(fminf(bv[0], bv[1]), bv[2]);
                       float m23 = fminf(fminf(bv[3], bv[4]), bv[5]);
                       theta = fminf(fminf(m01, m23), fminf(bv[6], bv[7]));
@@ -785,7 +810,7 @@ k_knn_tc(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUte
                     } else {
                       theta = fminf(fminf(bv[0], bv[1]), bv[2]);  // (KCT == 3 never reaches the streaming path)
                     }
-                    minpos = (int)(__float_as_uint(theta) & 7u);
+                    minpos = (int)(__float_as_uint(theta) & kSlot);
 #pragma unroll
                     for (int j = 0; j < 8; ++j) cur[8 * g + j] = (j == js) ? -CUDART_INF_F : cur[8 * g + j];
                     gm = fmaxf(fmaxf(cur[8 * g], cur[8 * g + 1]), cur[8 * g + 2]);
@@ -1005,8 +1030,8 @@ int aps_k_knn_tc(cudaStream_t s, int sm_count, const aps_tc_problem& p, cudaEven
     aps_set_error(APS_ERR_DIM, "", "tcgen05 path supports padded descriptor lengths 64 and 128 (got %d)", p.Dp);
     return APS_ERR_DIM;
   }
-  if (p.kcand != KC) {
-    aps_set_error(APS_ERR_ARGS, "", "kcand must be %d", KC);
+  if ((p.kcand != KC && p.kcand != KC_LARGE) || (p.kcand == KC_LARGE && p.dump)) {
+    aps_set_error(APS_ERR_ARGS, "", "kcand must be %d or %d (score dumps: %d)", KC, KC_LARGE, KC);
     return APS_ERR_ARGS;
   }
   if (p.q1 <= p.q0 || p.t1 <= p.t0) return APS_OK;
@@ -1039,7 +1064,7 @@ int aps_k_knn_tc(cudaStream_t s, int sm_count, const aps_tc_problem& p, cudaEven
   P.dump = p.dump;
   P.unit_table = nullptr;
   P.n_table_units = 0;
-  P.cand_stride = KC;
+  P.cand_stride = p.kcand;
   P.variant_flag = nullptr;
   P.variant_want = 0;
   P.idesc = p.operand_fp16 ? make_idesc_f16_f32acc(TM, TN) : make_idesc_bf16(TM, TN);
@@ -1051,8 +1076,7 @@ int aps_k_knn_tc(cudaStream_t s, int sm_count, const aps_tc_problem& p, cudaEven
     P.tiles_per_seg = sc.tiles_per_seg;
   }
   // every (row, list) slot is written by exactly one work unit (full-width units clear the unused lists)
-  const size_t smem = 1024 + (size_t)RB * TM * p.Dp * 2 + (size_t)NUM_B_STAGES * TN * p.Dp * 2 +
-                      (size_t)NUM_CS_STAGES * 2 * TN * sizeof(float) + (size_t)RB * CSPLIT * KC * TM * 4 + sizeof(Barriers);
+  const size_t smem = smem_bytes(p.Dp, CSPLIT, p.kcand);
   const int64_t units = sc.tail_balanced ? (int64_t)sc.units_full + (int64_t)sc.tail_balanced * sm_count
                                          : (int64_t)sc.units_full + (int64_t)sc.tail_units * sc.tail_seg;
   const unsigned grid = (unsigned)(units < sm_count ? units : sm_count);  // upper bound in second-pass mode
@@ -1063,7 +1087,12 @@ int aps_k_knn_tc(cudaStream_t s, int sm_count, const aps_tc_problem& p, cudaEven
     return APS_OK;
   };
   const bool pre = use_prefilter(sc, p);
-  if (p.dump)
+  if (p.kcand == KC_LARGE) {  // 6 <= k <= 12: one launch whatever the operands (the re-rank reads all 16 slots)
+    if (pre)
+      APS_TRY(p.bias ? launch(k_knn_tc<true, false, true, KC_LARGE>) : launch(k_knn_tc<false, false, true, KC_LARGE>));
+    else
+      APS_TRY(p.bias ? launch(k_knn_tc<true, false, false, KC_LARGE>) : launch(k_knn_tc<false, false, false, KC_LARGE>));
+  } else if (p.dump)
     APS_TRY(p.bias ? launch(k_knn_tc<true, true, false, KC>) : launch(k_knn_tc<false, true, false, KC>));
   else if (p.exact_flag && !p.nrows_dev) {
     // list size chosen by a device-side flag, no host round trip: both variants are launched, one exits at once
@@ -1137,8 +1166,7 @@ int aps_k_knn_tc_units(cudaStream_t s, int sm_count, const aps_tc_problem& p, co
   P.n_table_units = n_units;
   P.cand_stride = p.kcand;
   const int cs_groups = p.kcand == 3 ? 2 : CSPLIT;  // epilogue groups per row block of the variant launched below
-  const size_t smem = 1024 + (size_t)RB * TM * p.Dp * 2 + (size_t)NUM_B_STAGES * TN * p.Dp * 2 +
-                      (size_t)NUM_CS_STAGES * 2 * TN * sizeof(float) + (size_t)RB * cs_groups * KC * TM * 4 + sizeof(Barriers);
+  const size_t smem = smem_bytes(p.Dp, cs_groups, KC);
   const unsigned grid = (unsigned)(n_units < sm_count ? n_units : sm_count);
   const int threads = threads_for(cs_groups);
   auto launch = [&](auto kern) -> int {
