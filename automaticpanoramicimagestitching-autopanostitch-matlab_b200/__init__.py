@@ -7,7 +7,7 @@ from csrc/*.cu).  There is no CPU implementation in here: every call needs the C
 a B200, and fails loudly otherwise.
 """
 from . import _lib  # noqa: F401
-from ._lib import ApsError, Context, build_library, library_path  # noqa: F401
+from ._lib import ApsError, Context, DeviceGroup, build_library, library_path  # noqa: F401
 from .host import (  # noqa: F401
     ApsSemanticsWarning,
     GlobalPlan,

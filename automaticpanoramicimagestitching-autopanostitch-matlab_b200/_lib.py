@@ -143,6 +143,15 @@ def lib():
         "aps_pplan_match": (i32, [vp, dbl, dbl, i32, i32, pp]),
         "aps_pplan_set_method": (i32, [vp, i32, i64, C.c_uint64]),
         "aps_pplan_subset_table": (i32, [vp, i32, vp]),
+        "aps_group_create": (i32, [C.POINTER(i32), i32, pp]),
+        "aps_group_destroy": (None, [vp]),
+        "aps_group_size": (i32, [vp]),
+        "aps_group_ctx": (vp, [vp, i32]),
+        "aps_group_stage_times": (i32, [vp, i32, C.POINTER(dbl)]),
+        "aps_debug_group_create_shared": (i32, [i32, i32, pp]),
+        "aps_group_feature_matching_global": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, i32, dbl, i32, pp]),
+        "aps_group_feature_matching_pairwise": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, dbl, dbl, i32, i64,
+                                                      C.c_uint64, pp]),
         "aps_debug_tc_slots": (i32, [vp, i64, i64]),
         "aps_debug_pair_screen": (i32, [vp, vp, i64, vp, i64, i32, vp, vp, i32]),
         "aps_debug_tc_scores": (i32, [vp, vp, i64, vp, i64, i32, i32, vp, vp, vp]),
@@ -221,7 +230,8 @@ class Context:
 
     def close(self):
         if getattr(self, "_h", None):
-            lib().aps_ctx_destroy(self._h)
+            if getattr(self, "_owner", None) is None:   # a device group's member context is released with the group
+                lib().aps_ctx_destroy(self._h)
             self._h = None
 
     def __del__(self):
@@ -238,3 +248,69 @@ def default_context(device: int = 0) -> Context:
     if device not in _default_ctx:
         _default_ctx[device] = Context(device)
     return _default_ctx[device]
+
+
+class DeviceGroup:
+    """Several GPUs driven from this process (aps_group, include/apsmatch.h): the one-call global and pairwise entries
+    spread over the members and return lists bit-identical to a single Context's.  `devices` are CUDA ordinals."""
+
+    def __init__(self, devices, shared_members: int = 0):
+        """shared_members > 0 (tests): that many members, all on the single device devices[0]
+        (aps_debug_group_create_shared)."""
+        L = lib()
+        devs = [int(d) for d in devices]
+        h = C.c_void_p()
+        if shared_members:
+            devs = devs[:1] * int(shared_members)
+            check(L.aps_debug_group_create_shared(devs[0] if devs else 0, int(shared_members), C.byref(h)))
+        else:
+            arr = (C.c_int * max(len(devs), 1))(*devs)
+            check(L.aps_group_create(arr, len(devs), C.byref(h)))
+        self._h = h
+        self.devices = tuple(devs)
+        self._members = []
+        for i in range(len(devs)):
+            m = Context.__new__(Context)
+            m._h, m.device, m._owner = C.c_void_p(L.aps_group_ctx(h, i)), devs[i], self
+            self._members.append(m)
+
+    @property
+    def handle(self):
+        return self._h
+
+    def __len__(self):
+        return len(self.devices)
+
+    def ctx(self, i: int) -> Context:
+        """Member i's context: its knobs and the statistics of its share of the last call."""
+        return self._members[i]
+
+    def stage_times(self, i: int):
+        """Member i's device milliseconds of the last multi-member call: upload, exchange, search, finish."""
+        a = (C.c_double * 4)()
+        check(lib().aps_group_stage_times(self._h, int(i), a))
+        return {"upload": a[0], "exchange": a[1], "search": a[2], "finish": a[3]}
+
+    def close(self):
+        if getattr(self, "_h", None):
+            for m in self._members:
+                m._h = None
+            lib().aps_group_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+_default_group = {}
+
+
+def default_group(devices) -> DeviceGroup:
+    """One cached group per device list (in order), like default_context."""
+    key = tuple(int(d) for d in devices)
+    if key not in _default_group:
+        _default_group[key] = DeviceGroup(key)
+    return _default_group[key]

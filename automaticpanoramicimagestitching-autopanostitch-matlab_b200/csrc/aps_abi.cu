@@ -745,13 +745,20 @@ extern "C" void* aps_gplan_knn_idx_device(aps_gplan* p) { return p ? p->knn_idx.
 extern "C" void* aps_gplan_knn_dist_device(aps_gplan* p) { return p ? p->knn_dist.p : nullptr; }
 
 extern "C" int aps_gplan_upload(aps_gplan* p, const void* const* desc, int layout) {
+  return gplan_upload_images(p, desc, layout, 0, p ? p->n : 0);
+}
+
+// H2D of images [i0, i1) only, into their rows of the pooled matrix (a device group's members each upload one range)
+int gplan_upload_images(aps_gplan* p, const void* const* desc, int layout, int i0, int i1) {
   if (!p) APS_FAIL(APS_ERR_ARGS, "", "plan is NULL");
   aps_ctx* c = p->c;
   APS_CTX(c);
+  if (i0 < 0 || i1 > p->n || i0 > i1) APS_FAIL(APS_ERR_ARGS, "", "image range out of bounds");
   const int esz = p->dtype == APS_F32 ? 4 : 1;
   char* base = (char*)aps_gplan_desc_device(p);
-  if (layout == APS_COL_MAJOR && p->F > 0) APS_TRY(p->stage_tmp.alloc((size_t)p->F * p->D * esz, c->stream));
-  for (int i = 0; i < p->n; ++i) {
+  const int64_t r0 = p->off[i0], rows = p->off[i1] - r0;
+  if (layout == APS_COL_MAJOR && rows > 0) APS_TRY(p->stage_tmp.alloc((size_t)rows * p->D * esz, c->stream));
+  for (int i = i0; i < i1; ++i) {
     const int64_t Ni = p->counts[i];
     if (Ni == 0) continue;
     if (!desc || !desc[i]) APS_FAIL(APS_ERR_ARGS, "", "descriptor pointer %d is NULL but its count is %lld", i, (long long)Ni);
@@ -760,7 +767,7 @@ extern "C" int aps_gplan_upload(aps_gplan* p, const void* const* desc, int layou
     if (layout == APS_ROW_MAJOR) {
       APS_CUDA(cudaMemcpyAsync(dst, desc[i], bytes, cudaMemcpyHostToDevice, c->stream));
     } else {
-      char* st = (char*)p->stage_tmp.p + (size_t)p->off[i] * p->D * esz;
+      char* st = (char*)p->stage_tmp.p + (size_t)(p->off[i] - r0) * p->D * esz;
       APS_CUDA(cudaMemcpyAsync(st, desc[i], bytes, cudaMemcpyHostToDevice, c->stream));
       APS_TRY(aps_k_transpose_in(c->stream, st, Ni, p->D, esz, dst));
     }
@@ -788,9 +795,9 @@ extern "C" int aps_gplan_knn(aps_gplan* p, int64_t q0, int64_t q1) {
   aps_ctx* c = p->c;
   APS_CTX(c);
   if (q0 < 0 || q1 > p->F || q0 > q1) APS_FAIL(APS_ERR_ARGS, "", "query range out of bounds");
-  if (q0 == q1) return APS_OK;
-  c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
+  c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;  // an empty range reports an empty search
   c->h_flags[36] = 0;
+  if (q0 == q1) return APS_OK;
   if (p->dtype == APS_F32) {
     FloatSide s = p->fs.side();
     APS_TRY(float_knn(c, s, q0, q1, s, 0, p->F, p->D, p->k, /*metric*/ 0, /*bias*/ 0, p->fs.flags.p, 0,
@@ -902,6 +909,13 @@ extern "C" int aps_feature_matching_global(aps_ctx* c, const void* const* desc, 
                                            int dtype, int layout, int k, double ratio, int use_bf,
                                            aps_matchlist** out) {
   (void)use_bf;
+  return feature_matching_global_impl(c, desc, counts, n, D, dtype, layout, k, ratio, /*mutual*/ 0, out);
+}
+
+// the single-context pipeline behind aps_feature_matching_global (and a one-member aps_group); mutual != 0 adds the
+// opt-in cross-check of aps_gplan_filter_mutual
+int feature_matching_global_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
+                                 int layout, int k, double ratio, int mutual, aps_matchlist** out) {
   APS_CTX(c);
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
   *out = nullptr;
@@ -913,6 +927,7 @@ extern "C" int aps_feature_matching_global(aps_ctx* c, const void* const* desc, 
     if (rc == APS_OK) rc = aps_gplan_prepare(p);
     if (rc == APS_OK) rc = aps_gplan_knn(p, 0, p->F);
     if (rc == APS_OK) rc = aps_gplan_filter(p, 0, p->F, ratio);
+    if (rc == APS_OK && mutual) rc = aps_gplan_filter_mutual(p);
     if (rc == APS_OK) rc = aps_gplan_compact(p);
   }
   if (rc == APS_OK) rc = aps_gplan_download(p, out);

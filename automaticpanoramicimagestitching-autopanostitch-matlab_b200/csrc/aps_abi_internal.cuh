@@ -87,6 +87,14 @@ int hamming2_device(aps_ctx* c, const uint8_t* qpad, int64_t q0, int64_t N1, con
 int ssd2_device(aps_ctx* c, const FloatSide& Q, int64_t q0, int64_t N1, const FloatSide& T, int64_t t0, int64_t N2, int D,
                 const int32_t* flags, bool tc, int bias_mode, uint32_t* idx2, float* d1, float* d2);
 
+// ---- one-call pipelines over the staged plans (aps_abi.cu / aps_abi_pairwise.cu; aps_abi_group.cu runs them per member)
+int gplan_upload_images(aps_gplan* p, const void* const* desc, int layout, int i0, int i1);
+int feature_matching_global_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
+                                 int layout, int k, double ratio, int mutual, aps_matchlist** out);
+int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
+                                   int layout, double match_threshold, double max_ratio, int method, int64_t subset,
+                                   uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out);
+
 // ---- match lists: the n x n cell in CSR form -----------------------------------------------------------------------
 struct aps_matchlist {
   int n = 0;

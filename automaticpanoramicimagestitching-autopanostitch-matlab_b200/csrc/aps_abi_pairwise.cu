@@ -1011,9 +1011,9 @@ extern "C" int aps_pplan_match(aps_pplan* p, double match_threshold, double max_
   return APS_OK;
 }
 
-static int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D,
-                                          int dtype, int layout, double match_threshold, double max_ratio,
-                                          int pair_first, int pair_stride, aps_matchlist** out) {
+int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
+                                   int layout, double match_threshold, double max_ratio, int method, int64_t subset,
+                                   uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out) {
   APS_CTX(c);
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
   *out = nullptr;
@@ -1021,8 +1021,8 @@ static int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, c
     APS_FAIL(APS_ERR_ARGS, "", "bad arguments");
   aps_pplan* p = nullptr;
   APS_TRY(aps_pplan_create(c, counts, n, D, dtype, &p));
-  int rc = APS_OK;
-  if (p->F > 0 && n >= 2) {
+  int rc = aps_pplan_set_method(p, method, subset, seed);
+  if (rc == APS_OK && p->F > 0 && n >= 2) {
     rc = aps_pplan_upload(p, desc, layout);
     if (rc == APS_OK) rc = aps_pplan_prepare(p);  // an error here must not reach the pair classification (ps.big)
   }
@@ -1034,14 +1034,15 @@ static int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, c
 extern "C" int aps_feature_matching_pairwise(aps_ctx* c, const void* const* desc, const int64_t* counts, int n,
                                              int D, int dtype, int layout, double match_threshold, double max_ratio,
                                              aps_matchlist** out) {
-  return feature_matching_pairwise_impl(c, desc, counts, n, D, dtype, layout, match_threshold, max_ratio, 0, 1, out);
+  return feature_matching_pairwise_impl(c, desc, counts, n, D, dtype, layout, match_threshold, max_ratio,
+                                        APS_METHOD_EXHAUSTIVE, 12000, 0, 0, 1, out);
 }
 
 extern "C" int aps_feature_matching_pairwise_shard(aps_ctx* c, const void* const* desc, const int64_t* counts, int n,
                                                    int D, int dtype, int layout, double match_threshold,
                                                    double max_ratio, int pair_first, int pair_stride,
                                                    aps_matchlist** out) {
-  return feature_matching_pairwise_impl(c, desc, counts, n, D, dtype, layout, match_threshold, max_ratio, pair_first,
-                                        pair_stride, out);
+  return feature_matching_pairwise_impl(c, desc, counts, n, D, dtype, layout, match_threshold, max_ratio,
+                                        APS_METHOD_EXHAUSTIVE, 12000, 0, pair_first, pair_stride, out);
 }
 

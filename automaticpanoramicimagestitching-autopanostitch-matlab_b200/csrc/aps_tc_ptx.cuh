@@ -182,15 +182,17 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+// Resolved once per process; the function-local static makes the first call thread-safe (several host threads build
+// tensor maps at once when a device group runs its members in parallel).
 static PFN_encodeTiled get_encode() {
-  static PFN_encodeTiled fn = nullptr;
-  if (!fn) {
+  static const PFN_encodeTiled fn = []() -> PFN_encodeTiled {
     void* p = nullptr;
     cudaDriverEntryPointQueryResult qres;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
         qres == cudaDriverEntryPointSuccess)
-      fn = (PFN_encodeTiled)p;
-  }
+      return (PFN_encodeTiled)p;
+    return nullptr;
+  }();
   return fn;
 }
 

@@ -144,12 +144,32 @@ def _desc_args(mats, counts):
     return ptrs, cnt, layout, mats
 
 
+def _aps_gpus(input, ctx):
+    """input.apsGPUs: GPUs to spread the call over, 1-based like MATLAB's gpuDevice.  Returns (group or None, ctx):
+    a DeviceGroup when more than one GPU is listed; one GPU -> that GPU's default context (unless ctx is given)."""
+    gpus = _field(input, "apsGPUs", None)
+    if gpus is None:
+        return None, ctx or default_context()
+    g = np.atleast_1d(np.asarray(gpus, dtype=np.float64)).ravel()
+    if g.size and (not np.all(np.isfinite(g)) or np.any(g != np.round(g)) or np.any(g < 1)
+                   or len(set(g.tolist())) != g.size):
+        raise ValueError("input.apsGPUs must list distinct positive integer GPU indices (1-based, as gpuDevice)")
+    devices = [int(v) - 1 for v in g]
+    if len(devices) > 1:
+        if ctx is not None:
+            raise ValueError("input.apsGPUs with several GPUs and ctx= are alternative ways to choose the device")
+        return _lib.default_group(devices), None
+    return None, ctx or default_context(devices[0] if devices else 0)
+
+
 def featureMatchingGlobal(input, allDescriptors, numImg, ctx=None):
     """matches = featureMatchingGlobal(input, allDescriptors, numImg)   (featureMatchingGlobal.m:1-163)
 
     Returns an n x n nested list `matches[i][j]` (0-based): [M x 2] float64 index pairs (1-based
-    local feature indices, column 0 -> image i, column 1 -> image j) for i < j, empty elsewhere."""
-    ctx = ctx or default_context()
+    local feature indices, column 0 -> image i, column 1 -> image j) for i < j, empty elsewhere.
+    input.apsGPUs (1-based GPU indices) listing several GPUs spreads the call over them (aps_group_feature_matching_global,
+    same lists)."""
+    group, ctx = _aps_gpus(input, ctx)
     if not (np.isscalar(numImg) and np.isfinite(numImg) and numImg > 0):
         raise ValueError("numImg must be a positive finite scalar")  # arguments block :35-39
     k = int(_field(input, "k", required=True))
@@ -161,6 +181,13 @@ def featureMatchingGlobal(input, allDescriptors, numImg, ctx=None):
         return [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)]  # :49-52
     ptrs, cnt, layout, keep = _desc_args(mats, counts)
     h = C.c_void_p()
+    if group is not None:
+        check(lib().aps_group_feature_matching_global(group.handle, ptrs, cnt, n, int(D), APS_U8 if is_binary else APS_F32,
+                                                      layout, k, ratio, int(mutual), C.byref(h)))
+        try:
+            return _cells_from_matchlist(h, n)[0]
+        finally:
+            lib().aps_matchlist_free(h)
     if mutual:
         plan = GlobalPlan(ctx, counts, D, is_binary, k)
         try:
@@ -240,8 +267,12 @@ def featureMatchingPairwise(input, allDescriptors, numImg, ctx=None, return_metr
     the reference does (matchFeaturesScratch.m:611).
     shard=(first, stride): compute only every stride-th pair of the column-major pair list (one share
     per GPU rank); cells of other shares come back empty and are merged by `merge_pairwise_shards`.
-    csr=True returns the compacted lists as they leave the C ABI: (pair_ptr [n*n+1], rows [M x 2] uint32, metric [M])."""
-    ctx = ctx or default_context()
+    csr=True returns the compacted lists as they leave the C ABI: (pair_ptr [n*n+1], rows [M x 2] uint32, metric [M]).
+    input.apsGPUs (1-based GPU indices) listing several GPUs spreads the pairs over them in this process
+    (aps_group_feature_matching_pairwise, same lists); it cannot be combined with shard=."""
+    if shard is not None and _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs and shard= are alternative ways to split the image pairs; pass one of them")
+    group, ctx = _aps_gpus(input, ctx)
     if not (np.isscalar(numImg) and np.isfinite(numImg) and numImg > 0):
         raise ValueError("numImg must be a positive finite scalar")
     method = str(_field(input, "Matchingmethod", "Exhaustive")).lower()
@@ -259,7 +290,11 @@ def featureMatchingPairwise(input, allDescriptors, numImg, ctx=None, return_metr
     ptrs, cnt, layout, keep = _desc_args(mats, counts)
     h = C.c_void_p()
     first, stride = shard if shard is not None else (0, 1)
-    if aps_method != APS_METHOD["exhaustive"] and not is_binary:
+    if group is not None:
+        check(lib().aps_group_feature_matching_pairwise(group.handle, ptrs, cnt, n, int(D), APS_U8 if is_binary else APS_F32,
+                                                        layout, thr, ratio, aps_method, int(_field(input, "apsSubset", 12000)),
+                                                        int(_field(input, "apsSeed", 0)), C.byref(h)))
+    elif aps_method != APS_METHOD["exhaustive"] and not is_binary:
         ph = C.c_void_p()
         check(lib().aps_pplan_create(ctx.handle, cnt, n, int(D), APS_F32, C.byref(ph)))
         try:

@@ -304,6 +304,50 @@ int aps_pplan_subset_table(aps_pplan* p, int image, int32_t* out /* [subset] */)
 int aps_pplan_match(aps_pplan* p, double match_threshold, double max_ratio, int pair_first, int pair_stride,
                     aps_matchlist** out);
 
+/* ---- device group: single-process multi-GPU matching ------------------------------------------------------
+ * The reference's only parallelism is parfor over the image pairs (PP/featureMatching/featureMatchingPairwise.m:48-59),
+ * and a MATLAB process cannot join an NCCL world; a device group spreads one call of featureMatchingGlobal /
+ * featureMatchingPairwise over several GPUs of one process instead.  The lists are BIT-IDENTICAL to the
+ * single-context calls: the group runs the staged plans above on every member and exchanges only device buffers
+ * (cudaMemcpyPeerAsync; staged by the driver where the GPUs have no peer access).  One host thread per member issues
+ * that member's work, so the GPUs run concurrently even where the pairwise batches synchronise on host tables.
+ * A one-member group runs exactly the single-context code on its device.
+ *
+ * aps_group_create: one aps_ctx per listed CUDA ordinal -- distinct and in range (else APS_ERR_ARGS), sm_100a (else
+ *   APS_ERR_NOGPU, as without any device); where cudaDeviceCanAccessPeer allows, members get direct peer access to each
+ *   other's memory, including their default stream-ordered memory pools (cudaMemPoolSetAccess), which hold every
+ *   buffer the group exchanges.  This is process-wide state of those devices and is left in place by aps_group_destroy.
+ * aps_group_ctx: member i's context (knobs such as aps_ctx_set_float_engine, and per-member statistics: after a global
+ *   call aps_ctx_last_stats[0] of member i = the query rows it searched; after a pairwise call aps_ctx_pairwise_stats
+ *   = its share of the screened pairs).
+ * Failure of any member fails the whole call: no list is returned, every plan is released, and aps_last_error /
+ * aps_error_id of the CALLING thread carry the first failing member's message and id. */
+typedef struct aps_group aps_group;
+int aps_group_create(const int* devices, int ndev, aps_group** out);
+void aps_group_destroy(aps_group* g);
+int aps_group_size(const aps_group* g);
+aps_ctx* aps_group_ctx(aps_group* g, int i);
+/* featureMatchingGlobal (float and uint8, k <= APS_MAX_K; mutual != 0 = the opt-in cross-check of
+ * aps_gplan_filter_mutual).  Member i uploads a contiguous range of whole images (balanced by row count) and copies the
+ * other members' ranges peer-to-peer, so every member holds all descriptors; K1 runs on every member; member i searches
+ * query rows [q0, q1) = i-th block of equal multiples of 128 rows (members past F get an empty block) and filters them;
+ * the record slices are copied into member 0, which cross-checks (if asked), compacts and downloads. */
+int aps_group_feature_matching_global(aps_group* g, const void* const* desc, const int64_t* counts, int n, int D,
+                                      int dtype, int layout, int k, double ratio, int mutual, aps_matchlist** out);
+/* featureMatchingPairwise (float and uint8, every aps_method with its subset / seed as in aps_pplan_set_method).
+ * Member 0 uploads; its pooled matrix is copied peer-to-peer to the other members; member i computes the pairs whose
+ * column-major ordinal is congruent to i modulo the group size (aps_pplan_match(i, N)); the host lists are merged
+ * into one CSR in cell order. */
+int aps_group_feature_matching_pairwise(aps_group* g, const void* const* desc, const int64_t* counts, int n, int D,
+                                        int dtype, int layout, double match_threshold, double max_ratio, int method,
+                                        int64_t subset, uint64_t seed, aps_matchlist** out);
+/* Measurement hook: member i's device time (ms, CUDA events on its stream) of the last multi-member call, per stage:
+ * [0] host upload of its share, [1] peer exchange of the descriptors (includes waiting for the producers' uploads),
+ * [2] search = K1 + kNN + filter (global) or K1 + its pair share (pairwise), [3] member 0 of a global call: from the
+ * end of its own search to the lists on the host (waiting for the slowest member, record gather, cross-check,
+ * compaction, download).  Stages a member did not run, and one-member groups, report 0. */
+int aps_group_stage_times(aps_group* g, int i, double ms[4]);
+
 /* ---- diagnostics (tests only): raw output of the tcgen05 candidate kernel -----------------------
  * Q [nq x D], T [nt x D] ROW-major float (used as given, no normalisation).  scores [nq x nt]
  * receives (bf16(q).bf16(t))*scale_t + bias_t as the kernel's epilogue computes it (scale = 1,
@@ -316,6 +360,10 @@ int aps_debug_tc_slots(aps_ctx* ctx, int64_t nq, int64_t nt);
  * [N1 x dump_tiles x 64] the raw accumulator registers (two packed fp16 scores each) of the first dump_tiles tiles. */
 int aps_debug_pair_screen(aps_ctx* ctx, const float* A, int64_t N1, const float* B, int64_t N2, int D, float* b1b2,
                           uint32_t* dump, int dump_tiles);
+/* A device group of `nmembers` contexts that all live on `device` (aps_group_create refuses a repeated device): runs the
+ * multi-member pipelines -- one host thread per member, event-ordered device-to-device exchanges, the merge -- on a
+ * machine with one GPU.  The lists are the same as for any other group. */
+int aps_debug_group_create_shared(int device, int nmembers, aps_group** out);
 int aps_debug_tc_scores(aps_ctx* ctx, const float* Q, int64_t nq, const float* T, int64_t nt, int D, int nseg,
                         float* scores, uint32_t* cand_idx, float* cand_score);
 /* The candidate lists of one tcgen05 launch, prepared and scheduled as the float searches run it.  Q [nq x D], T [nt x D]

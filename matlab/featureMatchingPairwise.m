@@ -5,6 +5,8 @@ function matches = featureMatchingPairwise(input, allDescriptors, numImg)
     %   inputs.m default) / 'kdtree' (Euclidean searches, matchFeaturesScratch.m:142-155) / 'pca2nn' (PCA-48 + cosine, :130-141).
     %   (The MathWorks matchFeatures branch, input.useMATLABFeatureMatch = 1, is closed source; with this file on the
     %   path the scratch semantics are used and a warning says so.)
+    %   input.apsGPUs (optional, e.g. 1:gpuDeviceCount): spread the image pairs over these GPUs (gpuDevice numbering)
+    %   from this one process instead of parfor workers; the match lists are identical to the one-GPU call.
     arguments
         input struct
         allDescriptors cell
@@ -31,5 +33,10 @@ function matches = featureMatchingPairwise(input, allDescriptors, numImg)
                 error('Select a approximate method');
         end
     end
-    matches = aps_featureMatching_mex('pairwise', allDescriptors, numImg, input.Matchingthreshold, input.Ratiothreshold, method);
+    if isfield(input, 'apsGPUs')
+        matches = aps_featureMatching_mex('pairwise', allDescriptors, numImg, input.Matchingthreshold, ...
+            input.Ratiothreshold, method, double(input.apsGPUs));
+    else
+        matches = aps_featureMatching_mex('pairwise', allDescriptors, numImg, input.Matchingthreshold, input.Ratiothreshold, method);
+    end
 end

@@ -1,10 +1,12 @@
 // aps_featureMatching_mex.cpp -- batched gateway: the whole featureMatching/ stage in one device round trip.
-//   matches = aps_featureMatching_mex('global',   allDescriptors, numImg, k, ratioThr, useBF)
-//   matches = aps_featureMatching_mex('pairwise', allDescriptors, numImg, matchThreshold, maxRatio [, method])
+//   matches = aps_featureMatching_mex('global',   allDescriptors, numImg, k, ratioThr, useBF [, gpus])
+//   matches = aps_featureMatching_mex('pairwise', allDescriptors, numImg, matchThreshold, maxRatio [, method [, gpus]])
 //   [cand, IuptriIdx] = aps_featureMatching_mex('partners', matchesAll | countMatrix, m)
 // Called by the drop-in matlab/featureMatchingGlobal.m / featureMatchingPairwise.m (same signatures as
 // PP/featureMatching/featureMatchingGlobal.m:1 and featureMatchingPairwise.m:1) and by the two-line patch of
 // PP/imageMatching/imageMatching.m:75-100 shown in INTEGRATION.md.
+// gpus: optional vector of 1-based GPU indices (gpuDevice numbering).  Absent, [] or 1 = the single default context
+// (device 1); any other list runs the call on a device group of those GPUs (aps_group_*, same lists).
 #include "aps_mex_common.h"
 
 void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
@@ -38,6 +40,8 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     return;
   }
   if (!mxIsCell(prhs[1])) mexErrMsgIdAndTxt("apsmatch:args", "allDescriptors must be a cell array");
+  const std::vector<int> gpus = aps_mex_gpus(nrhs > 6 ? prhs[6] : nullptr);
+  const bool grouped = !gpus.empty() && !(gpus.size() == 1 && gpus[0] == 0);
   const int n = (int)mxGetScalar(prhs[2]);
   std::vector<const void*> ptrs;
   std::vector<int64_t> counts;
@@ -52,13 +56,22 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   int rc;
   if (mode == "global") {
     if (nrhs < 5) mexErrMsgIdAndTxt("apsmatch:args", "global: need k and ratio threshold");
-    rc = aps_feature_matching_global(aps_mex_ctx(), ptrs.data(), counts.data(), n, D, dtype, APS_COL_MAJOR,
-                                     (int)mxGetScalar(prhs[3]), mxGetScalar(prhs[4]),
-                                     nrhs > 5 ? (int)mxGetScalar(prhs[5]) : 0, &ml);
+    if (grouped) {
+      rc = aps_group_feature_matching_global(aps_mex_group(gpus), ptrs.data(), counts.data(), n, D, dtype, APS_COL_MAJOR,
+                                             (int)mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), /*mutual*/ 0, &ml);
+    } else {
+      rc = aps_feature_matching_global(aps_mex_ctx(), ptrs.data(), counts.data(), n, D, dtype, APS_COL_MAJOR,
+                                       (int)mxGetScalar(prhs[3]), mxGetScalar(prhs[4]),
+                                       nrhs > 5 ? (int)mxGetScalar(prhs[5]) : 0, &ml);
+    }
   } else if (mode == "pairwise") {
     if (nrhs < 5) mexErrMsgIdAndTxt("apsmatch:args", "pairwise: need MatchThreshold and MaxRatio");
     const int method = nrhs > 5 ? (int)mxGetScalar(prhs[5]) : APS_METHOD_EXHAUSTIVE;   // aps_method
-    if (method == APS_METHOD_EXHAUSTIVE || dtype == APS_U8) {
+    if (grouped) {
+      rc = aps_group_feature_matching_pairwise(aps_mex_group(gpus), ptrs.data(), counts.data(), n, D, dtype,
+                                               APS_COL_MAJOR, mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), method, 12000,
+                                               0, &ml);
+    } else if (method == APS_METHOD_EXHAUSTIVE || dtype == APS_U8) {
       rc = aps_feature_matching_pairwise(aps_mex_ctx(), ptrs.data(), counts.data(), n, D, dtype, APS_COL_MAJOR,
                                          mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), &ml);
     } else {   // 'subsetpdist2' / 'kdtree' (matchFeaturesScratch.m:142-155): staged plan with the Euclidean metric

@@ -12,9 +12,19 @@
 #include "mex.h"
 
 static aps_ctx* g_aps_ctx = nullptr;
+static aps_group* g_aps_group = nullptr;     // device group of the last multi-GPU call (one per process)
+static std::vector<int> g_aps_group_devices;  // its CUDA ordinals
+static bool g_aps_atexit = false;
 static void aps_mex_cleanup(void) {
   if (g_aps_ctx) aps_ctx_destroy(g_aps_ctx);
   g_aps_ctx = nullptr;
+  if (g_aps_group) aps_group_destroy(g_aps_group);
+  g_aps_group = nullptr;
+  g_aps_group_devices.clear();
+}
+static inline void aps_mex_register_cleanup(void) {
+  if (!g_aps_atexit) mexAtExit(aps_mex_cleanup);
+  g_aps_atexit = true;
 }
 static inline void aps_mex_fail(const char* fallback_id) {
   const char* id = aps_error_id();
@@ -23,9 +33,39 @@ static inline void aps_mex_fail(const char* fallback_id) {
 static inline aps_ctx* aps_mex_ctx(void) {
   if (!g_aps_ctx) {
     if (aps_ctx_create(0, &g_aps_ctx) != APS_OK) aps_mex_fail("apsmatch:nogpu");  // no CPU fallback
-    mexAtExit(aps_mex_cleanup);
+    aps_mex_register_cleanup();
   }
   return g_aps_ctx;
+}
+// Optional trailing `gpus` argument of the batched gateway: 1-based GPU indices (MATLAB's gpuDevice numbering), a
+// real double vector of distinct positive integers; [] or absent = the default device.  Returns 0-based ordinals.
+// Checked before any device is touched.
+static inline std::vector<int> aps_mex_gpus(const mxArray* a) {
+  std::vector<int> devs;
+  if (!a || mxIsEmpty(a)) return devs;
+  if (!mxIsDouble(a) || mxIsComplex(a) || mxGetNumberOfDimensions(a) != 2 || (mxGetM(a) != 1 && mxGetN(a) != 1))
+    mexErrMsgIdAndTxt("apsmatch:args", "gpus must be a real double vector of GPU indices (1-based, as gpuDevice)");
+  const double* v = mxGetPr(a);
+  for (size_t i = 0; i < mxGetNumberOfElements(a); ++i) {
+    if (!(v[i] >= 1.0 && v[i] <= 65536.0) || v[i] != (double)(int)v[i])
+      mexErrMsgIdAndTxt("apsmatch:args", "gpus(%d) = %g is not a positive integer GPU index", (int)i + 1, v[i]);
+    for (size_t j = 0; j < i; ++j)
+      if (v[j] == v[i]) mexErrMsgIdAndTxt("apsmatch:args", "GPU %d is listed twice in gpus", (int)v[i]);
+    devs.push_back((int)v[i] - 1);
+  }
+  return devs;
+}
+// One aps_group per process for the last device list used; a different list replaces it.
+static inline aps_group* aps_mex_group(const std::vector<int>& devs) {
+  if (g_aps_group && devs == g_aps_group_devices) return g_aps_group;
+  if (g_aps_group) aps_group_destroy(g_aps_group);
+  g_aps_group = nullptr;
+  g_aps_group_devices.clear();
+  const int rc = aps_group_create(devs.data(), (int)devs.size(), &g_aps_group);
+  if (rc != APS_OK) aps_mex_fail(rc == APS_ERR_ARGS ? "apsmatch:args" : "apsmatch:nogpu");  // e.g. a GPU that does not exist
+  g_aps_group_devices = devs;
+  aps_mex_register_cleanup();
+  return g_aps_group;
 }
 // allDescriptors{i}: numeric matrix, or a binaryFeatures object (its .Features, featureMatchingGlobal.m:56-75).
 // *is_binary: the element is a binaryFeatures OBJECT -- the reference decides "binary" by class alone (:56); a plain

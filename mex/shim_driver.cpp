@@ -23,7 +23,8 @@ static int expect_error(const char* want, int nlhs, int nrhs, const mxArray** in
 
 // ---- file mode: `gate file in.bin out.bin` ---------------------------------------------------------------------
 // in.bin : int32 nmat ; per matrix int32 cls (0 single, 1 uint8, 2 double, 4 uint8 wrapped in a binaryFeatures
-//          object), int32 rows, int32 cols, column-major payload ; int32 nscalars ; doubles.
+//          object), int32 rows, int32 cols, column-major payload ; int32 nscalars ; doubles ; optionally (batched
+//          gateway) int32 ngpus ; doubles = the trailing `gpus` vector (1-based GPU indices).
 // out.bin: int32 nout ; per output int32 cls (0 single, 1 uint8, 2 double, 3 uint32, -1 empty), rows, cols, payload.
 // tests/test_mex_gateways.py builds the inputs, runs the gateway on the GPU and compares the outputs with the oracle.
 static mxArray* read_matrix(FILE* f) {
@@ -63,6 +64,12 @@ static int file_mode(const char* in_path, const char* out_path) {
   if (std::fread(&nsc, 4, 1, f) != 1) return 2;
   std::vector<double> sc((size_t)nsc);
   if (nsc && std::fread(sc.data(), 8, (size_t)nsc, f) != (size_t)nsc) return 2;
+  int32_t ngpu = 0;
+  std::vector<double> gpus;
+  if (std::fread(&ngpu, 4, 1, f) == 1 && ngpu > 0) {
+    gpus.resize((size_t)ngpu);
+    if (std::fread(gpus.data(), 8, (size_t)ngpu, f) != (size_t)ngpu) return 2;
+  }
   std::fclose(f);
   mxArray* out[4] = {nullptr, nullptr, nullptr, nullptr};
   int nout = 0;
@@ -84,6 +91,11 @@ static int file_mode(const char* in_path, const char* out_path) {
     std::vector<const mxArray*> in = {mxCreateString(sc[0] == 0.0 ? "global" : "pairwise"), cells,
                                       mxCreateDoubleScalar((double)nmat)};
     for (size_t i = 1; i < sc.size(); ++i) in.push_back(mxCreateDoubleScalar(sc[i]));
+    if (!gpus.empty()) {  // after (k, ratio, useBF) / (MatchThreshold, MaxRatio, method)
+      mxArray* g = mxCreateDoubleMatrix(1, (mwSize)gpus.size(), mxREAL);
+      for (size_t i = 0; i < gpus.size(); ++i) mxGetPr(g)[i] = gpus[i];
+      in.push_back(g);
+    }
     mexFunction(1, out, (int)in.size(), in.data());
     for (int j = 0; j < nmat; ++j)   // upper-triangle cells in column-major order
       for (int i = 0; i < j; ++i) outs.push_back(mxGetCell(out[0], (mwIndex)(i + j * nmat)));
@@ -112,8 +124,43 @@ static int file_mode(const char* in_path, const char* out_path) {
   return 0;
 }
 
+#if defined(GATE_BATCHED)
+// `gate_batched gpus`: the trailing gpus argument of the batched gateway is validated before any device is touched;
+// without a GPU a well-formed multi-GPU list reaches aps_group_create and fails with apsmatch:nogpu.
+static int gpus_argument_checks() {
+  int bad = 0;
+  mxArray* cells = mxCreateCellMatrix(1, 2);
+  mxArray* a = mxCreateNumericMatrix(6, 8, mxSINGLE_CLASS, mxREAL);
+  mxSetCell(cells, 0, a);
+  mxSetCell(cells, 1, mxCreateNumericMatrix(6, 8, mxSINGLE_CLASS, mxREAL));
+  mxArray *n2 = mxCreateDoubleScalar(2), *k = mxCreateDoubleScalar(4), *r = mxCreateDoubleScalar(0.6);
+  mxArray* opt = mxCreateDoubleScalar(1);  // useBF / method
+  auto vec = [](std::vector<double> v) {
+    mxArray* g = mxCreateDoubleMatrix(1, (mwSize)v.size(), mxREAL);
+    for (size_t i = 0; i < v.size(); ++i) mxGetPr(g)[i] = v[i];
+    return g;
+  };
+  mxArray* bad_lists[] = {vec({0}), vec({1, 1.5}), vec({2, 2}), vec({-1, 2}), vec({1, NAN}), mxCreateString("1:2"),
+                          mxCreateNumericMatrix(1, 2, mxSINGLE_CLASS, mxREAL), mxCreateDoubleMatrix(2, 2, mxREAL)};
+  for (const char* mode : {"global", "pairwise"}) {
+    mxArray* m = mxCreateString(mode);
+    for (mxArray* g : bad_lists) {
+      const mxArray* in[] = {m, cells, n2, k, r, opt, g};
+      bad += expect_error("apsmatch:args", 1, 7, in);
+    }
+    const mxArray* in[] = {m, cells, n2, k, r, opt, vec({1, 2})};
+    bad += expect_error("apsmatch:nogpu", 1, 7, in);  // no CPU fallback for a device group either
+  }
+  std::printf(bad ? "FAILED (%d)\n" : "OK\n", bad);
+  return bad ? 1 : 0;
+}
+#endif
+
 int main(int argc, char** argv) {
   if (argc > 3 && !std::strcmp(argv[1], "file")) return file_mode(argv[2], argv[3]);
+#if defined(GATE_BATCHED)
+  if (argc > 1 && !std::strcmp(argv[1], "gpus")) return gpus_argument_checks();
+#endif
   const bool gpu = argc > 1 && !std::strcmp(argv[1], "gpu");
   int bad = 0;
 #if defined(GATE_FLANN)
