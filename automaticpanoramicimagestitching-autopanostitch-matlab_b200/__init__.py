@@ -16,6 +16,7 @@ from .host import (  # noqa: F401
     binaryFeatures,
     featureMatchingGlobal,
     featureMatchingGlobalDevice,
+    featureMatchingGlobalSets,
     estimateTransformationRANSAC,
     featureMatchingPairwise,
     imageMatching,

@@ -131,6 +131,8 @@ def lib():
         "aps_gplan_compact": (i32, [vp]),
         "aps_gplan_filter_mutual": (i32, [vp]),
         "aps_feature_matching_global_dev": (i32, [vp, vp, C.POINTER(i64), i32, i32, i32, i32, dbl, i32, pp]),
+        "aps_feature_matching_global_sets": (i32, [vp, i32, C.POINTER(i32), pp, C.POINTER(i64), i32, i32, i32, i32, dbl,
+                                                   i32, i32, pp]),
         "aps_gplan_download_knn": (i32, [vp, i64, i64, vp, vp]),
         "aps_gplan_download": (i32, [vp, pp]),
         "aps_gplan_pair_counts_device": (i32, [vp, pp]),

@@ -140,10 +140,19 @@ int aps_k_tile_bounds(cudaStream_t s, const float* colscale, const float* colbia
 int aps_k_knn_exact(cudaStream_t s, const float* Q, const float* sqQ, const int32_t* rows, const int32_t* nrows_dev,
                     int64_t q0, int64_t nq, const float* T, const float* sqT, int64_t t0, int64_t t1, int D,
                     int k, int metric, int64_t out_row0, uint32_t* idx, float* dist);
+// set-restricted search of the pooled rows X [F x D] (metric 0): group table {row0, rows <= 8, t0, t1} per CTA task,
+// neighbour indices 1-based over all F rows; ngroups_dev (optional): device-side group count (<= ngroups)
+int aps_k_knn_exact_groups(cudaStream_t s, const float* X, const int4* d_groups, int64_t ngroups,
+                           const int32_t* ngroups_dev, int D, int k, uint32_t* idx, float* dist);
+constexpr int APS_EXACT_GROUP_ROWS = 8;
 
 // K4 aps_hamming.cu : exact Hamming kNN, thread per query, k <= APS_MAX_K.  idx relative to t0, 1-based.
 int aps_k_knn_hamming(cudaStream_t s, const uint8_t* Q, int64_t q0, int64_t nq, const uint8_t* T, int64_t t0,
                       int64_t t1, int nb, int k, int64_t out_row0, uint32_t* idx, float* dist);
+// set-restricted Hamming search: one CTA per group {row0, rows <= aps_k_knn_hamming_group_rows(), t0, t1}
+int aps_k_knn_hamming_groups(cudaStream_t s, const uint8_t* X, const int4* d_groups, int64_t ngroups, int nb16, int k,
+                             uint32_t* idx, float* dist);
+int aps_k_knn_hamming_group_rows();
 
 // K2 aps_knn_tc.cu : tcgen05 candidate search.  See the file header.
 struct aps_tc_unit {  // explicit work unit of the batched launch
@@ -288,6 +297,12 @@ int aps_k_global_compact(cudaStream_t s, const int2* records /* [F]: (target ima
                          const int32_t* img_of_row, const int64_t* img_off, int n, int64_t F, int64_t* dir_counts /*n*n*/,
                          int64_t* pair_counts /*n*n*/, int64_t* pair_ptr /*n*n+1*/, int64_t* rank /*F*/,
                          uint32_t* rows /*2F*/);
+// the same over independent image sets: set s owns the cells [cell_off[s], cell_off[s] + n_s^2) (its own n_s x n_s
+// block), so the tables hold sum(n_s^2) cells; one scan over all of them
+int aps_k_global_compact_sets(cudaStream_t s, const int2* records, const int32_t* img_of_row, const int64_t* img_off,
+                              int nimg, int64_t F, const int32_t* img_set, const int32_t* set_img0, const int32_t* set_n,
+                              const int64_t* cell_off, int nsets, int max_n, int64_t cells, int64_t* dir_counts,
+                              int64_t* pair_counts, int64_t* pair_ptr, int64_t* rank, uint32_t* rows);
 int aps_k_hamming2_finalize(cudaStream_t s, int64_t N1, int64_t N2, int nb, const uint32_t* idx_k2,
                             const float* dist_k2, uint32_t* idx2, float* d1, float* d2);
 int aps_k_split_k2(cudaStream_t s, int64_t N1, const uint32_t* idx_k2, const float* dist_k2, uint32_t* idx2,

@@ -264,6 +264,130 @@ int aps_k_global_compact(cudaStream_t s, const int2* records,
 }
 
 // ------------------------------------------------------------------------------------------------
+// K5b over many independent image sets (aps_feature_matching_global_sets): the same cell order, but the cells of set s
+// are its own n_s x n_s block at cell_off[s] -- sum(n_s^2) cells instead of (sum n_s)^2.  Records hold pooled image ids;
+// a set's images are consecutive from set_img0[s], so local ids are pooled ids - set_img0[s].
+struct SetTables {
+  const int32_t* img_set;   // [images]: set of a pooled image
+  const int32_t* set_img0;  // [sets]: first pooled image
+  const int32_t* set_n;     // [sets]: images
+  const int64_t* cell_off;  // [sets + 1]: first cell
+};
+
+__global__ void k_rank_per_image_sets(const int2* __restrict__ records, const int64_t* __restrict__ img_off,
+                                      SetTables st, int64_t* __restrict__ dir_counts, int64_t* __restrict__ rank) {
+  extern __shared__ int cnt[];  // [n of this image's set]
+  const int i = blockIdx.x, lane = threadIdx.x;
+  const int set = st.img_set[i], n = st.set_n[set], i0 = st.set_img0[set];
+  for (int t = lane; t < n; t += 32) cnt[t] = 0;
+  __syncwarp();
+  const int64_t b = img_off[i], e = img_off[i + 1];
+  for (int64_t base = b; base < e; base += 32) {
+    const int64_t q = base + lane;
+    const int t = (q < e) ? records[q].x : 0;
+    const bool active = t > 0;
+    const unsigned amask = __ballot_sync(0xffffffffu, active);
+    int myrank = 0, cbase = 0;
+    unsigned peers = 0;
+    if (active) {
+      peers = __match_any_sync(amask, t);
+      cbase = cnt[t - 1 - i0];
+      myrank = __popc(peers & ((1u << lane) - 1u));
+    }
+    __syncwarp();
+    if (active) {
+      rank[q] = (int64_t)cbase + myrank;
+      if (myrank == 0) cnt[t - 1 - i0] = cbase + __popc(peers);
+    }
+    __syncwarp();
+  }
+  int64_t* dc = dir_counts + st.cell_off[set] + (int64_t)(i - i0) * n;
+  for (int t = lane; t < n; t += 32) dc[t] = cnt[t];
+}
+
+// pair_counts of every set's block (column-major a + b*n inside it) and ONE exclusive scan over all cells; single block
+__global__ void k_pair_counts_scan_sets(const int64_t* __restrict__ dir_counts, SetTables st, int nsets, int64_t cells,
+                                        int64_t* __restrict__ pair_counts, int64_t* __restrict__ pair_ptr) {
+  __shared__ int64_t s_part[1024];
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const int64_t per = (cells + nt - 1) / nt;
+  const int64_t c0 = min(cells, tid * per), c1 = min(cells, c0 + per);
+  int lo = 0, hi = nsets;  // set holding cell c0: the last s with cell_off[s] <= c0
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) / 2;
+    if (st.cell_off[mid] <= c0) lo = mid;
+    else hi = mid;
+  }
+  int64_t sum = 0;
+  for (int64_t c = c0, set = lo; c < c1; ++c) {
+    while (c >= st.cell_off[set + 1]) ++set;
+    const int64_t n = st.set_n[set], cb = st.cell_off[set], l = c - cb;
+    const int64_t a = l % n, b = l / n;
+    const int64_t v = (a < b) ? dir_counts[cb + a * n + b] + dir_counts[cb + b * n + a] : 0;
+    pair_counts[c] = v;
+    sum += v;
+  }
+  s_part[tid] = sum;
+  __syncthreads();
+  if (tid == 0) {
+    int64_t run = 0;
+    for (int t = 0; t < nt; ++t) {
+      int64_t v = s_part[t];
+      s_part[t] = run;
+      run += v;
+    }
+    pair_ptr[cells] = run;
+  }
+  __syncthreads();
+  int64_t run = s_part[tid];
+  for (int64_t c = c0; c < c1; ++c) {
+    pair_ptr[c] = run;
+    run += pair_counts[c];
+  }
+}
+
+__global__ void k_scatter_rows_sets(const int2* __restrict__ records, const int32_t* __restrict__ img_of_row,
+                                    const int64_t* __restrict__ img_off, SetTables st, int64_t F,
+                                    const int64_t* __restrict__ dir_counts, const int64_t* __restrict__ pair_ptr,
+                                    const int64_t* __restrict__ rank, uint32_t* __restrict__ rows) {
+  int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= F) return;
+  const int2 rec = records[q];
+  if (rec.x <= 0) return;
+  const int i = img_of_row[q], t = rec.x - 1, set = st.img_set[i], i0 = st.set_img0[set];
+  const int64_t n = st.set_n[set], cb = st.cell_off[set];
+  const uint32_t li = (uint32_t)(q - img_off[i] + 1), lj = (uint32_t)rec.y;
+  const int64_t a = min(i, t) - i0, b = max(i, t) - i0;
+  int64_t pos = pair_ptr[cb + a + b * n] + rank[q];
+  if (i > t) pos += dir_counts[cb + a * n + b];  // the lower image's queries come first
+  rows[2 * pos] = (i < t) ? li : lj;             // featureMatchingGlobal.m:155-159
+  rows[2 * pos + 1] = (i < t) ? lj : li;
+}
+
+int aps_k_global_compact_sets(cudaStream_t s, const int2* records, const int32_t* img_of_row, const int64_t* img_off,
+                              int nimg, int64_t F, const int32_t* img_set, const int32_t* set_img0, const int32_t* set_n,
+                              const int64_t* cell_off, int nsets, int max_n, int64_t cells, int64_t* dir_counts,
+                              int64_t* pair_counts, int64_t* pair_ptr, int64_t* rank, uint32_t* rows) {
+  if (nsets == 0) return APS_OK;
+  const SetTables st{img_set, set_img0, set_n, cell_off};
+  const size_t smem = (size_t)max_n * sizeof(int);
+  if (smem > 48 * 1024)
+    APS_CUDA(cudaFuncSetAttribute(k_rank_per_image_sets, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (nimg > 0) {
+    k_rank_per_image_sets<<<nimg, 32, smem, s>>>(records, img_off, st, dir_counts, rank);
+    APS_LAUNCHED();
+  }
+  k_pair_counts_scan_sets<<<1, 1024, 0, s>>>(dir_counts, st, nsets, cells, pair_counts, pair_ptr);
+  APS_LAUNCHED();
+  if (F > 0) {
+    k_scatter_rows_sets<<<(unsigned)aps_ceil_div(F, 256), 256, 0, s>>>(records, img_of_row, img_off, st, F, dir_counts,
+                                                                       pair_ptr, rank, rows);
+    APS_LAUNCHED();
+  }
+  return APS_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // Hamming 2-NN edge rows of the MEX contract (nearest2HammingExhaustiveMEX.cpp:42-45, 71-74).
 __global__ void k_hamming2_finalize(int64_t N1, int64_t N2, int nb, const uint32_t* __restrict__ idx_k2,
                                     const float* __restrict__ dist_k2, uint32_t* __restrict__ idx2,

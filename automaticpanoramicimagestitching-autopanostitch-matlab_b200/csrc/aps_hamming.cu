@@ -22,15 +22,28 @@ namespace {
 constexpr int HQ = 256;  // queries per CTA
 constexpr int HT = 512;  // train rows per shared-memory tile
 
-template <int NW, int KT>
+// SETS: CTA b takes group groups[b] = rows [g.x, g.x + g.y) (g.y <= HQ) searched against train rows [g.z, g.w) only,
+// neighbour indices 1-based over the whole matrix (q0, nq, t0, t1 unused)
+template <int NW, int KT, bool SETS = false>
 __global__ void __launch_bounds__(HQ) k_knn_hamming(const uint4* __restrict__ Q, int64_t q0, int64_t nq,
                                                      const uint4* __restrict__ T, int64_t t0, int64_t t1, int k,
                                                      int64_t out_row0, uint32_t* __restrict__ idx,
-                                                     float* __restrict__ dist) {
+                                                     float* __restrict__ dist, const int4* __restrict__ groups) {
   __shared__ uint4 ts[HT * NW];
   const int tid = threadIdx.x;
-  const int64_t q = q0 + (int64_t)blockIdx.x * HQ + tid;
-  const bool qvalid = q < q0 + nq;
+  int64_t q, ibase = t0;  // neighbour index = train row - ibase + 1
+  bool qvalid;
+  if (SETS) {
+    const int4 g = groups[blockIdx.x];
+    q = (int64_t)g.x + tid;
+    qvalid = tid < g.y;
+    t0 = g.z;
+    t1 = g.w;
+    ibase = 0;
+  } else {
+    q = q0 + (int64_t)blockIdx.x * HQ + tid;
+    qvalid = q < q0 + nq;
+  }
   uint4 a[NW];
 #pragma unroll
   for (int w = 0; w < NW; ++w) a[w] = qvalid ? Q[q * NW + w] : make_uint4(0, 0, 0, 0);
@@ -51,7 +64,7 @@ __global__ void __launch_bounds__(HQ) k_knn_hamming(const uint4* __restrict__ Q,
       const int h = hamming_words<NW>(a, ts + j * NW);
       if (h < bd[KT - 1]) {
         bd[KT - 1] = h;
-        bi[KT - 1] = (uint32_t)(j0 + j - t0 + 1);
+        bi[KT - 1] = (uint32_t)(j0 + j - ibase + 1);
 #pragma unroll
         for (int p = KT - 1; p > 0; --p) {
           if (bd[p] < bd[p - 1]) {
@@ -80,20 +93,56 @@ int launch_nw(cudaStream_t s, const uint8_t* Q, int64_t q0, int64_t nq, const ui
   const uint4* q4 = (const uint4*)Q;
   const uint4* t4 = (const uint4*)T;
   if (k <= 2)
-    k_knn_hamming<NW, 2><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist);
+    k_knn_hamming<NW, 2><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist, nullptr);
   else if (k <= 4)
-    k_knn_hamming<NW, 4><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist);
+    k_knn_hamming<NW, 4><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist, nullptr);
   else if (k <= 8)
-    k_knn_hamming<NW, 8><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist);
+    k_knn_hamming<NW, 8><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist, nullptr);
   else if (k <= 16)
-    k_knn_hamming<NW, 16><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist);
+    k_knn_hamming<NW, 16><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist, nullptr);
   else
-    k_knn_hamming<NW, 32><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist);
+    k_knn_hamming<NW, 32><<<grid, HQ, 0, s>>>(q4, q0, nq, t4, t0, t1, k, out_row0, idx, dist, nullptr);
+  APS_LAUNCHED();
+  return APS_OK;
+}
+
+template <int NW, int KT>
+void launch_groups(cudaStream_t s, const uint8_t* X, const int4* groups, int64_t ngroups, int k, uint32_t* idx,
+                   float* dist) {
+  const uint4* x4 = (const uint4*)X;
+  k_knn_hamming<NW, KT, true><<<(unsigned)ngroups, HQ, 0, s>>>(x4, 0, 0, x4, 0, 0, k, 0, idx, dist, groups);
+}
+
+template <int NW>
+int launch_groups_nw(cudaStream_t s, const uint8_t* X, const int4* groups, int64_t ngroups, int k, uint32_t* idx,
+                     float* dist) {
+  if (k <= 2) launch_groups<NW, 2>(s, X, groups, ngroups, k, idx, dist);
+  else if (k <= 4) launch_groups<NW, 4>(s, X, groups, ngroups, k, idx, dist);
+  else if (k <= 8) launch_groups<NW, 8>(s, X, groups, ngroups, k, idx, dist);
+  else if (k <= 16) launch_groups<NW, 16>(s, X, groups, ngroups, k, idx, dist);
+  else launch_groups<NW, 32>(s, X, groups, ngroups, k, idx, dist);
   APS_LAUNCHED();
   return APS_OK;
 }
 
 }  // namespace
+
+// Set-restricted search of the pooled rows X (padded to nb16): one launch, one CTA per group of up to 256 rows of one
+// set, each against its own set's rows (aps_k_knn_exact_groups' table with HQ-row groups).
+int aps_k_knn_hamming_groups(cudaStream_t s, const uint8_t* X, const int4* d_groups, int64_t ngroups, int nb16, int k,
+                             uint32_t* idx, float* dist) {
+  if (ngroups == 0) return APS_OK;
+  switch (nb16 / 16) {
+    case 1: return launch_groups_nw<1>(s, X, d_groups, ngroups, k, idx, dist);
+    case 2: return launch_groups_nw<2>(s, X, d_groups, ngroups, k, idx, dist);
+    case 3: return launch_groups_nw<3>(s, X, d_groups, ngroups, k, idx, dist);
+    case 4: return launch_groups_nw<4>(s, X, d_groups, ngroups, k, idx, dist);
+    default:
+      aps_set_error(APS_ERR_DIM, "hamm2nn:cols", "binary descriptors wider than 64 bytes are not supported (%d)", nb16);
+      return APS_ERR_DIM;
+  }
+}
+int aps_k_knn_hamming_group_rows() { return HQ; }
 
 // Q, T: rows padded to nb16 = multiple of 16 bytes (zero padded: pads XOR to zero), 16-byte aligned.
 int aps_k_knn_hamming(cudaStream_t s, const uint8_t* Q, int64_t q0, int64_t nq, const uint8_t* T, int64_t t0,

@@ -24,7 +24,10 @@ constexpr int TJ = 256;   // train rows per tile == threads per CTA
 constexpr int DC = 32;    // dimensions per staged chunk
 constexpr int TLD = DC + 4;
 
-template <int METRIC>
+// SETS: a group table drives the CTAs instead of (q0, nq, t0, t1): group g = rows [g.x, g.x + g.y) (g.y <= RQ) searched
+// against train rows [g.z, g.w) only, neighbour indices 1-based over the whole matrix (number of groups: *nrows_dev when
+// given -- a table built on the device -- else nq)
+template <int METRIC, bool SETS = false>
 __global__ void __launch_bounds__(TJ) k_knn_exact(const float* __restrict__ Q, const float* __restrict__ sqQ,
                                                    const int32_t* __restrict__ rows,
                                                    const int32_t* __restrict__ nrows_dev, int64_t q0, int64_t nq,
@@ -32,7 +35,7 @@ __global__ void __launch_bounds__(TJ) k_knn_exact(const float* __restrict__ Q, c
                                                    int64_t t0, int64_t t1, int D, int k, int64_t out_row0,
                                                    uint32_t* __restrict__ idx, float* __restrict__ dist,
                                                    int nsplit, int64_t split_cap, uint32_t* __restrict__ pidx,
-                                                   float* __restrict__ pdist) {
+                                                   float* __restrict__ pdist, const int4* __restrict__ groups) {
   extern __shared__ __align__(16) float smem[];
   const int Dpad = (D + DC - 1) / DC * DC;
   float* qs = smem;                       // [RQ][Dpad]
@@ -44,21 +47,29 @@ __global__ void __launch_bounds__(TJ) k_knn_exact(const float* __restrict__ Q, c
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int64_t total = rows ? (int64_t)(*nrows_dev) : nq;
-  const int64_t ngroups = (total + RQ - 1) / RQ;
+  const int64_t ngroups = SETS ? total : (total + RQ - 1) / RQ;
   const int nfull = D / 4;  // full groups of four (FLANN functor), then a scalar tail
   // few rows (the fallback list): split the train range over `ns` CTAs per row group, merge afterwards
-  const int ns = (nsplit > 1 && total <= split_cap) ? nsplit : 1;
+  const int ns = (!SETS && nsplit > 1 && total <= split_cap) ? nsplit : 1;
   const int64_t tiles_all = (t1 - t0 + TJ - 1) / TJ, tiles_per = (tiles_all + ns - 1) / ns;
 
   for (int64_t work = blockIdx.x; work < ngroups * ns; work += gridDim.x) {
     const int64_t grp = work / ns;
     const int sp = (int)(work - grp * ns);
+    int4 g = make_int4(0, 0, 0, 0);
+    if (SETS) {
+      g = groups[grp];
+      t0 = g.z;
+      t1 = g.w;
+    }
     const int64_t ts0 = t0 + (int64_t)sp * tiles_per * TJ;
-    const int64_t ts1 = min(t1, ts0 + tiles_per * TJ);
+    const int64_t ts1 = SETS ? t1 : min(t1, ts0 + tiles_per * TJ);
+    const int64_t ibase = SETS ? 0 : t0;  // neighbour index = train row - ibase + 1
     __syncthreads();
     if (tid < RQ) {
       int64_t i = grp * RQ + tid;
-      s_row[tid] = (i < total) ? (rows ? (int64_t)rows[i] : q0 + i) : -1;
+      if (SETS) s_row[tid] = tid < g.y ? (int64_t)g.x + tid : -1;
+      else s_row[tid] = (i < total) ? (rows ? (int64_t)rows[i] : q0 + i) : -1;
     }
     if (tid < RQ * APS_MAX_K) {
       topd[tid] = CUDART_INF_F;
@@ -168,7 +179,7 @@ __global__ void __launch_bounds__(TJ) k_knn_exact(const float* __restrict__ Q, c
                 --p;
               }
               topd[r * APS_MAX_K + p] = vl;
-              topi[r * APS_MAX_K + p] = (uint32_t)(j0 + 32 * i + l - t0 + 1);
+              topi[r * APS_MAX_K + p] = (uint32_t)(j0 + 32 * i + l - ibase + 1);
             }
             __syncwarp();
             worst = topd[r * APS_MAX_K + k - 1];
@@ -285,11 +296,11 @@ int aps_k_knn_exact(cudaStream_t s, const float* Q, const float* sqQ, const int3
   if (metric == 0) {
     APS_CUDA(cudaFuncSetAttribute(k_knn_exact<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_knn_exact<0><<<grid, TJ, smem, s>>>(Q, sqQ, rows, nrows_dev, q0, nq, T, sqT, t0, t1, D, k, out_row0, idx, dist,
-                                          nsplit, split_cap, pidx.p, pdist.p);
+                                          nsplit, split_cap, pidx.p, pdist.p, nullptr);
   } else {
     APS_CUDA(cudaFuncSetAttribute(k_knn_exact<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_knn_exact<1><<<grid, TJ, smem, s>>>(Q, sqQ, rows, nrows_dev, q0, nq, T, sqT, t0, t1, D, k, out_row0, idx, dist,
-                                          nsplit, split_cap, pidx.p, pdist.p);
+                                          nsplit, split_cap, pidx.p, pdist.p, nullptr);
   }
   APS_LAUNCHED();
   if (nsplit > 1) {
@@ -297,5 +308,27 @@ int aps_k_knn_exact(cudaStream_t s, const float* Q, const float* sqQ, const int3
         rows, nrows_dev, q0, nq, k, nsplit, split_cap, pidx.p, pdist.p, out_row0, idx, dist);
     APS_LAUNCHED();
   }
+  return APS_OK;
+}
+
+// Set-restricted search (global path, metric 0): every group of the table holds up to 8 query rows of ONE set and the
+// train range of that set, so rows never see another set's rows.  One launch for all sets; the neighbour indices are
+// 1-based rows of the whole matrix.  ngroups_dev != nullptr: the table holds *ngroups_dev groups (at most ngroups),
+// written on the device (e.g. the rows a re-rank could not prove).  Per row the result equals a search of the set alone:
+// the candidates are merged in ascending train order with ties to the lower index, whatever the tiling.
+int aps_k_knn_exact_groups(cudaStream_t s, const float* X, const int4* d_groups, int64_t ngroups,
+                           const int32_t* ngroups_dev, int D, int k, uint32_t* idx, float* dist) {
+  if (ngroups == 0) return APS_OK;
+  const int Dpad = (D + DC - 1) / DC * DC;
+  size_t smem = (size_t)(RQ * Dpad + TJ * TLD + RQ * TJ + 2 * RQ * APS_MAX_K) * sizeof(float);
+  if (smem > 200 * 1024) {
+    aps_set_error(APS_ERR_DIM, "", "descriptor dimension %d too large for the exact kernel", D);
+    return APS_ERR_DIM;
+  }
+  const unsigned grid = (unsigned)(ngroups < 148 * 4 ? ngroups : 148 * 4);
+  APS_CUDA(cudaFuncSetAttribute(k_knn_exact<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_knn_exact<0, true><<<grid, TJ, smem, s>>>(X, nullptr, ngroups_dev, ngroups_dev, 0, ngroups, X, nullptr, 0, 0, D, k,
+                                              0, idx, dist, 1, 0, nullptr, nullptr, d_groups);
+  APS_LAUNCHED();
   return APS_OK;
 }

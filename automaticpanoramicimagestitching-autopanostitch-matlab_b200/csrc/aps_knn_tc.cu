@@ -1137,8 +1137,9 @@ int aps_k_gather_rows(cudaStream_t s, const __nv_bfloat16* src, int Dp, const in
   return APS_OK;
 }
 
-// Batched (pairwise) launch: explicit work units, e.g. one per (256-row block of image i, image j).
-// One candidate list of 8 per row at candidate-buffer row (unit.out_row + row offset).
+// Batched launch: explicit work units, e.g. one per (256-row block of image i, image j) (pairwise) or per 256-row block
+// of one image set against that set's rows (aps_feature_matching_global_sets).  One candidate list of kcand per row at
+// candidate-buffer row (unit.out_row + row offset).
 int aps_k_knn_tc_units(cudaStream_t s, int sm_count, const aps_tc_problem& p, const aps_tc_unit* d_units,
                        int64_t n_units) {
   if (!aps_k_knn_tc_supported(p.Dp)) {
@@ -1166,7 +1167,7 @@ int aps_k_knn_tc_units(cudaStream_t s, int sm_count, const aps_tc_problem& p, co
   P.n_table_units = n_units;
   P.cand_stride = p.kcand;
   const int cs_groups = p.kcand == 3 ? 2 : CSPLIT;  // epilogue groups per row block of the variant launched below
-  const size_t smem = smem_bytes(p.Dp, cs_groups, KC);
+  const size_t smem = smem_bytes(p.Dp, cs_groups, p.kcand == KC_LARGE ? KC_LARGE : KC);
   const unsigned grid = (unsigned)(n_units < sm_count ? n_units : sm_count);
   const int threads = threads_for(cs_groups);
   auto launch = [&](auto kern) -> int {
@@ -1181,8 +1182,10 @@ int aps_k_knn_tc_units(cudaStream_t s, int sm_count, const aps_tc_problem& p, co
     APS_TRY(p.bias ? launch(k_knn_tc<true, false, false, 4>) : launch(k_knn_tc<false, false, false, 4>));
   else if (p.kcand == KC)
     APS_TRY(p.bias ? launch(k_knn_tc<true, false, false, KC>) : launch(k_knn_tc<false, false, false, KC>));
+  else if (p.kcand == KC_LARGE)  // the K' = 16 lists of 6 <= k <= 12 (batched global sets)
+    APS_TRY(p.bias ? launch(k_knn_tc<true, false, false, KC_LARGE>) : launch(k_knn_tc<false, false, false, KC_LARGE>));
   else {
-    aps_set_error(APS_ERR_ARGS, "", "kcand must be 3, 4 or %d", KC);
+    aps_set_error(APS_ERR_ARGS, "", "kcand must be 3, 4, %d or %d", KC, KC_LARGE);
     return APS_ERR_ARGS;
   }
   APS_LAUNCHED();

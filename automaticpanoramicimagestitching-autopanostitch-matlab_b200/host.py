@@ -209,6 +209,61 @@ def featureMatchingGlobal(input, allDescriptors, numImg, ctx=None):
     return matches
 
 
+def featureMatchingGlobalSets(input, allDescriptorsSets, numImgs, ctx=None):
+    """matchesSets = featureMatchingGlobalSets(input, allDescriptorsSets, numImgs)
+
+    featureMatchingGlobal over B independent image sets in one call (aps_feature_matching_global_sets): set b is
+    allDescriptorsSets[b] with numImgs[b] images.  Returns a list of B nested lists, element b exactly what
+    featureMatchingGlobal(input, allDescriptorsSets[b], numImgs[b]) returns (with input.apsMutual too).  All sets share
+    one descriptor kind (float or binaryFeatures) and width.  Device groups (input.apsGPUs) are not supported here."""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by featureMatchingGlobalSets; match the sets on one GPU")
+    sets = list(allDescriptorsSets) if allDescriptorsSets is not None else []
+    nums = list(np.atleast_1d(np.asarray(numImgs, dtype=np.float64)).ravel()) if np.size(numImgs) else []
+    if len(nums) != len(sets):
+        raise ValueError("numImgs must give one image count per descriptor set")
+    for v in nums:
+        if not (np.isfinite(v) and v > 0 and v == np.round(v)):
+            raise ValueError("every numImgs entry must be a positive integer")  # featureMatchingGlobal.m:35-39
+    k = int(_field(input, "k", required=True))
+    ratio = float(_field(input, "Ratiothreshold", required=True))
+    use_bf = bool(_field(input, "BFMatch", 0))
+    mutual = bool(int(_field(input, "apsMutual", 0)))
+    ns, all_mats, all_counts = [], [], []
+    kind = D = None
+    for cells, num in zip(sets, nums):
+        n, first, mats, counts, Db, is_binary = _describe(cells, num)
+        if first is None:
+            mats, counts = [None] * n, [0] * n
+        else:
+            if kind is not None and is_binary != kind:
+                raise ApsError(2, "flann_knn:type", "all descriptor sets must have the same class")
+            if D is not None and Db != D:
+                raise ApsError(4, "flann_knn:dim", "all descriptor sets must have the same number of columns")
+            kind, D = is_binary, Db
+        ns.append(n)
+        all_mats += mats
+        all_counts += counts
+    B = len(ns)
+    if kind is None:  # every set empty: cell(numImg) each, no device touched (featureMatchingGlobal.m:49-52)
+        return [[[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)] for n in ns]
+    ptrs, cnt, layout, keep = _desc_args(all_mats, all_counts)
+    simg = (C.c_int * max(B, 1))(*ns)
+    outs = (C.c_void_p * max(B, 1))()
+    ctx = ctx or default_context()
+    check(lib().aps_feature_matching_global_sets(ctx.handle, B, simg, ptrs, cnt, int(D),
+                                                 APS_U8 if kind else APS_F32, layout, k, ratio, int(use_bf),
+                                                 int(mutual), outs))
+    result = []
+    try:
+        for b in range(B):
+            result.append(_cells_from_matchlist(outs[b], ns[b])[0])
+    finally:
+        for b in range(B):
+            lib().aps_matchlist_free(outs[b])
+    return result
+
+
 class ApsSemanticsWarning(UserWarning):
     """The call was served with semantics that differ from what the reference's defaults select."""
 

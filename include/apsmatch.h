@@ -161,6 +161,21 @@ int aps_feature_matching_global(aps_ctx* ctx, const void* const* desc, const int
 int aps_feature_matching_global_dev(aps_ctx* ctx, const void* d_pooled, const int64_t* counts, int n, int D, int dtype,
                                     int k, double ratio, int mutual, aps_matchlist** out);
 
+/* featureMatchingGlobal over nsets independent image sets in one call.  Set b has set_images[b] images; desc / counts
+ * list the images of all sets one after another (set 0's images first).  Every set's match list is BIT-IDENTICAL to
+ * aps_feature_matching_global (mutual = 0) or to the staged plan with aps_gplan_filter_mutual (mutual != 0) on that set
+ * alone: rows of one set never see rows of another.  out[b] receives set b's list (n = set_images[b]); free each with
+ * aps_matchlist_free.  All sets share one D and dtype.  Argument errors carry the ids of aps_feature_matching_global
+ * (flann_knn:k, flann_knn:type, flann_knn:dim); nsets < 0, a negative count or a NULL out is APS_ERR_ARGS.
+ * All sets share ONE pass, whatever nsets: one normalisation, one tcgen05 unit-table search over the float sets the
+ * single-set call would search on the tensor path (each 256-row block against its own set's rows) with one re-rank and
+ * one set-restricted exact fallback, one set-restricted exact (float) or Hamming (binary) search over the other sets,
+ * one filter, one per-set compaction (sum of n_b^2 cells) and one download -- its launches and synchronisations do not
+ * depend on nsets.  nsets == 1 is exactly the single-set call. */
+int aps_feature_matching_global_sets(aps_ctx* ctx, int nsets, const int* set_images, const void* const* desc,
+                                     const int64_t* counts, int D, int dtype, int layout, int k, double ratio,
+                                     int use_bf, int mutual, aps_matchlist** out);
+
 /* ---- matches = featureMatchingPairwise(input, allDescriptors, numImg) ------------------------
  * PP/featureMatching/featureMatchingPairwise.m:1-63 with getMatches :103-120 on the
  * matchFeaturesScratch 'Exhaustive' branch (input.useMATLABFeatureMatch = 0), Unique = true. */
