@@ -17,6 +17,7 @@ from .host import (  # noqa: F401
     featureMatchingGlobal,
     featureMatchingGlobalDevice,
     featureMatchingGlobalSets,
+    featureMatchingPairwiseSets,
     estimateTransformationRANSAC,
     featureMatchingPairwise,
     imageMatching,

@@ -106,6 +106,8 @@ def lib():
         "aps_feature_matching_global": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, i32, dbl, i32, pp]),
         "aps_feature_matching_pairwise": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, dbl, dbl, pp]),
         "aps_feature_matching_pairwise_shard": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, dbl, dbl, i32, i32, pp]),
+        "aps_feature_matching_pairwise_sets": (i32, [vp, i32, C.POINTER(i32), pp, C.POINTER(i64), i32, i32, i32, dbl, dbl,
+                                                     i32, i64, C.c_uint64, pp]),
         "aps_matchlist_n": (i32, [vp]),
         "aps_matchlist_total": (i64, [vp]),
         "aps_matchlist_pair_ptr": (C.POINTER(i64), [vp]),

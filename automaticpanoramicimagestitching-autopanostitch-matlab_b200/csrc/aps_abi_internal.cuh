@@ -1,7 +1,9 @@
 // aps_abi_internal.cuh -- what the translation units behind include/apsmatch.h share (aps_abi.cu: context, kNN entries,
-// staged global pipeline; aps_abi_pairwise.cu: matchFeaturesScratch / featureMatchingPairwise, staged pairwise pipeline).
+// staged global pipeline; aps_abi_pairwise.cu: matchFeaturesScratch / featureMatchingPairwise, staged pairwise pipeline,
+// pairwise matching of many image sets; aps_abi_sets.cu: global matching of many image sets).
 #pragma once
 #include <string>
+#include <vector>
 
 #include "aps_common.cuh"
 
@@ -94,6 +96,14 @@ int feature_matching_global_impl(aps_ctx* c, const void* const* desc, const int6
 int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
                                    int layout, double match_threshold, double max_ratio, int method, int64_t subset,
                                    uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out);
+
+// ---- pooled upload of many images (aps_abi_sets.cu; the sets entries) ---------------------------------------------
+// img[r] = image of pooled row r (d_off: [nimg + 1] row offsets on the device)
+int sets_img_of_row(cudaStream_t s, const int64_t* d_off, int nimg, int64_t F, int32_t* img);
+// H2D of image i (host ptrs[i], off[i + 1] - off[i] rows) to rows [off[i], off[i + 1]) of the pooled row-major matrix
+// `raw`: one copy per image; column-major input is staged and transposed in ONE launch (needs img_of_row)
+int sets_upload(aps_ctx* c, const void* const* ptrs, const std::vector<int64_t>& off, const int64_t* d_off,
+                const int32_t* img_of_row, int D, int esz, int layout, void* raw);
 
 // ---- match lists: the n x n cell in CSR form -----------------------------------------------------------------------
 struct aps_matchlist {

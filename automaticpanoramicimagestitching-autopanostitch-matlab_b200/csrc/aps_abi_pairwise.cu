@@ -1,7 +1,10 @@
 // aps_abi_pairwise.cu -- the pairwise half of the extern "C" surface (include/apsmatch.h): matchFeaturesScratch for one
-// pair, featureMatchingPairwise in one call, and the staged pairwise pipeline aps_pplan_* (screen stage, exact stage,
-// subset views of 'subsetpdist2', PCA views of 'pca2nn').  No CPU compute path: without a CUDA device every entry fails.
+// pair, featureMatchingPairwise in one call, the staged pairwise pipeline aps_pplan_* (screen stage, exact stage,
+// subset views of 'subsetpdist2', PCA views of 'pca2nn') and featureMatchingPairwise over many image sets in one call.
+// No CPU compute path: without a CUDA device every entry fails.
+#include <algorithm>
 #include <chrono>
+#include <climits>
 #include <cstdlib>
 #include <cmath>
 #include <limits>
@@ -13,9 +16,18 @@
 // matchFeaturesScratch / featureMatchingPairwise
 // One image pair of a pairwise pass; results are appended to the host vectors in the order of the pair list.
 struct PairRef {
-  int i, j;
-  size_t ordinal;      // position in the full pair list (cell order)
+  int i, j;            // pooled image indices
+  size_t ordinal;      // position in the pass's pair list
   int64_t qbase = -1;  // 'pca2nn': first row of the pair's projected query rows in the batch buffers (else: the image's rows)
+  bool tensor = false; // the tensor engine (screen + tcgen05 candidates + exact re-rank) instead of the exact engine
+};
+// match lists of a pass, pair by pair: pair `ordinal` has cnt[ordinal] rows from row at[ordinal] of rows / metric (rows
+// in batch order; one append per batch, no allocation per pair)
+struct PairResults {
+  std::vector<int32_t> cnt;
+  std::vector<int64_t> at;
+  std::vector<uint32_t> rows;   // (col1, col2) per match
+  std::vector<double> metric;
 };
 // 'pca2nn': the rows one pass of the pairwise pipeline reads when they are NOT the set's own -- the query rows of a batch
 // projected with the train images' bases, and the projected train set
@@ -199,8 +211,9 @@ static int pairwise_finish(aps_ctx* c, PairwiseSets& ps, const int64_t* counts, 
 // Train view of the staged plan (after pairwise_finish): per-image norm bounds of the screen, and -- for 'subsetpdist2'
 // with images above `subset` rows -- the virtual subset images (matchFeaturesScratch.m:388-393: candB = randperm(N2,
 // subset), B2 = B(candB,:); here ONE subset per train image, drawn by a keyed bijection, instead of one per call).
+// key[j] (nullptr: j) keys image j's subset: its index in its own set.
 static int pairwise_build_train_view(aps_ctx* c, PairwiseSets& ps, const int64_t* counts, int n, int D, bool tensor,
-                                     int64_t subset, uint64_t seed) {
+                                     int64_t subset, uint64_t seed, const int32_t* key = nullptr) {
   cudaStream_t s = c->stream;
   const int64_t F = ps.off[n];
   ps.Freal = F;
@@ -219,12 +232,14 @@ static int pairwise_build_train_view(aps_ctx* c, PairwiseSets& ps, const int64_t
     ps.voff.assign(n, -1);
     ps.vcnt = subset;
     for (int b = 0; b < nbig; ++b) ps.voff[big[b]] = F + (int64_t)b * subset;
-    APS_TRY(ps.d_big.alloc((size_t)nbig, s));
+    for (int b = 0; b < nbig; ++b) big.push_back(key ? key[big[b]] : big[b]);   // [nbig, 2 nbig): key indices
+    APS_TRY(ps.d_big.alloc((size_t)nbig * 2, s));
     APS_TRY(ps.vsrc.alloc((size_t)V, s));
     APS_TRY(ps.vmap.alloc((size_t)V, s));
-    APS_CUDA(cudaMemcpyAsync(ps.d_big.p, big.data(), (size_t)nbig * 4, cudaMemcpyHostToDevice, s));
+    APS_CUDA(cudaMemcpyAsync(ps.d_big.p, big.data(), (size_t)nbig * 8, cudaMemcpyHostToDevice, s));
     APS_CUDA(cudaStreamSynchronize(s));   // `big` is pageable host memory
-    APS_TRY(aps_k_subset_rows(s, ps.d_img_off.p, ps.d_big.p, nbig, subset, seed, ps.vsrc.p, ps.vmap.p));
+    APS_TRY(aps_k_subset_rows(s, ps.d_img_off.p, ps.d_big.p, ps.d_big.p + nbig, nbig, subset, seed, ps.vsrc.p,
+                              ps.vmap.p));
     APS_TRY(ps.tv_ones.alloc((size_t)(F + V) + 256, s));
     APS_TRY(aps_k_fill_f32(s, ps.tv_ones.p, F + V + 256, 1.0f));
     for (int w = 0; w < 2; ++w) {
@@ -336,12 +351,9 @@ static int pairwise_screen_stage(aps_ctx* c, PairwiseSets& ps, std::vector<PairR
                                  bool norm, double match_threshold, double max_ratio, const PcaViews* pv = nullptr);
 static int pairwise_batch(aps_ctx* c, PairwiseSets& ps, const std::vector<PairRef>& pairs, const int64_t* counts, int D,
                           int dtype, bool norm, bool tensor, int dist_metric, double match_threshold, double max_ratio,
-                          std::vector<int32_t>& out_count, std::vector<std::vector<uint32_t>>& out_rows,
-                          std::vector<std::vector<double>>& out_metric, const PcaViews* pv = nullptr);
+                          PairResults& res, const PcaViews* pv = nullptr);
 static int pairwise_pca_batch(aps_ctx* c, PairwiseSets& ps, std::vector<PairRef> batch, const int64_t* counts, int D,
-                              bool norm, bool tensor, double match_threshold, double max_ratio,
-                              std::vector<int32_t>& cnt, std::vector<std::vector<uint32_t>>& prow,
-                              std::vector<std::vector<double>>& pmet) {
+                              bool norm, bool tensor, double match_threshold, double max_ratio, PairResults& res) {
   cudaStream_t s = c->stream;
   const int w = norm ? 1 : 0, P = ps.pcaP;
   const FloatSet& S = norm ? ps.normset : ps.rawset;
@@ -371,8 +383,7 @@ static int pairwise_pca_batch(aps_ctx* c, PairwiseSets& ps, std::vector<PairRef>
     pv.q_xh = qxh.p;
     if (c->pairwise_screen) APS_TRY(pairwise_screen_stage(c, ps, batch, counts, D, norm, match_threshold, max_ratio, &pv));
   }
-  return pairwise_batch(c, ps, batch, counts, D, APS_F32, norm, tensor, /*metric*/ 3, match_threshold, max_ratio, cnt, prow,
-                        pmet, &pv);
+  return pairwise_batch(c, ps, batch, counts, D, APS_F32, norm, tensor, /*metric*/ 3, match_threshold, max_ratio, res, &pv);
 }
 
 static int pairwise_prepare(aps_ctx* c, PairwiseSets& ps, const void* const* desc, const int64_t* counts, int n,
@@ -531,13 +542,11 @@ __global__ void k_gather_pairs(const uint32_t* __restrict__ src_m, const double*
   }
 }
 
-// One batch of pairs (all using the same descriptor view) through the batched pipeline; results are
-// appended to the host vectors in the order of `pairs`.
-
+// One batch of pairs (all using the same descriptor view and engine) through the batched pipeline; results are
+// appended to `res`.
 static int pairwise_batch(aps_ctx* c, PairwiseSets& ps, const std::vector<PairRef>& pairs, const int64_t* counts, int D,
                           int dtype, bool norm, bool tensor, int dist_metric, double match_threshold, double max_ratio,
-                          std::vector<int32_t>& out_count, std::vector<std::vector<uint32_t>>& out_rows,
-                          std::vector<std::vector<double>>& out_metric, const PcaViews* pv) {
+                          PairResults& res, const PcaViews* pv) {
   const int np = (int)pairs.size();
   if (np == 0) return APS_OK;
   cudaStream_t s = c->stream;
@@ -608,7 +617,7 @@ static int pairwise_batch(aps_ctx* c, PairwiseSets& ps, const std::vector<PairRe
     }
     c->stats[0] += E;
     if (tensor) {
-      c->stats[2] = 2;
+      c->stats[2] = 2;   // the tensor engine ran for some pair of the call
       std::vector<aps_tc_unit> units;
       for (int p = 0; p < np; ++p) {
         const int64_t nq = eoff[p + 1] - eoff[p];
@@ -679,7 +688,7 @@ static int pairwise_batch(aps_ctx* c, PairwiseSets& ps, const std::vector<PairRe
       APS_TRY(aps_k_pair_exact2(s, side.xn, side.sq, tv.xn, tv.sq, D, dist_metric, pt, fb.p, fb.p + E, E, i2.p, dd.p));
       APS_CUDA(cudaMemcpyAsync(c->h_flags + 33, fb.p + E, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     } else {
-      c->stats[2] = 1;
+      if (c->stats[2] == 0) c->stats[2] = 1;
       APS_CUDA(cudaStreamSynchronize(s));
       APS_TRY(aps_k_pair_exact2(s, side.xn, side.sq, tv.xn, tv.sq, D, dist_metric, pt, nullptr, nullptr, E, i2.p, dd.p));
     }
@@ -718,12 +727,13 @@ static int pairwise_batch(aps_ctx* c, PairwiseSets& ps, const std::vector<PairRe
     APS_CUDA(cudaMemcpyAsync(stage + (size_t)M * 8, met.p, (size_t)M * 8, cudaMemcpyDeviceToHost, s));
     APS_CUDA(cudaStreamSynchronize(s));
   }
+  const int64_t base = (int64_t)res.metric.size();
+  res.rows.insert(res.rows.end(), hrows, hrows + 2 * M);
+  res.metric.insert(res.metric.end(), hmet, hmet + M);
   for (int p = 0; p < np; ++p) {
     const size_t o = pairs[p].ordinal;
-    out_count[o] = hc[p];
-    if (hc[p] == 0) continue;
-    out_rows[o].assign(hrows + 2 * outoff[p], hrows + 2 * outoff[p + 1]);
-    out_metric[o].assign(hmet + outoff[p], hmet + outoff[p + 1]);
+    res.cnt[o] = hc[p];
+    res.at[o] = base + outoff[p];
   }
   return APS_OK;
 }
@@ -902,20 +912,86 @@ extern "C" int aps_pplan_set_method(aps_pplan* p, int method, int64_t subset, ui
   return APS_OK;
 }
 
+// One pass of the pairwise pipeline over an explicit pair list: pairs[o] (ordinal o, pooled image indices, engine) has
+// its list written to cell cell[o] of `m` (m->pair_ptr: ncells + 1 entries; cells no pair names stay empty).  Pairs
+// with an empty side are skipped (matchFeaturesScratch.m:84-88).  The pairs are grouped by view (raw / normalised,
+// :105-110 is a per-pair decision) and engine; tensor groups are screened first, then every group runs in batches of at
+// most ENTRY_BUDGET query rows.  Host work is O(pairs + match rows + ncells).
+static int pairwise_match_pairs(aps_ctx* c, PairwiseSets& ps, const int64_t* counts, int D, int dtype, int method,
+                                double match_threshold, double max_ratio, const std::vector<PairRef>& pairs,
+                                const std::vector<int64_t>& cell, int64_t ncells, aps_matchlist* m) {
+  // float descriptors: 1 = (a2 + b2) - 2 G of nearest2SSDExhaustive; 2 = Euclidean search squared afterwards ('kdtree'
+  // = exact KD-tree search, :142-148; 'subsetpdist2', :149-155, whose candidate subset is ALL of B while N2 <= subset)
+  const bool pca = dtype == APS_F32 && method == APS_METHOD_APPROX_PCA2NN;
+  const int metric = (dtype == APS_F32 && method != APS_METHOD_EXHAUSTIVE) ? 2 : 1;
+  const size_t NP = pairs.size();
+  // groups: [view * 2 + engine], raw before normalised, exact before tensor
+  std::vector<PairRef> grp[4];
+  for (const PairRef& pr : pairs) {
+    if (counts[pr.i] == 0 || counts[pr.j] == 0) continue;  // matchFeaturesScratch.m:84-88
+    const bool norm = dtype == APS_F32 && (ps.big[pr.i] || ps.big[pr.j]);  // :105-110 is a per-pair decision
+    grp[(norm ? 2 : 0) + (pr.tensor ? 1 : 0)].push_back(pr);
+  }
+  c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
+  int rc = APS_OK;
+  const bool dbg_t = getenv("APS_TIMING") != nullptr;
+  auto dbg_now = [&]() { cudaStreamSynchronize(c->stream); return std::chrono::steady_clock::now(); };
+  auto dbg_t0 = dbg_t ? dbg_now() : std::chrono::steady_clock::time_point();
+  if (c->pairwise_screen && !pca)
+    for (int g = 1; g < 4 && rc == APS_OK; g += 2)
+      rc = pairwise_screen_stage(c, ps, grp[g], counts, D, g >= 2, match_threshold, max_ratio);
+  auto dbg_t1 = dbg_t ? dbg_now() : dbg_t0;
+  PairResults res;
+  res.cnt.assign(NP, 0);
+  res.at.assign(NP, 0);
+  const int64_t ENTRY_BUDGET = (int64_t)1 << 25;  // entries per batch: bounds the candidate buffers to ~2 GB
+  for (int g = 0; g < 4 && rc == APS_OK; ++g) {
+    const std::vector<PairRef>& gp = grp[g];
+    const bool norm = g >= 2, tensor = (g & 1) != 0;
+    size_t a = 0;
+    while (a < gp.size() && rc == APS_OK) {
+      size_t b = a;
+      int64_t e = 0;
+      while (b < gp.size() && (b == a || e + counts[gp[b].i] <= ENTRY_BUDGET)) e += counts[gp[b++].i];
+      std::vector<PairRef> batch(gp.begin() + a, gp.begin() + b);
+      if (pca)   // projection with the train image's basis is a per-PAIR operation: screen and match batch by batch
+        rc = pairwise_pca_batch(c, ps, batch, counts, D, norm, tensor, match_threshold, max_ratio, res);
+      else
+        rc = pairwise_batch(c, ps, batch, counts, D, dtype, norm, tensor, metric, match_threshold, max_ratio, res);
+      a = b;
+    }
+  }
+  auto dbg_t2 = dbg_t ? dbg_now() : dbg_t0;
+  if (rc != APS_OK) return rc;
+  m->pair_ptr.assign((size_t)ncells + 1, 0);
+  for (size_t o = 0; o < NP; ++o) m->pair_ptr[(size_t)cell[o] + 1] = res.cnt[o];
+  for (int64_t q = 0; q < ncells; ++q) m->pair_ptr[(size_t)q + 1] += m->pair_ptr[(size_t)q];
+  m->total = m->pair_ptr[(size_t)ncells];
+  m->rows.resize((size_t)m->total * 2);
+  m->metric.resize((size_t)m->total);
+  for (size_t o = 0; o < NP; ++o) {
+    if (res.cnt[o] == 0) continue;
+    const int64_t dst = m->pair_ptr[(size_t)cell[o]], src = res.at[o];
+    std::copy(res.rows.begin() + 2 * src, res.rows.begin() + 2 * (src + res.cnt[o]), m->rows.begin() + 2 * dst);
+    std::copy(res.metric.begin() + src, res.metric.begin() + src + res.cnt[o], m->metric.begin() + dst);
+  }
+  if (dbg_t) {
+    auto dbg_t3 = dbg_now();
+    auto ms = [](auto a, auto b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
+    fprintf(stderr, "aps_pplan_match: screen %.2f ms, batches %.2f ms, assemble %.2f ms\n", ms(dbg_t0, dbg_t1), ms(dbg_t1, dbg_t2),
+            ms(dbg_t2, dbg_t3));
+  }
+  return APS_OK;
+}
+
 extern "C" int aps_pplan_match(aps_pplan* p, double match_threshold, double max_ratio, int pair_first, int pair_stride,
                                aps_matchlist** out) {
   if (!p || !out) APS_FAIL(APS_ERR_ARGS, "", "bad arguments");
   aps_ctx* c = p->c;
   APS_CTX(c);
   *out = nullptr;
-  // float descriptors: 1 = (a2 + b2) - 2 G of nearest2SSDExhaustive; 2 = Euclidean search squared afterwards ('kdtree'
-  // = exact KD-tree search, :142-148; 'subsetpdist2', :149-155, whose candidate subset is ALL of B while N2 <= subset)
-  const bool pca = p->dtype == APS_F32 && p->method == APS_METHOD_APPROX_PCA2NN;
-  const int metric = (p->dtype == APS_F32 && p->method != APS_METHOD_EXHAUSTIVE) ? 2 : 1;
-
   if (pair_stride < 1 || pair_first < 0 || pair_first >= pair_stride) APS_FAIL(APS_ERR_ARGS, "", "bad pair share");
-  const int n = p->n, D = p->D, dtype = p->dtype;
-  const int64_t* counts = p->counts.data();
+  const int n = p->n;
   c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
   aps_matchlist* m = new (std::nothrow) aps_matchlist();
   if (!m) APS_FAIL(APS_ERR_ALLOC, "", "out of host memory");
@@ -931,78 +1007,21 @@ extern "C" int aps_pplan_match(aps_pplan* p, double match_threshold, double max_
     delete m;
     APS_FAIL(APS_ERR_ARGS, "", "aps_pplan_prepare() has not run since the last upload");
   }
-  int rc = APS_OK;
-  {
-    const bool tensor = p->tensor;
-    PairwiseSets& ps = p->ps;
-    // pair list in column-major cell order (featureMatchingPairwise.m:48): j outer, i < j inner; this rank's
-    // share = every pair_stride-th pair (the reference's parfor distributes the same list over workers)
-    std::vector<PairRef> all, mine_raw, mine_norm;
-    for (int j = 0; j < n; ++j)
-      for (int i = 0; i < j; ++i) all.push_back(PairRef{i, j, all.size()});
-    const size_t NP = all.size();
-    for (size_t o = 0; o < NP; ++o) {
+  // pair list in column-major cell order (featureMatchingPairwise.m:48): j outer, i < j inner; this rank's
+  // share = every pair_stride-th pair (the reference's parfor distributes the same list over workers)
+  std::vector<PairRef> pairs;
+  std::vector<int64_t> cell;
+  size_t o = 0;
+  for (int j = 0; j < n; ++j)
+    for (int i = 0; i < j; ++i, ++o) {
       if ((int)(o % (size_t)pair_stride) != pair_first) continue;
-      const PairRef& pr = all[o];
-      if (counts[pr.i] == 0 || counts[pr.j] == 0) continue;  // matchFeaturesScratch.m:84-88
-      const bool norm = dtype == APS_F32 && (ps.big[pr.i] || ps.big[pr.j]);  // :105-110 is a per-pair decision
-      (norm ? mine_norm : mine_raw).push_back(pr);
+      PairRef pr{i, j, pairs.size()};
+      pr.tensor = p->tensor;
+      pairs.push_back(pr);
+      cell.push_back((int64_t)i + (int64_t)j * n);
     }
-    c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
-    const bool dbg_t = getenv("APS_TIMING") != nullptr;
-    auto dbg_now = [&]() { cudaStreamSynchronize(c->stream); return std::chrono::steady_clock::now(); };
-    auto dbg_t0 = dbg_t ? dbg_now() : std::chrono::steady_clock::time_point();
-    if (tensor && c->pairwise_screen && !pca) {
-      rc = pairwise_screen_stage(c, ps, mine_raw, counts, D, false, match_threshold, max_ratio);
-      if (rc == APS_OK) rc = pairwise_screen_stage(c, ps, mine_norm, counts, D, true, match_threshold, max_ratio);
-    }
-    auto dbg_t1 = dbg_t ? dbg_now() : dbg_t0;
-    std::vector<int32_t> cnt(NP, 0);
-    std::vector<std::vector<uint32_t>> prow(NP);
-    std::vector<std::vector<double>> pmet(NP);
-    const int64_t ENTRY_BUDGET = (int64_t)1 << 25;  // entries per batch: bounds the candidate buffers to ~2 GB
-    for (int g = 0; g < 2 && rc == APS_OK; ++g) {
-      const std::vector<PairRef>& grp = g ? mine_norm : mine_raw;
-      size_t a = 0;
-      while (a < grp.size() && rc == APS_OK) {
-        size_t b = a;
-        int64_t e = 0;
-        while (b < grp.size() && (b == a || e + counts[grp[b].i] <= ENTRY_BUDGET)) e += counts[grp[b++].i];
-        std::vector<PairRef> batch(grp.begin() + a, grp.begin() + b);
-        if (pca)   // projection with the train image's basis is a per-PAIR operation: screen and match batch by batch
-          rc = pairwise_pca_batch(c, ps, batch, counts, D, g == 1, tensor, match_threshold, max_ratio, cnt, prow, pmet);
-        else
-          rc = pairwise_batch(c, ps, batch, counts, D, dtype, g == 1, tensor, metric, match_threshold, max_ratio, cnt, prow,
-                              pmet);
-        a = b;
-      }
-    }
-    auto dbg_t2 = dbg_t ? dbg_now() : dbg_t0;
-    if (rc == APS_OK) {
-      size_t o = 0;
-      for (int j = 0; j < n; ++j)
-        for (int i = 0; i < n; ++i) {
-          const size_t cell = (size_t)i + (size_t)j * n;
-          int64_t add = 0;
-          if (i < j) add = cnt[o++];
-          m->pair_ptr[cell + 1] = m->pair_ptr[cell] + add;
-        }
-      m->total = m->pair_ptr[cells];
-      m->rows.reserve((size_t)m->total * 2);
-      m->metric.reserve((size_t)m->total);
-      for (size_t q = 0; q < NP; ++q) {
-        if (prow[q].empty()) continue;
-        m->rows.insert(m->rows.end(), prow[q].begin(), prow[q].end());
-        m->metric.insert(m->metric.end(), pmet[q].begin(), pmet[q].end());
-      }
-    }
-    if (dbg_t) {
-      auto dbg_t3 = dbg_now();
-      auto ms = [](auto a, auto b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
-      fprintf(stderr, "aps_pplan_match: screen %.2f ms, batches %.2f ms, assemble %.2f ms\n", ms(dbg_t0, dbg_t1), ms(dbg_t1, dbg_t2),
-              ms(dbg_t2, dbg_t3));
-    }
-  }
+  const int rc = pairwise_match_pairs(c, p->ps, p->counts.data(), p->D, p->dtype, p->method, match_threshold, max_ratio,
+                                      pairs, cell, (int64_t)cells, m);
   if (rc != APS_OK) {
     delete m;
     return rc;
@@ -1046,3 +1065,129 @@ extern "C" int aps_feature_matching_pairwise_shard(aps_ctx* c, const void* const
                                         APS_METHOD_EXHAUSTIVE, 12000, 0, pair_first, pair_stride, out);
 }
 
+// ------------------------------------------------------------------------------------------------
+// featureMatchingPairwise over many independent image sets in one call.  The reference runs the pairwise stage once per
+// dataset folder and once more per connected component; here all sets share ONE pooled plan (one upload, one K1, one
+// train view), one pair list that never crosses a set, and one pass of pairwise_match_pairs -- no host loop over sets
+// issues device work, so launches and synchronisations do not depend on nsets.
+static int pairwise_sets_pass(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
+                              const int64_t* counts, int nimg, int D, int dtype, int layout, double match_threshold,
+                              double max_ratio, int method, int64_t subset, uint64_t seed, aps_matchlist** out) {
+  // per image: its index in its own set (the key of its 'subsetpdist2' subset); per set: its first cell.  Set b's
+  // pairs: its own column-major strict-upper-triangle list, on the engine its single-set call chooses (aps_pplan_create)
+  std::vector<int32_t> local((size_t)nimg);
+  std::vector<int64_t> cell_off((size_t)nsets + 1, 0);
+  std::vector<PairRef> pairs;
+  std::vector<int64_t> cell;
+  bool any_tensor = false;
+  for (int b = 0, i0 = 0; b < nsets; i0 += set_images[b++]) {
+    const int n = set_images[b];
+    int64_t maxc = 0;
+    for (int i = 0; i < n; ++i) {
+      local[(size_t)i0 + i] = i;
+      maxc = counts[i0 + i] > maxc ? counts[i0 + i] : maxc;
+    }
+    const bool tensor = dtype == APS_F32 && tc_wanted(c, D, maxc, maxc * (int64_t)n, 2);
+    for (int j = 0; j < n; ++j)
+      for (int i = 0; i < j; ++i) {
+        if (counts[i0 + i] == 0 || counts[i0 + j] == 0) continue;  // matchFeaturesScratch.m:84-88
+        PairRef pr{i0 + i, i0 + j, pairs.size()};
+        pr.tensor = tensor;
+        any_tensor |= tensor;
+        pairs.push_back(pr);
+        cell.push_back(cell_off[b] + i + (int64_t)j * n);
+      }
+    cell_off[(size_t)b + 1] = cell_off[b] + (int64_t)n * n;
+  }
+  aps_matchlist pooled;
+  pooled.pair_ptr.assign((size_t)cell_off[nsets] + 1, 0);
+  if (!pairs.empty()) {
+    for (int i = 0; i < nimg; ++i)
+      if (counts[i] > 0 && (!desc || !desc[i])) APS_FAIL(APS_ERR_ARGS, "", "descriptor pointer %d is NULL", i);
+    PairwiseSets ps;
+    APS_TRY(pairwise_alloc(c, ps, counts, nimg, D, dtype));
+    const int64_t F = ps.off[nimg];
+    DevBuf<int64_t> d_off;
+    DevBuf<int32_t> img_of_row;
+    if (layout != APS_ROW_MAJOR) {   // the transpose needs each row's image
+      APS_TRY(d_off.alloc((size_t)nimg + 1, c->stream));
+      APS_TRY(img_of_row.alloc((size_t)F, c->stream));
+      APS_CUDA(cudaMemcpyAsync(d_off.p, ps.off.data(), ps.off.size() * 8, cudaMemcpyHostToDevice, c->stream));
+      APS_TRY(sets_img_of_row(c->stream, d_off.p, nimg, F, img_of_row.p));
+    }
+    APS_TRY(sets_upload(c, desc, ps.off, d_off.p, img_of_row.p, D, dtype == APS_F32 ? 4 : 1, layout,
+                        dtype == APS_F32 ? (void*)ps.rawset.raw.p : (void*)ps.u8raw.p));
+    APS_TRY(pairwise_finish(c, ps, counts, nimg, D, dtype, any_tensor));
+    if (dtype == APS_F32)
+      APS_TRY(pairwise_build_train_view(c, ps, counts, nimg, D, any_tensor,
+                                        method == APS_METHOD_APPROX_SUBSETPDIST2 ? subset : 0, seed, local.data()));
+    if (dtype == APS_F32 && method == APS_METHOD_APPROX_PCA2NN) APS_TRY(pairwise_build_pca(c, ps, counts, nimg, D));
+    APS_TRY(pairwise_match_pairs(c, ps, counts, D, dtype, method, match_threshold, max_ratio, pairs, cell,
+                                 cell_off[nsets], &pooled));
+  }
+  // split into one list per set: cells [cell_off[b], cell_off[b + 1]], rows from pair_ptr[cell_off[b]]
+  const std::vector<int64_t>& pp = pooled.pair_ptr;
+  for (int b = 0; b < nsets; ++b) {
+    aps_matchlist* m = new (std::nothrow) aps_matchlist();
+    if (!m) APS_FAIL(APS_ERR_ALLOC, "", "out of host memory");
+    out[b] = m;
+    m->n = set_images[b];
+    m->has_metric = true;
+    const int64_t c0 = cell_off[b], c1 = cell_off[(size_t)b + 1], r0 = pp[c0];
+    m->pair_ptr.resize((size_t)(c1 - c0) + 1);
+    for (int64_t q = c0; q <= c1; ++q) m->pair_ptr[(size_t)(q - c0)] = pp[q] - r0;
+    m->total = pp[c1] - r0;
+    m->rows.assign(pooled.rows.begin() + 2 * r0, pooled.rows.begin() + 2 * pp[c1]);
+    m->metric.assign(pooled.metric.begin() + r0, pooled.metric.begin() + pp[c1]);
+  }
+  return APS_OK;
+}
+
+extern "C" int aps_feature_matching_pairwise_sets(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
+                                                  const int64_t* counts, int D, int dtype, int layout,
+                                                  double match_threshold, double max_ratio, int method, int64_t subset,
+                                                  uint64_t seed, aps_matchlist** out) {
+  // arguments first (the statuses of the single-set call), then the device
+  if (nsets < 0) APS_FAIL(APS_ERR_ARGS, "", "nsets must be >= 0 (got %d)", nsets);
+  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
+  if (nsets > 0 && !set_images) APS_FAIL(APS_ERR_ARGS, "", "set_images is NULL");
+  for (int b = 0; b < nsets; ++b) out[b] = nullptr;
+  int64_t nimg = 0;
+  for (int b = 0; b < nsets; ++b) {
+    if (set_images[b] < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d has a negative image count", b);
+    nimg += set_images[b];
+  }
+  if (nimg > INT_MAX) APS_FAIL(APS_ERR_ARGS, "", "too many images");
+  if (nimg > 0 && !counts) APS_FAIL(APS_ERR_ARGS, "", "counts is NULL");
+  if (dtype != APS_F32 && dtype != APS_U8) APS_FAIL(APS_ERR_TYPE, "", "descriptors must be single or uint8");
+  if (method < APS_METHOD_EXHAUSTIVE || method > APS_METHOD_APPROX_PCA2NN)
+    APS_FAIL(APS_ERR_METHOD, "", "Select a approximate method");   // matchFeaturesScratch.m:156-157
+  if (subset < 1) APS_FAIL(APS_ERR_ARGS, "", "subset must be positive");
+  // pooled rows, the subset views included: one plan's limit
+  int64_t rows = 0;
+  for (int64_t i = 0; i < nimg; ++i) {
+    if (counts[i] < 0) APS_FAIL(APS_ERR_ARGS, "", "negative feature count");
+    rows += counts[i];
+    if (dtype == APS_F32 && method == APS_METHOD_APPROX_SUBSETPDIST2 && counts[i] > subset) rows += subset;
+  }
+  if (rows > 0 && D <= 0) APS_FAIL(APS_ERR_DIM, "", "descriptor dimension must be positive");
+  if (rows >= ((int64_t)1 << 31) - 512)
+    APS_FAIL(APS_ERR_ARGS, "", "%lld pooled descriptor rows (subset views included) exceed the limit of 2^31 - 512",
+             (long long)rows);
+  APS_CTX(c);
+  if (nsets == 0) return APS_OK;
+  if (nsets == 1)  // one set: the single-set call itself
+    return feature_matching_pairwise_impl(c, desc, counts, set_images[0], D, dtype, layout, match_threshold, max_ratio,
+                                          method, subset, seed, 0, 1, out);
+  c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
+  c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
+  c->h_flags[32] = 0;   // fallback rows of the call's tensor batches (aps_ctx_last_stats)
+  const int rc = pairwise_sets_pass(c, nsets, set_images, desc, counts, (int)nimg, D, dtype, layout, match_threshold,
+                                    max_ratio, method, subset, seed, out);
+  if (rc != APS_OK)
+    for (int b = 0; b < nsets; ++b) {
+      aps_matchlist_free(out[b]);
+      out[b] = nullptr;
+    }
+  return rc;
+}

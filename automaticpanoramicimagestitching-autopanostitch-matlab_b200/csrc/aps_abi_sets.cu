@@ -51,6 +51,45 @@ __global__ void k_sets_transpose_in(const T* __restrict__ src, const int32_t* __
   dst[e] = src[b * D + (int64_t)c * n + (r - b)];
 }
 
+}  // namespace
+
+int sets_img_of_row(cudaStream_t s, const int64_t* d_off, int nimg, int64_t F, int32_t* img) {
+  if (F == 0) return APS_OK;
+  k_sets_img_of_row<<<(unsigned)aps_ceil_div(F, 256), 256, 0, s>>>(d_off, nimg, F, img);
+  APS_LAUNCHED();
+  return APS_OK;
+}
+
+int sets_upload(aps_ctx* c, const void* const* ptrs, const std::vector<int64_t>& off, const int64_t* d_off,
+                const int32_t* img_of_row, int D, int esz, int layout, void* raw) {
+  cudaStream_t s = c->stream;
+  const int nimg = (int)off.size() - 1;
+  const int64_t F = off.back();
+  if (F == 0) return APS_OK;
+  // row-major images land in place; column-major ones are staged and transposed in one launch
+  DevBuf<uint8_t> stage;
+  uint8_t* dst = (uint8_t*)raw;
+  if (layout != APS_ROW_MAJOR) {
+    APS_TRY(stage.alloc((size_t)F * D * esz, s));
+    dst = stage.p;
+  }
+  for (int i = 0; i < nimg; ++i)
+    if (off[i + 1] > off[i])
+      APS_CUDA(cudaMemcpyAsync(dst + (size_t)off[i] * D * esz, ptrs[i], (size_t)(off[i + 1] - off[i]) * D * esz,
+                               cudaMemcpyHostToDevice, s));
+  if (layout != APS_ROW_MAJOR) {
+    const unsigned grid = (unsigned)aps_ceil_div(F * D, 256);
+    if (esz == 4)
+      k_sets_transpose_in<float><<<grid, 256, 0, s>>>((const float*)stage.p, img_of_row, d_off, F, D, (float*)raw);
+    else
+      k_sets_transpose_in<uint8_t><<<grid, 256, 0, s>>>(stage.p, img_of_row, d_off, F, D, (uint8_t*)raw);
+    APS_LAUNCHED();   // `stage` is released in stream order
+  }
+  return APS_OK;
+}
+
+namespace {
+
 // rows the tensor pass could not prove -> one K2f group each, searched against its own set's rows (device-side list)
 __global__ void k_sets_fallback_groups(const int32_t* __restrict__ fb, const int32_t* __restrict__ nfb,
                                        const int32_t* __restrict__ img_of_row, const int64_t* __restrict__ img_off,
@@ -130,7 +169,7 @@ int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std
     DevBuf<int32_t> d_tabs, img_of_row, flags, fb;
     DevBuf<int4> d_groups, fb_groups;
     DevBuf<aps_tc_unit> d_units;
-    DevBuf<uint8_t> raw, stage, u8pad, keep;
+    DevBuf<uint8_t> raw, u8pad, keep;
     DevBuf<float> xn, sq, invn, knn_dist, colscale, colbias, cscore;
     DevBuf<__nv_bfloat16> xb;
     DevBuf<uint32_t> knn_idx, rows, cidx;
@@ -155,26 +194,8 @@ int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std
       APS_CUDA(cudaMemcpyAsync(d_groups.p, groups.data(), groups.size() * sizeof(int4), cudaMemcpyHostToDevice, s));
     if (!units.empty())
       APS_CUDA(cudaMemcpyAsync(d_units.p, units.data(), units.size() * sizeof(aps_tc_unit), cudaMemcpyHostToDevice, s));
-    k_sets_img_of_row<<<(unsigned)aps_ceil_div(F, 256), 256, 0, s>>>(d_off.p, nimg, F, img_of_row.p);
-    APS_LAUNCHED();
-    // upload: row-major images land in place; column-major ones are staged and transposed in one launch
-    uint8_t* dst = layout == APS_ROW_MAJOR ? raw.p : nullptr;
-    if (!dst) {
-      APS_TRY(stage.alloc((size_t)F * D * esz, s));
-      dst = stage.p;
-    }
-    for (int i = 0; i < nimg; ++i)
-      if (off[i + 1] > off[i])
-        APS_CUDA(cudaMemcpyAsync(dst + (size_t)off[i] * D * esz, ptrs[i], (size_t)(off[i + 1] - off[i]) * D * esz,
-                                 cudaMemcpyHostToDevice, s));
-    if (layout != APS_ROW_MAJOR) {
-      const unsigned grid = (unsigned)aps_ceil_div(F * D, 256);
-      if (esz == 4)
-        k_sets_transpose_in<float><<<grid, 256, 0, s>>>((const float*)stage.p, img_of_row.p, d_off.p, F, D, (float*)raw.p);
-      else
-        k_sets_transpose_in<uint8_t><<<grid, 256, 0, s>>>(stage.p, img_of_row.p, d_off.p, F, D, raw.p);
-      APS_LAUNCHED();
-    }
+    APS_TRY(sets_img_of_row(s, d_off.p, nimg, F, img_of_row.p));
+    APS_TRY(sets_upload(c, ptrs.data(), off, d_off.p, img_of_row.p, D, esz, layout, raw.p));
     APS_TRY(knn_idx.alloc((size_t)F * k, s));
     APS_TRY(knn_dist.alloc((size_t)F * k, s));
     if (dtype == APS_F32) {

@@ -254,9 +254,10 @@ int aps_k_image_sq_bounds(cudaStream_t s, const float* sq, const int64_t* d_star
 int aps_k_pair_screen(cudaStream_t s, int sm_count, const void* xh_q, int64_t Fq, const void* xh_t, int64_t Ft, int Dp,
                       const aps_pair_screen_tables& t, aps_tc_unit* d_units, int64_t n_units, uint32_t* out,
                       uint32_t* dump = nullptr, int dump_tiles = 0);
-// virtual (subset) images: vsrc[v] = global source row of virtual row v, chosen by a keyed bijection of [0, N_j)
-int aps_k_subset_rows(cudaStream_t s, const int64_t* d_img_off, const int32_t* d_big_img, int nbig, int64_t subset,
-                      uint64_t seed, int32_t* vsrc, int32_t* vmap);
+// virtual (subset) images: vsrc[v] = global source row of virtual row v, chosen by a keyed bijection of [0, N_j) whose
+// key is (seed, d_key_img[b]) for big image b = d_big_img[b]
+int aps_k_subset_rows(cudaStream_t s, const int64_t* d_img_off, const int32_t* d_big_img, const int32_t* d_key_img,
+                      int nbig, int64_t subset, uint64_t seed, int32_t* vsrc, int32_t* vmap);
 int aps_k_gather_f32_rows(cudaStream_t s, const float* src, const int32_t* rows, int64_t nrows, int D, float* dst);
 int aps_k_gather_u16_rows(cudaStream_t s, const uint16_t* src, const int32_t* rows, int64_t nrows, int Dp, uint16_t* dst);
 int aps_k_pair_screen_decide(cudaStream_t s, const uint32_t* scr, const float* sq, const aps_pair_screen_tables& t,

@@ -350,11 +350,14 @@ __device__ __forceinline__ uint32_t perm_in_range(uint32_t x, uint32_t N, uint64
   } while (x >= N);
   return x;
 }
-__global__ void k_subset_rows(const int64_t* __restrict__ img_off, const int32_t* __restrict__ big_img, int64_t subset,
-                              uint64_t seed, int32_t* __restrict__ vsrc, int32_t* __restrict__ vmap) {
+// key_img[b]: the index that keys big image b's bijection -- its image index in the set it belongs to, so that a set
+// matched inside a pooled call draws the subsets of its call alone
+__global__ void k_subset_rows(const int64_t* __restrict__ img_off, const int32_t* __restrict__ big_img,
+                              const int32_t* __restrict__ key_img, int64_t subset, uint64_t seed,
+                              int32_t* __restrict__ vsrc, int32_t* __restrict__ vmap) {
   const int b = blockIdx.y, j = big_img[b];
   const uint32_t N = (uint32_t)(img_off[j + 1] - img_off[j]);
-  const uint64_t key = seed * 0x9E3779B97F4A7C15ull + (uint64_t)(j + 1) * 0xD1B54A32D192ED03ull;
+  const uint64_t key = seed * 0x9E3779B97F4A7C15ull + (uint64_t)(key_img[b] + 1) * 0xD1B54A32D192ED03ull;
   for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < subset; r += (int64_t)gridDim.x * blockDim.x) {
     const uint32_t loc = perm_in_range((uint32_t)r, N, key);
     vmap[b * subset + r] = (int32_t)loc;
@@ -380,11 +383,11 @@ __global__ void k_gather_u16_rows(const uint4* __restrict__ src, const int32_t* 
 
 }  // namespace
 
-int aps_k_subset_rows(cudaStream_t s, const int64_t* d_img_off, const int32_t* d_big_img, int nbig, int64_t subset,
-                      uint64_t seed, int32_t* vsrc, int32_t* vmap) {
+int aps_k_subset_rows(cudaStream_t s, const int64_t* d_img_off, const int32_t* d_big_img, const int32_t* d_key_img,
+                      int nbig, int64_t subset, uint64_t seed, int32_t* vsrc, int32_t* vmap) {
   if (nbig == 0 || subset == 0) return APS_OK;
   dim3 grid((unsigned)aps_min64(aps_ceil_div(subset, 256), 64), (unsigned)nbig);
-  k_subset_rows<<<grid, 256, 0, s>>>(d_img_off, d_big_img, subset, seed, vsrc, vmap);
+  k_subset_rows<<<grid, 256, 0, s>>>(d_img_off, d_big_img, d_key_img, subset, seed, vsrc, vmap);
   APS_LAUNCHED();
   return APS_OK;
 }

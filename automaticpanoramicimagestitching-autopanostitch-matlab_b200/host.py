@@ -373,6 +373,76 @@ def featureMatchingPairwise(input, allDescriptors, numImg, ctx=None, return_metr
     return (matches, metrics) if return_metric else matches
 
 
+def featureMatchingPairwiseSets(input, allDescriptorsSets, numImgs, ctx=None, return_metric=False):
+    """matchesSets = featureMatchingPairwiseSets(input, allDescriptorsSets, numImgs)
+
+    featureMatchingPairwise over B independent image sets in one call (aps_feature_matching_pairwise_sets): set b is
+    allDescriptorsSets[b] with numImgs[b] images.  Returns a list of B elements, element b exactly what
+    featureMatchingPairwise(input, allDescriptorsSets[b], numImgs[b], return_metric=return_metric) returns.  Reads the
+    fields featureMatchingPairwise reads (Matchingmethod, ApproxFloatNNMethod, Matchingthreshold, Ratiothreshold,
+    apsSubset, apsSeed) and warns the same way for useMATLABFeatureMatch=1.  All sets share one descriptor kind (float
+    or binaryFeatures) and width.  Device groups (input.apsGPUs) are not supported here."""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by featureMatchingPairwiseSets; match the sets on one GPU")
+    sets = list(allDescriptorsSets) if allDescriptorsSets is not None else []
+    nums = list(np.atleast_1d(np.asarray(numImgs, dtype=np.float64)).ravel()) if np.size(numImgs) else []
+    if len(nums) != len(sets):
+        raise ValueError("numImgs must give one image count per descriptor set")
+    for v in nums:
+        if not (np.isfinite(v) and v > 0 and v == np.round(v)):
+            raise ValueError("every numImgs entry must be a positive integer")  # featureMatchingPairwise.m arguments
+    method = str(_field(input, "Matchingmethod", "Exhaustive")).lower()
+    if method not in ("exhaustive", "approximate"):
+        raise ValueError(f"Unknown Method: {method}")  # matchFeaturesScratch.m:164-165
+    aps_method = _resolve_method(input, method)
+    thr = float(_field(input, "Matchingthreshold", required=True))
+    ratio = float(_field(input, "Ratiothreshold", required=True))
+    ns, empty, all_mats, all_counts = [], [], [], []
+    kind = D = None
+    for cells, num in zip(sets, nums):
+        n, first, mats, counts, Db, is_binary = _describe(cells, num)
+        if first is None:
+            mats, counts = [None] * n, [0] * n
+        else:
+            if kind is not None and is_binary != kind:
+                raise ApsError(2, "flann_knn:type", "all descriptor sets must have the same class")
+            if D is not None and Db != D:
+                raise ApsError(4, "flann_knn:dim", "all descriptor sets must have the same number of columns")
+            kind, D = is_binary, Db
+        ns.append(n)
+        empty.append(first is None)
+        all_mats += mats
+        all_counts += counts
+
+    def empty_cells(n):   # featureMatchingPairwise on a set without descriptors: cell(numImg), no device touched
+        m = [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)]
+        return (m, [[None] * n for _ in range(n)]) if return_metric else m
+
+    B = len(ns)
+    if kind is None:
+        return [empty_cells(n) for n in ns]
+    ptrs, cnt, layout, keep = _desc_args(all_mats, all_counts)
+    simg = (C.c_int * max(B, 1))(*ns)
+    outs = (C.c_void_p * max(B, 1))()
+    ctx = ctx or default_context()
+    check(lib().aps_feature_matching_pairwise_sets(ctx.handle, B, simg, ptrs, cnt, int(D), APS_U8 if kind else APS_F32,
+                                                   layout, thr, ratio, aps_method, int(_field(input, "apsSubset", 12000)),
+                                                   int(_field(input, "apsSeed", 0)), outs))
+    result = []
+    try:
+        for b in range(B):
+            if empty[b]:
+                result.append(empty_cells(ns[b]))
+                continue
+            matches, metrics, _, _ = _cells_from_matchlist(outs[b], ns[b], want_metric=True)
+            _fill_upper_cells(matches, ns[b])
+            result.append((matches, metrics) if return_metric else matches)
+    finally:
+        for b in range(B):
+            lib().aps_matchlist_free(outs[b])
+    return result
+
+
 def _fill_upper_cells(matches, n):
     """featureMatchingPairwise fills EVERY upper-triangle cell (possibly 0 x 2), featureMatchingPairwise.m:62."""
     empty = np.zeros((0, 2))

@@ -190,6 +190,28 @@ int aps_feature_matching_pairwise_shard(aps_ctx* ctx, const void* const* desc, c
                                         int dtype, int layout, double match_threshold, double max_ratio,
                                         int pair_first, int pair_stride, aps_matchlist** out);
 
+/* featureMatchingPairwise over nsets independent image sets in one call.  Set b has set_images[b] images; desc / counts
+ * list the images of all sets one after another (set 0's images first).  out[b] receives set b's list (n =
+ * set_images[b], with metric); free each with aps_matchlist_free.  Every list is BIT-IDENTICAL in pair_ptr, rows and
+ * metric to set b matched alone with the same method, subset and seed -- aps_feature_matching_pairwise for
+ * APS_METHOD_EXHAUSTIVE, the staged plan with aps_pplan_set_method otherwise (aps_method; binary descriptors run the
+ * exhaustive Hamming search for every method): pairs never cross a set, and an image's 'subsetpdist2' subset is keyed
+ * by its index in its own set.  All sets share one D and dtype.  Argument errors carry the single-set call's statuses;
+ * nsets < 0, a negative count or a NULL out is APS_ERR_ARGS, and so is a call whose pooled rows, the subset views
+ * included, reach the one-plan limit of 2^31 - 512.  nsets == 0 succeeds and returns nothing; a set with fewer than two
+ * non-empty images gets an all-empty list; nsets == 1 is exactly the single-set call.
+ * All sets share ONE pass, whatever nsets: one upload (one transpose launch for column-major input), one K1, one train
+ * view, one pair list of every set's column-major strict upper triangle, each set's pairs on the engine its single-set
+ * call chooses (fp16 screen + tcgen05 + exact re-rank, or the exact engine), batches bounded by rows, not by sets, and
+ * one split into the nsets lists (sum of n_b^2 cells) -- its launches and synchronisations do not depend on nsets.
+ * The flag words of a view (exactness, max |x|^2, the screen's bound) are pooled over all sets: one set's values can
+ * let more pairs through another set's screen and send more of its rows to the exact fallback; the lists do not change.
+ * aps_ctx_last_stats and aps_ctx_pairwise_stats report sums over the call; last_stats[2] is 2 when any set ran on the
+ * tensor path. */
+int aps_feature_matching_pairwise_sets(aps_ctx* ctx, int nsets, const int* set_images, const void* const* desc,
+                                       const int64_t* counts, int D, int dtype, int layout, double match_threshold,
+                                       double max_ratio, int method, int64_t subset, uint64_t seed, aps_matchlist** out);
+
 /* ---- match list: the n x n cell in CSR form ---------------------------------------------------
  * cell (i,j) (0-based, i<j) is linear index c = i + j*n (MATLAB's column-major cell index);
  * its rows are rows[2*pair_ptr[c] .. 2*pair_ptr[c+1]) interleaved (col1,col2) = (index into image i,

@@ -2,74 +2,118 @@
 //   matches = aps_featureMatching_mex('global',   allDescriptors, numImg, k, ratioThr, useBF [, gpus])
 //   matchesSets = aps_featureMatching_mex('globalsets', {allDesc_1, ..., allDesc_B}, numImgs, k, ratioThr, useBF [, mutual])
 //   matches = aps_featureMatching_mex('pairwise', allDescriptors, numImg, matchThreshold, maxRatio [, method [, gpus]])
+//   matchesSets = aps_featureMatching_mex('pairwisesets', {allDesc_1, ..., allDesc_B}, numImgs, matchThreshold, maxRatio [, method])
 //   [cand, IuptriIdx] = aps_featureMatching_mex('partners', matchesAll | countMatrix, m)
 // Called by the drop-in matlab/featureMatchingGlobal.m / featureMatchingPairwise.m (same signatures as
 // PP/featureMatching/featureMatchingGlobal.m:1 and featureMatchingPairwise.m:1), matlab/featureMatchingGlobalSets.m
-// ('globalsets'), and by the two-line patch of
+// ('globalsets'), matlab/featureMatchingPairwiseSets.m ('pairwisesets'), and by the two-line patch of
 // PP/imageMatching/imageMatching.m:75-100 shown in INTEGRATION.md.
 // gpus: optional vector of 1-based GPU indices (gpuDevice numbering).  Absent, [] or 1 = the single default context
 // (device 1); any other list runs the call on a device group of those GPUs (aps_group_*, same lists).
 // 'globalsets': B independent image sets in one call (aps_feature_matching_global_sets); returns a 1 x B cell whose
-// element b is set b's numImgs(b) x numImgs(b) cell, exactly as 'global' returns it.  Every set uses one descriptor
-// class and width.
+// element b is set b's numImgs(b) x numImgs(b) cell, exactly as 'global' returns it.  'pairwisesets': the same for
+// 'pairwise' (aps_feature_matching_pairwise_sets, subset 12000, seed 0).  Every set uses one descriptor class and width.
 #include "aps_mex_common.h"
 
-static void global_sets(int nrhs, mxArray* plhs[], const mxArray* prhs[]) {
-  if (nrhs < 5) mexErrMsgIdAndTxt("apsmatch:args", "globalsets: need the sets, numImgs, k and ratio threshold");
+// The descriptor sets of 'globalsets' / 'pairwisesets' (prhs[1], counts prhs[2]), checked before any device is touched:
+// every image of every set one after another in ptrs / counts; dtype < 0 when every set is empty.  set_dtype[b] < 0
+// marks a set without descriptors.
+struct MexSets {
+  std::vector<int> set_images, set_dtype;
+  std::vector<const void*> ptrs;
+  std::vector<int64_t> counts;
+  std::vector<std::vector<std::vector<float>>> keep;  // converted matrices of every set stay alive
+  int dtype = -1, D = 0;
+};
+static void collect_sets(const char* verb, const char* scalars, int nrhs, const mxArray* prhs[], MexSets& S) {
+  if (nrhs < 5) mexErrMsgIdAndTxt("apsmatch:args", "%s: need the sets, numImgs, %s", verb, scalars);
   const mxArray* sets = prhs[1];
-  if (!mxIsCell(sets)) mexErrMsgIdAndTxt("apsmatch:args", "globalsets: the descriptor sets must be a cell array of cell arrays");
+  if (!mxIsCell(sets)) mexErrMsgIdAndTxt("apsmatch:args", "%s: the descriptor sets must be a cell array of cell arrays", verb);
   const int B = (int)mxGetNumberOfElements(sets);
   const mxArray* nimg = prhs[2];
   if (!mxIsDouble(nimg) || mxIsComplex(nimg) || (int)mxGetNumberOfElements(nimg) != B)
-    mexErrMsgIdAndTxt("apsmatch:args", "globalsets: numImgs must be a real double vector with one count per set");
-  std::vector<int> set_images((size_t)B);
-  std::vector<const void*> ptrs;
-  std::vector<int64_t> counts;
-  std::vector<std::vector<std::vector<float>>> keep((size_t)B);  // converted matrices of every set stay alive
-  int dtype = -1, D = 0;
+    mexErrMsgIdAndTxt("apsmatch:args", "%s: numImgs must be a real double vector with one count per set", verb);
+  S.set_images.assign((size_t)B, 0);
+  S.set_dtype.assign((size_t)B, -1);
+  S.keep.resize((size_t)B);
   for (int b = 0; b < B; ++b) {
     const double v = mxGetPr(nimg)[b];
     if (!(v >= 1.0 && v <= 2147483647.0) || v != (double)(int64_t)v)
-      mexErrMsgIdAndTxt("apsmatch:args", "globalsets: numImgs(%d) = %g is not a positive integer", b + 1, v);
+      mexErrMsgIdAndTxt("apsmatch:args", "%s: numImgs(%d) = %g is not a positive integer", verb, b + 1, v);
     const mxArray* cellb = mxGetCell(sets, (mwIndex)b);
-    if (!cellb || !mxIsCell(cellb)) mexErrMsgIdAndTxt("apsmatch:args", "globalsets: set %d is not a cell array", b + 1);
-    set_images[b] = (int)v;
+    if (!cellb || !mxIsCell(cellb)) mexErrMsgIdAndTxt("apsmatch:args", "%s: set %d is not a cell array", verb, b + 1);
+    S.set_images[b] = (int)v;
     std::vector<const void*> pb;
     std::vector<int64_t> cb;
     int dt, Db;
-    aps_mex_collect(cellb, set_images[b], pb, cb, dt, Db, keep[b]);
+    aps_mex_collect(cellb, S.set_images[b], pb, cb, dt, Db, S.keep[b]);
     if (dt >= 0) {  // one ABI call takes one class and one width
-      if (dtype >= 0 && dt != dtype) mexErrMsgIdAndTxt("apsmatch:args", "globalsets: set %d has another descriptor class", b + 1);
-      if (dtype >= 0 && Db != D) mexErrMsgIdAndTxt("apsmatch:args", "globalsets: set %d has another descriptor width", b + 1);
-      dtype = dt;
-      D = Db;
+      if (S.dtype >= 0 && dt != S.dtype) mexErrMsgIdAndTxt("apsmatch:args", "%s: set %d has another descriptor class", verb, b + 1);
+      if (S.dtype >= 0 && Db != S.D) mexErrMsgIdAndTxt("apsmatch:args", "%s: set %d has another descriptor width", verb, b + 1);
+      S.dtype = dt;
+      S.D = Db;
     }
-    ptrs.insert(ptrs.end(), pb.begin(), pb.end());
-    counts.insert(counts.end(), cb.begin(), cb.end());
+    S.set_dtype[b] = dt;
+    S.ptrs.insert(S.ptrs.end(), pb.begin(), pb.end());
+    S.counts.insert(S.counts.end(), cb.begin(), cb.end());
   }
-  const int mutual = nrhs > 6 ? (int)mxGetScalar(prhs[6]) : 0;
-  std::vector<aps_matchlist*> ml((size_t)B, nullptr);
-  if (dtype >= 0 && aps_feature_matching_global_sets(aps_mex_ctx(), B, set_images.data(), ptrs.data(), counts.data(), D,
-                                                     dtype, APS_COL_MAJOR, (int)mxGetScalar(prhs[3]),
-                                                     mxGetScalar(prhs[4]), nrhs > 5 ? (int)mxGetScalar(prhs[5]) : 0,
-                                                     mutual, ml.data()) != APS_OK)
-    aps_mex_fail("apsmatch:args");
+}
+
+// 1 x B cell of the sets' lists; a set without descriptors gets cell(numImgs(b)), as the single-set verbs return it
+static void sets_output(mxArray* plhs[], const MexSets& S, std::vector<aps_matchlist*>& ml, bool pairwise) {
+  const int B = (int)S.set_images.size();
   plhs[0] = mxCreateCellMatrix(1, (mwSize)B);
-  for (int b = 0; b < B; ++b) {  // every set empty: cell(numImg) each, no GPU touched (featureMatchingGlobal.m:49-52)
-    mxSetCell(plhs[0], (mwIndex)b, ml[b] ? aps_mex_cells(ml[b], set_images[b], false)
-                                         : mxCreateCellMatrix((mwSize)set_images[b], (mwSize)set_images[b]));
+  for (int b = 0; b < B; ++b) {
+    const int n = S.set_images[b];
+    const bool listed = ml[b] && (!pairwise || S.set_dtype[b] >= 0);
+    mxSetCell(plhs[0], (mwIndex)b, listed ? aps_mex_cells(ml[b], n, pairwise) : mxCreateCellMatrix((mwSize)n, (mwSize)n));
     aps_matchlist_free(ml[b]);
   }
 }
 
+static void global_sets(int nrhs, mxArray* plhs[], const mxArray* prhs[]) {
+  MexSets S;
+  collect_sets("globalsets", "k and ratio threshold", nrhs, prhs, S);
+  const int B = (int)S.set_images.size();
+  const int mutual = nrhs > 6 ? (int)mxGetScalar(prhs[6]) : 0;
+  std::vector<aps_matchlist*> ml((size_t)B, nullptr);
+  if (S.dtype >= 0 && aps_feature_matching_global_sets(aps_mex_ctx(), B, S.set_images.data(), S.ptrs.data(),
+                                                       S.counts.data(), S.D, S.dtype, APS_COL_MAJOR,
+                                                       (int)mxGetScalar(prhs[3]), mxGetScalar(prhs[4]),
+                                                       nrhs > 5 ? (int)mxGetScalar(prhs[5]) : 0, mutual,
+                                                       ml.data()) != APS_OK)
+    aps_mex_fail("apsmatch:args");
+  sets_output(plhs, S, ml, false);  // every set empty: cell(numImg) each, no GPU touched (featureMatchingGlobal.m:49-52)
+}
+
+// as 'pairwise' per set, with its subset (12000) and seed (0)
+static void pairwise_sets(int nrhs, mxArray* plhs[], const mxArray* prhs[]) {
+  MexSets S;
+  collect_sets("pairwisesets", "MatchThreshold and MaxRatio", nrhs, prhs, S);
+  const int B = (int)S.set_images.size();
+  const int method = nrhs > 5 ? (int)mxGetScalar(prhs[5]) : APS_METHOD_EXHAUSTIVE;   // aps_method
+  std::vector<aps_matchlist*> ml((size_t)B, nullptr);
+  if (S.dtype >= 0 && aps_feature_matching_pairwise_sets(aps_mex_ctx(), B, S.set_images.data(), S.ptrs.data(),
+                                                         S.counts.data(), S.D, S.dtype, APS_COL_MAJOR,
+                                                         mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), method, 12000, 0,
+                                                         ml.data()) != APS_OK)
+    aps_mex_fail("apsmatch:args");
+  sets_output(plhs, S, ml, true);
+}
+
 void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   if (nrhs < 3 || !mxIsChar(prhs[0]))
-    mexErrMsgIdAndTxt("apsmatch:args", "first argument must be 'global', 'globalsets', 'pairwise' or 'partners'");
+    mexErrMsgIdAndTxt("apsmatch:args",
+                      "first argument must be 'global', 'globalsets', 'pairwise', 'pairwisesets' or 'partners'");
   char* m = mxArrayToString(prhs[0]);
   const std::string mode = m ? m : "";
   if (m) mxFree(m);
   if (mode == "globalsets") {
     global_sets(nrhs, plhs, prhs);
+    return;
+  }
+  if (mode == "pairwisesets") {
+    pairwise_sets(nrhs, plhs, prhs);
     return;
   }
   if (mode == "partners") {

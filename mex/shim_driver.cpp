@@ -86,7 +86,9 @@ static int file_mode(const char* in_path, const char* out_path) {
     mexFunction(3, out, 2, in);
     outs = {out[0], out[1], out[2]};
 #elif defined(GATE_BATCHED)  // scalars: mode (0 global, 1 pairwise), then (k, ratio, useBF) or (MatchThreshold, MaxRatio)
-    if (sc[0] == 2.0) {  // 'globalsets': scalars 2, B, numImgs(1..B), k, ratio, useBF, mutual; matrices = all sets' images
+    // 'globalsets': scalars 2, B, numImgs(1..B), k, ratio, useBF, mutual; 'pairwisesets': scalars 3, B, numImgs(1..B),
+    // MatchThreshold, MaxRatio, method; matrices = all sets' images
+    if (sc[0] == 2.0 || sc[0] == 3.0) {
       const int B = (int)sc[1];
       mxArray* sets = mxCreateCellMatrix(1, (mwSize)B);
       mxArray* nimg = mxCreateDoubleMatrix(1, (mwSize)B, mxREAL);
@@ -98,7 +100,7 @@ static int file_mode(const char* in_path, const char* out_path) {
         m0 += n;
         mxSetCell(sets, (mwIndex)b, cb);
       }
-      std::vector<const mxArray*> in = {mxCreateString("globalsets"), sets, nimg};
+      std::vector<const mxArray*> in = {mxCreateString(sc[0] == 2.0 ? "globalsets" : "pairwisesets"), sets, nimg};
       for (size_t i = 2 + B; i < sc.size(); ++i) in.push_back(mxCreateDoubleScalar(sc[i]));
       mexFunction(1, out, (int)in.size(), in.data());
       for (int b = 0; b < B; ++b) {  // per set: upper-triangle cells in column-major order
@@ -178,57 +180,59 @@ static int gpus_argument_checks() {
   return bad ? 1 : 0;
 }
 
-// `gate_batched sets [nogpu]`: the 'globalsets' verb's argument checks, all made before any device is touched; with
-// `nogpu` a well-formed call must then fail with apsmatch:nogpu (no CPU fallback)
+// `gate_batched sets [nogpu]`: the argument checks of the 'globalsets' and 'pairwisesets' verbs, all made before any
+// device is touched; with `nogpu` a well-formed call must then fail with apsmatch:nogpu (no CPU fallback)
 static int sets_argument_checks(bool nogpu) {
   int bad = 0;
-  auto set_of = [](std::vector<mxArray*> m) {
-    mxArray* c = mxCreateCellMatrix(1, (mwSize)m.size());
-    for (size_t i = 0; i < m.size(); ++i) mxSetCell(c, (mwIndex)i, m[i]);
-    return c;
-  };
-  auto vec = [](std::vector<double> v) {
-    mxArray* g = mxCreateDoubleMatrix(1, (mwSize)v.size(), mxREAL);
-    for (size_t i = 0; i < v.size(); ++i) mxGetPr(g)[i] = v[i];
-    return g;
-  };
-  mxArray* f8 = mxCreateNumericMatrix(6, 8, mxSINGLE_CLASS, mxREAL);
-  mxArray* f16 = mxCreateNumericMatrix(6, 16, mxSINGLE_CLASS, mxREAL);
-  mxArray* orb = new mxArray();
-  orb->cls = mxUNKNOWN_CLASS;
-  orb->dims = {1, 1};
-  orb->class_name = "binaryFeatures";
-  orb->properties.push_back({"Features", mxCreateNumericMatrix(6, 32, mxUINT8_CLASS, mxREAL)});
-  mxArray *mode = mxCreateString("globalsets"), *k = mxCreateDoubleScalar(4), *r = mxCreateDoubleScalar(0.6);
-  mxArray* good = set_of({set_of({f8, f8}), set_of({f8})});
-  {  // too few arguments, sets not a cell of cells, numImgs of the wrong length / not positive integers
-    const mxArray* in[] = {mode, good, vec({2, 1}), k};
-    bad += expect_error("apsmatch:args", 1, 4, in);
-  }
-  for (mxArray* sets : {f8, set_of({f8, f8})}) {
-    const mxArray* in[] = {mode, sets, vec({2, 1}), k, r};
-    bad += expect_error("apsmatch:args", 1, 5, in);
-  }
-  for (mxArray* n : {vec({2}), vec({2, 0}), vec({2, 1.5}), vec({2, NAN})}) {
-    const mxArray* in[] = {mode, good, n, k, r};
-    bad += expect_error("apsmatch:args", 1, 5, in);
-  }
-  {  // sets of different classes or widths
-    const mxArray* in1[] = {mode, set_of({set_of({f8}), set_of({orb})}), vec({1, 1}), k, r};
-    bad += expect_error("apsmatch:args", 1, 5, in1);
-    const mxArray* in2[] = {mode, set_of({set_of({f8}), set_of({f16})}), vec({1, 1}), k, r};
-    bad += expect_error("apsmatch:args", 1, 5, in2);
-  }
-  {  // every set empty: 1 x B cell of cell(numImgs(b)) without touching the GPU
-    mxArray* out[1] = {nullptr};
-    const mxArray* in[] = {mode, set_of({mxCreateCellMatrix(1, 2), mxCreateCellMatrix(1, 3)}), vec({2, 3}), k, r};
-    mexFunction(1, out, 5, in);
-    const mxArray* c1 = out[0] ? mxGetCell(out[0], 1) : nullptr;
-    bad += !(out[0] && mxGetN(out[0]) == 2 && c1 && mxIsCell(c1) && mxGetM(c1) == 3 && mxGetN(c1) == 3);
-  }
-  if (nogpu) {
-    const mxArray* in[] = {mode, good, vec({2, 1}), k, r};
-    bad += expect_error("apsmatch:nogpu", 1, 5, in);
+  for (const char* verb : {"globalsets", "pairwisesets"}) {
+    auto set_of = [](std::vector<mxArray*> m) {
+      mxArray* c = mxCreateCellMatrix(1, (mwSize)m.size());
+      for (size_t i = 0; i < m.size(); ++i) mxSetCell(c, (mwIndex)i, m[i]);
+      return c;
+    };
+    auto vec = [](std::vector<double> v) {
+      mxArray* g = mxCreateDoubleMatrix(1, (mwSize)v.size(), mxREAL);
+      for (size_t i = 0; i < v.size(); ++i) mxGetPr(g)[i] = v[i];
+      return g;
+    };
+    mxArray* f8 = mxCreateNumericMatrix(6, 8, mxSINGLE_CLASS, mxREAL);
+    mxArray* f16 = mxCreateNumericMatrix(6, 16, mxSINGLE_CLASS, mxREAL);
+    mxArray* orb = new mxArray();
+    orb->cls = mxUNKNOWN_CLASS;
+    orb->dims = {1, 1};
+    orb->class_name = "binaryFeatures";
+    orb->properties.push_back({"Features", mxCreateNumericMatrix(6, 32, mxUINT8_CLASS, mxREAL)});
+    mxArray *mode = mxCreateString(verb), *k = mxCreateDoubleScalar(4), *r = mxCreateDoubleScalar(0.6);
+    mxArray* good = set_of({set_of({f8, f8}), set_of({f8})});
+    {  // too few arguments, sets not a cell of cells, numImgs of the wrong length / not positive integers
+      const mxArray* in[] = {mode, good, vec({2, 1}), k};
+      bad += expect_error("apsmatch:args", 1, 4, in);
+    }
+    for (mxArray* sets : {f8, set_of({f8, f8})}) {
+      const mxArray* in[] = {mode, sets, vec({2, 1}), k, r};
+      bad += expect_error("apsmatch:args", 1, 5, in);
+    }
+    for (mxArray* n : {vec({2}), vec({2, 0}), vec({2, 1.5}), vec({2, NAN})}) {
+      const mxArray* in[] = {mode, good, n, k, r};
+      bad += expect_error("apsmatch:args", 1, 5, in);
+    }
+    {  // sets of different classes or widths
+      const mxArray* in1[] = {mode, set_of({set_of({f8}), set_of({orb})}), vec({1, 1}), k, r};
+      bad += expect_error("apsmatch:args", 1, 5, in1);
+      const mxArray* in2[] = {mode, set_of({set_of({f8}), set_of({f16})}), vec({1, 1}), k, r};
+      bad += expect_error("apsmatch:args", 1, 5, in2);
+    }
+    {  // every set empty: 1 x B cell of cell(numImgs(b)) without touching the GPU
+      mxArray* out[1] = {nullptr};
+      const mxArray* in[] = {mode, set_of({mxCreateCellMatrix(1, 2), mxCreateCellMatrix(1, 3)}), vec({2, 3}), k, r};
+      mexFunction(1, out, 5, in);
+      const mxArray* c1 = out[0] ? mxGetCell(out[0], 1) : nullptr;
+      bad += !(out[0] && mxGetN(out[0]) == 2 && c1 && mxIsCell(c1) && mxGetM(c1) == 3 && mxGetN(c1) == 3);
+    }
+    if (nogpu) {
+      const mxArray* in[] = {mode, good, vec({2, 1}), k, r};
+      bad += expect_error("apsmatch:nogpu", 1, 5, in);
+    }
   }
   std::printf(bad ? "FAILED (%d)\n" : "OK\n", bad);
   return bad ? 1 : 0;
