@@ -22,6 +22,7 @@ from .host import (  # noqa: F401
     featureMatchingPairwise,
     imageMatching,
     imageMatchingBatch,
+    imageMatchingSets,
     ransacSampleTable,
     flann_knn_win,
     matchFeaturesScratch,
@@ -31,5 +32,6 @@ from .host import (  # noqa: F401
     nearest2HammingExhaustiveOMPMEX,
     nearest2SSDExhaustive,
     selectImagePartners,
+    selectImagePartnersSets,
 )
 from . import multigpu, synth  # noqa: F401

@@ -115,10 +115,13 @@ def lib():
         "aps_matchlist_metric": (C.POINTER(dbl), [vp]),
         "aps_matchlist_free": (None, [vp]),
         "aps_select_partners": (i32, [vp, vp, i32, i32, vp, vp, C.POINTER(i64)]),
+        "aps_select_partners_sets": (i32, [vp, i32, vp, vp, i32, vp, vp, vp]),
         "aps_ransac_sample_table": (i32, [vp, vp, i64, i64, C.c_uint64, vp]),
         "aps_image_matching_batch": (i32, [vp, i64, vp, vp, vp, dbl, dbl, i32, vp, i64, C.c_uint64, vp, vp, vp, vp, vp, vp]),
         "aps_image_matching": (i32, [vp, i32, vp, vp, vp, vp, vp, i64, dbl, dbl, i32, vp, i64, C.c_uint64, vp, vp, vp, vp,
                                      vp, vp, vp]),
+        "aps_image_matching_sets": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, vp, dbl, dbl, i32, vp, i64, C.c_uint64, vp,
+                                          vp, vp, vp, vp, vp, vp]),
         "aps_gplan_create": (i32, [vp, C.POINTER(i64), i32, i32, i32, i32, pp]),
         "aps_gplan_destroy": (None, [vp]),
         "aps_gplan_total": (i64, [vp]),

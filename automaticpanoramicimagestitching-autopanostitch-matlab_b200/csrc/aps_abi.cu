@@ -997,6 +997,52 @@ extern "C" int aps_select_partners(aps_ctx* c, const int64_t* counts, int n, int
   return APS_OK;
 }
 
+// imageMatching.m:75-100 for nsets sets: one upload (counts and the set tables), K6 over every set's block, the
+// device-side find(), one download, whatever nsets
+extern "C" int aps_select_partners_sets(aps_ctx* c, int nsets, const int* set_images, const int64_t* counts, int m,
+                                        uint8_t* cand, int64_t* pairs_lin, int64_t* set_pair_ptr) {
+  if (nsets < 0 || (nsets > 0 && !set_images) || !set_pair_ptr) APS_FAIL(APS_ERR_ARGS, "", "bad set list");
+  int64_t rows = 0, cells = 0, pair_cap = 0;
+  for (int b = 0; b < nsets; ++b) {
+    const int64_t n = set_images[b];
+    if (n < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d: negative image count", b + 1);
+    rows += n;
+    cells += n * n;
+    pair_cap += n * (n - 1) / 2;
+  }
+  if (rows > INT32_MAX) APS_FAIL(APS_ERR_ARGS, "", "more than 2^31 - 1 images");
+  if (cells > 0 && (!counts || !cand || !pairs_lin)) APS_FAIL(APS_ERR_ARGS, "", "NULL argument");
+  APS_CTX(c);
+  for (int b = 0; b <= nsets; ++b) set_pair_ptr[b] = 0;
+  if (cells == 0) return APS_OK;
+  // host / device layout [set_img | cell_off (nsets + 1 each) | counts (cells)], results [set_pair_ptr | pairs_lin | cand]
+  const size_t nt = (size_t)nsets + 1, in_words = 2 * nt + (size_t)cells, out_words = nt + (size_t)pair_cap;
+  std::vector<int64_t> in(in_words);
+  in[0] = in[nt] = 0;
+  for (int b = 0; b < nsets; ++b) {
+    in[b + 1] = in[b] + set_images[b];
+    in[nt + b + 1] = in[nt + b] + (int64_t)set_images[b] * set_images[b];
+  }
+  std::memcpy(in.data() + 2 * nt, counts, (size_t)cells * 8);
+  cudaStream_t s = c->stream;
+  DevBuf<int64_t> din, dout;
+  APS_TRY(din.alloc(in_words, s));
+  APS_TRY(dout.alloc(out_words + aps_ceil_div(cells, 8), s));
+  uint8_t* dcand = (uint8_t*)(dout.p + out_words);
+  uint8_t* h = (uint8_t*)aps_ctx_stage(c, out_words * 8 + (size_t)cells);
+  if (!h) APS_FAIL(APS_ERR_ALLOC, "", "pinned staging allocation failed");
+  APS_CUDA(cudaMemcpyAsync(din.p, in.data(), in_words * 8, cudaMemcpyHostToDevice, s));
+  APS_TRY(aps_k_select_partners_sets(s, din.p + 2 * nt, (int)rows, cells, din.p, din.p + nt, nsets, m, dcand));
+  APS_TRY(aps_k_select_compact(s, dcand, cells, din.p + nt, nsets, dout.p + nt, dout.p));
+  APS_CUDA(cudaMemcpyAsync(h, dout.p, out_words * 8 + (size_t)cells, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaStreamSynchronize(s));  // `in` stays alive until here
+  const int64_t* hw = (const int64_t*)h;
+  std::memcpy(set_pair_ptr, hw, nt * 8);
+  std::memcpy(pairs_lin, hw + nt, (size_t)hw[nsets] * 8);
+  std::memcpy(cand, h + out_words * 8, (size_t)cells);
+  return APS_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // diagnostics: run the tcgen05 candidate kernel alone and return what its epilogue saw
 extern "C" int aps_debug_tc_slots(aps_ctx* c, int64_t nq, int64_t nt) {

@@ -316,6 +316,13 @@ int aps_k_pair_filter_unique(cudaStream_t s, const uint32_t* idx2, const float* 
 
 // K6 aps_select.cu
 int aps_k_select_partners(cudaStream_t s, const int64_t* counts_cm, int n, int m, uint8_t* cand_cm);
+// the same for nsets image sets: n_rows = sum n_b pooled images, set_img / cell_off [nsets + 1] = first pooled image and
+// first cell of each set's n_b x n_b column-major block (cells = cell_off[nsets])
+int aps_k_select_partners_sets(cudaStream_t s, const int64_t* counts, int n_rows, int64_t cells, const int64_t* set_img,
+                               const int64_t* cell_off, int nsets, int m, uint8_t* cand);
+// find() of every set's block: pairs_lin = cell indices inside the set's block, set-major; set_pair_ptr [nsets + 1]
+int aps_k_select_compact(cudaStream_t s, const uint8_t* cand, int64_t cells, const int64_t* cell_off, int nsets,
+                         int64_t* pairs_lin, int64_t* set_pair_ptr);
 
 // aps_pairwise.cu : batched pairwise stages (see the file header)
 // X / sq: query rows ; XT / sqT: train view (the same arrays unless the train view carries subset images)

@@ -547,35 +547,111 @@ int aps_k_pair_filter_unique(cudaStream_t s, const uint32_t* idx2, const float* 
 }
 
 // ------------------------------------------------------------------------------------------------
-// K6  imageMatching.m:75-100.  Stable descending order == rank by (value desc, column asc).
-__global__ void k_select_rows(const int64_t* __restrict__ counts, int n, int take, uint8_t* __restrict__ P) {
-  const int i = blockIdx.x;
-  for (int j = threadIdx.x; j < n; j += blockDim.x) {
-    const int64_t sj = (i == j) ? 0 : counts[i + (int64_t)j * n] + counts[j + (int64_t)i * n];  // :82-83
+// K6  imageMatching.m:75-100 for every image set of a call.  Set b owns pooled images [set_img[b], set_img[b + 1]) and
+// the n_b x n_b column-major block of cells at cell_off[b] (both tables [nsets + 1]); NULL tables = one set of n images.
+// Stable descending order == rank by (value desc, column asc).
+struct SelectSet {
+  int64_t img0, cell0;
+  int n;
+};
+// the set whose range [tab[b], tab[b + 1]) holds x (tab non-decreasing: empty sets are skipped)
+__device__ __forceinline__ int select_set_of(const int64_t* __restrict__ tab, int nsets, int64_t x) {
+  int lo = 0, hi = nsets;  // last b with tab[b] <= x
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (tab[mid] <= x) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+__device__ __forceinline__ SelectSet select_set(const int64_t* __restrict__ set_img, const int64_t* __restrict__ cell_off,
+                                                int nsets, int n, const int64_t* __restrict__ tab, int64_t x) {
+  if (!set_img) return SelectSet{0, 0, n};
+  const int b = select_set_of(tab, nsets, x);
+  return SelectSet{set_img[b], cell_off[b], (int)(set_img[b + 1] - set_img[b])};
+}
+
+// one CTA per pooled image row: that row's partners ranked inside its own set's block
+__global__ void k_select_rows(const int64_t* __restrict__ counts, int n, const int64_t* __restrict__ set_img,
+                              const int64_t* __restrict__ cell_off, int nsets, int m, uint8_t* __restrict__ P) {
+  const SelectSet S = select_set(set_img, cell_off, nsets, n, set_img, blockIdx.x);
+  const int i = (int)(blockIdx.x - S.img0), nb = S.n;
+  const int take = m < nb - 1 ? (m < 0 ? 0 : m) : nb - 1;
+  const int64_t* C = counts + S.cell0;
+  for (int j = threadIdx.x; j < nb; j += blockDim.x) {
+    const int64_t sj = (i == j) ? 0 : C[i + (int64_t)j * nb] + C[j + (int64_t)i * nb];  // :82-83
     int r = 0;
-    for (int c = 0; c < n; ++c) {
-      const int64_t sc = (i == c) ? 0 : counts[i + (int64_t)c * n] + counts[c + (int64_t)i * n];
+    for (int c = 0; c < nb; ++c) {
+      const int64_t sc = (i == c) ? 0 : C[i + (int64_t)c * nb] + C[c + (int64_t)i * nb];
       r += (sc > sj) || (sc == sj && c < j);
     }
-    P[i + (int64_t)j * n] = r < take;  // :86-91
+    P[S.cell0 + i + (int64_t)j * nb] = r < take;  // :86-91
   }
 }
-__global__ void k_select_sym(const uint8_t* __restrict__ P, int n, uint8_t* __restrict__ cand) {
+__global__ void k_select_sym(const uint8_t* __restrict__ P, int n, const int64_t* __restrict__ set_img,
+                             const int64_t* __restrict__ cell_off, int nsets, int64_t cells, uint8_t* __restrict__ cand) {
   int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= (int64_t)n * n) return;
-  int i = (int)(c % n), j = (int)(c / n);
-  cand[c] = (i < j) && (P[i + (int64_t)j * n] || P[j + (int64_t)i * n]);  // :94-96
+  if (c >= cells) return;
+  const SelectSet S = select_set(set_img, cell_off, nsets, n, cell_off, c);
+  const int64_t l = c - S.cell0;
+  const int i = (int)(l % S.n), j = (int)(l / S.n);
+  cand[c] = (i < j) && (P[S.cell0 + i + (int64_t)j * S.n] || P[S.cell0 + j + (int64_t)i * S.n]);  // :94-96
+}
+
+// find(candidatePairs) of every set in one CTA: ascending cell order == set-major, find() order inside a set.
+// pairs_lin receives cell indices inside each set's block, set_pair_ptr [nsets + 1] the per-set offsets.
+__global__ void __launch_bounds__(1024) k_select_compact(const uint8_t* __restrict__ cand, int64_t cells,
+                                                         const int64_t* __restrict__ cell_off, int nsets,
+                                                         int64_t* __restrict__ pairs_lin, int64_t* __restrict__ set_pair_ptr) {
+  __shared__ int warp_cnt[32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int64_t base = 0;
+  for (int64_t c0 = 0; c0 < cells; c0 += blockDim.x) {
+    const int64_t c = c0 + threadIdx.x;
+    const bool sel = c < cells && cand[c];
+    const unsigned bal = __ballot_sync(0xffffffffu, sel);
+    if (lane == 0) warp_cnt[w] = __popc(bal);
+    __syncthreads();
+    int before = 0, tot = 0;
+    for (int k = 0; k < nw; ++k) {
+      before += k < w ? warp_cnt[k] : 0;
+      tot += warp_cnt[k];
+    }
+    if (sel) pairs_lin[base + before + __popc(bal & ((1u << lane) - 1u))] = c;
+    base += tot;
+    __syncthreads();
+  }
+  for (int b = threadIdx.x; b <= nsets; b += blockDim.x) {  // pairs in cells before set b's block
+    int64_t lo = 0, hi = base;
+    while (lo < hi) {
+      const int64_t mid = (lo + hi) >> 1;
+      if (pairs_lin[mid] < cell_off[b]) lo = mid + 1; else hi = mid;
+    }
+    set_pair_ptr[b] = lo;
+  }
+  __syncthreads();
+  for (int64_t k = threadIdx.x; k < base; k += blockDim.x)
+    pairs_lin[k] -= cell_off[select_set_of(cell_off, nsets, pairs_lin[k])];
+}
+
+int aps_k_select_partners_sets(cudaStream_t s, const int64_t* counts, int n_rows, int64_t cells, const int64_t* set_img,
+                               const int64_t* cell_off, int nsets, int m, uint8_t* cand) {
+  if (n_rows == 0) return APS_OK;
+  DevBuf<uint8_t> P;
+  APS_TRY(P.alloc((size_t)cells, s));
+  k_select_rows<<<n_rows, 128, 0, s>>>(counts, n_rows, set_img, cell_off, nsets, m, P.p);
+  APS_LAUNCHED();
+  k_select_sym<<<(unsigned)aps_ceil_div(cells, 256), 256, 0, s>>>(P.p, n_rows, set_img, cell_off, nsets, cells, cand);
+  APS_LAUNCHED();
+  return APS_OK;
 }
 
 int aps_k_select_partners(cudaStream_t s, const int64_t* counts_cm, int n, int m, uint8_t* cand_cm) {
-  if (n == 0) return APS_OK;
-  int take = m < n - 1 ? m : n - 1;
-  if (take < 0) take = 0;
-  DevBuf<uint8_t> P;
-  APS_TRY(P.alloc((size_t)n * n, s));
-  k_select_rows<<<n, 128, 0, s>>>(counts_cm, n, take, P.p);
-  APS_LAUNCHED();
-  k_select_sym<<<(unsigned)aps_ceil_div((int64_t)n * n, 256), 256, 0, s>>>(P.p, n, cand_cm);
+  return aps_k_select_partners_sets(s, counts_cm, n, (int64_t)n * n, nullptr, nullptr, 1, m, cand_cm);
+}
+
+int aps_k_select_compact(cudaStream_t s, const uint8_t* cand, int64_t cells, const int64_t* cell_off, int nsets,
+                         int64_t* pairs_lin, int64_t* set_pair_ptr) {
+  k_select_compact<<<1, 1024, 0, s>>>(cand, cells, cell_off, nsets, pairs_lin, set_pair_ptr);
   APS_LAUNCHED();
   return APS_OK;
 }

@@ -262,10 +262,12 @@ __device__ __forceinline__ uint64_t splitmix64(uint64_t& s) {
   return z ^ (z >> 31);
 }
 
-// K-R1: four distinct indices per (pair, draw), uniform without replacement (stand-in for randperm(n, 4))
-__global__ void k_ransac_samples(const int64_t* __restrict__ pt_ptr, int64_t n_draws, uint64_t seed,
-                                 uint32_t* __restrict__ samples) {
+// K-R1: four distinct indices per (pair, draw), uniform without replacement (stand-in for randperm(n, 4)).  The draws
+// of pair p are keyed by keys[p] (its index in its own set's candidate list), or by p when keys is NULL.
+__global__ void k_ransac_samples(const int64_t* __restrict__ pt_ptr, const int64_t* __restrict__ keys, int64_t n_draws,
+                                 uint64_t seed, uint32_t* __restrict__ samples) {
   const int64_t pair = blockIdx.y;
+  const int64_t key = keys ? keys[pair] : pair;
   const int64_t d = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (d >= n_draws) return;
   const int64_t n = pt_ptr[pair + 1] - pt_ptr[pair];
@@ -274,7 +276,7 @@ __global__ void k_ransac_samples(const int64_t* __restrict__ pt_ptr, int64_t n_d
     out[0] = out[1] = out[2] = out[3] = 0;
     return;
   }
-  uint64_t s = seed ^ (0xD1B54A32D192ED03ull * (uint64_t)(pair + 1)) ^ (0x8CB92BA72F3D8DD7ull * (uint64_t)(d + 1));
+  uint64_t s = seed ^ (0xD1B54A32D192ED03ull * (uint64_t)(key + 1)) ^ (0x8CB92BA72F3D8DD7ull * (uint64_t)(d + 1));
   uint32_t c[4];
   for (int k = 0; k < 4; ++k) {
     uint32_t r = (uint32_t)(splitmix64(s) % (uint64_t)(n - k));
@@ -592,13 +594,14 @@ __global__ void k_gather_matched_points(const int64_t* __restrict__ pt_ptr, cons
 
 // ---- launchers ------------------------------------------------------------------------------------------------
 static int ransac_device(aps_ctx* c, int64_t n_pairs, int64_t total, const int64_t* d_ptr, const double2* d_p1,
-                         const double2* d_p2, uint32_t* d_samples, bool have_samples, int64_t n_draws, uint64_t seed,
-                         double max_distance, double confidence, int max_trials, double* d_models, double* d_minv,
-                         uint8_t* d_inl, int32_t* d_ninl, uint8_t* d_acc, int32_t* d_used) {
+                         const double2* d_p2, uint32_t* d_samples, bool have_samples, const int64_t* d_keys,
+                         int64_t n_draws, uint64_t seed, double max_distance, double confidence, int max_trials,
+                         double* d_models, double* d_minv, uint8_t* d_inl, int32_t* d_ninl, uint8_t* d_acc,
+                         int32_t* d_used) {
   cudaStream_t s = c->stream;
   const dim3 gd((unsigned)((n_draws + 127) / 128), (unsigned)n_pairs);
   if (!have_samples) {
-    k_ransac_samples<<<gd, 128, 0, s>>>(d_ptr, n_draws, seed, d_samples);
+    k_ransac_samples<<<gd, 128, 0, s>>>(d_ptr, d_keys, n_draws, seed, d_samples);
     APS_LAUNCHED();
   }
   DevBuf<int32_t> cnt, best;
@@ -634,12 +637,17 @@ static int ransac_device(aps_ctx* c, int64_t n_pairs, int64_t total, const int64
   return APS_OK;
 }
 
+static int ransac_params(int64_t n_draws, int max_trials, double confidence) {
+  if (n_draws <= 0 || max_trials <= 0) APS_FAIL(APS_ERR_ARGS, "", "n_draws and max_trials must be positive");
+  if (!(confidence > 0.0 && confidence < 100.0)) APS_FAIL(APS_ERR_ARGS, "", "confidence must be in (0, 100)");
+  return APS_OK;
+}
+
 static int ransac_args(aps_ctx* c, int64_t n_pairs, const int64_t* pt_ptr, int64_t n_draws, int max_trials,
                        double confidence) {
   if (!c) APS_FAIL(APS_ERR_NOGPU, "apsmatch:nogpu", "context is NULL (no GPU context; there is no CPU path)");
   if (n_pairs < 0 || (n_pairs > 0 && !pt_ptr)) APS_FAIL(APS_ERR_ARGS, "", "bad pair list");
-  if (n_draws <= 0 || max_trials <= 0) APS_FAIL(APS_ERR_ARGS, "", "n_draws and max_trials must be positive");
-  if (!(confidence > 0.0 && confidence < 100.0)) APS_FAIL(APS_ERR_ARGS, "", "confidence must be in (0, 100)");
+  APS_TRY(ransac_params(n_draws, max_trials, confidence));
   if (n_pairs > 65535) APS_FAIL(APS_ERR_ARGS, "", "at most 65535 candidate pairs per call");
   for (int64_t p = 0; p < n_pairs; ++p)
     if (pt_ptr[p + 1] < pt_ptr[p]) APS_FAIL(APS_ERR_ARGS, "", "pt_ptr must be non-decreasing");
@@ -658,7 +666,7 @@ extern "C" int aps_ransac_sample_table(aps_ctx* c, const int64_t* pt_ptr, int64_
   APS_TRY(ds.alloc((size_t)(n_pairs * n_draws * 4), c->stream));
   APS_CUDA(cudaMemcpyAsync(dptr.p, pt_ptr, (size_t)(n_pairs + 1) * 8, cudaMemcpyHostToDevice, c->stream));
   const dim3 gd((unsigned)((n_draws + 127) / 128), (unsigned)n_pairs);
-  k_ransac_samples<<<gd, 128, 0, c->stream>>>(dptr.p, n_draws, seed, ds.p);
+  k_ransac_samples<<<gd, 128, 0, c->stream>>>(dptr.p, nullptr, n_draws, seed, ds.p);
   APS_LAUNCHED();
   APS_CUDA(cudaMemcpyAsync(samples, ds.p, (size_t)(n_pairs * n_draws * 4) * 4, cudaMemcpyDeviceToHost, c->stream));
   APS_CUDA(cudaStreamSynchronize(c->stream));
@@ -702,8 +710,8 @@ extern "C" int aps_image_matching_batch(aps_ctx* c, int64_t n_pairs, const int64
   }
   if (samples)
     APS_CUDA(cudaMemcpyAsync(ds.p, samples, (size_t)(n_pairs * n_draws * 4) * 4, cudaMemcpyHostToDevice, s));
-  APS_TRY(ransac_device(c, n_pairs, total, dptr.p, dp1.p, dp2.p, ds.p, samples != nullptr, n_draws, seed, max_distance,
-                        confidence, max_trials, dm.p, dmi.p, dinl.p, dni.p, dacc.p, dused.p));
+  APS_TRY(ransac_device(c, n_pairs, total, dptr.p, dp1.p, dp2.p, ds.p, samples != nullptr, nullptr, n_draws, seed,
+                        max_distance, confidence, max_trials, dm.p, dmi.p, dinl.p, dni.p, dacc.p, dused.p));
   APS_CUDA(cudaMemcpyAsync(models, dm.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
   APS_CUDA(cudaMemcpyAsync(models_inv, dmi.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
   if (total > 0) APS_CUDA(cudaMemcpyAsync(inliers, dinl.p, (size_t)total, cudaMemcpyDeviceToHost, s));
@@ -787,8 +795,8 @@ extern "C" int aps_image_matching(aps_ctx* c, int n_images, const int64_t* pair_
   }
   if (samples)
     APS_CUDA(cudaMemcpyAsync(ds.p, samples, (size_t)(n_pairs * n_draws * 4) * 4, cudaMemcpyHostToDevice, s));
-  APS_TRY(ransac_device(c, n_pairs, total, dptr.p, dp1.p, dp2.p, ds.p, samples != nullptr, n_draws, seed, max_distance,
-                        confidence, max_trials, dm.p, dmi.p, dinl.p, dni.p, dacc.p, dused.p));
+  APS_TRY(ransac_device(c, n_pairs, total, dptr.p, dp1.p, dp2.p, ds.p, samples != nullptr, nullptr, n_draws, seed,
+                        max_distance, confidence, max_trials, dm.p, dmi.p, dinl.p, dni.p, dacc.p, dused.p));
   APS_CUDA(cudaMemcpyAsync(models, dm.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
   APS_CUDA(cudaMemcpyAsync(models_inv, dmi.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
   if (total > 0) APS_CUDA(cudaMemcpyAsync(inliers, dinl.p, (size_t)total, cudaMemcpyDeviceToHost, s));
@@ -796,5 +804,131 @@ extern "C" int aps_image_matching(aps_ctx* c, int n_images, const int64_t* pair_
   APS_CUDA(cudaMemcpyAsync(accepted, dacc.p, (size_t)n_pairs, cudaMemcpyDeviceToHost, s));
   APS_CUDA(cudaMemcpyAsync(draws_used, dused.p, (size_t)n_pairs * 4, cudaMemcpyDeviceToHost, s));
   APS_CUDA(cudaStreamSynchronize(s));  // crow / ptr / ii / jj stay alive until here
+  return APS_OK;
+}
+
+// imageMatching.m:121-156 for every candidate pair of nsets image sets.  Set b's pairs are
+// set_pair_ptr[b] .. set_pair_ptr[b + 1] of pairs_lin (cells of its own n_b x n_b block); its images are the pooled
+// images g_b .. g_b + n_b of img_off / keypoints.  Pair p of set b draws its samples under key p - set_pair_ptr[b], the
+// key its single-set call gives it, so every set gets the single-set call's bits.  The gather and the RANSAC chain
+// run in chunks of pairs: gridDim.y holds at most 65535 pairs, and the per-draw tables (kSetsDrawBytes per draw and
+// pair) stay within kSetsChunkBytes.  pt_ptr offsets are absolute, so a chunk only offsets the per-pair pointers.
+static constexpr int64_t kSetsDrawBytes = 16 + 72 + 4 + 8;  // sample table, Htab, cnt, err
+static constexpr int64_t kSetsChunkBytes = (int64_t)1 << 30;
+
+extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_images, const int64_t* const* pair_ptr,
+                                       const uint32_t* const* rows, const double* keypoints, const int64_t* img_off,
+                                       const int64_t* set_pair_ptr, const int64_t* pairs_lin, double max_distance,
+                                       double confidence, int max_trials, const uint32_t* samples, int64_t n_draws,
+                                       uint64_t seed, int64_t* pt_ptr_out, double* models, double* models_inv,
+                                       uint8_t* inliers, int32_t* n_inliers, uint8_t* accepted, int32_t* draws_used) {
+  if (nsets < 0 || (nsets > 0 && (!set_images || !set_pair_ptr))) APS_FAIL(APS_ERR_ARGS, "", "bad set list");
+  std::vector<int64_t> img0((size_t)nsets + 1, 0);
+  for (int b = 0; b < nsets; ++b) {
+    if (set_images[b] < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d: negative image count", b + 1);
+    img0[b + 1] = img0[b] + set_images[b];
+  }
+  if (img0[nsets] > INT32_MAX) APS_FAIL(APS_ERR_ARGS, "", "more than 2^31 - 1 images");
+  if (nsets > 0 && set_pair_ptr[0] != 0) APS_FAIL(APS_ERR_ARGS, "", "set_pair_ptr[0] must be 0");
+  for (int b = 0; b < nsets; ++b)
+    if (set_pair_ptr[b + 1] < set_pair_ptr[b]) APS_FAIL(APS_ERR_ARGS, "", "set_pair_ptr must be non-decreasing");
+  APS_TRY(ransac_params(n_draws, max_trials, confidence));
+  const int64_t n_pairs = nsets > 0 ? set_pair_ptr[nsets] : 0, G = img0[nsets];
+  if (n_pairs > 0 && (!pair_ptr || !rows || !pairs_lin || !img_off || !pt_ptr_out || !models || !models_inv ||
+                      !n_inliers || !accepted || !draws_used))
+    APS_FAIL(APS_ERR_ARGS, "", "NULL argument");
+  std::vector<int64_t> ptr((size_t)n_pairs + 1, 0), keys((size_t)n_pairs);
+  std::vector<int32_t> ii((size_t)n_pairs), jj((size_t)n_pairs);
+  for (int b = 0; b < nsets; ++b) {
+    const int64_t n = set_images[b];
+    for (int64_t p = set_pair_ptr[b]; p < set_pair_ptr[b + 1]; ++p) {
+      const int64_t lin = pairs_lin[p];
+      if (!pair_ptr[b] || lin < 0 || lin >= n * n) APS_FAIL(APS_ERR_ARGS, "", "set %d: pair index out of range", b + 1);
+      const int64_t cnt = pair_ptr[b][lin + 1] - pair_ptr[b][lin];
+      if (cnt < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d: pair_ptr must be non-decreasing", b + 1);
+      ii[p] = (int32_t)(img0[b] + lin % n);
+      jj[p] = (int32_t)(img0[b] + lin / n);
+      keys[p] = p - set_pair_ptr[b];
+      ptr[p + 1] = ptr[p] + cnt;
+    }
+  }
+  const int64_t total = ptr[n_pairs], F = n_pairs > 0 ? img_off[G] : 0;
+  if (total > 0 && (!keypoints || !inliers)) APS_FAIL(APS_ERR_ARGS, "", "NULL argument");
+  std::vector<uint32_t> crow((size_t)(2 * total));
+  for (int b = 0; b < nsets; ++b)
+    for (int64_t p = set_pair_ptr[b]; p < set_pair_ptr[b + 1]; ++p) {  // refineMatch:214-221
+      const int64_t a = pair_ptr[b][pairs_lin[p]], cntp = ptr[p + 1] - ptr[p];
+      const int64_t ni = img_off[ii[p] + 1] - img_off[ii[p]], nj = img_off[jj[p] + 1] - img_off[jj[p]];
+      if (cntp > 0 && !rows[b]) APS_FAIL(APS_ERR_ARGS, "", "set %d: rows is NULL", b + 1);
+      for (int64_t r = 0; r < cntp; ++r) {
+        const uint32_t ra = rows[b][2 * (a + r)], rb = rows[b][2 * (a + r) + 1];
+        if (ra < 1 || rb < 1 || (int64_t)ra > ni || (int64_t)rb > nj)
+          APS_FAIL(APS_ERR_ARGS, "refineMatch:MatchIndexOutOfBounds",
+                   "Match indices exceed keypoint array sizes (set %d).", b + 1);
+        crow[2 * (ptr[p] + r)] = ra;
+        crow[2 * (ptr[p] + r) + 1] = rb;
+      }
+    }
+  if (!c) APS_FAIL(APS_ERR_NOGPU, "apsmatch:nogpu", "context is NULL (no GPU context; there is no CPU path)");
+  APS_CUDA(cudaSetDevice(c->device));
+  if (pt_ptr_out)
+    for (int64_t p = 0; p <= n_pairs; ++p) pt_ptr_out[p] = ptr[p];
+  if (n_pairs == 0) return APS_OK;
+  const int64_t by_bytes = kSetsChunkBytes / (n_draws * kSetsDrawBytes);
+  const int64_t chunk = aps_min64(65535, by_bytes > 0 ? by_bytes : 1);
+  cudaStream_t s = c->stream;
+  DevBuf<int64_t> dptr, doff, dkeys;
+  DevBuf<int32_t> dii, djj, dni, dused;
+  DevBuf<uint32_t> drows, ds;
+  DevBuf<double2> dkp, dp1, dp2;
+  DevBuf<double> dm, dmi;
+  DevBuf<uint8_t> dinl, dacc;
+  const size_t tot = (size_t)(total > 0 ? total : 1);
+  APS_TRY(dptr.alloc((size_t)n_pairs + 1, s));
+  APS_TRY(doff.alloc((size_t)G + 1, s));
+  APS_TRY(dkeys.alloc((size_t)n_pairs, s));
+  APS_TRY(dii.alloc((size_t)n_pairs, s));
+  APS_TRY(djj.alloc((size_t)n_pairs, s));
+  APS_TRY(drows.alloc(2 * tot, s));
+  APS_TRY(dkp.alloc((size_t)(F > 0 ? F : 1), s));
+  APS_TRY(dp1.alloc(tot, s));
+  APS_TRY(dp2.alloc(tot, s));
+  APS_TRY(ds.alloc((size_t)(aps_min64(chunk, n_pairs) * n_draws * 4), s));
+  APS_TRY(dm.alloc((size_t)n_pairs * 9, s));
+  APS_TRY(dmi.alloc((size_t)n_pairs * 9, s));
+  APS_TRY(dinl.alloc(tot, s));
+  APS_TRY(dacc.alloc((size_t)n_pairs, s));
+  APS_TRY(dni.alloc((size_t)n_pairs, s));
+  APS_TRY(dused.alloc((size_t)n_pairs, s));
+  APS_CUDA(cudaMemcpyAsync(dptr.p, ptr.data(), (size_t)(n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
+  APS_CUDA(cudaMemcpyAsync(doff.p, img_off, (size_t)(G + 1) * 8, cudaMemcpyHostToDevice, s));
+  APS_CUDA(cudaMemcpyAsync(dkeys.p, keys.data(), (size_t)n_pairs * 8, cudaMemcpyHostToDevice, s));
+  APS_CUDA(cudaMemcpyAsync(dii.p, ii.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
+  APS_CUDA(cudaMemcpyAsync(djj.p, jj.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
+  if (total > 0) {
+    APS_CUDA(cudaMemcpyAsync(drows.p, crow.data(), (size_t)total * 8, cudaMemcpyHostToDevice, s));
+    APS_CUDA(cudaMemcpyAsync(dkp.p, keypoints, (size_t)F * 16, cudaMemcpyHostToDevice, s));
+  }
+  for (int64_t p0 = 0; p0 < n_pairs; p0 += chunk) {
+    const int64_t np = aps_min64(chunk, n_pairs - p0);
+    if (ptr[p0 + np] > ptr[p0]) {
+      k_gather_matched_points<<<dim3(8, (unsigned)np), 256, 0, s>>>(dptr.p + p0, drows.p, dii.p + p0, djj.p + p0, doff.p,
+                                                                    dkp.p, dp1.p, dp2.p);
+      APS_LAUNCHED();
+    }
+    if (samples)
+      APS_CUDA(cudaMemcpyAsync(ds.p, samples + p0 * n_draws * 4, (size_t)(np * n_draws * 4) * 4, cudaMemcpyHostToDevice,
+                               s));
+    APS_TRY(ransac_device(c, np, total, dptr.p + p0, dp1.p, dp2.p, ds.p, samples != nullptr, dkeys.p + p0, n_draws, seed,
+                          max_distance, confidence, max_trials, dm.p + 9 * p0, dmi.p + 9 * p0, dinl.p, dni.p + p0,
+                          dacc.p + p0, dused.p + p0));
+  }
+  APS_CUDA(cudaMemcpyAsync(models, dm.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(models_inv, dmi.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
+  if (total > 0) APS_CUDA(cudaMemcpyAsync(inliers, dinl.p, (size_t)total, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(n_inliers, dni.p, (size_t)n_pairs * 4, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(accepted, dacc.p, (size_t)n_pairs, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaMemcpyAsync(draws_used, dused.p, (size_t)n_pairs * 4, cudaMemcpyDeviceToHost, s));
+  APS_CUDA(cudaStreamSynchronize(s));  // crow / ptr / keys / ii / jj stay alive until here
   return APS_OK;
 }

@@ -643,18 +643,22 @@ def nearest2SSDExhaustive(A, B, ctx=None):
     return np.arange(1, N1 + 1, dtype=np.float64), idx2, d1, d2
 
 
+def _putative_counts(matchesAll):
+    """putativeCount of imageMatching.m:76: rows of every cell of the n x n nested list (or an integer count matrix)"""
+    if isinstance(matchesAll, np.ndarray):
+        return matchesAll.astype(np.int64)
+    n = len(matchesAll)
+    return np.array([[np.asarray(matchesAll[i][j]).shape[0] if np.asarray(matchesAll[i][j]).ndim == 2 else 0
+                      for j in range(n)] for i in range(n)], np.int64)
+
+
 def selectImagePartners(matchesAll, m, ctx=None):
     """Top-m candidate selection of imageMatching.m:75-100.
 
     matchesAll: n x n nested list of [M x 2] arrays (or an [n x n] integer count matrix).
     Returns (candidatePairs [n x n] bool, IuptriIdx: 1-based column-major linear indices)."""
     ctx = ctx or default_context()
-    if isinstance(matchesAll, np.ndarray):
-        counts = matchesAll.astype(np.int64)
-    else:
-        n = len(matchesAll)
-        counts = np.array([[np.asarray(matchesAll[i][j]).shape[0] if np.asarray(matchesAll[i][j]).ndim == 2 else 0
-                            for j in range(n)] for i in range(n)], np.int64)
+    counts = _putative_counts(matchesAll)
     n = counts.shape[0]
     if counts.shape != (n, n):
         raise ValueError("matchesAll must be an n-by-n cell array.")  # imageMatching.m:58-60
@@ -785,8 +789,137 @@ def imageMatching(input, n, keypoints, matchesAll, imagesProcessed=None, samples
         numMatches[i, j] = ni[p]
         tforms[i][j], tforms[j][i] = models[p], minv[p]  # :150-151, :165-166
     imageMatching.last = dict(pairs_lin=lin, pt_ptr=ptr, n_inliers=ni, accepted=acc.astype(bool), draws_used=du,
-                              models=models, inliers=inl[:total].astype(bool))
+                              models=models, models_inv=minv, inliers=inl[:total].astype(bool))
     return allMatches, numMatches, tforms
+
+
+def _set_counts(matchesAll):
+    c = _putative_counts(matchesAll)
+    return c.reshape(0, 0) if c.size == 0 and c.ndim == 1 else c   # a set without images: a 0 x 0 block
+
+
+def _select_partners_sets(ctx, counts_sets, m):
+    """aps_select_partners_sets over [n_b x n_b] count matrices -> (cand blocks, 0-based pairs_lin, set_pair_ptr)"""
+    ns = [c.shape[0] for c in counts_sets]
+    B, cells = len(ns), sum(n * n for n in ns)
+    cm = (np.concatenate([np.ascontiguousarray(c.T).ravel() for c in counts_sets]).astype(np.int64) if cells
+          else np.zeros(0, np.int64))  # column-major blocks, set after set
+    cand = np.zeros(cells, np.uint8)
+    pairs = np.zeros(sum(n * (n - 1) // 2 for n in ns), np.int64)
+    spp = np.zeros(B + 1, np.int64)
+    simg = (C.c_int * max(B, 1))(*ns)
+    check(lib().aps_select_partners_sets(ctx.handle, B, simg, _ptr(cm), int(m), _ptr(cand), _ptr(pairs), _ptr(spp)))
+    return cand, pairs[:spp[-1]], spp
+
+
+def selectImagePartnersSets(matchesAllSets, m, ctx=None):
+    """selectImagePartners over B independent image sets in one call (aps_select_partners_sets): element b of the
+    returned list is exactly selectImagePartners(matchesAllSets[b], m) -- (candidatePairs, 1-based IuptriIdx)."""
+    ctx = ctx or default_context()
+    counts = [_set_counts(mb) for mb in matchesAllSets]
+    for b, c in enumerate(counts):
+        if c.shape != (c.shape[0], c.shape[0]):
+            raise ValueError(f"matchesAllSets[{b}] must be an n-by-n cell array.")
+    cand, pairs, spp = _select_partners_sets(ctx, counts, m)
+    out, c0 = [], 0
+    for b, c in enumerate(counts):
+        n = c.shape[0]
+        out.append((cand[c0:c0 + n * n].reshape(n, n).T.astype(bool), pairs[spp[b]:spp[b + 1]] + 1))
+        c0 += n * n
+    return out
+
+
+def imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets, seed=0, samples=None, ctx=None):
+    """[allMatchesSets, numMatchesSets, tformsSets] = imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets)
+
+    imageMatching over B independent image sets in one call (aps_select_partners_sets, then aps_image_matching_sets):
+    set b is keypointsSets[b] / matchesAllSets[b] with numImgs[b] images.  Returns a list of B tuples, element b exactly
+    what imageMatching(input, numImgs[b], keypointsSets[b], matchesAllSets[b], seed=seed) returns.  samples: None (drawn
+    on the device, each set as its single-set call draws) or one table per set, each what imageMatching's `samples`
+    would be for that set.  Device groups (input.apsGPUs) are not supported here."""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by imageMatchingSets; verify the sets on one GPU")
+    kps_sets, m_sets = list(keypointsSets), list(matchesAllSets)
+    nums = list(np.atleast_1d(np.asarray(numImgs, dtype=np.float64)).ravel()) if np.size(numImgs) else []
+    if len(nums) != len(kps_sets) or len(nums) != len(m_sets):
+        raise ValueError("numImgs must give one image count per keypoint set and per match set")
+    for v in nums:
+        if not (np.isfinite(v) and v >= 0 and v == np.round(v)):
+            raise ValueError("every numImgs entry must be a non-negative integer")
+    if str(_field(input, "imageMatchingMethod", "ransac")).lower() != "ransac" or int(_field(input, "useMATLABImageMatching", 0)):
+        raise ValueError("only input.imageMatchingMethod = 'ransac' with useMATLABImageMatching = 0 is built")
+    if str(_field(input, "transformationType", "projective")).lower() != "projective":
+        raise ValueError("only input.transformationType = 'projective' is built")
+    ns = [int(v) for v in nums]
+    for b, (n, kps, mall) in enumerate(zip(ns, kps_sets, m_sets)):
+        if len(mall) != n or any(len(r) != n for r in mall):
+            raise ValueError(f"matchesAllSets[{b}] must be an n-by-n cell array.")  # imageMatching:InvalidMatchesAllSize
+        if len(kps) != n:
+            raise ValueError(f"keypointsSets[{b}] must contain n elements (one per image).")
+    ctx = ctx or default_context()
+    B = len(ns)
+    _, lin, spp = _select_partners_sets(ctx, [_set_counts(mall) for mall in m_sets], int(_field(input, "mBrownLowe", 6)))
+    result = [([[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)], np.zeros((n, n)), [[None] * n for _ in range(n)])
+              for n in ns]
+    imageMatchingSets.last = [dict(pairs_lin=np.zeros(0, np.int64), pt_ptr=np.zeros(1, np.int64)) for _ in ns]
+    P = int(spp[-1])
+    if P == 0:
+        return result
+    # per set: CSR of the cell (column-major cell index c = i + j*n, strict upper triangle), as imageMatching builds it
+    pps, rows = [], []
+    for n, mall in zip(ns, m_sets):
+        pp, segs = np.zeros(n * n + 1, np.int64), []
+        for j in range(n):
+            for i in range(j):
+                a = np.asarray(mall[i][j])
+                if a.ndim == 2 and a.shape[0]:
+                    pp[i + j * n + 1] = a.shape[0]
+                    segs.append(np.ascontiguousarray(a, np.float64).astype(np.uint32))
+        pps.append(np.cumsum(pp))
+        rows.append(np.ascontiguousarray(np.vstack(segs), np.uint32) if segs else np.zeros((0, 2), np.uint32))
+    kps = [np.asarray(k, np.float64).reshape(-1, 2) for ks in kps_sets for k in ks]
+    img_off = np.concatenate([[0], np.cumsum([k.shape[0] for k in kps], dtype=np.int64)]).astype(np.int64)
+    kp = np.ascontiguousarray(np.vstack(kps)) if img_off[-1] else np.zeros((0, 2))
+    md, conf, mt = _ransac_params(input)
+    n_draws = 2 * mt
+    if samples is not None:
+        tabs = [np.ascontiguousarray(t, np.uint32) for t in samples]
+        if len(tabs) != B:
+            raise ValueError("samples must hold one table per set")
+        n_draws = next((t.size // (4 * (spp[b + 1] - spp[b])) for b, t in enumerate(tabs) if spp[b + 1] > spp[b]), 0)
+        samples = np.ascontiguousarray(np.concatenate([t.reshape(spp[b + 1] - spp[b], n_draws, 4)
+                                                       for b, t in enumerate(tabs)]))
+    ptr = np.zeros(P + 1, np.int64)
+    total = 0
+    for b in range(B):
+        total += int(sum(pps[b][c + 1] - pps[b][c] for c in lin[spp[b]:spp[b + 1]]))
+    models, minv = np.full((P, 3, 3), np.nan), np.full((P, 3, 3), np.nan)
+    inl, ni = np.zeros(total, np.uint8), np.zeros(P, np.int32)
+    acc, du = np.zeros(P, np.uint8), np.zeros(P, np.int32)
+    simg = (C.c_int * B)(*ns)
+    pp_arr = (C.c_void_p * B)(*[p.ctypes.data for p in pps])
+    rows_arr = (C.c_void_p * B)(*[r.ctypes.data if r.size else None for r in rows])
+    check(lib().aps_image_matching_sets(ctx.handle, B, simg, pp_arr, rows_arr, _ptr(kp), _ptr(img_off), _ptr(spp),
+                                        _ptr(lin), md, conf, mt, _ptr(samples) if samples is not None else C.c_void_p(0),
+                                        int(n_draws), int(seed), _ptr(ptr), _ptr(models), _ptr(minv), _ptr(inl), _ptr(ni),
+                                        _ptr(acc), _ptr(du)))
+    for b, (n, mall) in enumerate(zip(ns, m_sets)):
+        p0, p1 = int(spp[b]), int(spp[b + 1])
+        allMatches, numMatches, tforms = result[b]
+        for p in range(p0, p1):
+            if not acc[p]:
+                continue
+            c = lin[p]
+            i, j = int(c % n), int(c // n)
+            mij = np.asarray(mall[i][j], np.float64)
+            allMatches[i][j] = mij[inl[ptr[p]:ptr[p + 1]].astype(bool)]  # imageMatching.m:148
+            numMatches[i, j] = ni[p]
+            tforms[i][j], tforms[j][i] = models[p], minv[p]  # :150-151, :165-166
+        t0, t1 = ptr[p0], ptr[p1]
+        imageMatchingSets.last[b] = dict(pairs_lin=lin[p0:p1], pt_ptr=ptr[p0:p1 + 1] - t0, n_inliers=ni[p0:p1],
+                                         accepted=acc[p0:p1].astype(bool), draws_used=du[p0:p1], models=models[p0:p1],
+                                         models_inv=minv[p0:p1], inliers=inl[t0:t1].astype(bool))
+    return result
 
 
 RECORD_PAD = 16384  # APS_RECORD_PAD of include/apsmatch.h: rows the record buffer holds beyond F

@@ -230,6 +230,15 @@ void aps_matchlist_free(aps_matchlist* m);
  * NULL) receives find(candidatePairs) as 0-based linear indices, *npairs their number. */
 int aps_select_partners(aps_ctx* ctx, const int64_t* counts, int n, int m, uint8_t* cand, int64_t* pairs_lin,
                         int64_t* npairs);
+/* The same for nsets independent image sets in one call.  Set b has set_images[b] images; counts holds, for each set,
+ * its n_b x n_b column-major putativeCount block at cell_off[b] = sum_{c<b} n_c^2 (the cell layout of
+ * aps_feature_matching_global_sets' compaction); cand [sum n_b^2] the blocks of candidatePairs.  pairs_lin [<= sum
+ * n_b (n_b - 1) / 2] receives the 0-based linear cell indices INSIDE each set's block, set-major and ascending within a
+ * set (find() order); set_pair_ptr [nsets + 1] the offset of each set's pairs.  Set b's results are bit-identical to
+ * aps_select_partners on set b alone.  One upload, one download and one synchronisation, whatever nsets.  nsets < 0, a
+ * negative image count or a NULL argument is APS_ERR_ARGS (checked before the context). */
+int aps_select_partners_sets(aps_ctx* ctx, int nsets, const int* set_images, const int64_t* counts, int m,
+                             uint8_t* cand, int64_t* pairs_lin, int64_t* set_pair_ptr);
 
 /* ---- consumer of the match lists: batched RANSAC homographies (SURVEY.md 8(f) rank 1) ---------------
  * Replaces the parfor of PP/imageMatching/imageMatching.m:121-156 with its callee
@@ -268,6 +277,23 @@ int aps_image_matching(aps_ctx* ctx, int n_images, const int64_t* pair_ptr, cons
                        double max_distance, double confidence, int max_trials, const uint32_t* samples,
                        int64_t n_draws, uint64_t seed, int64_t* pt_ptr_out, double* models, double* models_inv,
                        uint8_t* inliers, int32_t* n_inliers, uint8_t* accepted, int32_t* draws_used);
+/* aps_image_matching for every candidate pair of nsets independent image sets in one pass.  pair_ptr[b] / rows[b] =
+ * set b's CSR (what aps_matchlist_pair_ptr / _rows return for its list); keypoints = pooled [F x 2] ROW-major doubles of
+ * all images of all sets (set 0's images first), img_off [sum n_b + 1]; set_pair_ptr / pairs_lin as
+ * aps_select_partners_sets returns them.  Outputs are pooled in that pair order and mean what aps_image_matching's
+ * mean: pt_ptr_out [n_pairs + 1] are offsets into the pooled `inliers`.  samples = [n_pairs x n_draws x 4] pooled in
+ * the same order, or NULL to draw them on the device, pair p of set b keyed by p - set_pair_ptr[b] (its index in its
+ * own set's list).  Every set's outputs are BIT-IDENTICAL to aps_image_matching on that set alone with the same seed.
+ * Argument errors (checked before the context): nsets < 0, a negative image count or a bad pair index is APS_ERR_ARGS;
+ * a match index outside a set's keypoints is refineMatch:MatchIndexOutOfBounds naming the set, and the call returns
+ * nothing.  No limit on the number of pairs: the gather and the RANSAC chain run in chunks of at most 65535 pairs and
+ * about 1 GiB of per-draw tables; launches grow with the chunks, never with nsets. */
+int aps_image_matching_sets(aps_ctx* ctx, int nsets, const int* set_images, const int64_t* const* pair_ptr,
+                            const uint32_t* const* rows, const double* keypoints, const int64_t* img_off,
+                            const int64_t* set_pair_ptr, const int64_t* pairs_lin, double max_distance,
+                            double confidence, int max_trials, const uint32_t* samples, int64_t n_draws,
+                            uint64_t seed, int64_t* pt_ptr_out, double* models, double* models_inv,
+                            uint8_t* inliers, int32_t* n_inliers, uint8_t* accepted, int32_t* draws_used);
 
 /* ---- staged global pipeline (building block of the multi-GPU host; bench.py times these) -----
  * The stages of PP/featureMatching/featureMatchingGlobal.m as separate calls: pooling + normalisation :70-97

@@ -131,6 +131,28 @@ static int file_mode(const char* in_path, const char* out_path) {
                            mxCreateDoubleScalar(sc[2]), uq};
     mexFunction(2, out, 6, in);
     outs = {out[0], out[1]};
+#elif defined(GATE_IMATCH_SETS)  // scalars: B, numImgs(1..B), m, maxDistance, confidence, maxIter, seed ; matrices: per
+    // set its n_b keypoint matrices, then its n_b^2 matchesAll cells in column-major order.  outputs per set: the n_b^2
+    // allMatches cells (column-major), numMatches, the n_b^2 tforms cells
+    const int B = (int)sc[0];
+    mxArray *kps = mxCreateCellMatrix(1, (mwSize)B), *mcs = mxCreateCellMatrix(1, (mwSize)B);
+    for (int b = 0, m0 = 0; b < B; ++b) {
+      const int n = (int)sc[1 + b];
+      mxArray *kc = mxCreateCellMatrix(1, (mwSize)n), *mc = mxCreateCellMatrix((mwSize)n, (mwSize)n);
+      for (int i = 0; i < n; ++i) mxSetCell(kc, (mwIndex)i, mats[m0++]);
+      for (int c = 0; c < n * n; ++c) mxSetCell(mc, (mwIndex)c, mats[m0++]);
+      mxSetCell(kps, (mwIndex)b, kc);
+      mxSetCell(mcs, (mwIndex)b, mc);
+    }
+    std::vector<const mxArray*> in = {kps, mcs};
+    for (size_t i = 1 + B; i < sc.size(); ++i) in.push_back(mxCreateDoubleScalar(sc[i]));
+    mexFunction(3, out, (int)in.size(), in.data());
+    for (int b = 0; b < B; ++b) {
+      const int n = (int)sc[1 + b];
+      for (int c = 0; c < n * n; ++c) outs.push_back(mxGetCell(mxGetCell(out[0], (mwIndex)b), (mwIndex)c));
+      outs.push_back(mxGetCell(out[1], (mwIndex)b));
+      for (int c = 0; c < n * n; ++c) outs.push_back(mxGetCell(mxGetCell(out[2], (mwIndex)b), (mwIndex)c));
+    }
 #else
     (void)out;
     return 3;
@@ -348,6 +370,64 @@ int main(int argc, char** argv) {
     for (int r = 0; r < 10; ++r) mxGetPr(m12)[r] = (r % 5) + 1;
     mxSetCell(kp, 0, k1); mxSetCell(kp, 1, k2); mxSetCell(mm, 2, m12);
     const mxArray* in[] = {kp, mm, six, md, cf, it};
+    bad += expect_error("apsmatch:nogpu", 3, 6, in);  // no CPU fallback
+  }
+#elif defined(GATE_IMATCH_SETS)
+  // two sets: set 1 = two images whose second is the first shifted by (10, -5) (40 correspondences, 30 exact), set 2 =
+  // one image (no candidate pair)
+  const int N = 40;
+  mxArray *k1 = mxCreateDoubleMatrix(N, 2, mxREAL), *k2 = mxCreateDoubleMatrix(N, 2, mxREAL), *m12 = mxCreateDoubleMatrix(N, 2, mxREAL);
+  for (int r = 0; r < N; ++r) {
+    const double x = (double)((r * 37) % 101) * 7.0, y = (double)((r * 53) % 89) * 9.0;
+    mxGetPr(k1)[r] = x; mxGetPr(k1)[r + N] = y;
+    mxGetPr(k2)[r] = (r < 30) ? x - 10.0 : (double)((r * 11) % 97) * 5.0;
+    mxGetPr(k2)[r + N] = (r < 30) ? y + 5.0 : (double)((r * 29) % 83) * 3.0;
+    mxGetPr(m12)[r] = r + 1; mxGetPr(m12)[r + N] = r + 1;
+  }
+  auto cell_of = [](int m, int n, std::vector<mxArray*> e) {
+    mxArray* c = mxCreateCellMatrix((mwSize)m, (mwSize)n);
+    for (size_t i = 0; i < e.size(); ++i) mxSetCell(c, (mwIndex)i, e[i]);
+    return c;
+  };
+  mxArray* kp1 = cell_of(1, 2, {k1, k2});
+  mxArray* mm1 = cell_of(2, 2, {nullptr, nullptr, m12, nullptr});
+  mxArray* kps = cell_of(1, 2, {kp1, cell_of(1, 1, {k1})});
+  mxArray* mms = cell_of(1, 2, {mm1, mxCreateCellMatrix(1, 1)});
+  mxArray *six = mxCreateDoubleScalar(6), *md = mxCreateDoubleScalar(5.5), *cf = mxCreateDoubleScalar(99.9), *it = mxCreateDoubleScalar(500);
+  { const mxArray* in[] = {kps, mms, six}; bad += expect_error("apsmatch:args", 3, 3, in); }
+  { const mxArray* in[] = {kp1, mms, six, md, cf, it}; bad += expect_error("apsmatch:args", 3, 6, in); }   // not one per set
+  { const mxArray* in[] = {six, mms, six, md, cf, it}; bad += expect_error("apsmatch:args", 3, 6, in); }   // not a cell
+  { const mxArray* in[] = {kps, cell_of(1, 2, {mm1, cell_of(1, 2, {nullptr, nullptr})}), six, md, cf, it};
+    bad += expect_error("apsmatch:args", 3, 6, in); }                                                      // not n x n
+  { const mxArray* in[] = {cell_of(1, 2, {kp1, cell_of(1, 2, {k1, k2})}), mms, six, md, cf, it};
+    bad += expect_error("apsmatch:args", 3, 6, in); }                                                      // keypoints != n
+  { const mxArray* in[] = {kps, mms, six, md, cf, mxCreateString("500")}; bad += expect_error("apsmatch:args", 3, 6, in); }
+  if (gpu) {
+    {  // a match index outside the keypoints of set 2 fails the whole call (the library checks it on the host, but the
+       // gateway creates its context first)
+      mxArray* m12b = mxCreateDoubleMatrix(N, 2, mxREAL);
+      for (int r = 0; r < 2 * N; ++r) mxGetPr(m12b)[r] = mxGetPr(m12)[r];
+      mxGetPr(m12b)[3] = N + 1;
+      const mxArray* in[] = {cell_of(1, 2, {cell_of(1, 1, {k1}), kp1}),
+                             cell_of(1, 2, {mxCreateCellMatrix(1, 1), cell_of(2, 2, {nullptr, nullptr, m12b, nullptr})}),
+                             six, md, cf, it};
+      bad += expect_error("refineMatch:MatchIndexOutOfBounds", 3, 6, in);
+    }
+    mxArray* out[3] = {nullptr, nullptr, nullptr};
+    const mxArray* in[] = {kps, mms, six, md, cf, it};
+    mexFunction(3, out, 6, in);
+    const mxArray* a12 = mxGetCell(mxGetCell(out[0], 0), 2);
+    const mxArray* t12 = mxGetCell(mxGetCell(out[2], 0), 2);
+    bad += !(mxGetN(out[0]) == 2 && a12 && mxGetM(a12) == 30 && mxGetPr(mxGetCell(out[1], 0))[2] == 30.0);
+    if (t12) {  // model maps image 2 keypoints to image 1: translation (+10, -5); column-major 3x3
+      const double* t = mxGetPr(t12);
+      bad += !(std::fabs(t[6] / t[8] - 10.0) < 1e-6 && std::fabs(t[7] / t[8] + 5.0) < 1e-6);
+    } else {
+      ++bad;
+    }
+    bad += !(mxGetM(mxGetCell(out[0], 1)) == 1 && mxGetCell(mxGetCell(out[0], 1), 0) == nullptr);
+  } else {
+    const mxArray* in[] = {kps, mms, six, md, cf, it};
     bad += expect_error("apsmatch:nogpu", 3, 6, in);  // no CPU fallback
   }
 #elif defined(GATE_MATCHF)
