@@ -1,6 +1,7 @@
 // aps_abi.cu -- the extern "C" surface declared in include/apsmatch.h: argument checks with the
 // reference's error identifiers, host<->device staging, and the kernel pipelines.
 // No CPU compute path exists here: without a CUDA device every entry fails with APS_ERR_NOGPU.
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <limits>
@@ -971,29 +972,15 @@ extern "C" int aps_feature_matching_global_dev(aps_ctx* c, const void* d_pooled,
 }
 
 // ------------------------------------------------------------------------------------------------
-// imageMatching.m:75-100
+// imageMatching.m:75-100: the one-set case of aps_select_partners_sets (pairs_lin may be NULL here)
 extern "C" int aps_select_partners(aps_ctx* c, const int64_t* counts, int n, int m, uint8_t* cand,
                                    int64_t* pairs_lin, int64_t* npairs) {
   APS_CTX(c);
   if (n < 0 || (n > 0 && (!counts || !cand))) APS_FAIL(APS_ERR_ARGS, "", "bad arguments");
-  if (npairs) *npairs = 0;
-  if (n == 0) return APS_OK;
-  const size_t cells = (size_t)n * n;
-  DevBuf<int64_t> dc;
-  DevBuf<uint8_t> dcand;
-  APS_TRY(dc.alloc(cells, c->stream));
-  APS_TRY(dcand.alloc(cells, c->stream));
-  APS_CUDA(cudaMemcpyAsync(dc.p, counts, cells * 8, cudaMemcpyHostToDevice, c->stream));
-  APS_TRY(aps_k_select_partners(c->stream, dc.p, n, m, dcand.p));
-  APS_CUDA(cudaMemcpyAsync(cand, dcand.p, cells, cudaMemcpyDeviceToHost, c->stream));
-  APS_CUDA(cudaStreamSynchronize(c->stream));
-  int64_t np = 0;
-  for (size_t i = 0; i < cells; ++i)  // find(): ascending linear index (imageMatching.m:99)
-    if (cand[i]) {
-      if (pairs_lin) pairs_lin[np] = (int64_t)i;
-      ++np;
-    }
-  if (npairs) *npairs = np;
+  std::vector<int64_t> scratch(pairs_lin ? 0 : (size_t)n * (n - 1) / 2 + 1);
+  int64_t set_pair_ptr[2] = {0, 0};
+  APS_TRY(aps_select_partners_sets(c, 1, &n, counts, m, cand, pairs_lin ? pairs_lin : scratch.data(), set_pair_ptr));
+  if (npairs) *npairs = set_pair_ptr[1];
   return APS_OK;
 }
 
@@ -1001,16 +988,15 @@ extern "C" int aps_select_partners(aps_ctx* c, const int64_t* counts, int n, int
 // device-side find(), one download, whatever nsets
 extern "C" int aps_select_partners_sets(aps_ctx* c, int nsets, const int* set_images, const int64_t* counts, int m,
                                         uint8_t* cand, int64_t* pairs_lin, int64_t* set_pair_ptr) {
-  if (nsets < 0 || (nsets > 0 && !set_images) || !set_pair_ptr) APS_FAIL(APS_ERR_ARGS, "", "bad set list");
-  int64_t rows = 0, cells = 0, pair_cap = 0;
+  std::vector<int64_t> img0;
+  APS_TRY(sets_image_offsets(nsets, set_images, img0));
+  if (!set_pair_ptr) APS_FAIL(APS_ERR_ARGS, "", "set_pair_ptr is NULL");
+  int64_t cells = 0, pair_cap = 0;
   for (int b = 0; b < nsets; ++b) {
     const int64_t n = set_images[b];
-    if (n < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d: negative image count", b + 1);
-    rows += n;
     cells += n * n;
     pair_cap += n * (n - 1) / 2;
   }
-  if (rows > INT32_MAX) APS_FAIL(APS_ERR_ARGS, "", "more than 2^31 - 1 images");
   if (cells > 0 && (!counts || !cand || !pairs_lin)) APS_FAIL(APS_ERR_ARGS, "", "NULL argument");
   APS_CTX(c);
   for (int b = 0; b <= nsets; ++b) set_pair_ptr[b] = 0;
@@ -1018,11 +1004,9 @@ extern "C" int aps_select_partners_sets(aps_ctx* c, int nsets, const int* set_im
   // host / device layout [set_img | cell_off (nsets + 1 each) | counts (cells)], results [set_pair_ptr | pairs_lin | cand]
   const size_t nt = (size_t)nsets + 1, in_words = 2 * nt + (size_t)cells, out_words = nt + (size_t)pair_cap;
   std::vector<int64_t> in(in_words);
-  in[0] = in[nt] = 0;
-  for (int b = 0; b < nsets; ++b) {
-    in[b + 1] = in[b] + set_images[b];
-    in[nt + b + 1] = in[nt + b] + (int64_t)set_images[b] * set_images[b];
-  }
+  std::copy(img0.begin(), img0.end(), in.begin());
+  in[nt] = 0;
+  for (int b = 0; b < nsets; ++b) in[nt + b + 1] = in[nt + b] + (int64_t)set_images[b] * set_images[b];
   std::memcpy(in.data() + 2 * nt, counts, (size_t)cells * 8);
   cudaStream_t s = c->stream;
   DevBuf<int64_t> din, dout;
@@ -1032,7 +1016,7 @@ extern "C" int aps_select_partners_sets(aps_ctx* c, int nsets, const int* set_im
   uint8_t* h = (uint8_t*)aps_ctx_stage(c, out_words * 8 + (size_t)cells);
   if (!h) APS_FAIL(APS_ERR_ALLOC, "", "pinned staging allocation failed");
   APS_CUDA(cudaMemcpyAsync(din.p, in.data(), in_words * 8, cudaMemcpyHostToDevice, s));
-  APS_TRY(aps_k_select_partners_sets(s, din.p + 2 * nt, (int)rows, cells, din.p, din.p + nt, nsets, m, dcand));
+  APS_TRY(aps_k_select_partners_sets(s, din.p + 2 * nt, (int)img0[nsets], cells, din.p, din.p + nt, nsets, m, dcand));
   APS_TRY(aps_k_select_compact(s, dcand, cells, din.p + nt, nsets, dout.p + nt, dout.p));
   APS_CUDA(cudaMemcpyAsync(h, dout.p, out_words * 8 + (size_t)cells, cudaMemcpyDeviceToHost, s));
   APS_CUDA(cudaStreamSynchronize(s));  // `in` stays alive until here

@@ -97,7 +97,16 @@ int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const in
                                    int layout, double match_threshold, double max_ratio, int method, int64_t subset,
                                    uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out);
 
-// ---- pooled upload of many images (aps_abi_sets.cu; the sets entries) ---------------------------------------------
+// ---- lists of image sets and pooled upload of many images (aps_abi_sets.cu; the sets entries) ---------------------
+// Checks the set list of a sets entry (nsets >= 0, set_images[b] >= 0, at most INT_MAX images in all) and returns
+// img0 [nsets + 1], the first pooled image of each set.  Messages number the sets from 1.
+int sets_image_offsets(int nsets, const int* set_images, std::vector<int64_t>& img0);
+// Splits a pooled match list whose cells are nsets column-major blocks (block j: cells [cell_off[j], cell_off[j + 1])
+// of an n[j] x n[j] matrix) into one list per block, stored in out[slot[j]] (out[j] when slot is NULL).  metric: the
+// pooled metric, or NULL for lists without one.
+int sets_split_lists(int nsets, const std::vector<int64_t>& pair_ptr, const std::vector<uint32_t>& rows,
+                     const std::vector<double>* metric, const std::vector<int64_t>& cell_off, const int* n,
+                     const int* slot, aps_matchlist** out);
 // img[r] = image of pooled row r (d_off: [nimg + 1] row offsets on the device)
 int sets_img_of_row(cudaStream_t s, const int64_t* d_off, int nimg, int64_t F, int32_t* img);
 // H2D of image i (host ptrs[i], off[i + 1] - off[i] rows) to rows [off[i], off[i + 1]) of the pooled row-major matrix

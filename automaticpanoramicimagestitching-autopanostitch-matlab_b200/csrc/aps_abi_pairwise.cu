@@ -1125,22 +1125,8 @@ static int pairwise_sets_pass(aps_ctx* c, int nsets, const int* set_images, cons
     APS_TRY(pairwise_match_pairs(c, ps, counts, D, dtype, method, match_threshold, max_ratio, pairs, cell,
                                  cell_off[nsets], &pooled));
   }
-  // split into one list per set: cells [cell_off[b], cell_off[b + 1]], rows from pair_ptr[cell_off[b]]
-  const std::vector<int64_t>& pp = pooled.pair_ptr;
-  for (int b = 0; b < nsets; ++b) {
-    aps_matchlist* m = new (std::nothrow) aps_matchlist();
-    if (!m) APS_FAIL(APS_ERR_ALLOC, "", "out of host memory");
-    out[b] = m;
-    m->n = set_images[b];
-    m->has_metric = true;
-    const int64_t c0 = cell_off[b], c1 = cell_off[(size_t)b + 1], r0 = pp[c0];
-    m->pair_ptr.resize((size_t)(c1 - c0) + 1);
-    for (int64_t q = c0; q <= c1; ++q) m->pair_ptr[(size_t)(q - c0)] = pp[q] - r0;
-    m->total = pp[c1] - r0;
-    m->rows.assign(pooled.rows.begin() + 2 * r0, pooled.rows.begin() + 2 * pp[c1]);
-    m->metric.assign(pooled.metric.begin() + r0, pooled.metric.begin() + pp[c1]);
-  }
-  return APS_OK;
+  // one list per set: cells [cell_off[b], cell_off[b + 1]], rows from pair_ptr[cell_off[b]]
+  return sets_split_lists(nsets, pooled.pair_ptr, pooled.rows, &pooled.metric, cell_off, set_images, nullptr, out);
 }
 
 extern "C" int aps_feature_matching_pairwise_sets(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
@@ -1148,16 +1134,11 @@ extern "C" int aps_feature_matching_pairwise_sets(aps_ctx* c, int nsets, const i
                                                   double match_threshold, double max_ratio, int method, int64_t subset,
                                                   uint64_t seed, aps_matchlist** out) {
   // arguments first (the statuses of the single-set call), then the device
-  if (nsets < 0) APS_FAIL(APS_ERR_ARGS, "", "nsets must be >= 0 (got %d)", nsets);
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
-  if (nsets > 0 && !set_images) APS_FAIL(APS_ERR_ARGS, "", "set_images is NULL");
   for (int b = 0; b < nsets; ++b) out[b] = nullptr;
-  int64_t nimg = 0;
-  for (int b = 0; b < nsets; ++b) {
-    if (set_images[b] < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d has a negative image count", b);
-    nimg += set_images[b];
-  }
-  if (nimg > INT_MAX) APS_FAIL(APS_ERR_ARGS, "", "too many images");
+  std::vector<int64_t> img_first;
+  APS_TRY(sets_image_offsets(nsets, set_images, img_first));
+  const int64_t nimg = img_first[nsets];
   if (nimg > 0 && !counts) APS_FAIL(APS_ERR_ARGS, "", "counts is NULL");
   if (dtype != APS_F32 && dtype != APS_U8) APS_FAIL(APS_ERR_TYPE, "", "descriptors must be single or uint8");
   if (method < APS_METHOD_EXHAUSTIVE || method > APS_METHOD_APPROX_PCA2NN)

@@ -88,6 +88,39 @@ int sets_upload(aps_ctx* c, const void* const* ptrs, const std::vector<int64_t>&
   return APS_OK;
 }
 
+int sets_image_offsets(int nsets, const int* set_images, std::vector<int64_t>& img0) {
+  if (nsets < 0) APS_FAIL(APS_ERR_ARGS, "", "nsets must be >= 0 (got %d)", nsets);
+  if (nsets > 0 && !set_images) APS_FAIL(APS_ERR_ARGS, "", "set_images is NULL");
+  img0.assign((size_t)nsets + 1, 0);
+  for (int b = 0; b < nsets; ++b) {
+    if (set_images[b] < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d has a negative image count", b + 1);
+    img0[b + 1] = img0[b] + set_images[b];
+  }
+  if (img0[nsets] > INT_MAX) APS_FAIL(APS_ERR_ARGS, "", "more than 2^31 - 1 images");
+  return APS_OK;
+}
+
+int sets_split_lists(int nsets, const std::vector<int64_t>& pair_ptr, const std::vector<uint32_t>& rows,
+                     const std::vector<double>* metric, const std::vector<int64_t>& cell_off, const int* n,
+                     const int* slot, aps_matchlist** out) {
+  for (int j = 0; j < nsets; ++j) {
+    aps_matchlist* m = new (std::nothrow) aps_matchlist();
+    if (!m) APS_FAIL(APS_ERR_ALLOC, "", "out of host memory");
+    out[slot ? slot[j] : j] = m;
+    m->n = n[j];
+    const int64_t c0 = cell_off[j], c1 = cell_off[j + 1], r0 = pair_ptr[c0], r1 = pair_ptr[c1];
+    m->pair_ptr.resize((size_t)(c1 - c0) + 1);
+    for (int64_t c = c0; c <= c1; ++c) m->pair_ptr[(size_t)(c - c0)] = pair_ptr[c] - r0;
+    m->total = r1 - r0;
+    m->rows.assign(rows.begin() + 2 * r0, rows.begin() + 2 * r1);
+    if (metric) {
+      m->has_metric = true;
+      m->metric.assign(metric->begin() + r0, metric->begin() + r1);
+    }
+  }
+  return APS_OK;
+}
+
 namespace {
 
 // rows the tensor pass could not prove -> one K2f group each, searched against its own set's rows (device-side list)
@@ -295,18 +328,8 @@ int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std
       APS_CUDA(cudaStreamSynchronize(s));
     }
   }
-  // split into one list per set (cells of set j: [cell_off[j], cell_off[j + 1]], rows from pp[cell_off[j]])
-  for (int j = 0; j < nsets; ++j) {
-    aps_matchlist* m = new (std::nothrow) aps_matchlist();
-    if (!m) APS_FAIL(APS_ERR_ALLOC, "", "out of host memory");
-    out[sets[j]] = m;
-    m->n = set_n[j];
-    const int64_t c0 = cell_off[j], c1 = cell_off[j + 1], r0 = pp[c0];
-    m->pair_ptr.resize((size_t)(c1 - c0) + 1);
-    for (int64_t cc = c0; cc <= c1; ++cc) m->pair_ptr[(size_t)(cc - c0)] = pp[cc] - r0;
-    m->total = pp[c1] - r0;
-    m->rows.assign(rows_h.begin() + 2 * r0, rows_h.begin() + 2 * pp[c1]);
-  }
+  // one list per set (cells of set j: [cell_off[j], cell_off[j + 1]], rows from pp[cell_off[j]])
+  APS_TRY(sets_split_lists(nsets, pp, rows_h, nullptr, cell_off, set_n.data(), sets.data(), out));
   // statistics of the call, as the single-set call reports them: rows searched; the engine (tcgen05 when any set took
   // the tensor path); rows its proof left to K2f (no second tensor pass here: first-pass unproven == fallback rows);
   // operands exact for every float row
@@ -326,17 +349,11 @@ extern "C" int aps_feature_matching_global_sets(aps_ctx* c, int nsets, const int
                                                 double ratio, int use_bf, int mutual, aps_matchlist** out) {
   (void)use_bf;
   // arguments first (the ids of aps_feature_matching_global), then the device
-  if (nsets < 0) APS_FAIL(APS_ERR_ARGS, "", "nsets must be >= 0 (got %d)", nsets);
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
-  if (nsets > 0 && !set_images) APS_FAIL(APS_ERR_ARGS, "", "set_images is NULL");
   for (int b = 0; b < nsets; ++b) out[b] = nullptr;
-  std::vector<int64_t> img_first((size_t)nsets + 1, 0);
-  for (int b = 0; b < nsets; ++b) {
-    if (set_images[b] < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d has a negative image count", b);
-    img_first[b + 1] = img_first[b] + set_images[b];
-  }
+  std::vector<int64_t> img_first;
+  APS_TRY(sets_image_offsets(nsets, set_images, img_first));
   const int64_t nimg = img_first[nsets];
-  if (nimg > INT_MAX) APS_FAIL(APS_ERR_ARGS, "", "too many images");
   if (nimg > 0 && !counts) APS_FAIL(APS_ERR_ARGS, "", "counts is NULL");
   std::vector<int64_t> set_rows((size_t)nsets, 0);
   int64_t F = 0;

@@ -314,9 +314,7 @@ int aps_k_pair_filter_unique(cudaStream_t s, const uint32_t* idx2, const float* 
                              int unique, unsigned long long* best_by_train /*N2*/, unsigned long long* keys /*2*N1*/,
                              int32_t* count_dev, uint32_t* matches /*2*N1*/, double* metric /*N1*/);
 
-// K6 aps_select.cu
-int aps_k_select_partners(cudaStream_t s, const int64_t* counts_cm, int n, int m, uint8_t* cand_cm);
-// the same for nsets image sets: n_rows = sum n_b pooled images, set_img / cell_off [nsets + 1] = first pooled image and
+// K6 (aps_filter.cu): top-m partner selection of nsets image sets: n_rows = sum n_b pooled images, set_img / cell_off [nsets + 1] = first pooled image and
 // first cell of each set's n_b x n_b column-major block (cells = cell_off[nsets])
 int aps_k_select_partners_sets(cudaStream_t s, const int64_t* counts, int n_rows, int64_t cells, const int64_t* set_img,
                                const int64_t* cell_off, int nsets, int m, uint8_t* cand);

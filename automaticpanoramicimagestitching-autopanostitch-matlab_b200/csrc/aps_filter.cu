@@ -548,7 +548,7 @@ int aps_k_pair_filter_unique(cudaStream_t s, const uint32_t* idx2, const float* 
 
 // ------------------------------------------------------------------------------------------------
 // K6  imageMatching.m:75-100 for every image set of a call.  Set b owns pooled images [set_img[b], set_img[b + 1]) and
-// the n_b x n_b column-major block of cells at cell_off[b] (both tables [nsets + 1]); NULL tables = one set of n images.
+// the n_b x n_b column-major block of cells at cell_off[b] (both tables [nsets + 1]).
 // Stable descending order == rank by (value desc, column asc).
 struct SelectSet {
   int64_t img0, cell0;
@@ -564,16 +564,15 @@ __device__ __forceinline__ int select_set_of(const int64_t* __restrict__ tab, in
   return lo;
 }
 __device__ __forceinline__ SelectSet select_set(const int64_t* __restrict__ set_img, const int64_t* __restrict__ cell_off,
-                                                int nsets, int n, const int64_t* __restrict__ tab, int64_t x) {
-  if (!set_img) return SelectSet{0, 0, n};
+                                                int nsets, const int64_t* __restrict__ tab, int64_t x) {
   const int b = select_set_of(tab, nsets, x);
   return SelectSet{set_img[b], cell_off[b], (int)(set_img[b + 1] - set_img[b])};
 }
 
 // one CTA per pooled image row: that row's partners ranked inside its own set's block
-__global__ void k_select_rows(const int64_t* __restrict__ counts, int n, const int64_t* __restrict__ set_img,
+__global__ void k_select_rows(const int64_t* __restrict__ counts, const int64_t* __restrict__ set_img,
                               const int64_t* __restrict__ cell_off, int nsets, int m, uint8_t* __restrict__ P) {
-  const SelectSet S = select_set(set_img, cell_off, nsets, n, set_img, blockIdx.x);
+  const SelectSet S = select_set(set_img, cell_off, nsets, set_img, blockIdx.x);
   const int i = (int)(blockIdx.x - S.img0), nb = S.n;
   const int take = m < nb - 1 ? (m < 0 ? 0 : m) : nb - 1;
   const int64_t* C = counts + S.cell0;
@@ -587,11 +586,11 @@ __global__ void k_select_rows(const int64_t* __restrict__ counts, int n, const i
     P[S.cell0 + i + (int64_t)j * nb] = r < take;  // :86-91
   }
 }
-__global__ void k_select_sym(const uint8_t* __restrict__ P, int n, const int64_t* __restrict__ set_img,
+__global__ void k_select_sym(const uint8_t* __restrict__ P, const int64_t* __restrict__ set_img,
                              const int64_t* __restrict__ cell_off, int nsets, int64_t cells, uint8_t* __restrict__ cand) {
   int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= cells) return;
-  const SelectSet S = select_set(set_img, cell_off, nsets, n, cell_off, c);
+  const SelectSet S = select_set(set_img, cell_off, nsets, cell_off, c);
   const int64_t l = c - S.cell0;
   const int i = (int)(l % S.n), j = (int)(l / S.n);
   cand[c] = (i < j) && (P[S.cell0 + i + (int64_t)j * S.n] || P[S.cell0 + j + (int64_t)i * S.n]);  // :94-96
@@ -638,15 +637,11 @@ int aps_k_select_partners_sets(cudaStream_t s, const int64_t* counts, int n_rows
   if (n_rows == 0) return APS_OK;
   DevBuf<uint8_t> P;
   APS_TRY(P.alloc((size_t)cells, s));
-  k_select_rows<<<n_rows, 128, 0, s>>>(counts, n_rows, set_img, cell_off, nsets, m, P.p);
+  k_select_rows<<<n_rows, 128, 0, s>>>(counts, set_img, cell_off, nsets, m, P.p);
   APS_LAUNCHED();
-  k_select_sym<<<(unsigned)aps_ceil_div(cells, 256), 256, 0, s>>>(P.p, n_rows, set_img, cell_off, nsets, cells, cand);
+  k_select_sym<<<(unsigned)aps_ceil_div(cells, 256), 256, 0, s>>>(P.p, set_img, cell_off, nsets, cells, cand);
   APS_LAUNCHED();
   return APS_OK;
-}
-
-int aps_k_select_partners(cudaStream_t s, const int64_t* counts_cm, int n, int m, uint8_t* cand_cm) {
-  return aps_k_select_partners_sets(s, counts_cm, n, (int64_t)n * n, nullptr, nullptr, 1, m, cand_cm);
 }
 
 int aps_k_select_compact(cudaStream_t s, const uint8_t* cand, int64_t cells, const int64_t* cell_off, int nsets,

@@ -27,15 +27,7 @@
 // correspondence read by every thread of a pair at the same time (broadcast from L1).
 #include <math_constants.h>
 
-#include "aps_common.cuh"
-
-#ifndef APS_FAIL
-#define APS_FAIL(code, id, ...)           \
-  do {                                    \
-    aps_set_error(code, id, __VA_ARGS__); \
-    return code;                          \
-  } while (0)
-#endif
+#include "aps_abi_internal.cuh"
 
 namespace {
 
@@ -722,6 +714,8 @@ extern "C" int aps_image_matching_batch(aps_ctx* c, int64_t n_pairs, const int64
   return APS_OK;
 }
 
+// The one-set case of aps_image_matching_sets.  What differs is the front: the context is checked first, a call without
+// pairs succeeds whatever the RANSAC parameters, and one call takes at most 65535 pairs (DESIGN.md).
 extern "C" int aps_image_matching(aps_ctx* c, int n_images, const int64_t* pair_ptr, const uint32_t* rows,
                                   const double* keypoints, const int64_t* img_off, const int64_t* pairs_lin,
                                   int64_t n_pairs, double max_distance, double confidence, int max_trials,
@@ -729,82 +723,13 @@ extern "C" int aps_image_matching(aps_ctx* c, int n_images, const int64_t* pair_
                                   double* models, double* models_inv, uint8_t* inliers, int32_t* n_inliers,
                                   uint8_t* accepted, int32_t* draws_used) {
   if (!c) APS_FAIL(APS_ERR_NOGPU, "apsmatch:nogpu", "context is NULL (no GPU context; there is no CPU path)");
-  if (n_images < 0 || n_pairs < 0 || (n_pairs > 0 && (!pair_ptr || !pairs_lin || !img_off || !pt_ptr_out)))
-    APS_FAIL(APS_ERR_ARGS, "", "bad arguments");
+  if (n_images < 0 || n_pairs < 0) APS_FAIL(APS_ERR_ARGS, "", "bad arguments");
   if (n_pairs == 0) return APS_OK;
-  std::vector<int64_t> ptr((size_t)n_pairs + 1, 0);
-  std::vector<int32_t> ii((size_t)n_pairs), jj((size_t)n_pairs);
-  for (int64_t p = 0; p < n_pairs; ++p) {
-    const int64_t lin = pairs_lin[p];
-    if (lin < 0 || lin >= (int64_t)n_images * n_images) APS_FAIL(APS_ERR_ARGS, "", "pair index out of range");
-    ii[p] = (int32_t)(lin % n_images);
-    jj[p] = (int32_t)(lin / n_images);
-    ptr[p + 1] = ptr[p] + (pair_ptr[lin + 1] - pair_ptr[lin]);
-  }
-  for (int64_t p = 0; p <= n_pairs; ++p) pt_ptr_out[p] = ptr[p];
-  APS_TRY(ransac_args(c, n_pairs, ptr.data(), n_draws, max_trials, confidence));
-  APS_CUDA(cudaSetDevice(c->device));
-  const int64_t total = ptr[n_pairs], F = img_off[n_images];
-  if ((total > 0 && (!rows || !keypoints || !inliers)) || !models || !models_inv || !n_inliers || !accepted || !draws_used)
-    APS_FAIL(APS_ERR_ARGS, "", "NULL argument");
-  std::vector<uint32_t> crow((size_t)(2 * total));
-  for (int64_t p = 0; p < n_pairs; ++p) {  // refineMatch:214-221: indices must lie inside the keypoint arrays
-    const int64_t lin = pairs_lin[p], a = pair_ptr[lin], cntp = ptr[p + 1] - ptr[p];
-    const int64_t ni = img_off[ii[p] + 1] - img_off[ii[p]], nj = img_off[jj[p] + 1] - img_off[jj[p]];
-    for (int64_t r = 0; r < cntp; ++r) {
-      const uint32_t ra = rows[2 * (a + r)], rb = rows[2 * (a + r) + 1];
-      if (ra < 1 || rb < 1 || (int64_t)ra > ni || (int64_t)rb > nj)
-        APS_FAIL(APS_ERR_ARGS, "refineMatch:MatchIndexOutOfBounds", "Match indices exceed keypoint array sizes.");
-      crow[2 * (ptr[p] + r)] = ra;
-      crow[2 * (ptr[p] + r) + 1] = rb;
-    }
-  }
-  cudaStream_t s = c->stream;
-  DevBuf<int64_t> dptr, doff;
-  DevBuf<int32_t> dii, djj, dni, dused;
-  DevBuf<uint32_t> drows, ds;
-  DevBuf<double2> dkp, dp1, dp2;
-  DevBuf<double> dm, dmi;
-  DevBuf<uint8_t> dinl, dacc;
-  const size_t tot = (size_t)(total > 0 ? total : 1);
-  APS_TRY(dptr.alloc((size_t)n_pairs + 1, s));
-  APS_TRY(doff.alloc((size_t)n_images + 1, s));
-  APS_TRY(dii.alloc((size_t)n_pairs, s));
-  APS_TRY(djj.alloc((size_t)n_pairs, s));
-  APS_TRY(drows.alloc(2 * tot, s));
-  APS_TRY(dkp.alloc((size_t)(F > 0 ? F : 1), s));
-  APS_TRY(dp1.alloc(tot, s));
-  APS_TRY(dp2.alloc(tot, s));
-  APS_TRY(ds.alloc((size_t)(n_pairs * n_draws * 4), s));
-  APS_TRY(dm.alloc((size_t)n_pairs * 9, s));
-  APS_TRY(dmi.alloc((size_t)n_pairs * 9, s));
-  APS_TRY(dinl.alloc(tot, s));
-  APS_TRY(dacc.alloc((size_t)n_pairs, s));
-  APS_TRY(dni.alloc((size_t)n_pairs, s));
-  APS_TRY(dused.alloc((size_t)n_pairs, s));
-  APS_CUDA(cudaMemcpyAsync(dptr.p, ptr.data(), (size_t)(n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
-  APS_CUDA(cudaMemcpyAsync(doff.p, img_off, (size_t)(n_images + 1) * 8, cudaMemcpyHostToDevice, s));
-  APS_CUDA(cudaMemcpyAsync(dii.p, ii.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
-  APS_CUDA(cudaMemcpyAsync(djj.p, jj.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
-  if (total > 0) {
-    APS_CUDA(cudaMemcpyAsync(drows.p, crow.data(), (size_t)total * 8, cudaMemcpyHostToDevice, s));
-    APS_CUDA(cudaMemcpyAsync(dkp.p, keypoints, (size_t)F * 16, cudaMemcpyHostToDevice, s));
-    k_gather_matched_points<<<dim3(8, (unsigned)n_pairs), 256, 0, s>>>(dptr.p, drows.p, dii.p, djj.p, doff.p, dkp.p,
-                                                                       dp1.p, dp2.p);
-    APS_LAUNCHED();
-  }
-  if (samples)
-    APS_CUDA(cudaMemcpyAsync(ds.p, samples, (size_t)(n_pairs * n_draws * 4) * 4, cudaMemcpyHostToDevice, s));
-  APS_TRY(ransac_device(c, n_pairs, total, dptr.p, dp1.p, dp2.p, ds.p, samples != nullptr, nullptr, n_draws, seed,
-                        max_distance, confidence, max_trials, dm.p, dmi.p, dinl.p, dni.p, dacc.p, dused.p));
-  APS_CUDA(cudaMemcpyAsync(models, dm.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
-  APS_CUDA(cudaMemcpyAsync(models_inv, dmi.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
-  if (total > 0) APS_CUDA(cudaMemcpyAsync(inliers, dinl.p, (size_t)total, cudaMemcpyDeviceToHost, s));
-  APS_CUDA(cudaMemcpyAsync(n_inliers, dni.p, (size_t)n_pairs * 4, cudaMemcpyDeviceToHost, s));
-  APS_CUDA(cudaMemcpyAsync(accepted, dacc.p, (size_t)n_pairs, cudaMemcpyDeviceToHost, s));
-  APS_CUDA(cudaMemcpyAsync(draws_used, dused.p, (size_t)n_pairs * 4, cudaMemcpyDeviceToHost, s));
-  APS_CUDA(cudaStreamSynchronize(s));  // crow / ptr / ii / jj stay alive until here
-  return APS_OK;
+  if (n_pairs > 65535) APS_FAIL(APS_ERR_ARGS, "", "at most 65535 candidate pairs per call");
+  const int64_t set_pair_ptr[2] = {0, n_pairs};
+  return aps_image_matching_sets(c, 1, &n_images, &pair_ptr, &rows, keypoints, img_off, set_pair_ptr, pairs_lin,
+                                 max_distance, confidence, max_trials, samples, n_draws, seed, pt_ptr_out, models,
+                                 models_inv, inliers, n_inliers, accepted, draws_used);
 }
 
 // imageMatching.m:121-156 for every candidate pair of nsets image sets.  Set b's pairs are
@@ -822,13 +747,11 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
                                        double confidence, int max_trials, const uint32_t* samples, int64_t n_draws,
                                        uint64_t seed, int64_t* pt_ptr_out, double* models, double* models_inv,
                                        uint8_t* inliers, int32_t* n_inliers, uint8_t* accepted, int32_t* draws_used) {
-  if (nsets < 0 || (nsets > 0 && (!set_images || !set_pair_ptr))) APS_FAIL(APS_ERR_ARGS, "", "bad set list");
-  std::vector<int64_t> img0((size_t)nsets + 1, 0);
-  for (int b = 0; b < nsets; ++b) {
-    if (set_images[b] < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d: negative image count", b + 1);
-    img0[b + 1] = img0[b] + set_images[b];
-  }
-  if (img0[nsets] > INT32_MAX) APS_FAIL(APS_ERR_ARGS, "", "more than 2^31 - 1 images");
+  std::vector<int64_t> img0;
+  APS_TRY(sets_image_offsets(nsets, set_images, img0));
+  if (nsets > 0 && !set_pair_ptr) APS_FAIL(APS_ERR_ARGS, "", "set_pair_ptr is NULL");
+  // messages name the set only when there are several (one set: the messages of aps_image_matching)
+  auto in_set = [nsets](int b) { return nsets > 1 ? " (set " + std::to_string(b + 1) + ")" : std::string(); };
   if (nsets > 0 && set_pair_ptr[0] != 0) APS_FAIL(APS_ERR_ARGS, "", "set_pair_ptr[0] must be 0");
   for (int b = 0; b < nsets; ++b)
     if (set_pair_ptr[b + 1] < set_pair_ptr[b]) APS_FAIL(APS_ERR_ARGS, "", "set_pair_ptr must be non-decreasing");
@@ -843,9 +766,10 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
     const int64_t n = set_images[b];
     for (int64_t p = set_pair_ptr[b]; p < set_pair_ptr[b + 1]; ++p) {
       const int64_t lin = pairs_lin[p];
-      if (!pair_ptr[b] || lin < 0 || lin >= n * n) APS_FAIL(APS_ERR_ARGS, "", "set %d: pair index out of range", b + 1);
+      if (!pair_ptr[b] || lin < 0 || lin >= n * n)
+        APS_FAIL(APS_ERR_ARGS, "", "pair index out of range%s", in_set(b).c_str());
       const int64_t cnt = pair_ptr[b][lin + 1] - pair_ptr[b][lin];
-      if (cnt < 0) APS_FAIL(APS_ERR_ARGS, "", "set %d: pair_ptr must be non-decreasing", b + 1);
+      if (cnt < 0) APS_FAIL(APS_ERR_ARGS, "", "pair_ptr must be non-decreasing%s", in_set(b).c_str());
       ii[p] = (int32_t)(img0[b] + lin % n);
       jj[p] = (int32_t)(img0[b] + lin / n);
       keys[p] = p - set_pair_ptr[b];
@@ -859,12 +783,12 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
     for (int64_t p = set_pair_ptr[b]; p < set_pair_ptr[b + 1]; ++p) {  // refineMatch:214-221
       const int64_t a = pair_ptr[b][pairs_lin[p]], cntp = ptr[p + 1] - ptr[p];
       const int64_t ni = img_off[ii[p] + 1] - img_off[ii[p]], nj = img_off[jj[p] + 1] - img_off[jj[p]];
-      if (cntp > 0 && !rows[b]) APS_FAIL(APS_ERR_ARGS, "", "set %d: rows is NULL", b + 1);
+      if (cntp > 0 && !rows[b]) APS_FAIL(APS_ERR_ARGS, "", "rows is NULL%s", in_set(b).c_str());
       for (int64_t r = 0; r < cntp; ++r) {
         const uint32_t ra = rows[b][2 * (a + r)], rb = rows[b][2 * (a + r) + 1];
         if (ra < 1 || rb < 1 || (int64_t)ra > ni || (int64_t)rb > nj)
           APS_FAIL(APS_ERR_ARGS, "refineMatch:MatchIndexOutOfBounds",
-                   "Match indices exceed keypoint array sizes (set %d).", b + 1);
+                   "Match indices exceed keypoint array sizes%s.", in_set(b).c_str());
         crow[2 * (ptr[p] + r)] = ra;
         crow[2 * (ptr[p] + r) + 1] = rb;
       }
@@ -876,6 +800,8 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
   if (n_pairs == 0) return APS_OK;
   const int64_t by_bytes = kSetsChunkBytes / (n_draws * kSetsDrawBytes);
   const int64_t chunk = aps_min64(65535, by_bytes > 0 ? by_bytes : 1);
+  // one set in one chunk: keys[p] == p, which is what k_ransac_samples takes a NULL key table to mean
+  const bool keyed = nsets > 1 || n_pairs > chunk;
   cudaStream_t s = c->stream;
   DevBuf<int64_t> dptr, doff, dkeys;
   DevBuf<int32_t> dii, djj, dni, dused;
@@ -886,7 +812,7 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
   const size_t tot = (size_t)(total > 0 ? total : 1);
   APS_TRY(dptr.alloc((size_t)n_pairs + 1, s));
   APS_TRY(doff.alloc((size_t)G + 1, s));
-  APS_TRY(dkeys.alloc((size_t)n_pairs, s));
+  if (keyed) APS_TRY(dkeys.alloc((size_t)n_pairs, s));
   APS_TRY(dii.alloc((size_t)n_pairs, s));
   APS_TRY(djj.alloc((size_t)n_pairs, s));
   APS_TRY(drows.alloc(2 * tot, s));
@@ -902,7 +828,7 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
   APS_TRY(dused.alloc((size_t)n_pairs, s));
   APS_CUDA(cudaMemcpyAsync(dptr.p, ptr.data(), (size_t)(n_pairs + 1) * 8, cudaMemcpyHostToDevice, s));
   APS_CUDA(cudaMemcpyAsync(doff.p, img_off, (size_t)(G + 1) * 8, cudaMemcpyHostToDevice, s));
-  APS_CUDA(cudaMemcpyAsync(dkeys.p, keys.data(), (size_t)n_pairs * 8, cudaMemcpyHostToDevice, s));
+  if (keyed) APS_CUDA(cudaMemcpyAsync(dkeys.p, keys.data(), (size_t)n_pairs * 8, cudaMemcpyHostToDevice, s));
   APS_CUDA(cudaMemcpyAsync(dii.p, ii.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
   APS_CUDA(cudaMemcpyAsync(djj.p, jj.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, s));
   if (total > 0) {
@@ -919,7 +845,7 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
     if (samples)
       APS_CUDA(cudaMemcpyAsync(ds.p, samples + p0 * n_draws * 4, (size_t)(np * n_draws * 4) * 4, cudaMemcpyHostToDevice,
                                s));
-    APS_TRY(ransac_device(c, np, total, dptr.p + p0, dp1.p, dp2.p, ds.p, samples != nullptr, dkeys.p + p0, n_draws, seed,
+    APS_TRY(ransac_device(c, np, total, dptr.p + p0, dp1.p, dp2.p, ds.p, samples != nullptr, keyed ? dkeys.p + p0 : nullptr, n_draws, seed,
                           max_distance, confidence, max_trials, dm.p + 9 * p0, dmi.p + 9 * p0, dinl.p, dni.p + p0,
                           dacc.p + p0, dused.p + p0));
   }

@@ -209,15 +209,10 @@ def featureMatchingGlobal(input, allDescriptors, numImg, ctx=None):
     return matches
 
 
-def featureMatchingGlobalSets(input, allDescriptorsSets, numImgs, ctx=None):
-    """matchesSets = featureMatchingGlobalSets(input, allDescriptorsSets, numImgs)
-
-    featureMatchingGlobal over B independent image sets in one call (aps_feature_matching_global_sets): set b is
-    allDescriptorsSets[b] with numImgs[b] images.  Returns a list of B nested lists, element b exactly what
-    featureMatchingGlobal(input, allDescriptorsSets[b], numImgs[b]) returns (with input.apsMutual too).  All sets share
-    one descriptor kind (float or binaryFeatures) and width.  Device groups (input.apsGPUs) are not supported here."""
-    if _field(input, "apsGPUs", None) is not None:
-        raise ValueError("input.apsGPUs is not supported by featureMatchingGlobalSets; match the sets on one GPU")
+def _pool_descriptor_sets(allDescriptorsSets, numImgs):
+    """The descriptor sets of a sets call, pooled image after image -> (ns, empty, mats, counts, kind, D): image counts,
+    which sets have no descriptors, pooled matrices and row counts (None / 0 for the images of an empty set), and the
+    one descriptor kind (is_binary, None when every set is empty) and width all sets share."""
     sets = list(allDescriptorsSets) if allDescriptorsSets is not None else []
     nums = list(np.atleast_1d(np.asarray(numImgs, dtype=np.float64)).ravel()) if np.size(numImgs) else []
     if len(nums) != len(sets):
@@ -225,11 +220,7 @@ def featureMatchingGlobalSets(input, allDescriptorsSets, numImgs, ctx=None):
     for v in nums:
         if not (np.isfinite(v) and v > 0 and v == np.round(v)):
             raise ValueError("every numImgs entry must be a positive integer")  # featureMatchingGlobal.m:35-39
-    k = int(_field(input, "k", required=True))
-    ratio = float(_field(input, "Ratiothreshold", required=True))
-    use_bf = bool(_field(input, "BFMatch", 0))
-    mutual = bool(int(_field(input, "apsMutual", 0)))
-    ns, all_mats, all_counts = [], [], []
+    ns, empty, all_mats, all_counts = [], [], [], []
     kind = D = None
     for cells, num in zip(sets, nums):
         n, first, mats, counts, Db, is_binary = _describe(cells, num)
@@ -242,8 +233,26 @@ def featureMatchingGlobalSets(input, allDescriptorsSets, numImgs, ctx=None):
                 raise ApsError(4, "flann_knn:dim", "all descriptor sets must have the same number of columns")
             kind, D = is_binary, Db
         ns.append(n)
+        empty.append(first is None)
         all_mats += mats
         all_counts += counts
+    return ns, empty, all_mats, all_counts, kind, D
+
+
+def featureMatchingGlobalSets(input, allDescriptorsSets, numImgs, ctx=None):
+    """matchesSets = featureMatchingGlobalSets(input, allDescriptorsSets, numImgs)
+
+    featureMatchingGlobal over B independent image sets in one call (aps_feature_matching_global_sets): set b is
+    allDescriptorsSets[b] with numImgs[b] images.  Returns a list of B nested lists, element b exactly what
+    featureMatchingGlobal(input, allDescriptorsSets[b], numImgs[b]) returns (with input.apsMutual too).  All sets share
+    one descriptor kind (float or binaryFeatures) and width.  Device groups (input.apsGPUs) are not supported here."""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by featureMatchingGlobalSets; match the sets on one GPU")
+    ns, _, all_mats, all_counts, kind, D = _pool_descriptor_sets(allDescriptorsSets, numImgs)
+    k = int(_field(input, "k", required=True))
+    ratio = float(_field(input, "Ratiothreshold", required=True))
+    use_bf = bool(_field(input, "BFMatch", 0))
+    mutual = bool(int(_field(input, "apsMutual", 0)))
     B = len(ns)
     if kind is None:  # every set empty: cell(numImg) each, no device touched (featureMatchingGlobal.m:49-52)
         return [[[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)] for n in ns]
@@ -384,35 +393,13 @@ def featureMatchingPairwiseSets(input, allDescriptorsSets, numImgs, ctx=None, re
     or binaryFeatures) and width.  Device groups (input.apsGPUs) are not supported here."""
     if _field(input, "apsGPUs", None) is not None:
         raise ValueError("input.apsGPUs is not supported by featureMatchingPairwiseSets; match the sets on one GPU")
-    sets = list(allDescriptorsSets) if allDescriptorsSets is not None else []
-    nums = list(np.atleast_1d(np.asarray(numImgs, dtype=np.float64)).ravel()) if np.size(numImgs) else []
-    if len(nums) != len(sets):
-        raise ValueError("numImgs must give one image count per descriptor set")
-    for v in nums:
-        if not (np.isfinite(v) and v > 0 and v == np.round(v)):
-            raise ValueError("every numImgs entry must be a positive integer")  # featureMatchingPairwise.m arguments
+    ns, empty, all_mats, all_counts, kind, D = _pool_descriptor_sets(allDescriptorsSets, numImgs)
     method = str(_field(input, "Matchingmethod", "Exhaustive")).lower()
     if method not in ("exhaustive", "approximate"):
         raise ValueError(f"Unknown Method: {method}")  # matchFeaturesScratch.m:164-165
     aps_method = _resolve_method(input, method)
     thr = float(_field(input, "Matchingthreshold", required=True))
     ratio = float(_field(input, "Ratiothreshold", required=True))
-    ns, empty, all_mats, all_counts = [], [], [], []
-    kind = D = None
-    for cells, num in zip(sets, nums):
-        n, first, mats, counts, Db, is_binary = _describe(cells, num)
-        if first is None:
-            mats, counts = [None] * n, [0] * n
-        else:
-            if kind is not None and is_binary != kind:
-                raise ApsError(2, "flann_knn:type", "all descriptor sets must have the same class")
-            if D is not None and Db != D:
-                raise ApsError(4, "flann_knn:dim", "all descriptor sets must have the same number of columns")
-            kind, D = is_binary, Db
-        ns.append(n)
-        empty.append(first is None)
-        all_mats += mats
-        all_counts += counts
 
     def empty_cells(n):   # featureMatchingPairwise on a set without descriptors: cell(numImg), no device touched
         m = [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)]
@@ -745,41 +732,65 @@ def imageMatching(input, n, keypoints, matchesAll, imagesProcessed=None, samples
         raise ValueError("keypoints must contain n elements (one per image).")
     if str(_field(input, "imageMatchingMethod", "ransac")).lower() != "ransac" or int(_field(input, "useMATLABImageMatching", 0)):
         raise ValueError("only input.imageMatchingMethod = 'ransac' with useMATLABImageMatching = 0 is built")
-    allMatches = [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)]
-    numMatches = np.zeros((n, n))
-    tforms = [[None] * n for _ in range(n)]
     _, lin1 = selectImagePartners(matchesAll, int(_field(input, "mBrownLowe", 6)), ctx)
     if lin1.size == 0:
-        return allMatches, numMatches, tforms
+        return _fill_image_matching(n, matchesAll, lin1, np.zeros(1, np.int64), None)[:3]
     lin = np.ascontiguousarray(lin1 - 1, np.int64)
-    # CSR of the cell (column-major cell index c = i + j*n), pooled keypoints
-    pair_ptr = np.zeros(n * n + 1, np.int64)
-    segs = []
-    for j in range(n):
-        for i in range(n):
-            a = np.asarray(matchesAll[i][j])
-            cnt = a.shape[0] if (a.ndim == 2 and i < j) else 0
-            pair_ptr[i + j * n + 1] = cnt
-            if cnt:
-                segs.append(np.ascontiguousarray(a, np.float64).astype(np.uint32))
-    pair_ptr = np.cumsum(pair_ptr)
-    rows = np.ascontiguousarray(np.vstack(segs), np.uint32) if segs else np.zeros((0, 2), np.uint32)
-    kps = [np.asarray(k, np.float64).reshape(-1, 2) for k in keypoints]
-    img_off = np.concatenate([[0], np.cumsum([k.shape[0] for k in kps])]).astype(np.int64)
-    kp = np.ascontiguousarray(np.vstack(kps)) if img_off[-1] else np.zeros((0, 2))
+    pair_ptr, rows = _match_csr(n, matchesAll)
+    kp, img_off = _pool_keypoints(keypoints)
     md, conf, mt = _ransac_params(input)
     P = lin.size
-    total = int(sum(pair_ptr[c + 1] - pair_ptr[c] for c in lin))
+    total = int(np.diff(pair_ptr)[lin].sum())
     if samples is not None:
         samples = np.ascontiguousarray(samples, np.uint32).reshape(P, -1, 4)
     n_draws = samples.shape[1] if samples is not None else 2 * mt
     ptr = np.zeros(P + 1, np.int64)
-    models, minv = np.full((P, 3, 3), np.nan), np.full((P, 3, 3), np.nan)
-    inl, ni = np.zeros(max(total, 1), np.uint8), np.zeros(P, np.int32)
-    acc, du = np.zeros(P, np.uint8), np.zeros(P, np.int32)
+    outputs = _ransac_outputs(P, total)
     check(lib().aps_image_matching(ctx.handle, n, _ptr(pair_ptr), _ptr(rows), _ptr(kp), _ptr(img_off), _ptr(lin), P, md,
                                    conf, mt, _ptr(samples) if samples is not None else C.c_void_p(0), n_draws, int(seed),
-                                   _ptr(ptr), _ptr(models), _ptr(minv), _ptr(inl), _ptr(ni), _ptr(acc), _ptr(du)))
+                                   _ptr(ptr), *[_ptr(a) for a in outputs]))
+    *result, imageMatching.last = _fill_image_matching(n, matchesAll, lin, ptr, outputs)
+    return tuple(result)
+
+
+def _match_csr(n, matchesAll):
+    """CSR of the n x n cell's strict upper triangle (column-major cell index c = i + j*n) -> (pair_ptr [n*n + 1],
+    rows [M x 2] uint32 1-based index pairs)"""
+    pair_ptr, segs = np.zeros(n * n + 1, np.int64), []
+    for j in range(n):
+        for i in range(j):
+            a = np.asarray(matchesAll[i][j])
+            if a.ndim == 2 and a.shape[0]:
+                pair_ptr[i + j * n + 1] = a.shape[0]
+                segs.append(np.ascontiguousarray(a, np.float64).astype(np.uint32))
+    rows = np.ascontiguousarray(np.vstack(segs), np.uint32) if segs else np.zeros((0, 2), np.uint32)
+    return np.cumsum(pair_ptr), rows
+
+
+def _pool_keypoints(keypoints):
+    """[Ni x 2] keypoint arrays -> (pooled row-major [F x 2] float64, img_off [n + 1])"""
+    kps = [np.asarray(k, np.float64).reshape(-1, 2) for k in keypoints]
+    img_off = np.concatenate([[0], np.cumsum([k.shape[0] for k in kps], dtype=np.int64)]).astype(np.int64)
+    return (np.ascontiguousarray(np.vstack(kps)) if img_off[-1] else np.zeros((0, 2))), img_off
+
+
+def _ransac_outputs(P, total):
+    """output buffers of the image-matching entries: models, models_inv [P x 3 x 3], inliers [total], n_inliers,
+    accepted, draws_used [P]"""
+    return (np.full((P, 3, 3), np.nan), np.full((P, 3, 3), np.nan), np.zeros(total, np.uint8), np.zeros(P, np.int32),
+            np.zeros(P, np.uint8), np.zeros(P, np.int32))
+
+
+def _fill_image_matching(n, matchesAll, lin, ptr, outputs):
+    """imageMatching's results for one set from the RANSAC outputs of its candidate pairs (lin: 0-based cells, ptr:
+    their [P + 1] offsets into outputs' inliers, from 0; outputs None: no pairs) ->
+    (allMatches, numMatches, tforms, last)"""
+    allMatches = [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)]
+    numMatches = np.zeros((n, n))
+    tforms = [[None] * n for _ in range(n)]
+    if outputs is None:
+        return allMatches, numMatches, tforms, dict(pairs_lin=np.zeros(0, np.int64), pt_ptr=ptr)
+    models, minv, inl, ni, acc, du = outputs
     for p, c in enumerate(lin):
         if not acc[p]:
             continue
@@ -788,9 +799,9 @@ def imageMatching(input, n, keypoints, matchesAll, imagesProcessed=None, samples
         allMatches[i][j] = m[inl[ptr[p]:ptr[p + 1]].astype(bool)]  # imageMatching.m:148
         numMatches[i, j] = ni[p]
         tforms[i][j], tforms[j][i] = models[p], minv[p]  # :150-151, :165-166
-    imageMatching.last = dict(pairs_lin=lin, pt_ptr=ptr, n_inliers=ni, accepted=acc.astype(bool), draws_used=du,
-                              models=models, models_inv=minv, inliers=inl[:total].astype(bool))
-    return allMatches, numMatches, tforms
+    last = dict(pairs_lin=lin, pt_ptr=ptr, n_inliers=ni, accepted=acc.astype(bool), draws_used=du, models=models,
+                models_inv=minv, inliers=inl[:ptr[-1]].astype(bool))
+    return allMatches, numMatches, tforms, last
 
 
 def _set_counts(matchesAll):
@@ -859,27 +870,13 @@ def imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets, seed=0, sam
     ctx = ctx or default_context()
     B = len(ns)
     _, lin, spp = _select_partners_sets(ctx, [_set_counts(mall) for mall in m_sets], int(_field(input, "mBrownLowe", 6)))
-    result = [([[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)], np.zeros((n, n)), [[None] * n for _ in range(n)])
-              for n in ns]
-    imageMatchingSets.last = [dict(pairs_lin=np.zeros(0, np.int64), pt_ptr=np.zeros(1, np.int64)) for _ in ns]
     P = int(spp[-1])
     if P == 0:
-        return result
-    # per set: CSR of the cell (column-major cell index c = i + j*n, strict upper triangle), as imageMatching builds it
-    pps, rows = [], []
-    for n, mall in zip(ns, m_sets):
-        pp, segs = np.zeros(n * n + 1, np.int64), []
-        for j in range(n):
-            for i in range(j):
-                a = np.asarray(mall[i][j])
-                if a.ndim == 2 and a.shape[0]:
-                    pp[i + j * n + 1] = a.shape[0]
-                    segs.append(np.ascontiguousarray(a, np.float64).astype(np.uint32))
-        pps.append(np.cumsum(pp))
-        rows.append(np.ascontiguousarray(np.vstack(segs), np.uint32) if segs else np.zeros((0, 2), np.uint32))
-    kps = [np.asarray(k, np.float64).reshape(-1, 2) for ks in kps_sets for k in ks]
-    img_off = np.concatenate([[0], np.cumsum([k.shape[0] for k in kps], dtype=np.int64)]).astype(np.int64)
-    kp = np.ascontiguousarray(np.vstack(kps)) if img_off[-1] else np.zeros((0, 2))
+        result = [_fill_image_matching(n, None, None, np.zeros(1, np.int64), None) for n in ns]
+        imageMatchingSets.last = [r[3] for r in result]
+        return [r[:3] for r in result]
+    csrs = [_match_csr(n, mall) for n, mall in zip(ns, m_sets)]
+    kp, img_off = _pool_keypoints([k for ks in kps_sets for k in ks])
     md, conf, mt = _ransac_params(input)
     n_draws = 2 * mt
     if samples is not None:
@@ -890,36 +887,22 @@ def imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets, seed=0, sam
         samples = np.ascontiguousarray(np.concatenate([t.reshape(spp[b + 1] - spp[b], n_draws, 4)
                                                        for b, t in enumerate(tabs)]))
     ptr = np.zeros(P + 1, np.int64)
-    total = 0
-    for b in range(B):
-        total += int(sum(pps[b][c + 1] - pps[b][c] for c in lin[spp[b]:spp[b + 1]]))
-    models, minv = np.full((P, 3, 3), np.nan), np.full((P, 3, 3), np.nan)
-    inl, ni = np.zeros(total, np.uint8), np.zeros(P, np.int32)
-    acc, du = np.zeros(P, np.uint8), np.zeros(P, np.int32)
+    total = int(sum(pp[c + 1] - pp[c] for b, (pp, _) in enumerate(csrs) for c in lin[spp[b]:spp[b + 1]]))
+    outputs = _ransac_outputs(P, total)
     simg = (C.c_int * B)(*ns)
-    pp_arr = (C.c_void_p * B)(*[p.ctypes.data for p in pps])
-    rows_arr = (C.c_void_p * B)(*[r.ctypes.data if r.size else None for r in rows])
+    pp_arr = (C.c_void_p * B)(*[pp.ctypes.data for pp, _ in csrs])
+    rows_arr = (C.c_void_p * B)(*[r.ctypes.data if r.size else None for _, r in csrs])
     check(lib().aps_image_matching_sets(ctx.handle, B, simg, pp_arr, rows_arr, _ptr(kp), _ptr(img_off), _ptr(spp),
                                         _ptr(lin), md, conf, mt, _ptr(samples) if samples is not None else C.c_void_p(0),
-                                        int(n_draws), int(seed), _ptr(ptr), _ptr(models), _ptr(minv), _ptr(inl), _ptr(ni),
-                                        _ptr(acc), _ptr(du)))
+                                        int(n_draws), int(seed), _ptr(ptr), *[_ptr(a) for a in outputs]))
+    models, minv, inl, ni, acc, du = outputs
+    result = []
     for b, (n, mall) in enumerate(zip(ns, m_sets)):
-        p0, p1 = int(spp[b]), int(spp[b + 1])
-        allMatches, numMatches, tforms = result[b]
-        for p in range(p0, p1):
-            if not acc[p]:
-                continue
-            c = lin[p]
-            i, j = int(c % n), int(c // n)
-            mij = np.asarray(mall[i][j], np.float64)
-            allMatches[i][j] = mij[inl[ptr[p]:ptr[p + 1]].astype(bool)]  # imageMatching.m:148
-            numMatches[i, j] = ni[p]
-            tforms[i][j], tforms[j][i] = models[p], minv[p]  # :150-151, :165-166
-        t0, t1 = ptr[p0], ptr[p1]
-        imageMatchingSets.last[b] = dict(pairs_lin=lin[p0:p1], pt_ptr=ptr[p0:p1 + 1] - t0, n_inliers=ni[p0:p1],
-                                         accepted=acc[p0:p1].astype(bool), draws_used=du[p0:p1], models=models[p0:p1],
-                                         models_inv=minv[p0:p1], inliers=inl[t0:t1].astype(bool))
-    return result
+        p, t0, t1 = slice(spp[b], spp[b + 1]), ptr[spp[b]], ptr[spp[b + 1]]
+        result.append(_fill_image_matching(n, mall, lin[p], ptr[spp[b]:spp[b + 1] + 1] - t0,
+                                           (models[p], minv[p], inl[t0:t1], ni[p], acc[p], du[p])))
+    imageMatchingSets.last = [r[3] for r in result]
+    return [r[:3] for r in result]
 
 
 RECORD_PAD = 16384  # APS_RECORD_PAD of include/apsmatch.h: rows the record buffer holds beyond F

@@ -227,7 +227,8 @@ void aps_matchlist_free(aps_matchlist* m);
 /* ---- top-m image-partner selection ------------------------- PP/imageMatching/imageMatching.m:75-100
  * counts: putativeCount [n x n] column-major (counts[i + j*n] = size(matchesAll{i,j},1)), m =
  * input.mBrownLowe.  cand [n x n] column-major logical (strict upper triangle); pairs_lin (may be
- * NULL) receives find(candidatePairs) as 0-based linear indices, *npairs their number. */
+ * NULL) receives find(candidatePairs) as 0-based linear indices, *npairs their number.  The one-set case of
+ * aps_select_partners_sets, except that the context is checked first. */
 int aps_select_partners(aps_ctx* ctx, const int64_t* counts, int n, int m, uint8_t* cand, int64_t* pairs_lin,
                         int64_t* npairs);
 /* The same for nsets independent image sets in one call.  Set b has set_images[b] images; counts holds, for each set,
@@ -271,7 +272,9 @@ int aps_image_matching_batch(aps_ctx* ctx, int64_t n_pairs, const int64_t* pt_pt
  * img_off [n_images + 1], pairs_lin = find(candidatePairs) from aps_select_partners.  The matched points are
  * gathered on the device (refineMatch, imageMatching.m:224-227; out-of-range indices -> error id
  * refineMatch:MatchIndexOutOfBounds).  pt_ptr_out [n_pairs + 1] receives the offsets of each pair's
- * correspondences inside `inliers` (allMatches{ii,jj} = matches(inliers,:)). */
+ * correspondences inside `inliers` (allMatches{ii,jj} = matches(inliers,:)).  The one-set case of
+ * aps_image_matching_sets, except that the context is checked first, n_pairs == 0 succeeds before the RANSAC
+ * parameters are checked, and at most 65535 pairs are taken per call. */
 int aps_image_matching(aps_ctx* ctx, int n_images, const int64_t* pair_ptr, const uint32_t* rows,
                        const double* keypoints, const int64_t* img_off, const int64_t* pairs_lin, int64_t n_pairs,
                        double max_distance, double confidence, int max_trials, const uint32_t* samples,

@@ -21,7 +21,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     if (!mxIsDouble(prhs[i]) || mxGetNumberOfElements(prhs[i]) != 1)
       mexErrMsgIdAndTxt("apsmatch:args", "m, maxDistance, confidence, maxIter and seed must be double scalars");
   std::vector<int> ns((size_t)B);
-  std::vector<int64_t> off(1, 0), counts, cell0(1, 0);
+  std::vector<int64_t> off(1, 0), counts;
   std::vector<double> kp;
   std::vector<std::vector<int64_t>> pair_ptr((size_t)B);
   std::vector<std::vector<uint32_t>> rows((size_t)B);
@@ -34,40 +34,8 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     if ((int)mxGetNumberOfElements(kpc) != n)
       mexErrMsgIdAndTxt("apsmatch:args", "set %d: keypoints must contain n elements (one per image).", b + 1);
     ns[b] = n;
-    for (int i = 0; i < n; ++i) {  // pooled keypoints, row-major [F x 2]
-      const mxArray* k = mxGetCell(kpc, i);
-      if (k && !mxIsEmpty(k) && (!mxIsDouble(k) || mxGetN(k) != 2))
-        mexErrMsgIdAndTxt("apsmatch:args", "set %d: keypoints{%d} must be [Ni x 2] double", b + 1, i + 1);
-      const int64_t ni = k ? (int64_t)mxGetM(k) : 0;  // rows, as aps_imageMatching_mex counts them
-      const double* d = (k && !mxIsEmpty(k)) ? mxGetPr(k) : nullptr;  // an [Ni x 0] array has no coordinates: zeros
-      for (int64_t r = 0; r < ni; ++r) {
-        kp.push_back(d ? d[r] : 0.0);
-        kp.push_back(d ? d[r + ni] : 0.0);
-      }
-      off.push_back(off.back() + ni);
-    }
-    // CSR of the set's cell (strict upper triangle) + putative counts of every cell (imageMatching.m:76)
-    const size_t cells = (size_t)n * n;
-    std::vector<int64_t>& pp = pair_ptr[b];
-    pp.assign(cells + 1, 0);
-    for (size_t c = 0; c < cells; ++c) {
-      const mxArray* e = mxGetCell(mc, c);
-      counts.push_back(e ? (int64_t)mxGetM(e) : 0);
-      const bool upper = (int)(c % n) < (int)(c / n);
-      const bool used = upper && e && mxGetN(e) == 2 && mxGetM(e) > 0;
-      if (used && !mxIsDouble(e)) mexErrMsgIdAndTxt("apsmatch:args", "set %d: matchesAll{i,j} must be double", b + 1);
-      pp[c + 1] = pp[c] + (used ? (int64_t)mxGetM(e) : 0);
-    }
-    rows[b].resize((size_t)(2 * pp[cells]));
-    for (size_t c = 0; c < cells; ++c) {
-      const int64_t a = pp[c], m = pp[c + 1] - a;
-      const double* d = m ? mxGetPr(mxGetCell(mc, c)) : nullptr;
-      for (int64_t r = 0; r < m; ++r) {
-        rows[b][2 * (a + r)] = (uint32_t)d[r];
-        rows[b][2 * (a + r) + 1] = (uint32_t)d[r + m];
-      }
-    }
-    cell0.push_back(cell0.back() + (int64_t)cells);
+    aps_mex_pool_keypoints(kpc, n, b + 1, kp, off);
+    aps_mex_match_csr(mc, n, b + 1, pair_ptr[b], rows[b], counts);
   }
   mxArray* allM = mxCreateCellMatrix(1, (mwSize)B);
   mxArray* numM = mxCreateCellMatrix(1, (mwSize)B);
@@ -83,7 +51,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   if (B == 0) return;
   int64_t cap = 0;
   for (int n : ns) cap += (int64_t)n * (n - 1) / 2;
-  std::vector<uint8_t> cand((size_t)cell0[B] + 1);
+  std::vector<uint8_t> cand(counts.size() + 1);
   std::vector<int64_t> lin((size_t)cap + 1), spp((size_t)B + 1);
   if (aps_select_partners_sets(aps_mex_ctx(), B, ns.data(), counts.data(), (int)mxGetScalar(prhs[2]), cand.data(),
                                lin.data(), spp.data()) != APS_OK)
@@ -109,32 +77,8 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
                               2 * (int64_t)max_iter, seed, ptr.data(), models.data(), minv.data(), inl.data(), ni.data(),
                               acc.data(), used.data()) != APS_OK)
     aps_mex_fail("apsmatch:args");
-  for (int b = 0; b < B; ++b) {
-    const int64_t n = ns[b];
-    mxArray *am_b = mxGetCell(allM, b), *tf_b = mxGetCell(tfs, b);
-    double* num_b = mxGetPr(mxGetCell(numM, b));
-    for (int64_t p = spp[b]; p < spp[b + 1]; ++p) {
-      if (!acc[p]) continue;
-      const int64_t c = lin[p], i = c % n, j = c / n, a = pair_ptr[b][c], m = ptr[p + 1] - ptr[p];
-      mxArray* am = mxCreateDoubleMatrix((mwSize)ni[p], 2, mxREAL);  // matches(inliers,:), :148
-      double* d = mxGetPr(am);
-      int64_t w = 0;
-      for (int64_t r = 0; r < m; ++r)
-        if (inl[ptr[p] + r]) {
-          d[w] = (double)rows[b][2 * (a + r)];
-          d[w + ni[p]] = (double)rows[b][2 * (a + r) + 1];
-          ++w;
-        }
-      mxSetCell(am_b, (mwIndex)c, am);
-      num_b[c] = (double)ni[p];
-      mxArray *t1 = mxCreateDoubleMatrix(3, 3, mxREAL), *t2 = mxCreateDoubleMatrix(3, 3, mxREAL);
-      for (int rr = 0; rr < 3; ++rr)
-        for (int cc = 0; cc < 3; ++cc) {  // row-major -> MATLAB column-major
-          mxGetPr(t1)[rr + 3 * cc] = models[9 * p + 3 * rr + cc];
-          mxGetPr(t2)[rr + 3 * cc] = minv[9 * p + 3 * rr + cc];
-        }
-      mxSetCell(tf_b, (mwIndex)(i + j * n), t1);  // tforms(IuptriIdx) = tforms_ij  (:165)
-      mxSetCell(tf_b, (mwIndex)(j + i * n), t2);  // tforms(IlowtriIdx) = tforms_ji (:166)
-    }
-  }
+  for (int b = 0; b < B; ++b)
+    aps_mex_put_matches(ns[b], pair_ptr[b].data(), rows[b].data(), lin.data(), spp[b], spp[b + 1], ptr.data(),
+                        models.data(), minv.data(), inl.data(), ni.data(), acc.data(), mxGetCell(allM, b),
+                        mxGetPr(mxGetCell(numM, b)), mxGetCell(tfs, b));
 }

@@ -18,53 +18,19 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   if ((int)mxGetN(mc) != n) mexErrMsgIdAndTxt("imageMatching:InvalidMatchesAllSize", "matchesAll must be an n-by-n cell array.");
   if ((int)mxGetNumberOfElements(kpc) != n)
     mexErrMsgIdAndTxt("imageMatching:InvalidKeypointsLength", "keypoints must contain n elements (one per image).");
-  // pooled keypoints, row-major [F x 2]
-  std::vector<int64_t> off((size_t)n + 1, 0);
-  for (int i = 0; i < n; ++i) {
-    const mxArray* k = mxGetCell(kpc, i);
-    if (k && !mxIsEmpty(k) && (!mxIsDouble(k) || mxGetN(k) != 2)) mexErrMsgIdAndTxt("apsmatch:args", "keypoints{i} must be [Ni x 2] double");
-    off[i + 1] = off[i] + (k ? (int64_t)mxGetM(k) : 0);
-  }
-  std::vector<double> kp((size_t)(2 * off[n]));
-  for (int i = 0; i < n; ++i) {
-    const mxArray* k = mxGetCell(kpc, i);
-    const int64_t ni = off[i + 1] - off[i];
-    if (!ni) continue;
-    const double* d = mxGetPr(k);
-    for (int64_t r = 0; r < ni; ++r) {
-      kp[2 * (off[i] + r)] = d[r];
-      kp[2 * (off[i] + r) + 1] = d[r + ni];
-    }
-  }
-  // CSR of the cell (strict upper triangle) + putative counts
-  const size_t cells = (size_t)n * n;
-  std::vector<int64_t> pair_ptr(cells + 1, 0), counts(cells, 0);
-  for (size_t c = 0; c < cells; ++c) {
-    const mxArray* e = mxGetCell(mc, c);
-    counts[c] = e ? (int64_t)mxGetM(e) : 0;  // putativeCount (:76) counts every cell
-    const bool upper = (int)(c % n) < (int)(c / n);
-    pair_ptr[c + 1] = pair_ptr[c] + ((upper && e && mxGetN(e) == 2) ? (int64_t)mxGetM(e) : 0);
-  }
-  std::vector<uint32_t> rows((size_t)(2 * pair_ptr[cells]));
-  for (size_t c = 0; c < cells; ++c) {
-    const int64_t a = pair_ptr[c], m = pair_ptr[c + 1] - a;
-    if (!m) continue;
-    const mxArray* e = mxGetCell(mc, c);
-    if (!mxIsDouble(e)) mexErrMsgIdAndTxt("apsmatch:args", "matchesAll{i,j} must be double");
-    const double* d = mxGetPr(e);
-    for (int64_t r = 0; r < m; ++r) {
-      rows[2 * (a + r)] = (uint32_t)d[r];
-      rows[2 * (a + r) + 1] = (uint32_t)d[r + m];
-    }
-  }
+  std::vector<int64_t> off(1, 0), pair_ptr, counts;
+  std::vector<double> kp;
+  std::vector<uint32_t> rows;
+  aps_mex_pool_keypoints(kpc, n, 0, kp, off);
+  aps_mex_match_csr(mc, n, 0, pair_ptr, rows, counts);
   plhs[0] = mxCreateCellMatrix((mwSize)n, (mwSize)n);
   mxArray* numM = mxCreateDoubleMatrix((mwSize)n, (mwSize)n, mxREAL);
   mxArray* tf = mxCreateCellMatrix((mwSize)n, (mwSize)n);
   if (nlhs > 1) plhs[1] = numM;
   if (nlhs > 2) plhs[2] = tf;
   if (n == 0) return;
-  std::vector<uint8_t> cand(cells);
-  std::vector<int64_t> lin(cells + 1);
+  std::vector<uint8_t> cand((size_t)n * n);
+  std::vector<int64_t> lin((size_t)n * n + 1);
   int64_t np = 0;
   if (aps_select_partners(aps_mex_ctx(), counts.data(), n, (int)mxGetScalar(prhs[2]), cand.data(), lin.data(), &np) != APS_OK)
     aps_mex_fail("apsmatch:args");
@@ -81,27 +47,6 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
                          mxGetScalar(prhs[3]), mxGetScalar(prhs[4]), max_iter, nullptr, 2 * (int64_t)max_iter, seed,
                          ptr.data(), models.data(), minv.data(), inl.data(), ni.data(), acc.data(), used.data()) != APS_OK)
     aps_mex_fail("apsmatch:args");
-  for (int64_t p = 0; p < np; ++p) {
-    if (!acc[p]) continue;
-    const int64_t c = lin[p], i = c % n, j = c / n, a = pair_ptr[c], m = ptr[p + 1] - ptr[p];
-    mxArray* am = mxCreateDoubleMatrix((mwSize)ni[p], 2, mxREAL);  // matches(inliers,:), :148
-    double* d = mxGetPr(am);
-    int64_t w = 0;
-    for (int64_t r = 0; r < m; ++r)
-      if (inl[ptr[p] + r]) {
-        d[w] = (double)rows[2 * (a + r)];
-        d[w + ni[p]] = (double)rows[2 * (a + r) + 1];
-        ++w;
-      }
-    mxSetCell(plhs[0], (mwIndex)c, am);
-    mxGetPr(numM)[c] = (double)ni[p];
-    mxArray *t1 = mxCreateDoubleMatrix(3, 3, mxREAL), *t2 = mxCreateDoubleMatrix(3, 3, mxREAL);
-    for (int rr = 0; rr < 3; ++rr)
-      for (int cc = 0; cc < 3; ++cc) {  // row-major -> MATLAB column-major
-        mxGetPr(t1)[rr + 3 * cc] = models[9 * p + 3 * rr + cc];
-        mxGetPr(t2)[rr + 3 * cc] = minv[9 * p + 3 * rr + cc];
-      }
-    mxSetCell(tf, (mwIndex)(i + j * n), t1);  // tforms(IuptriIdx) = tforms_ij  (:165)
-    mxSetCell(tf, (mwIndex)(j + i * n), t2);  // tforms(IlowtriIdx) = tforms_ji (:166)
-  }
+  aps_mex_put_matches(n, pair_ptr.data(), rows.data(), lin.data(), 0, np, ptr.data(), models.data(), minv.data(),
+                      inl.data(), ni.data(), acc.data(), plhs[0], mxGetPr(numM), tf);
 }

@@ -140,3 +140,80 @@ static inline mxArray* aps_mex_cells(const aps_matchlist* ml, int n, bool fill_u
     }
   return out;
 }
+// "" or " (set b)" after a gateway message: the sets gateway names the set (1-based), the single-set one does not
+static inline std::string aps_mex_in_set(int set) {
+  return set > 0 ? " (set " + std::to_string(set) + ")" : std::string();
+}
+// keypoints{i} (1 x n or n x 1 cell of [Ni x 2] double) appended to the pooled row-major [F x 2] keypoints and their
+// row offsets (off starts with {0}).  An empty [Ni x 0] element counts Ni rows with zero coordinates.
+static inline void aps_mex_pool_keypoints(const mxArray* kpc, int n, int set, std::vector<double>& kp,
+                                          std::vector<int64_t>& off) {
+  for (int i = 0; i < n; ++i) {
+    const mxArray* k = mxGetCell(kpc, i);
+    if (k && !mxIsEmpty(k) && (!mxIsDouble(k) || mxGetN(k) != 2))
+      mexErrMsgIdAndTxt("apsmatch:args", "keypoints{%d} must be [Ni x 2] double%s", i + 1, aps_mex_in_set(set).c_str());
+    const int64_t ni = k ? (int64_t)mxGetM(k) : 0;
+    const double* d = (k && !mxIsEmpty(k)) ? mxGetPr(k) : nullptr;
+    for (int64_t r = 0; r < ni; ++r) {
+      kp.push_back(d ? d[r] : 0.0);
+      kp.push_back(d ? d[r + ni] : 0.0);
+    }
+    off.push_back(off.back() + ni);
+  }
+}
+// CSR of the n x n cell's strict upper triangle (pair_ptr [n*n + 1], rows = 1-based index pairs) and the putativeCount
+// of every cell (imageMatching.m:76), appended to counts
+static inline void aps_mex_match_csr(const mxArray* mc, int n, int set, std::vector<int64_t>& pair_ptr,
+                                     std::vector<uint32_t>& rows, std::vector<int64_t>& counts) {
+  const size_t cells = (size_t)n * n;
+  pair_ptr.assign(cells + 1, 0);
+  for (size_t c = 0; c < cells; ++c) {
+    const mxArray* e = mxGetCell(mc, c);
+    counts.push_back(e ? (int64_t)mxGetM(e) : 0);
+    const bool upper = (int)(c % n) < (int)(c / n);
+    const bool used = upper && e && mxGetN(e) == 2 && mxGetM(e) > 0;
+    if (used && !mxIsDouble(e))
+      mexErrMsgIdAndTxt("apsmatch:args", "matchesAll{i,j} must be double%s", aps_mex_in_set(set).c_str());
+    pair_ptr[c + 1] = pair_ptr[c] + (used ? (int64_t)mxGetM(e) : 0);
+  }
+  rows.resize((size_t)(2 * pair_ptr[cells]));
+  for (size_t c = 0; c < cells; ++c) {
+    const int64_t a = pair_ptr[c], m = pair_ptr[c + 1] - a;
+    const double* d = m ? mxGetPr(mxGetCell(mc, c)) : nullptr;
+    for (int64_t r = 0; r < m; ++r) {
+      rows[2 * (a + r)] = (uint32_t)d[r];
+      rows[2 * (a + r) + 1] = (uint32_t)d[r + m];
+    }
+  }
+}
+// One set's imageMatching outputs (imageMatching.m:148-166) from the RANSAC results of its candidate pairs [p0, p1):
+// allMatches{c} = matches(inliers,:), numMatches(c) = ni, tforms{i,j} = model (maps image j to image i), tforms{j,i} =
+// its inverse.  lin: cells of the set's block; pair_ptr / rows: the set's CSR; ptr: absolute offsets into inl.
+static inline void aps_mex_put_matches(int64_t n, const int64_t* pair_ptr, const uint32_t* rows, const int64_t* lin,
+                                       int64_t p0, int64_t p1, const int64_t* ptr, const double* models,
+                                       const double* minv, const uint8_t* inl, const int32_t* ni, const uint8_t* acc,
+                                       mxArray* allM, double* numM, mxArray* tf) {
+  for (int64_t p = p0; p < p1; ++p) {
+    if (!acc[p]) continue;
+    const int64_t c = lin[p], i = c % n, j = c / n, a = pair_ptr[c], m = ptr[p + 1] - ptr[p];
+    mxArray* am = mxCreateDoubleMatrix((mwSize)ni[p], 2, mxREAL);
+    double* d = mxGetPr(am);
+    int64_t w = 0;
+    for (int64_t r = 0; r < m; ++r)
+      if (inl[ptr[p] + r]) {
+        d[w] = (double)rows[2 * (a + r)];
+        d[w + ni[p]] = (double)rows[2 * (a + r) + 1];
+        ++w;
+      }
+    mxSetCell(allM, (mwIndex)c, am);
+    numM[c] = (double)ni[p];
+    mxArray *t1 = mxCreateDoubleMatrix(3, 3, mxREAL), *t2 = mxCreateDoubleMatrix(3, 3, mxREAL);
+    for (int rr = 0; rr < 3; ++rr)
+      for (int cc = 0; cc < 3; ++cc) {  // row-major -> MATLAB column-major
+        mxGetPr(t1)[rr + 3 * cc] = models[9 * p + 3 * rr + cc];
+        mxGetPr(t2)[rr + 3 * cc] = minv[9 * p + 3 * rr + cc];
+      }
+    mxSetCell(tf, (mwIndex)(i + j * n), t1);
+    mxSetCell(tf, (mwIndex)(j + i * n), t2);
+  }
+}

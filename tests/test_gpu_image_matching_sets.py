@@ -3,6 +3,7 @@ against imageMatching on each set alone with the same seed: candidate pairs, cor
 bits, inlier masks, n_inliers, accepted and draws_used must be identical.  Also the partner selection per set, the
 oracle with given samples, launch counts that do not depend on the number of sets, more than 65535 pairs in one call,
 errors, the end-to-end chain from featureMatchingGlobalSets, and the MEX gateway."""
+import ctypes as C
 import os
 
 import numpy as np
@@ -101,6 +102,15 @@ def test_partner_selection_equals_single_set_call(aps):
                 continue
             rc, rl = aps.selectImagePartners(c, m)
             assert np.array_equal(cand, rc) and np.array_equal(lin, rl)
+    # aps_select_partners without pairs_lin: the count alone
+    L, ctx = aps._lib.lib(), aps._lib.default_context()
+    for c in sets[:20]:
+        n = c.shape[0]
+        cm = np.ascontiguousarray(c.T, np.int64)
+        cand, npairs = np.zeros(max(n * n, 1), np.uint8), C.c_int64(-1)
+        assert L.aps_select_partners(ctx.handle, C.c_void_p(cm.ctypes.data), n, 4, C.c_void_p(cand.ctypes.data), None,
+                                     C.byref(npairs)) == 0
+        assert npairs.value == aps.selectImagePartners(c, 4)[1].size
 
 
 def test_given_samples_equal_device_draws_and_the_oracle(aps, orc):

@@ -96,6 +96,48 @@ def test_image_matching_sets_argument_errors(aps):
     assert eid == "refineMatch:MatchIndexOutOfBounds"
 
 
+def _ctx(aps, real):
+    """a real context when a GPU is present; otherwise zeroed memory standing for one, which the checks under test
+    return before reading (were it read, its device 0 would fail without a GPU)"""
+    import torch
+
+    if not real:
+        return None
+    if torch.cuda.is_available():
+        return aps._lib.default_context().handle
+    _ctx.fake = C.create_string_buffer(4096)
+    return C.cast(_ctx.fake, C.c_void_p)
+
+
+@pytest.mark.parametrize("case", [
+    dict(entry="match", ctx=False, n_images=-1, n_pairs=1, want=6),      # the context first, before bad arguments
+    dict(entry="match", ctx=False, n_images=2, n_pairs=0, want=6),
+    dict(entry="match", ctx=True, n_images=2, n_pairs=0, max_trials=0, want=0),   # no pairs: OK whatever the RANSAC
+    dict(entry="match", ctx=True, n_images=2, n_pairs=65536, want=1),     # the single-set entry's pair limit
+    dict(entry="match", ctx=True, n_images=-1, n_pairs=0, want=1),
+    dict(entry="select", ctx=False, n_images=2, want=6),                  # pairs_lin may be NULL
+    dict(entry="select", ctx=False, n_images=-1, want=6),
+])
+def test_single_set_entries_check_the_context_first(aps, case):
+    """aps_image_matching and aps_select_partners are the one-set case of the sets entries, with their own front"""
+    L = _library(aps)
+    ctx, n = _ctx(aps, case["ctx"]), case["n_images"]
+    if case["entry"] == "select":
+        cnt, cand, npairs = (C.c_int64 * 4)(0, 3, 3, 0), (C.c_uint8 * 4)(), C.c_int64(-1)
+        assert L.aps_select_partners(ctx, cnt, n, 4, cand, None, C.byref(npairs)) == case["want"]
+        return
+    P = case["n_pairs"]
+    pp, rows, kp, img_off = np.array([0, 0, 0, 4, 4], np.int64), np.ones(8, np.uint32), np.zeros((6, 2)), np.array(
+        [0, 3, 6], np.int64)
+    lin, ptr = np.full(max(P, 1), 2, np.int64), np.zeros(P + 1, np.int64)
+    out = [np.zeros(9 * max(P, 1)), np.zeros(9 * max(P, 1)), np.zeros(4 * max(P, 1), np.uint8)] + [
+        np.zeros(max(P, 1), t) for t in (np.int32, np.uint8, np.int32)]
+    v = lambda a: C.c_void_p(a.ctypes.data)  # noqa: E731
+    rc = L.aps_image_matching(ctx, n, v(pp), v(rows), v(kp), v(img_off), v(lin), P, 5.5, 99.9,
+                              case.get("max_trials", 500), None, 1000, 0, v(ptr), *[v(a) for a in out])
+    assert rc == case["want"], L.aps_last_error().decode()
+
+
 def test_well_formed_calls_without_gpu_are_nogpu(aps):
     L = _no_gpu(aps)
     assert _select(L, 2, [2, 0], [0, 3, 3, 0]) == 6              # APS_ERR_NOGPU
