@@ -21,6 +21,8 @@ from .host import (  # noqa: F401
     estimateTransformationRANSAC,
     featureMatchingPairwise,
     imageMatching,
+    globalImageMatching,
+    globalImageMatchingSets,
     imageMatchingBatch,
     imageMatchingSets,
     ransacSampleTable,

@@ -122,6 +122,24 @@ def lib():
                                      vp, vp, vp]),
         "aps_image_matching_sets": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, vp, dbl, dbl, i32, vp, i64, C.c_uint64, vp,
                                           vp, vp, vp, vp, vp, vp]),
+        "aps_global_image_matching_sets": (i32, [vp, i32, C.POINTER(i32), pp, C.POINTER(i64), i32, i32, i32, i32, dbl,
+                                                 i32, i32, vp, i32, dbl, dbl, i32, C.c_uint64, i32, pp]),
+        "aps_global_image_matching": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, i32, dbl, i32, i32, vp, i32, dbl,
+                                            dbl, i32, C.c_uint64, i32, pp]),
+        "aps_image_matches_nsets": (i32, [vp]),
+        "aps_image_matches_pairs": (i64, [vp]),
+        "aps_image_matches_set_pair_ptr": (C.POINTER(i64), [vp]),
+        "aps_image_matches_pairs_lin": (C.POINTER(i64), [vp]),
+        "aps_image_matches_pt_ptr": (C.POINTER(i64), [vp]),
+        "aps_image_matches_match_ptr": (C.POINTER(i64), [vp]),
+        "aps_image_matches_match_rows": (C.POINTER(C.c_uint32), [vp]),
+        "aps_image_matches_models": (C.POINTER(dbl), [vp]),
+        "aps_image_matches_models_inv": (C.POINTER(dbl), [vp]),
+        "aps_image_matches_n_inliers": (C.POINTER(C.c_int32), [vp]),
+        "aps_image_matches_accepted": (C.POINTER(C.c_uint8), [vp]),
+        "aps_image_matches_draws_used": (C.POINTER(C.c_int32), [vp]),
+        "aps_image_matches_list": (vp, [vp, i32]),
+        "aps_image_matches_free": (None, [vp]),
         "aps_gplan_create": (i32, [vp, C.POINTER(i64), i32, i32, i32, i32, pp]),
         "aps_gplan_destroy": (None, [vp]),
         "aps_gplan_total": (i64, [vp]),

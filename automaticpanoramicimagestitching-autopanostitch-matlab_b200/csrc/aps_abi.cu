@@ -923,17 +923,30 @@ int feature_matching_global_impl(aps_ctx* c, const void* const* desc, const int6
   aps_gplan* p = nullptr;
   APS_TRY(aps_gplan_create(c, counts, n, D, dtype, k, &p));
   int rc = APS_OK;
-  if (p->F > 0) {  // featureMatchingGlobal.m:49-52,65-67: all empty -> cell(numImg)
-    rc = aps_gplan_upload(p, desc, layout);
-    if (rc == APS_OK) rc = aps_gplan_prepare(p);
-    if (rc == APS_OK) rc = aps_gplan_knn(p, 0, p->F);
-    if (rc == APS_OK) rc = aps_gplan_filter(p, 0, p->F, ratio);
-    if (rc == APS_OK && mutual) rc = aps_gplan_filter_mutual(p);
-    if (rc == APS_OK) rc = aps_gplan_compact(p);
-  }
+  if (p->F > 0) rc = gplan_run(p, desc, layout, ratio, mutual);  // featureMatchingGlobal.m:49-52,65-67: all empty -> cell(numImg)
   if (rc == APS_OK) rc = aps_gplan_download(p, out);
   aps_gplan_destroy(p);
   return rc;
+}
+
+int gplan_run(aps_gplan* p, const void* const* desc, int layout, double ratio, int mutual) {
+  APS_TRY(aps_gplan_upload(p, desc, layout));
+  APS_TRY(aps_gplan_prepare(p));
+  APS_TRY(aps_gplan_knn(p, 0, p->F));
+  APS_TRY(aps_gplan_filter(p, 0, p->F, ratio));
+  if (mutual) APS_TRY(aps_gplan_filter_mutual(p));
+  return aps_gplan_compact(p);
+}
+
+void gplan_lists(aps_gplan* p, GlobalLists& L) {
+  L.plan = p;
+  L.order.assign(1, 0);
+  L.cell_off = {0, (int64_t)p->n * p->n};
+  L.pair_counts = p->pair_counts.p;
+  L.pair_ptr = p->pair_ptr.p;
+  L.rows = p->rows.p;
+  L.F = p->F;
+  L.Ft = p->dtype == APS_F32 && p->tensor ? p->F : 0;
 }
 
 // Same with the pooled descriptors ALREADY ON THE DEVICE (a GPU extractor's output, or a previous stage's buffer):

@@ -1,6 +1,7 @@
 // aps_abi_internal.cuh -- what the translation units behind include/apsmatch.h share (aps_abi.cu: context, kNN entries,
 // staged global pipeline; aps_abi_pairwise.cu: matchFeaturesScratch / featureMatchingPairwise, staged pairwise pipeline,
-// pairwise matching of many image sets; aps_abi_sets.cu: global matching of many image sets).
+// pairwise matching of many image sets; aps_abi_sets.cu: global matching of many image sets; aps_ransac.cu: RANSAC
+// chunks; aps_global_image_matching.cu: global matching through image matching in one call).
 #pragma once
 #include <string>
 #include <vector>
@@ -113,6 +114,54 @@ int sets_img_of_row(cudaStream_t s, const int64_t* d_off, int nimg, int64_t F, i
 // `raw`: one copy per image; column-major input is staged and transposed in ONE launch (needs img_of_row)
 int sets_upload(aps_ctx* c, const void* const* ptrs, const std::vector<int64_t>& off, const int64_t* d_off,
                 const int32_t* img_of_row, int D, int esz, int layout, void* raw);
+
+// ---- global match lists kept on the device (aps_abi.cu, aps_abi_sets.cu; aps_global_image_matching_sets) ----------
+// The compaction outputs of one global pass over nsets sets, in PASS order: pass position j is the caller's set
+// order[j], its n x n block is cells [cell_off[j], cell_off[j + 1]) of pair_counts / pair_ptr (column-major, strict
+// upper triangle filled), and cell c's rows are rows[2 * pair_ptr[c] .. 2 * pair_ptr[c + 1]).
+struct GlobalLists {
+  std::vector<int> order;
+  std::vector<int64_t> cell_off;
+  const int64_t* pair_counts = nullptr;  // [cells]
+  const int64_t* pair_ptr = nullptr;     // [cells + 1]
+  const uint32_t* rows = nullptr;
+  DevBuf<int64_t> counts_buf, ptr_buf;   // owners for a pass over several sets
+  DevBuf<uint32_t> rows_buf;
+  aps_gplan* plan = nullptr;             // owner for one set
+  int64_t F = 0, Ft = 0;                 // rows searched, rows of the tensor-path sets (statistics)
+  GlobalLists() = default;
+  GlobalLists(const GlobalLists&) = delete;
+  GlobalLists& operator=(const GlobalLists&) = delete;
+  ~GlobalLists() { aps_gplan_destroy(plan); }
+};
+// Checks the arguments of aps_feature_matching_global_sets (ids of aps_feature_matching_global) and returns the first
+// pooled image of each set and the rows of each set.
+int global_sets_args(int nsets, const int* set_images, const int64_t* counts, int D, int dtype, int k,
+                     std::vector<int64_t>& img_first, std::vector<int64_t>& set_rows);
+// Runs the global pass of aps_feature_matching_global_sets up to the compaction and leaves the lists on the device in
+// L; the arguments must have passed global_sets_args, the context must be current and some set must have rows.
+// Nothing is synchronised; global_lists_stats sets the context's statistics once the stream has been synchronised.
+int global_lists_device(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
+                        const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D,
+                        int dtype, int layout, int k, double ratio, int mutual, GlobalLists& L);
+void global_lists_stats(aps_ctx* c, int dtype, const GlobalLists& L);
+// The one-set pass (aps_abi.cu): the staged plan from upload to compaction, and its lists handed to L.
+int gplan_run(aps_gplan* p, const void* const* desc, int layout, double ratio, int mutual);
+void gplan_lists(aps_gplan* p, GlobalLists& L);
+
+// ---- RANSAC over candidate pairs whose tables are on the device (aps_ransac.cu) ------------------------------------
+// The gather and the RANSAC chain of aps_image_matching_sets over n_pairs pairs: pair p's correspondences are
+// d_ptr[p] .. d_ptr[p + 1] of d_rows (packed 1-based match rows, images d_ii[p] / d_jj[p] of d_img_off / d_kp), its
+// samples keyed by d_keys[p] (NULL: p).  Chunks of at most 65535 pairs and about 1 GiB of per-draw tables;
+// ptr_host (may be NULL) lets chunks without correspondences skip the gather.  Outputs are device arrays.
+int ransac_chunks(aps_ctx* c, int64_t n_pairs, int64_t total, const int64_t* d_ptr, const int64_t* ptr_host,
+                  const uint32_t* d_rows, const int32_t* d_ii, const int32_t* d_jj, const int64_t* d_img_off,
+                  const double2* d_kp, const int64_t* d_keys, const uint32_t* samples, int64_t n_draws, uint64_t seed,
+                  double max_distance, double confidence, int max_trials, double* d_models, double* d_minv,
+                  uint8_t* d_inl, int32_t* d_ni, uint8_t* d_acc, int32_t* d_used);
+// pairs one chunk of ransac_chunks holds
+int64_t ransac_chunk_pairs(int64_t n_draws);
+int ransac_params(int64_t n_draws, int max_trials, double confidence);
 
 // ---- match lists: the n x n cell in CSR form -----------------------------------------------------------------------
 struct aps_matchlist {

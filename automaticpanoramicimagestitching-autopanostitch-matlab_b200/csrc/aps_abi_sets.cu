@@ -136,9 +136,9 @@ __global__ void k_sets_fallback_groups(const int32_t* __restrict__ fb, const int
 
 // The pooled pass over the sets listed in `sets` (indices into the call's sets).  The first `ntensor` of them are float
 // sets the single-set call would search on the tensor path: they occupy rows [0, Ft) of the pooled matrix.
-int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std::vector<int64_t>& img_first,
-                const int* set_images, const void* const* desc, const int64_t* counts, int D, int dtype, int layout,
-                int k, double ratio, int mutual, aps_matchlist** out) {
+int pooled_pass_device(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std::vector<int64_t>& img_first,
+                       const int* set_images, const void* const* desc, const int64_t* counts, int D, int dtype,
+                       int layout, int k, double ratio, int mutual, GlobalLists& L) {
   cudaStream_t s = c->stream;
   const int nsets = (int)sets.size();
   // pooled images, offsets and set tables
@@ -162,8 +162,10 @@ int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std
   const int nimg = (int)img_set.size();
   const int64_t F = off.back(), cells = cell_off.back();
   const int64_t Ft = ntensor < nsets ? off[set_img0[ntensor]] : F;  // rows of the tensor-path sets
-  std::vector<int64_t> pp((size_t)cells + 1, 0);
-  std::vector<uint32_t> rows_h;
+  L.order = sets;
+  L.cell_off = cell_off;
+  L.F = F;
+  L.Ft = Ft;
   c->h_flags[32] = c->h_flags[34] = c->h_flags[35] = c->h_flags[37] = 0;
   if (F > 0) {
     for (int i = 0; i < nimg; ++i)
@@ -198,14 +200,17 @@ int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std
       }
     }
     const int esz = dtype == APS_F32 ? 4 : 1;
-    DevBuf<int64_t> d_off, d_cell_off, dir_counts, pair_counts, pair_ptr, rank;
+    DevBuf<int64_t> d_off, d_cell_off, dir_counts, rank;
+    DevBuf<int64_t>& pair_counts = L.counts_buf;
+    DevBuf<int64_t>& pair_ptr = L.ptr_buf;
     DevBuf<int32_t> d_tabs, img_of_row, flags, fb;
     DevBuf<int4> d_groups, fb_groups;
     DevBuf<aps_tc_unit> d_units;
     DevBuf<uint8_t> raw, u8pad, keep;
     DevBuf<float> xn, sq, invn, knn_dist, colscale, colbias, cscore;
     DevBuf<__nv_bfloat16> xb;
-    DevBuf<uint32_t> knn_idx, rows, cidx;
+    DevBuf<uint32_t> knn_idx, cidx;
+    DevBuf<uint32_t>& rows = L.rows_buf;
     DevBuf<int2> records;
     APS_TRY(d_off.alloc((size_t)nimg + 1, s));
     APS_TRY(d_cell_off.alloc((size_t)nsets + 1, s));
@@ -320,16 +325,51 @@ int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std
     APS_TRY(aps_k_global_compact_sets(s, records.p, img_of_row.p, d_off.p, nimg, F, d_img_set, d_set_img0, d_set_n,
                                       d_cell_off.p, nsets, max_n, cells, dir_counts.p, pair_counts.p, pair_ptr.p,
                                       rank.p, rows.p));
-    APS_CUDA(cudaMemcpyAsync(pp.data(), pair_ptr.p, pp.size() * 8, cudaMemcpyDeviceToHost, s));
+    L.pair_counts = pair_counts.p;
+    L.pair_ptr = pair_ptr.p;
+    L.rows = rows.p;
+  }
+  return APS_OK;
+}
+
+// pooled_pass_device, then one download split into the nsets lists
+int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std::vector<int64_t>& img_first,
+                const int* set_images, const void* const* desc, const int64_t* counts, int D, int dtype, int layout,
+                int k, double ratio, int mutual, aps_matchlist** out) {
+  cudaStream_t s = c->stream;
+  const int nsets = (int)sets.size();
+  GlobalLists L;
+  APS_TRY(pooled_pass_device(c, sets, ntensor, img_first, set_images, desc, counts, D, dtype, layout, k, ratio, mutual,
+                             L));
+  const int64_t cells = L.cell_off.back();
+  std::vector<int64_t> pp((size_t)cells + 1, 0);
+  std::vector<uint32_t> rows_h;
+  if (L.F > 0) {
+    APS_CUDA(cudaMemcpyAsync(pp.data(), L.pair_ptr, pp.size() * 8, cudaMemcpyDeviceToHost, s));
     APS_CUDA(cudaStreamSynchronize(s));
     rows_h.resize((size_t)pp[cells] * 2);
     if (pp[cells] > 0) {
-      APS_CUDA(cudaMemcpyAsync(rows_h.data(), rows.p, rows_h.size() * 4, cudaMemcpyDeviceToHost, s));
+      APS_CUDA(cudaMemcpyAsync(rows_h.data(), L.rows, rows_h.size() * 4, cudaMemcpyDeviceToHost, s));
       APS_CUDA(cudaStreamSynchronize(s));
     }
   }
   // one list per set (cells of set j: [cell_off[j], cell_off[j + 1]], rows from pp[cell_off[j]])
-  APS_TRY(sets_split_lists(nsets, pp, rows_h, nullptr, cell_off, set_n.data(), sets.data(), out));
+  std::vector<int> set_n;
+  for (int b : sets) set_n.push_back(set_images[b]);
+  APS_TRY(sets_split_lists(nsets, pp, rows_h, nullptr, L.cell_off, set_n.data(), sets.data(), out));
+  global_lists_stats(c, dtype, L);
+  return APS_OK;
+}
+
+}  // namespace
+
+void global_lists_stats(aps_ctx* c, int dtype, const GlobalLists& L) {
+  const int64_t F = L.F, Ft = L.Ft;
+  if (L.plan) {  // one set: what aps_gplan_download reports (aps_gplan_knn set the rest)
+    if (Ft > 0) c->stats[1] = c->h_flags[32];
+    if (dtype == APS_F32 && F > 0) c->stats[3] = c->h_flags[35];
+    return;
+  }
   // statistics of the call, as the single-set call reports them: rows searched; the engine (tcgen05 when any set took
   // the tensor path); rows its proof left to K2f (no second tensor pass here: first-pass unproven == fallback rows);
   // operands exact for every float row
@@ -339,23 +379,14 @@ int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std
   c->h_flags[34] = c->h_flags[32];
   c->stats[3] = dtype == APS_F32 && F > 0 && (Ft == 0 || c->h_flags[35]) && (F == Ft || c->h_flags[37]);
   c->h_flags[36] = 0;
-  return APS_OK;
 }
 
-}  // namespace
-
-extern "C" int aps_feature_matching_global_sets(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
-                                                const int64_t* counts, int D, int dtype, int layout, int k,
-                                                double ratio, int use_bf, int mutual, aps_matchlist** out) {
-  (void)use_bf;
-  // arguments first (the ids of aps_feature_matching_global), then the device
-  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
-  for (int b = 0; b < nsets; ++b) out[b] = nullptr;
-  std::vector<int64_t> img_first;
+int global_sets_args(int nsets, const int* set_images, const int64_t* counts, int D, int dtype, int k,
+                     std::vector<int64_t>& img_first, std::vector<int64_t>& set_rows) {
   APS_TRY(sets_image_offsets(nsets, set_images, img_first));
   const int64_t nimg = img_first[nsets];
   if (nimg > 0 && !counts) APS_FAIL(APS_ERR_ARGS, "", "counts is NULL");
-  std::vector<int64_t> set_rows((size_t)nsets, 0);
+  set_rows.assign((size_t)nsets, 0);
   int64_t F = 0;
   for (int b = 0; b < nsets; ++b)
     for (int64_t i = img_first[b]; i < img_first[b + 1]; ++i) {
@@ -369,18 +400,54 @@ extern "C" int aps_feature_matching_global_sets(aps_ctx* c, int nsets, const int
   if (k > APS_MAX_K) APS_FAIL(APS_ERR_K, "flann_knn:k", "k must be <= %d in this implementation", APS_MAX_K);
   if (F > 0 && D <= 0) APS_FAIL(APS_ERR_DIM, "flann_knn:dim", "descriptor dimension must be positive");
   if (F >= ((int64_t)1 << 31) - 1) APS_FAIL(APS_ERR_ARGS, "", "more than 2^31 descriptors are not supported");
+  return APS_OK;
+}
+
+// pass order: float sets the single-set call would search on the tensor path first (rows [0, Ft) of the pooled matrix,
+// one tcgen05 unit-table launch), then the sets it would search with the exact engines; returns the tensor sets' number
+static int pass_order(aps_ctx* c, int nsets, const std::vector<int64_t>& set_rows, int D, int dtype, int k,
+                      std::vector<int>& order) {
+  std::vector<int> rest;
+  order.clear();
+  for (int b = 0; b < nsets; ++b)
+    (dtype == APS_F32 && set_rows[b] > 0 && tc_wanted(c, D, set_rows[b], set_rows[b], k) ? order : rest).push_back(b);
+  const int ntensor = (int)order.size();
+  order.insert(order.end(), rest.begin(), rest.end());
+  return ntensor;
+}
+
+int global_lists_device(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
+                        const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D,
+                        int dtype, int layout, int k, double ratio, int mutual, GlobalLists& L) {
+  if (nsets == 1) {  // one set: the single-set call's plan
+    aps_gplan* p = nullptr;
+    APS_TRY(aps_gplan_create(c, counts, set_images[0], D, dtype, k, &p));
+    gplan_lists(p, L);  // L owns the plan from here
+    return gplan_run(p, desc, layout, ratio, mutual);
+  }
+  std::vector<int> order;
+  const int ntensor = pass_order(c, nsets, set_rows, D, dtype, k, order);
+  return pooled_pass_device(c, order, ntensor, img_first, set_images, desc, counts, D, dtype, layout, k, ratio, mutual,
+                            L);
+}
+
+extern "C" int aps_feature_matching_global_sets(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
+                                                const int64_t* counts, int D, int dtype, int layout, int k,
+                                                double ratio, int use_bf, int mutual, aps_matchlist** out) {
+  (void)use_bf;
+  // arguments first (the ids of aps_feature_matching_global), then the device
+  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
+  for (int b = 0; b < nsets; ++b) out[b] = nullptr;
+  std::vector<int64_t> img_first, set_rows;
+  APS_TRY(global_sets_args(nsets, set_images, counts, D, dtype, k, img_first, set_rows));
   APS_CTX(c);
   if (nsets == 0) return APS_OK;
   if (nsets == 1)  // one set: the single-set call itself
     return feature_matching_global_impl(c, desc, counts, set_images[0], D, dtype, layout, k, ratio, mutual, out);
 
-  // one pass for every set: float sets the single-set call would search on the tensor path first (rows [0, Ft) of the
-  // pooled matrix, one tcgen05 unit-table launch), then the sets it would search with the exact engines
-  std::vector<int> order, rest;
-  for (int b = 0; b < nsets; ++b)
-    (dtype == APS_F32 && set_rows[b] > 0 && tc_wanted(c, D, set_rows[b], set_rows[b], k) ? order : rest).push_back(b);
-  const int ntensor = (int)order.size();
-  order.insert(order.end(), rest.begin(), rest.end());
+  // one pass for every set
+  std::vector<int> order;
+  const int ntensor = pass_order(c, nsets, set_rows, D, dtype, k, order);
   const int rc = pooled_pass(c, order, ntensor, img_first, set_images, desc, counts, D, dtype, layout, k, ratio, mutual,
                              out);
   if (rc != APS_OK)

@@ -629,7 +629,7 @@ static int ransac_device(aps_ctx* c, int64_t n_pairs, int64_t total, const int64
   return APS_OK;
 }
 
-static int ransac_params(int64_t n_draws, int max_trials, double confidence) {
+int ransac_params(int64_t n_draws, int max_trials, double confidence) {
   if (n_draws <= 0 || max_trials <= 0) APS_FAIL(APS_ERR_ARGS, "", "n_draws and max_trials must be positive");
   if (!(confidence > 0.0 && confidence < 100.0)) APS_FAIL(APS_ERR_ARGS, "", "confidence must be in (0, 100)");
   return APS_OK;
@@ -741,6 +741,42 @@ extern "C" int aps_image_matching(aps_ctx* c, int n_images, const int64_t* pair_
 static constexpr int64_t kSetsDrawBytes = 16 + 72 + 4 + 8;  // sample table, Htab, cnt, err
 static constexpr int64_t kSetsChunkBytes = (int64_t)1 << 30;
 
+int64_t ransac_chunk_pairs(int64_t n_draws) {
+  const int64_t by_bytes = kSetsChunkBytes / (n_draws * kSetsDrawBytes);
+  return aps_min64(65535, by_bytes > 0 ? by_bytes : 1);
+}
+
+int ransac_chunks(aps_ctx* c, int64_t n_pairs, int64_t total, const int64_t* d_ptr, const int64_t* ptr_host,
+                  const uint32_t* d_rows, const int32_t* d_ii, const int32_t* d_jj, const int64_t* d_img_off,
+                  const double2* d_kp, const int64_t* d_keys, const uint32_t* samples, int64_t n_draws, uint64_t seed,
+                  double max_distance, double confidence, int max_trials, double* d_models, double* d_minv,
+                  uint8_t* d_inl, int32_t* d_ni, uint8_t* d_acc, int32_t* d_used) {
+  if (n_pairs == 0) return APS_OK;
+  const int64_t chunk = ransac_chunk_pairs(n_draws);
+  cudaStream_t s = c->stream;
+  DevBuf<uint32_t> ds;
+  DevBuf<double2> dp1, dp2;
+  const size_t tot = (size_t)(total > 0 ? total : 1);
+  APS_TRY(dp1.alloc(tot, s));
+  APS_TRY(dp2.alloc(tot, s));
+  APS_TRY(ds.alloc((size_t)(aps_min64(chunk, n_pairs) * n_draws * 4), s));
+  for (int64_t p0 = 0; p0 < n_pairs; p0 += chunk) {
+    const int64_t np = aps_min64(chunk, n_pairs - p0);
+    if (ptr_host ? ptr_host[p0 + np] > ptr_host[p0] : total > 0) {
+      k_gather_matched_points<<<dim3(8, (unsigned)np), 256, 0, s>>>(d_ptr + p0, d_rows, d_ii + p0, d_jj + p0,
+                                                                    d_img_off, d_kp, dp1.p, dp2.p);
+      APS_LAUNCHED();
+    }
+    if (samples)
+      APS_CUDA(cudaMemcpyAsync(ds.p, samples + p0 * n_draws * 4, (size_t)(np * n_draws * 4) * 4, cudaMemcpyHostToDevice,
+                               s));
+    APS_TRY(ransac_device(c, np, total, d_ptr + p0, dp1.p, dp2.p, ds.p, samples != nullptr,
+                          d_keys ? d_keys + p0 : nullptr, n_draws, seed, max_distance, confidence, max_trials,
+                          d_models + 9 * p0, d_minv + 9 * p0, d_inl, d_ni + p0, d_acc + p0, d_used + p0));
+  }
+  return APS_OK;
+}
+
 extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_images, const int64_t* const* pair_ptr,
                                        const uint32_t* const* rows, const double* keypoints, const int64_t* img_off,
                                        const int64_t* set_pair_ptr, const int64_t* pairs_lin, double max_distance,
@@ -798,15 +834,14 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
   if (pt_ptr_out)
     for (int64_t p = 0; p <= n_pairs; ++p) pt_ptr_out[p] = ptr[p];
   if (n_pairs == 0) return APS_OK;
-  const int64_t by_bytes = kSetsChunkBytes / (n_draws * kSetsDrawBytes);
-  const int64_t chunk = aps_min64(65535, by_bytes > 0 ? by_bytes : 1);
+  const int64_t chunk = ransac_chunk_pairs(n_draws);
   // one set in one chunk: keys[p] == p, which is what k_ransac_samples takes a NULL key table to mean
   const bool keyed = nsets > 1 || n_pairs > chunk;
   cudaStream_t s = c->stream;
   DevBuf<int64_t> dptr, doff, dkeys;
   DevBuf<int32_t> dii, djj, dni, dused;
-  DevBuf<uint32_t> drows, ds;
-  DevBuf<double2> dkp, dp1, dp2;
+  DevBuf<uint32_t> drows;
+  DevBuf<double2> dkp;
   DevBuf<double> dm, dmi;
   DevBuf<uint8_t> dinl, dacc;
   const size_t tot = (size_t)(total > 0 ? total : 1);
@@ -817,9 +852,6 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
   APS_TRY(djj.alloc((size_t)n_pairs, s));
   APS_TRY(drows.alloc(2 * tot, s));
   APS_TRY(dkp.alloc((size_t)(F > 0 ? F : 1), s));
-  APS_TRY(dp1.alloc(tot, s));
-  APS_TRY(dp2.alloc(tot, s));
-  APS_TRY(ds.alloc((size_t)(aps_min64(chunk, n_pairs) * n_draws * 4), s));
   APS_TRY(dm.alloc((size_t)n_pairs * 9, s));
   APS_TRY(dmi.alloc((size_t)n_pairs * 9, s));
   APS_TRY(dinl.alloc(tot, s));
@@ -835,20 +867,9 @@ extern "C" int aps_image_matching_sets(aps_ctx* c, int nsets, const int* set_ima
     APS_CUDA(cudaMemcpyAsync(drows.p, crow.data(), (size_t)total * 8, cudaMemcpyHostToDevice, s));
     APS_CUDA(cudaMemcpyAsync(dkp.p, keypoints, (size_t)F * 16, cudaMemcpyHostToDevice, s));
   }
-  for (int64_t p0 = 0; p0 < n_pairs; p0 += chunk) {
-    const int64_t np = aps_min64(chunk, n_pairs - p0);
-    if (ptr[p0 + np] > ptr[p0]) {
-      k_gather_matched_points<<<dim3(8, (unsigned)np), 256, 0, s>>>(dptr.p + p0, drows.p, dii.p + p0, djj.p + p0, doff.p,
-                                                                    dkp.p, dp1.p, dp2.p);
-      APS_LAUNCHED();
-    }
-    if (samples)
-      APS_CUDA(cudaMemcpyAsync(ds.p, samples + p0 * n_draws * 4, (size_t)(np * n_draws * 4) * 4, cudaMemcpyHostToDevice,
-                               s));
-    APS_TRY(ransac_device(c, np, total, dptr.p + p0, dp1.p, dp2.p, ds.p, samples != nullptr, keyed ? dkeys.p + p0 : nullptr, n_draws, seed,
-                          max_distance, confidence, max_trials, dm.p + 9 * p0, dmi.p + 9 * p0, dinl.p, dni.p + p0,
-                          dacc.p + p0, dused.p + p0));
-  }
+  APS_TRY(ransac_chunks(c, n_pairs, total, dptr.p, ptr.data(), drows.p, dii.p, djj.p, doff.p, dkp.p,
+                        keyed ? dkeys.p : nullptr, samples, n_draws, seed, max_distance, confidence, max_trials, dm.p,
+                        dmi.p, dinl.p, dni.p, dacc.p, dused.p));
   APS_CUDA(cudaMemcpyAsync(models, dm.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
   APS_CUDA(cudaMemcpyAsync(models_inv, dmi.p, (size_t)n_pairs * 72, cudaMemcpyDeviceToHost, s));
   if (total > 0) APS_CUDA(cudaMemcpyAsync(inliers, dinl.p, (size_t)total, cudaMemcpyDeviceToHost, s));

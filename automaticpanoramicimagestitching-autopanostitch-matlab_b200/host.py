@@ -840,6 +840,13 @@ def selectImagePartnersSets(matchesAllSets, m, ctx=None):
     return out
 
 
+def _check_ransac_projective(input):
+    if str(_field(input, "imageMatchingMethod", "ransac")).lower() != "ransac" or int(_field(input, "useMATLABImageMatching", 0)):
+        raise ValueError("only input.imageMatchingMethod = 'ransac' with useMATLABImageMatching = 0 is built")
+    if str(_field(input, "transformationType", "projective")).lower() != "projective":
+        raise ValueError("only input.transformationType = 'projective' is built")
+
+
 def imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets, seed=0, samples=None, ctx=None):
     """[allMatchesSets, numMatchesSets, tformsSets] = imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets)
 
@@ -857,10 +864,7 @@ def imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets, seed=0, sam
     for v in nums:
         if not (np.isfinite(v) and v >= 0 and v == np.round(v)):
             raise ValueError("every numImgs entry must be a non-negative integer")
-    if str(_field(input, "imageMatchingMethod", "ransac")).lower() != "ransac" or int(_field(input, "useMATLABImageMatching", 0)):
-        raise ValueError("only input.imageMatchingMethod = 'ransac' with useMATLABImageMatching = 0 is built")
-    if str(_field(input, "transformationType", "projective")).lower() != "projective":
-        raise ValueError("only input.transformationType = 'projective' is built")
+    _check_ransac_projective(input)
     ns = [int(v) for v in nums]
     for b, (n, kps, mall) in enumerate(zip(ns, kps_sets, m_sets)):
         if len(mall) != n or any(len(r) != n for r in mall):
@@ -903,6 +907,122 @@ def imageMatchingSets(input, numImgs, keypointsSets, matchesAllSets, seed=0, sam
                                            (models[p], minv[p], inl[t0:t1], ni[p], acc[p], du[p])))
     imageMatchingSets.last = [r[3] for r in result]
     return [r[:3] for r in result]
+
+
+def _global_image_matching(input, allDescriptorsSets, numImgs, keypointsSets, seed, return_matches, ctx, one_set):
+    """featureMatchingGlobal + imageMatching of every set in one call (aps_global_image_matching[_sets]) ->
+    (per set (allMatches, numMatches, tforms), per set `last`, per set match lists or None)"""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by globalImageMatching[Sets]; match the sets on one GPU")
+    _check_ransac_projective(input)
+    ns, _, all_mats, all_counts, kind, D = _pool_descriptor_sets(allDescriptorsSets, numImgs)
+    kps_sets = list(keypointsSets)
+    if len(kps_sets) != len(ns):
+        raise ValueError("keypointsSets must hold one keypoint set per descriptor set")
+    kps = []
+    for b, (n, ks) in enumerate(zip(ns, kps_sets)):
+        if len(ks) != n:
+            raise ValueError(f"keypointsSets[{b}] must contain n elements (one per image).")
+        kps += list(ks)
+    pooled = []
+    for g, (kp, cnt) in enumerate(zip(kps, all_counts)):
+        if cnt:  # images without descriptors take part in no match
+            kp = np.asarray(kp, np.float64).reshape(-1, 2)
+            if kp.shape[0] != cnt:
+                raise ValueError(f"image {g + 1}: the keypoints must have one row per descriptor row")
+            pooled.append(kp)
+    kp = np.ascontiguousarray(np.vstack(pooled)) if pooled else np.zeros((0, 2))
+    k = int(_field(input, "k", required=True))
+    ratio = float(_field(input, "Ratiothreshold", required=True))
+    use_bf = bool(_field(input, "BFMatch", 0))
+    mutual = bool(int(_field(input, "apsMutual", 0)))
+    m = int(_field(input, "mBrownLowe", 6))
+    md, conf, mt = _ransac_params(input)
+    ptrs, cnt, layout, keep = _desc_args(all_mats, all_counts)
+    dtype = APS_U8 if kind else APS_F32
+    B = len(ns)
+    ctx = ctx or default_context()
+    h = C.c_void_p()
+    if one_set:
+        check(lib().aps_global_image_matching(ctx.handle, ptrs, cnt, ns[0], int(D or 0), dtype, layout, k, ratio,
+                                              int(use_bf), int(mutual), _ptr(kp), m, md, conf, mt, int(seed),
+                                              int(return_matches), C.byref(h)))
+    else:
+        check(lib().aps_global_image_matching_sets(ctx.handle, B, (C.c_int * max(B, 1))(*ns), ptrs, cnt, int(D or 0),
+                                                   dtype, layout, k, ratio, int(use_bf), int(mutual), _ptr(kp), m, md,
+                                                   conf, mt, int(seed), int(return_matches), C.byref(h)))
+    try:
+        return _image_matches_result(h, ns, return_matches)
+    finally:
+        lib().aps_image_matches_free(h)
+
+
+def _image_matches_result(h, ns, want_lists):
+    L = lib()
+    P = L.aps_image_matches_pairs(h)
+
+    def arr(p, n, dt):
+        return np.ctypeslib.as_array(p, shape=(n,)).astype(dt) if n else np.zeros(0, dt)
+
+    spp = arr(L.aps_image_matches_set_pair_ptr(h), len(ns) + 1, np.int64)
+    lin = arr(L.aps_image_matches_pairs_lin(h), P, np.int64)
+    pt = arr(L.aps_image_matches_pt_ptr(h), P + 1, np.int64)
+    mp = arr(L.aps_image_matches_match_ptr(h), P + 1, np.int64)
+    rows = arr(L.aps_image_matches_match_rows(h), 2 * int(mp[-1]), np.uint32).reshape(-1, 2).astype(np.float64)
+    models = arr(L.aps_image_matches_models(h), 9 * P, np.float64).reshape(P, 3, 3)
+    minv = arr(L.aps_image_matches_models_inv(h), 9 * P, np.float64).reshape(P, 3, 3)
+    ni = arr(L.aps_image_matches_n_inliers(h), P, np.int32)
+    acc = arr(L.aps_image_matches_accepted(h), P, np.uint8).astype(bool)
+    du = arr(L.aps_image_matches_draws_used(h), P, np.int32)
+    results, lasts = [], []
+    for b, n in enumerate(ns):
+        p0, p1 = int(spp[b]), int(spp[b + 1])
+        allMatches = [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)]
+        numMatches = np.zeros((n, n))
+        tforms = [[None] * n for _ in range(n)]
+        for q in range(p0, p1):
+            if acc[q]:
+                i, j = int(lin[q] % n), int(lin[q] // n)
+                allMatches[i][j] = rows[mp[q]:mp[q + 1]]           # imageMatching.m:148
+                numMatches[i, j] = ni[q]
+                tforms[i][j], tforms[j][i] = models[q], minv[q]   # :150-151, :165-166
+        results.append((allMatches, numMatches, tforms))
+        lasts.append(dict(pairs_lin=lin[p0:p1], pt_ptr=pt[p0:p1 + 1] - pt[p0], n_inliers=ni[p0:p1],
+                          accepted=acc[p0:p1], draws_used=du[p0:p1], models=models[p0:p1], models_inv=minv[p0:p1]))
+    lists = [_cells_from_matchlist(L.aps_image_matches_list(h, b), n)[0] for b, n in enumerate(ns)] if want_lists else None
+    return results, lasts, lists
+
+
+def globalImageMatchingSets(input, allDescriptorsSets, numImgs, keypointsSets, seed=0, return_matches=False, ctx=None):
+    """[allMatchesSets, numMatchesSets, tformsSets] = globalImageMatchingSets(input, allDescriptorsSets, numImgs,
+    keypointsSets)
+
+    featureMatchingGlobalSets followed by imageMatchingSets in one call (aps_global_image_matching_sets): the match
+    lists stay on the device between the two stages.  Set b is allDescriptorsSets[b] / keypointsSets[b] with numImgs[b]
+    images; image i's keypoints have one row per descriptor row (images without descriptors may have any keypoints).
+    Returns a list of B tuples, element b exactly what
+    imageMatchingSets(input, numImgs, keypointsSets, featureMatchingGlobalSets(input, ...), seed=seed)[b] returns.
+    return_matches=True also returns the putative lists, exactly featureMatchingGlobalSets' result:
+    (results, matchesSets).  globalImageMatchingSets.last: per set what imageMatchingSets.last holds, without the
+    per-correspondence `inliers` (the call does not download them).  Device groups (input.apsGPUs) are not supported."""
+    results, globalImageMatchingSets.last, lists = _global_image_matching(
+        input, allDescriptorsSets, numImgs, keypointsSets, seed, return_matches, ctx, one_set=False)
+    return (results, lists) if return_matches else results
+
+
+def globalImageMatching(input, allDescriptors, numImg, keypoints, seed=0, return_matches=False, ctx=None):
+    """[allMatches, numMatches, tforms] = globalImageMatching(input, allDescriptors, numImg, keypoints)
+
+    featureMatchingGlobal followed by imageMatching in one call (aps_global_image_matching, the one-set case of
+    globalImageMatchingSets): the same results as imageMatching(input, numImg, keypoints,
+    featureMatchingGlobal(input, allDescriptors, numImg), seed=seed).  return_matches=True returns
+    ((allMatches, numMatches, tforms), matches).  globalImageMatching.last as globalImageMatchingSets.last[0]."""
+    if not (np.isscalar(numImg) and np.isfinite(numImg) and numImg > 0):
+        raise ValueError("numImg must be a positive finite scalar")  # featureMatchingGlobal.m:35-39
+    results, lasts, lists = _global_image_matching(input, [allDescriptors], [numImg], [keypoints], seed,
+                                                   return_matches, ctx, one_set=True)
+    globalImageMatching.last = lasts[0]
+    return (results[0], lists[0]) if return_matches else results[0]
 
 
 RECORD_PAD = 16384  # APS_RECORD_PAD of include/apsmatch.h: rows the record buffer holds beyond F

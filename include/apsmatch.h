@@ -298,6 +298,59 @@ int aps_image_matching_sets(aps_ctx* ctx, int nsets, const int* set_images, cons
                             uint64_t seed, int64_t* pt_ptr_out, double* models, double* models_inv,
                             uint8_t* inliers, int32_t* n_inliers, uint8_t* accepted, int32_t* draws_used);
 
+/* ---- featureMatchingGlobal followed by imageMatching, in one call -------------------------------------------------
+ * The reference's default run (PP/inputs.m:46, input.matchFeaturesPairwise = 0) calls featureMatchingGlobal
+ * (PP/main.m:98) and then imageMatching (imageMatchingPanoramaConComps.m:40) on each image set.  This entry is the
+ * pair aps_feature_matching_global_sets + aps_image_matching_sets with the match lists kept on the device in between:
+ * partner selection reads the pass's putative counts, the candidate pairs' correspondences are packed from the pass's
+ * rows, RANSAC runs as in aps_image_matching_sets, and allMatches is compacted on the device.  One synchronisation in
+ * the middle (the number of candidate pairs and of correspondences, which size the RANSAC) and one download at the end.
+ *
+ * Arguments: those of aps_feature_matching_global_sets (sets, descriptors, k = input.k, ratio = input.Ratiothreshold,
+ * use_bf, mutual); keypoints = pooled [F x 2] ROW-major doubles of all images of all sets in the same order as the
+ * descriptors, image i holding counts[i] rows (keypoints and descriptors of an image come from the same extractor);
+ * m = input.mBrownLowe; max_distance / confidence / max_trials = input.maxDistance / inliersConfidence / maxIter.
+ * Samples are drawn on the device from `seed`, 2 * max_trials draws per pair (what aps_image_matching_sets draws with
+ * samples = NULL and n_draws = 2 * max_trials).  Argument errors come before the context: the ids of
+ * aps_feature_matching_global_sets (flann_knn:k, flann_knn:type, flann_knn:dim), APS_ERR_ARGS for bad RANSAC parameters
+ * (max_trials <= 0, confidence outside (0, 100)), for keypoints == NULL with F > 0 and for out == NULL.
+ *
+ * *out receives a result to free with aps_image_matches_free, in the caller's set order: set_pair_ptr [nsets + 1],
+ * pairs_lin [pairs] (0-based cell indices inside each set's n_b x n_b block, find() order), pt_ptr [pairs + 1] (each
+ * pair's putative correspondences), models / models_inv [pairs x 9] ROW-major, n_inliers, accepted, draws_used [pairs]:
+ * set b's pairs are set_pair_ptr[b] .. set_pair_ptr[b + 1], and every value is BIT-IDENTICAL to
+ * aps_feature_matching_global_sets followed by aps_select_partners_sets and aps_image_matching_sets with the same
+ * seed (pt_ptr runs over all sets as aps_image_matching_sets' pt_ptr_out does).  match_ptr [pairs + 1] / match_rows
+ * [2 * match_ptr[pairs]]: allMatches{ii,jj} = matches(inliers,:) of each accepted pair (imageMatching.m:148), rows
+ * interleaved as in aps_matchlist_rows; rejected pairs own no rows.  The per-correspondence inlier mask and the putative
+ * rows are not returned; with want_lists != 0, aps_image_matches_list(r, b) is set b's putative match list, equal to
+ * what aps_feature_matching_global_sets returns (NULL otherwise; owned by the result).
+ * Launches and synchronisations do not depend on nsets (more than 65535 candidate pairs add RANSAC chunks);
+ * aps_global_image_matching is the one-set case. */
+typedef struct aps_image_matches aps_image_matches;
+int aps_global_image_matching_sets(aps_ctx* ctx, int nsets, const int* set_images, const void* const* desc,
+                                   const int64_t* counts, int D, int dtype, int layout, int k, double ratio, int use_bf,
+                                   int mutual, const double* keypoints, int m, double max_distance, double confidence,
+                                   int max_trials, uint64_t seed, int want_lists, aps_image_matches** out);
+int aps_global_image_matching(aps_ctx* ctx, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
+                              int layout, int k, double ratio, int use_bf, int mutual, const double* keypoints, int m,
+                              double max_distance, double confidence, int max_trials, uint64_t seed, int want_lists,
+                              aps_image_matches** out);
+int aps_image_matches_nsets(const aps_image_matches* r);
+int64_t aps_image_matches_pairs(const aps_image_matches* r);
+const int64_t* aps_image_matches_set_pair_ptr(const aps_image_matches* r); /* nsets + 1 */
+const int64_t* aps_image_matches_pairs_lin(const aps_image_matches* r);    /* pairs */
+const int64_t* aps_image_matches_pt_ptr(const aps_image_matches* r);       /* pairs + 1 */
+const int64_t* aps_image_matches_match_ptr(const aps_image_matches* r);    /* pairs + 1 */
+const uint32_t* aps_image_matches_match_rows(const aps_image_matches* r);  /* 2 * match_ptr[pairs] */
+const double* aps_image_matches_models(const aps_image_matches* r);        /* pairs x 9 */
+const double* aps_image_matches_models_inv(const aps_image_matches* r);    /* pairs x 9 */
+const int32_t* aps_image_matches_n_inliers(const aps_image_matches* r);
+const uint8_t* aps_image_matches_accepted(const aps_image_matches* r);
+const int32_t* aps_image_matches_draws_used(const aps_image_matches* r);
+const aps_matchlist* aps_image_matches_list(const aps_image_matches* r, int b);
+void aps_image_matches_free(aps_image_matches* r);
+
 /* ---- staged global pipeline (building block of the multi-GPU host; bench.py times these) -----
  * The stages of PP/featureMatching/featureMatchingGlobal.m as separate calls: pooling + normalisation :70-97
  * (create / upload), global kNN :106-120 (knn), per-feature filter loop :123-161 (filter, then compact after the
