@@ -25,6 +25,8 @@ from .host import (  # noqa: F401
     globalImageMatchingSets,
     imageMatchingBatch,
     imageMatchingSets,
+    pairwiseImageMatching,
+    pairwiseImageMatchingSets,
     ransacSampleTable,
     flann_knn_win,
     matchFeaturesScratch,

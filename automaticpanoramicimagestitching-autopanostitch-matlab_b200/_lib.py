@@ -126,6 +126,10 @@ def lib():
                                                  i32, i32, vp, i32, dbl, dbl, i32, C.c_uint64, i32, pp]),
         "aps_global_image_matching": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, i32, dbl, i32, i32, vp, i32, dbl,
                                             dbl, i32, C.c_uint64, i32, pp]),
+        "aps_pairwise_image_matching_sets": (i32, [vp, i32, C.POINTER(i32), pp, C.POINTER(i64), i32, i32, i32, dbl, dbl,
+                                                   i32, i64, C.c_uint64, vp, i32, dbl, dbl, i32, C.c_uint64, i32, pp]),
+        "aps_pairwise_image_matching": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, dbl, dbl, i32, i64, C.c_uint64,
+                                              vp, i32, dbl, dbl, i32, C.c_uint64, i32, pp]),
         "aps_image_matches_nsets": (i32, [vp]),
         "aps_image_matches_pairs": (i64, [vp]),
         "aps_image_matches_set_pair_ptr": (C.POINTER(i64), [vp]),

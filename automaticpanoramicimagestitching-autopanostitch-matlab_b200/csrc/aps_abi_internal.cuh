@@ -1,7 +1,7 @@
 // aps_abi_internal.cuh -- what the translation units behind include/apsmatch.h share (aps_abi.cu: context, kNN entries,
 // staged global pipeline; aps_abi_pairwise.cu: matchFeaturesScratch / featureMatchingPairwise, staged pairwise pipeline,
 // pairwise matching of many image sets; aps_abi_sets.cu: global matching of many image sets; aps_ransac.cu: RANSAC
-// chunks; aps_global_image_matching.cu: global matching through image matching in one call).
+// chunks; aps_global_image_matching.cu: global and pairwise matching through image matching in one call).
 #pragma once
 #include <string>
 #include <vector>
@@ -125,8 +125,10 @@ struct GlobalLists {
   const int64_t* pair_counts = nullptr;  // [cells]
   const int64_t* pair_ptr = nullptr;     // [cells + 1]
   const uint32_t* rows = nullptr;
+  const double* metric = nullptr;        // [rows] pairwise lists' metric (NULL: lists without one)
   DevBuf<int64_t> counts_buf, ptr_buf;   // owners for a pass over several sets
   DevBuf<uint32_t> rows_buf;
+  DevBuf<double> metric_buf;
   aps_gplan* plan = nullptr;             // owner for one set
   int64_t F = 0, Ft = 0;                 // rows searched, rows of the tensor-path sets (statistics)
   GlobalLists() = default;
@@ -148,6 +150,28 @@ void global_lists_stats(aps_ctx* c, int dtype, const GlobalLists& L);
 // The one-set pass (aps_abi.cu): the staged plan from upload to compaction, and its lists handed to L.
 int gplan_run(aps_gplan* p, const void* const* desc, int layout, double ratio, int mutual);
 void gplan_lists(aps_gplan* p, GlobalLists& L);
+
+// ---- pairwise match lists kept on the device (aps_abi_pairwise.cu; aps_pairwise_image_matching_sets) -------------
+// The outputs of one pairwise pass over nsets sets, in the caller's set order: set j's n x n block is cells
+// [cell_off[j], cell_off[j + 1]); rows / metric hold the M match rows in batch order.  The npairs pairs with rows are
+// the table tab = [cell (npairs) | count (npairs) | src (npairs)]: pair q's rows are rows[2 * src[q] ..] and belong to
+// cell cell[q].  Cells no pair names have no rows.
+struct PairwiseRows {
+  std::vector<int64_t> cell_off, tab;
+  int64_t npairs = 0, M = 0;
+  DevBuf<uint32_t> rows;
+  DevBuf<double> metric;
+};
+// Checks the arguments of aps_feature_matching_pairwise_sets (its statuses) and returns the first pooled image of
+// each set.
+int pairwise_sets_args(int nsets, const int* set_images, const int64_t* counts, int D, int dtype, int method,
+                       int64_t subset, std::vector<int64_t>& img_first);
+// The pass of aps_feature_matching_pairwise_sets over every set (one set included) with its lists left on the device
+// in R; the arguments must have passed pairwise_sets_args and the context must be current.  Its only synchronisations
+// are those of the pass (the per-batch match counts among them); the pass's own buffers are released on return.
+int pairwise_rows_device(aps_ctx* c, int nsets, const int* set_images, const void* const* desc, const int64_t* counts,
+                         int nimg, int D, int dtype, int layout, double match_threshold, double max_ratio, int method,
+                         int64_t subset, uint64_t seed, PairwiseRows& R);
 
 // ---- RANSAC over candidate pairs whose tables are on the device (aps_ransac.cu) ------------------------------------
 // The gather and the RANSAC chain of aps_image_matching_sets over n_pairs pairs: pair p's correspondences are

@@ -7,6 +7,7 @@
 #include <climits>
 #include <cstdlib>
 #include <cmath>
+#include <deque>
 #include <limits>
 #include <new>
 
@@ -22,12 +23,17 @@ struct PairRef {
   bool tensor = false; // the tensor engine (screen + tcgen05 candidates + exact re-rank) instead of the exact engine
 };
 // match lists of a pass, pair by pair: pair `ordinal` has cnt[ordinal] rows from row at[ordinal] of rows / metric (rows
-// in batch order; one append per batch, no allocation per pair)
+// in batch order; one append per batch, no allocation per pair).  device: each batch's compacted rows and metric stay
+// in their device buffers d_rows / d_met instead, and `at` counts rows over all batches (M so far).
 struct PairResults {
   std::vector<int32_t> cnt;
   std::vector<int64_t> at;
   std::vector<uint32_t> rows;   // (col1, col2) per match
   std::vector<double> metric;
+  bool device = false;
+  int64_t M = 0;
+  std::deque<DevBuf<uint32_t>> d_rows;
+  std::deque<DevBuf<double>> d_met;
 };
 // 'pca2nn': the rows one pass of the pairwise pipeline reads when they are NOT the set's own -- the query rows of a batch
 // projected with the train images' bases, and the projected train set
@@ -708,14 +714,18 @@ static int pairwise_batch(aps_ctx* c, PairwiseSets& ps, const std::vector<PairRe
   for (int p = 0; p < np; ++p) outoff[p + 1] = outoff[p] + hc[p];
   const int64_t M = outoff[np];
   // rows and metric of the batch land in ONE pinned staging area (a pageable destination is copied through the
-  // driver's bounce buffers at a fraction of the PCIe rate) and are split per pair from there
-  uint8_t* stage = M > 0 ? (uint8_t*)aps_ctx_stage(c, (size_t)M * 16) : nullptr;
-  if (M > 0 && !stage) APS_FAIL(APS_ERR_ALLOC, "", "out of pinned host memory (%lld match rows)", (long long)M);
+  // driver's bounce buffers at a fraction of the PCIe rate) and are split per pair from there; in device mode they
+  // stay in the batch's device buffers
+  uint8_t* stage = M > 0 && !res.device ? (uint8_t*)aps_ctx_stage(c, (size_t)M * 16) : nullptr;
+  if (M > 0 && !res.device && !stage)
+    APS_FAIL(APS_ERR_ALLOC, "", "out of pinned host memory (%lld match rows)", (long long)M);
   const uint32_t* hrows = (const uint32_t*)stage;
-  const double* hmet = (const double*)(stage + (size_t)M * 8);
+  const double* hmet = stage ? (const double*)(stage + (size_t)M * 8) : nullptr;
   if (M > 0) {
-    DevBuf<uint32_t> rows;
-    DevBuf<double> met;
+    DevBuf<uint32_t> rows_host_mode;
+    DevBuf<double> met_host_mode;
+    DevBuf<uint32_t>& rows = res.device ? res.d_rows.emplace_back() : rows_host_mode;
+    DevBuf<double>& met = res.device ? res.d_met.emplace_back() : met_host_mode;
     DevBuf<int64_t> d_outoff;
     APS_TRY(rows.alloc((size_t)M * 2, s));
     APS_TRY(met.alloc((size_t)M, s));
@@ -723,13 +733,19 @@ static int pairwise_batch(aps_ctx* c, PairwiseSets& ps, const std::vector<PairRe
     APS_CUDA(cudaMemcpyAsync(d_outoff.p, outoff.data(), (np + 1) * 8, cudaMemcpyHostToDevice, s));
     k_gather_pairs<<<(unsigned)np, 128, 0, s>>>(matches.p, metric.p, d_eoff.p, d_outoff.p, rows.p, met.p);
     APS_LAUNCHED();
-    APS_CUDA(cudaMemcpyAsync(stage, rows.p, (size_t)M * 8, cudaMemcpyDeviceToHost, s));
-    APS_CUDA(cudaMemcpyAsync(stage + (size_t)M * 8, met.p, (size_t)M * 8, cudaMemcpyDeviceToHost, s));
-    APS_CUDA(cudaStreamSynchronize(s));
+    if (!res.device) {
+      APS_CUDA(cudaMemcpyAsync(stage, rows.p, (size_t)M * 8, cudaMemcpyDeviceToHost, s));
+      APS_CUDA(cudaMemcpyAsync(stage + (size_t)M * 8, met.p, (size_t)M * 8, cudaMemcpyDeviceToHost, s));
+      APS_CUDA(cudaStreamSynchronize(s));
+    }
   }
-  const int64_t base = (int64_t)res.metric.size();
-  res.rows.insert(res.rows.end(), hrows, hrows + 2 * M);
-  res.metric.insert(res.metric.end(), hmet, hmet + M);
+  const int64_t base = res.device ? res.M : (int64_t)res.metric.size();
+  if (res.device) {
+    res.M += M;
+  } else {
+    res.rows.insert(res.rows.end(), hrows, hrows + 2 * M);
+    res.metric.insert(res.metric.end(), hmet, hmet + M);
+  }
   for (int p = 0; p < np; ++p) {
     const size_t o = pairs[p].ordinal;
     res.cnt[o] = hc[p];
@@ -912,14 +928,46 @@ extern "C" int aps_pplan_set_method(aps_pplan* p, int method, int64_t subset, ui
   return APS_OK;
 }
 
+// Device mode of a pass: the batches' rows and metric joined in batch order into dev.rows / dev.metric (one
+// device-to-device copy per batch, the batch buffers released), and the table of the pairs that have rows.
+static int pairwise_join_rows(aps_ctx* c, PairResults& res, const std::vector<int64_t>& cell, PairwiseRows& dev) {
+  cudaStream_t s = c->stream;
+  dev.M = res.M;
+  APS_TRY(dev.rows.alloc((size_t)dev.M * 2, s));
+  APS_TRY(dev.metric.alloc((size_t)dev.M, s));
+  int64_t at = 0;
+  for (size_t b = 0; b < res.d_met.size(); ++b) {
+    const size_t n = res.d_met[b].n;
+    APS_CUDA(cudaMemcpyAsync(dev.rows.p + 2 * at, res.d_rows[b].p, n * 8, cudaMemcpyDeviceToDevice, s));
+    APS_CUDA(cudaMemcpyAsync(dev.metric.p + at, res.d_met[b].p, n * 8, cudaMemcpyDeviceToDevice, s));
+    at += (int64_t)n;
+  }
+  res.d_rows.clear();
+  res.d_met.clear();
+  std::vector<int64_t> src;
+  dev.tab.clear();
+  for (size_t o = 0; o < res.cnt.size(); ++o)
+    if (res.cnt[o] > 0) {
+      dev.tab.push_back(cell[o]);
+      src.push_back(res.at[o]);
+    }
+  dev.npairs = (int64_t)src.size();
+  for (size_t o = 0; o < res.cnt.size(); ++o)
+    if (res.cnt[o] > 0) dev.tab.push_back(res.cnt[o]);
+  dev.tab.insert(dev.tab.end(), src.begin(), src.end());
+  return APS_OK;
+}
+
 // One pass of the pairwise pipeline over an explicit pair list: pairs[o] (ordinal o, pooled image indices, engine) has
 // its list written to cell cell[o] of `m` (m->pair_ptr: ncells + 1 entries; cells no pair names stay empty).  Pairs
 // with an empty side are skipped (matchFeaturesScratch.m:84-88).  The pairs are grouped by view (raw / normalised,
 // :105-110 is a per-pair decision) and engine; tensor groups are screened first, then every group runs in batches of at
-// most ENTRY_BUDGET query rows.  Host work is O(pairs + match rows + ncells).
+// most ENTRY_BUDGET query rows.  Host work is O(pairs + match rows + ncells).  dev != NULL: the lists stay on the
+// device instead (pairwise_rows_device), m is not used and host work is O(pairs + batches).
 static int pairwise_match_pairs(aps_ctx* c, PairwiseSets& ps, const int64_t* counts, int D, int dtype, int method,
                                 double match_threshold, double max_ratio, const std::vector<PairRef>& pairs,
-                                const std::vector<int64_t>& cell, int64_t ncells, aps_matchlist* m) {
+                                const std::vector<int64_t>& cell, int64_t ncells, aps_matchlist* m,
+                                PairwiseRows* dev = nullptr) {
   // float descriptors: 1 = (a2 + b2) - 2 G of nearest2SSDExhaustive; 2 = Euclidean search squared afterwards ('kdtree'
   // = exact KD-tree search, :142-148; 'subsetpdist2', :149-155, whose candidate subset is ALL of B while N2 <= subset)
   const bool pca = dtype == APS_F32 && method == APS_METHOD_APPROX_PCA2NN;
@@ -944,6 +992,7 @@ static int pairwise_match_pairs(aps_ctx* c, PairwiseSets& ps, const int64_t* cou
   PairResults res;
   res.cnt.assign(NP, 0);
   res.at.assign(NP, 0);
+  res.device = dev != nullptr;
   const int64_t ENTRY_BUDGET = (int64_t)1 << 25;  // entries per batch: bounds the candidate buffers to ~2 GB
   for (int g = 0; g < 4 && rc == APS_OK; ++g) {
     const std::vector<PairRef>& gp = grp[g];
@@ -963,6 +1012,7 @@ static int pairwise_match_pairs(aps_ctx* c, PairwiseSets& ps, const int64_t* cou
   }
   auto dbg_t2 = dbg_t ? dbg_now() : dbg_t0;
   if (rc != APS_OK) return rc;
+  if (dev) return pairwise_join_rows(c, res, cell, *dev);
   m->pair_ptr.assign((size_t)ncells + 1, 0);
   for (size_t o = 0; o < NP; ++o) m->pair_ptr[(size_t)cell[o] + 1] = res.cnt[o];
   for (int64_t q = 0; q < ncells; ++q) m->pair_ptr[(size_t)q + 1] += m->pair_ptr[(size_t)q];
@@ -1070,9 +1120,11 @@ extern "C" int aps_feature_matching_pairwise_shard(aps_ctx* c, const void* const
 // dataset folder and once more per connected component; here all sets share ONE pooled plan (one upload, one K1, one
 // train view), one pair list that never crosses a set, and one pass of pairwise_match_pairs -- no host loop over sets
 // issues device work, so launches and synchronisations do not depend on nsets.
+// dev != NULL: the lists stay on the device in *dev (pairwise_rows_device) and out is not used.
 static int pairwise_sets_pass(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
                               const int64_t* counts, int nimg, int D, int dtype, int layout, double match_threshold,
-                              double max_ratio, int method, int64_t subset, uint64_t seed, aps_matchlist** out) {
+                              double max_ratio, int method, int64_t subset, uint64_t seed, aps_matchlist** out,
+                              PairwiseRows* dev = nullptr) {
   // per image: its index in its own set (the key of its 'subsetpdist2' subset); per set: its first cell.  Set b's
   // pairs: its own column-major strict-upper-triangle list, on the engine its single-set call chooses (aps_pplan_create)
   std::vector<int32_t> local((size_t)nimg);
@@ -1123,7 +1175,11 @@ static int pairwise_sets_pass(aps_ctx* c, int nsets, const int* set_images, cons
                                         method == APS_METHOD_APPROX_SUBSETPDIST2 ? subset : 0, seed, local.data()));
     if (dtype == APS_F32 && method == APS_METHOD_APPROX_PCA2NN) APS_TRY(pairwise_build_pca(c, ps, counts, nimg, D));
     APS_TRY(pairwise_match_pairs(c, ps, counts, D, dtype, method, match_threshold, max_ratio, pairs, cell,
-                                 cell_off[nsets], &pooled));
+                                 cell_off[nsets], &pooled, dev));
+  }   // the pass's buffers (ps) are released here: only the lists leave it
+  if (dev) {
+    dev->cell_off = cell_off;
+    return APS_OK;
   }
   // one list per set: cells [cell_off[b], cell_off[b + 1]], rows from pair_ptr[cell_off[b]]
   return sets_split_lists(nsets, pooled.pair_ptr, pooled.rows, &pooled.metric, cell_off, set_images, nullptr, out);
@@ -1137,6 +1193,28 @@ extern "C" int aps_feature_matching_pairwise_sets(aps_ctx* c, int nsets, const i
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
   for (int b = 0; b < nsets; ++b) out[b] = nullptr;
   std::vector<int64_t> img_first;
+  APS_TRY(pairwise_sets_args(nsets, set_images, counts, D, dtype, method, subset, img_first));
+  const int64_t nimg = img_first[nsets];
+  APS_CTX(c);
+  if (nsets == 0) return APS_OK;
+  if (nsets == 1)  // one set: the single-set call itself
+    return feature_matching_pairwise_impl(c, desc, counts, set_images[0], D, dtype, layout, match_threshold, max_ratio,
+                                          method, subset, seed, 0, 1, out);
+  c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
+  c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
+  c->h_flags[32] = 0;   // fallback rows of the call's tensor batches (aps_ctx_last_stats)
+  const int rc = pairwise_sets_pass(c, nsets, set_images, desc, counts, (int)nimg, D, dtype, layout, match_threshold,
+                                    max_ratio, method, subset, seed, out);
+  if (rc != APS_OK)
+    for (int b = 0; b < nsets; ++b) {
+      aps_matchlist_free(out[b]);
+      out[b] = nullptr;
+    }
+  return rc;
+}
+
+int pairwise_sets_args(int nsets, const int* set_images, const int64_t* counts, int D, int dtype, int method,
+                       int64_t subset, std::vector<int64_t>& img_first) {
   APS_TRY(sets_image_offsets(nsets, set_images, img_first));
   const int64_t nimg = img_first[nsets];
   if (nimg > 0 && !counts) APS_FAIL(APS_ERR_ARGS, "", "counts is NULL");
@@ -1155,20 +1233,15 @@ extern "C" int aps_feature_matching_pairwise_sets(aps_ctx* c, int nsets, const i
   if (rows >= ((int64_t)1 << 31) - 512)
     APS_FAIL(APS_ERR_ARGS, "", "%lld pooled descriptor rows (subset views included) exceed the limit of 2^31 - 512",
              (long long)rows);
-  APS_CTX(c);
-  if (nsets == 0) return APS_OK;
-  if (nsets == 1)  // one set: the single-set call itself
-    return feature_matching_pairwise_impl(c, desc, counts, set_images[0], D, dtype, layout, match_threshold, max_ratio,
-                                          method, subset, seed, 0, 1, out);
+  return APS_OK;
+}
+
+int pairwise_rows_device(aps_ctx* c, int nsets, const int* set_images, const void* const* desc, const int64_t* counts,
+                         int nimg, int D, int dtype, int layout, double match_threshold, double max_ratio, int method,
+                         int64_t subset, uint64_t seed, PairwiseRows& R) {
   c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
   c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
-  c->h_flags[32] = 0;   // fallback rows of the call's tensor batches (aps_ctx_last_stats)
-  const int rc = pairwise_sets_pass(c, nsets, set_images, desc, counts, (int)nimg, D, dtype, layout, match_threshold,
-                                    max_ratio, method, subset, seed, out);
-  if (rc != APS_OK)
-    for (int b = 0; b < nsets; ++b) {
-      aps_matchlist_free(out[b]);
-      out[b] = nullptr;
-    }
-  return rc;
+  c->h_flags[32] = 0;
+  return pairwise_sets_pass(c, nsets, set_images, desc, counts, nimg, D, dtype, layout, match_threshold, max_ratio,
+                            method, subset, seed, nullptr, &R);
 }

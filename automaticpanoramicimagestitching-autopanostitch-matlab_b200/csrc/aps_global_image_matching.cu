@@ -1,14 +1,16 @@
-// aps_global_image_matching.cu -- featureMatchingGlobal followed by imageMatching in one call
-// (aps_global_image_matching_sets, include/apsmatch.h).
+// aps_global_image_matching.cu -- featureMatchingGlobal or featureMatchingPairwise followed by imageMatching in one
+// call (aps_global_image_matching_sets, aps_pairwise_image_matching_sets, include/apsmatch.h).
 //
-// The reference's default run (input.matchFeaturesPairwise = 0) calls featureMatchingGlobal and then imageMatching on
-// the same image set.  As two calls, the match lists travel to the host and back: downloaded and split per set, turned
-// into cells, counted and packed again on the host, uploaded again.  Here they stay where the global pass left them:
-//   global pass (aps_feature_matching_global_sets up to its compaction: pair_counts, pair_ptr, rows in pass order) ->
+// The reference calls featureMatchingGlobal (input.matchFeaturesPairwise = 0) or featureMatchingPairwise (= 1) and then
+// imageMatching on the same image set.  As two calls, the match lists travel to the host and back: downloaded and split
+// per set, turned into cells, counted and packed again on the host, uploaded again.  Here they stay on the device:
+//   global pass (aps_feature_matching_global_sets up to its compaction: pair_counts, pair_ptr, rows in pass order), or
+//   pairwise pass (aps_feature_matching_pairwise_sets with each batch's rows kept on the device) -> k_scatter_counts
+//   (pair_counts) -> k_scan_counts (pair_ptr) -> k_place_rows (rows and metric in cell order), then the shared tail:
 //   K6 partner selection directly on pair_counts (k_select_rows / k_select_sym / k_select_compact) ->
 //   k_candidate_tables (images, key, cell and putative count of every candidate pair) -> k_scan_counts (pt_ptr) ->
-//   k_pack_rows (the candidate pairs' match rows, packed) -> the only synchronisation: number of pairs and of
-//   correspondences -> the gather + RANSAC chunks of aps_image_matching_sets -> k_scan_counts (allMatches offsets) ->
+//   k_pack_rows (the candidate pairs' match rows, packed) -> the only synchronisation of the tail: number of pairs and
+//   of correspondences -> the gather + RANSAC chunks of aps_image_matching_sets -> k_scan_counts (allMatches offsets) ->
 //   k_all_matches (rows with the inlier flag set, accepted pairs only) -> one download, reordered into the caller's set
 //   order on the host.
 // A set's candidate pairs are keyed by their index in that set's own list, so pass order changes nothing: every output
@@ -160,6 +162,28 @@ __global__ void __launch_bounds__(256) k_all_matches(const int64_t* __restrict__
   }
 }
 
+// pair_counts[cell[q]] = count[q] for every pair q with rows of a pairwise pass (PairwiseRows::tab); the other cells
+// keep the zero of a memset
+__global__ void k_scatter_counts(const int64_t* __restrict__ tab, int64_t np, int64_t* __restrict__ pair_counts) {
+  const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q < np) pair_counts[tab[q]] = tab[np + q];
+}
+
+// One CTA per pair with rows of a pairwise pass: its rows (and metric, when met != NULL) from batch order to its cell's
+// place pair_ptr[cell] of the cell-ordered lists
+__global__ void __launch_bounds__(128) k_place_rows(const int64_t* __restrict__ tab, int64_t np,
+                                                    const int64_t* __restrict__ pair_ptr,
+                                                    const uint2* __restrict__ src_rows,
+                                                    const double* __restrict__ src_met, uint2* __restrict__ rows,
+                                                    double* __restrict__ met) {
+  const int64_t q = blockIdx.x;
+  const int64_t n = tab[np + q], s0 = tab[2 * np + q], d0 = pair_ptr[tab[q]];
+  for (int64_t t = threadIdx.x; t < n; t += blockDim.x) {
+    rows[d0 + t] = src_rows[s0 + t];
+    if (met) met[d0 + t] = src_met[s0 + t];
+  }
+}
+
 // candidate pairs a set can have at most: every image marks at most min(m, n - 1) partners (imageMatching.m:86-91)
 int64_t pair_bound(const std::vector<int>& ns, int m) {
   int64_t cap = 0;
@@ -207,27 +231,15 @@ void reorder(const std::vector<int>& order, const std::vector<int64_t>& spp, con
   }
 }
 
-int run(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
-        const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D, int dtype,
-        int layout, int k, double ratio, int mutual, const double* keypoints, int m, double max_distance,
-        double confidence, int max_trials, uint64_t seed, int want_lists, aps_image_matches* r) {
+// imageMatching of every set on lists L that are on the device (both entries): partner selection, candidate tables,
+// packed rows, RANSAC, allMatches and the download into r.  F: pooled keypoint rows; row_bound: a bound on the rows of
+// L's lists (sizes the packed correspondences).  With want_lists, r->lists are L's lists (with L.metric when set).
+int match_lists(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
+                const int64_t* counts, int64_t F, const double* keypoints, const GlobalLists& L, int64_t row_bound,
+                int m, double max_distance, double confidence, int max_trials, uint64_t seed, int want_lists,
+                aps_image_matches* r) {
   cudaStream_t s = c->stream;
   const int G = (int)img_first[nsets];
-  int64_t F = 0;
-  for (int64_t F_b : set_rows) F += F_b;
-  GlobalLists L;
-  if (F > 0) {
-    APS_TRY(global_lists_device(c, nsets, set_images, img_first, set_rows, desc, counts, D, dtype, layout, k, ratio,
-                                mutual, L));
-  } else {  // no descriptor anywhere: every putative count is 0 (partner selection still runs, imageMatching.m:75-100)
-    for (int b = 0; b < nsets; ++b) L.order.push_back(b);
-    L.cell_off.assign(1, 0);
-    for (int b = 0; b < nsets; ++b) L.cell_off.push_back(L.cell_off.back() + (int64_t)set_images[b] * set_images[b]);
-    const int64_t cells = L.cell_off.back();
-    APS_TRY(L.counts_buf.alloc((size_t)cells + 1, s));
-    APS_CUDA(cudaMemsetAsync(L.counts_buf.p, 0, ((size_t)cells + 1) * 8, s));
-    L.pair_counts = L.pair_ptr = L.counts_buf.p;  // zero counts, zero offsets
-  }
   const std::vector<int>& order = L.order;
   const int64_t cells = L.cell_off.back();
   std::vector<int> ns;
@@ -271,7 +283,7 @@ int run(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>
   APS_TRY(keys.alloc((size_t)cap, s));
   APS_TRY(cnt.alloc((size_t)cap, s));
   APS_TRY(pt.alloc((size_t)cap + 1, s));
-  APS_TRY(packed.alloc((size_t)(F > 0 ? 2 * F : 2), s));  // a query row yields at most one match row
+  APS_TRY(packed.alloc((size_t)(row_bound > 0 ? 2 * row_bound : 2), s));
   if (cap > 0) {
     k_candidate_tables<<<(unsigned)aps_ceil_div(cap, 256), 256, 0, s>>>(lin.p, sel.p, nsets, cap, t, L.pair_ptr,
                                                                          cell.p, ii.p, jj.p, keys.p, cnt.p);
@@ -279,8 +291,8 @@ int run(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>
   }
   k_scan_counts<<<1, 1024, 0, s>>>(CountOf{cnt.p}, cap, pt.p, sel.p + nt);
   APS_LAUNCHED();
-  if (F > 0 && cap > 0) {
-    k_pack_rows<<<(unsigned)aps_min64(aps_ceil_div(F, 256), 8 * (int64_t)c->sm_count), 256, 0, s>>>(
+  if (row_bound > 0 && cap > 0) {
+    k_pack_rows<<<(unsigned)aps_min64(aps_ceil_div(row_bound, 256), 8 * (int64_t)c->sm_count), 256, 0, s>>>(
         sel.p, nsets, pt.p, cell.p, L.pair_ptr, (const uint2*)L.rows, (uint2*)packed.p);
     APS_LAUNCHED();
   }
@@ -290,7 +302,6 @@ int run(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>
   APS_CUDA(cudaMemcpyAsync(h, sel.p + nsets, 16, cudaMemcpyDeviceToHost, s));
   APS_CUDA(cudaStreamSynchronize(s));
   const int64_t P = h[0], T = h[1];
-  if (F > 0) global_lists_stats(c, dtype, L);
   const size_t tot = (size_t)(T > 0 ? T : 1);
   APS_TRY(models.alloc((size_t)P * 9, s));
   APS_TRY(minv.alloc((size_t)P * 9, s));
@@ -341,20 +352,118 @@ int run(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>
   std::vector<uint32_t> h_am_rows((size_t)(2 * h_am[P]));
   std::vector<int64_t> pp;
   std::vector<uint32_t> rows_h;
+  std::vector<double> met_h;
   if (want_lists) {
     pp.assign(h_pp, h_pp + cells + 1);
     rows_h.resize((size_t)(2 * pp[cells]));
+    if (L.metric) met_h.resize((size_t)pp[cells]);
   }
   if (!h_am_rows.empty())
     APS_CUDA(cudaMemcpyAsync(h_am_rows.data(), am_rows.p, h_am_rows.size() * 4, cudaMemcpyDeviceToHost, s));
   if (!rows_h.empty()) APS_CUDA(cudaMemcpyAsync(rows_h.data(), L.rows, rows_h.size() * 4, cudaMemcpyDeviceToHost, s));
+  if (!met_h.empty()) APS_CUDA(cudaMemcpyAsync(met_h.data(), L.metric, met_h.size() * 8, cudaMemcpyDeviceToHost, s));
   if (!h_am_rows.empty() || !rows_h.empty()) APS_CUDA(cudaStreamSynchronize(s));
   const std::vector<int64_t> spp(h_spp, h_spp + nt);
   reorder(order, spp, h_lin, h_pt, h_am, h_am_rows.data(), h_models, h_minv, h_ni, h_acc, h_used, r);
   if (want_lists) {
     r->lists.assign((size_t)nsets, nullptr);
-    APS_TRY(sets_split_lists(nsets, pp, rows_h, nullptr, L.cell_off, ns.data(), order.data(), r->lists.data()));
+    APS_TRY(sets_split_lists(nsets, pp, rows_h, L.metric ? &met_h : nullptr, L.cell_off, ns.data(), order.data(),
+                             r->lists.data()));
   }
+  return APS_OK;
+}
+
+int run_global(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
+               const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D, int dtype,
+               int layout, int k, double ratio, int mutual, const double* keypoints, int m, double max_distance,
+               double confidence, int max_trials, uint64_t seed, int want_lists, aps_image_matches* r) {
+  cudaStream_t s = c->stream;
+  int64_t F = 0;
+  for (int64_t F_b : set_rows) F += F_b;
+  GlobalLists L;
+  if (F > 0) {
+    APS_TRY(global_lists_device(c, nsets, set_images, img_first, set_rows, desc, counts, D, dtype, layout, k, ratio,
+                                mutual, L));
+  } else {  // no descriptor anywhere: every putative count is 0 (partner selection still runs, imageMatching.m:75-100)
+    for (int b = 0; b < nsets; ++b) L.order.push_back(b);
+    L.cell_off.assign(1, 0);
+    for (int b = 0; b < nsets; ++b) L.cell_off.push_back(L.cell_off.back() + (int64_t)set_images[b] * set_images[b]);
+    const int64_t cells = L.cell_off.back();
+    APS_TRY(L.counts_buf.alloc((size_t)cells + 1, s));
+    APS_CUDA(cudaMemsetAsync(L.counts_buf.p, 0, ((size_t)cells + 1) * 8, s));
+    L.pair_counts = L.pair_ptr = L.counts_buf.p;  // zero counts, zero offsets
+  }
+  // a query row yields at most one match row: F bounds the rows of the lists
+  APS_TRY(match_lists(c, nsets, set_images, img_first, counts, F, keypoints, L, F, m, max_distance, confidence,
+                      max_trials, seed, want_lists, r));
+  if (F > 0) global_lists_stats(c, dtype, L);
+  return APS_OK;
+}
+
+int run_pairwise(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
+                 const void* const* desc, const int64_t* counts, int D, int dtype, int layout, double match_threshold,
+                 double max_ratio, int method, int64_t subset, uint64_t subset_seed, const double* keypoints, int m,
+                 double max_distance, double confidence, int max_trials, uint64_t seed, int want_lists,
+                 aps_image_matches* r) {
+  cudaStream_t s = c->stream;
+  const int nimg = (int)img_first[nsets];
+  int64_t F = 0;
+  for (int g = 0; g < nimg; ++g) F += counts[g];
+  GlobalLists L;
+  for (int b = 0; b < nsets; ++b) L.order.push_back(b);  // the pass keeps the caller's set order
+  int64_t M = 0;
+  {
+    PairwiseRows R;
+    APS_TRY(pairwise_rows_device(c, nsets, set_images, desc, counts, nimg, D, dtype, layout, match_threshold,
+                                 max_ratio, method, subset, subset_seed, R));
+    // the lists in cell order, as GlobalLists: counts scattered into zeroed cells, offsets scanned, rows placed
+    L.cell_off = R.cell_off;
+    const int64_t cells = L.cell_off.back(), np = R.npairs;
+    M = R.M;
+    DevBuf<int64_t> dtab;
+    APS_TRY(L.counts_buf.alloc((size_t)cells + 1, s));
+    APS_TRY(L.ptr_buf.alloc((size_t)cells + 1, s));
+    APS_TRY(L.rows_buf.alloc((size_t)(M > 0 ? 2 * M : 2), s));
+    if (want_lists) APS_TRY(L.metric_buf.alloc((size_t)(M > 0 ? M : 1), s));
+    APS_CUDA(cudaMemsetAsync(L.counts_buf.p, 0, ((size_t)cells + 1) * 8, s));
+    if (np > 0) {
+      APS_TRY(dtab.alloc(R.tab.size(), s));
+      APS_CUDA(cudaMemcpyAsync(dtab.p, R.tab.data(), R.tab.size() * 8, cudaMemcpyHostToDevice, s));
+      k_scatter_counts<<<(unsigned)aps_ceil_div(np, 256), 256, 0, s>>>(dtab.p, np, L.counts_buf.p);
+      APS_LAUNCHED();
+    }
+    k_scan_counts<<<1, 1024, 0, s>>>(CountOf{L.counts_buf.p}, cells, L.ptr_buf.p, nullptr);
+    APS_LAUNCHED();
+    if (np > 0) {
+      k_place_rows<<<(unsigned)np, 128, 0, s>>>(dtab.p, np, L.ptr_buf.p, (const uint2*)R.rows.p, R.metric.p,
+                                                (uint2*)L.rows_buf.p, want_lists ? L.metric_buf.p : nullptr);
+      APS_LAUNCHED();
+    }
+  }  // the batch-ordered rows are released before the RANSAC allocates
+  L.pair_counts = L.counts_buf.p;
+  L.pair_ptr = L.ptr_buf.p;
+  L.rows = L.rows_buf.p;
+  L.metric = want_lists ? L.metric_buf.p : nullptr;
+  // a query row can match once in every pair of its image: the pass's M rows bound the lists
+  return match_lists(c, nsets, set_images, img_first, counts, F, keypoints, L, M, m, max_distance, confidence,
+                     max_trials, seed, want_lists, r);
+}
+
+// a result for nsets sets, filled by fill(r) when nsets > 0; *out set only on success
+template <class Fill>
+int new_result(int nsets, aps_image_matches** out, Fill fill) {
+  aps_image_matches* r = new (std::nothrow) aps_image_matches();
+  if (!r) APS_FAIL(APS_ERR_ALLOC, "", "out of host memory");
+  r->nsets = nsets;
+  r->set_pair_ptr.assign((size_t)nsets + 1, 0);
+  r->pt_ptr.assign(1, 0);
+  r->match_ptr.assign(1, 0);
+  const int rc = nsets > 0 ? fill(r) : APS_OK;
+  if (rc != APS_OK) {
+    delete r;
+    return rc;
+  }
+  *out = r;
   return APS_OK;
 }
 
@@ -376,21 +485,10 @@ extern "C" int aps_global_image_matching_sets(aps_ctx* c, int nsets, const int* 
   for (int64_t F_b : set_rows) F += F_b;
   if (F > 0 && !keypoints) APS_FAIL(APS_ERR_ARGS, "", "keypoints is NULL");
   APS_CTX(c);
-  aps_image_matches* r = new (std::nothrow) aps_image_matches();
-  if (!r) APS_FAIL(APS_ERR_ALLOC, "", "out of host memory");
-  r->nsets = nsets;
-  r->set_pair_ptr.assign((size_t)nsets + 1, 0);
-  r->pt_ptr.assign(1, 0);
-  r->match_ptr.assign(1, 0);
-  const int rc = nsets > 0 ? run(c, nsets, set_images, img_first, set_rows, desc, counts, D, dtype, layout, k, ratio,
-                                 mutual, keypoints, m, max_distance, confidence, max_trials, seed, want_lists, r)
-                           : APS_OK;
-  if (rc != APS_OK) {
-    delete r;
-    return rc;
-  }
-  *out = r;
-  return APS_OK;
+  return new_result(nsets, out, [&](aps_image_matches* r) {
+    return run_global(c, nsets, set_images, img_first, set_rows, desc, counts, D, dtype, layout, k, ratio, mutual,
+                      keypoints, m, max_distance, confidence, max_trials, seed, want_lists, r);
+  });
 }
 
 extern "C" int aps_global_image_matching(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D,
@@ -399,6 +497,39 @@ extern "C" int aps_global_image_matching(aps_ctx* c, const void* const* desc, co
                                          int max_trials, uint64_t seed, int want_lists, aps_image_matches** out) {
   return aps_global_image_matching_sets(c, 1, &n, desc, counts, D, dtype, layout, k, ratio, use_bf, mutual, keypoints,
                                         m, max_distance, confidence, max_trials, seed, want_lists, out);
+}
+
+extern "C" int aps_pairwise_image_matching_sets(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
+                                                const int64_t* counts, int D, int dtype, int layout,
+                                                double match_threshold, double max_ratio, int method, int64_t subset,
+                                                uint64_t subset_seed, const double* keypoints, int m,
+                                                double max_distance, double confidence, int max_trials, uint64_t seed,
+                                                int want_lists, aps_image_matches** out) {
+  // arguments first (the statuses of aps_feature_matching_pairwise_sets, then the RANSAC parameters), then the device
+  std::vector<int64_t> img_first;
+  APS_TRY(pairwise_sets_args(nsets, set_images, counts, D, dtype, method, subset, img_first));
+  APS_TRY(ransac_params(2 * (int64_t)max_trials, max_trials, confidence));
+  int64_t F = 0;
+  for (int64_t g = 0; g < img_first[nsets]; ++g) F += counts[g];
+  if (F > 0 && !keypoints) APS_FAIL(APS_ERR_ARGS, "", "keypoints is NULL");
+  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
+  *out = nullptr;
+  APS_CTX(c);
+  return new_result(nsets, out, [&](aps_image_matches* r) {
+    return run_pairwise(c, nsets, set_images, img_first, desc, counts, D, dtype, layout, match_threshold, max_ratio,
+                        method, subset, subset_seed, keypoints, m, max_distance, confidence, max_trials, seed,
+                        want_lists, r);
+  });
+}
+
+extern "C" int aps_pairwise_image_matching(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D,
+                                           int dtype, int layout, double match_threshold, double max_ratio, int method,
+                                           int64_t subset, uint64_t subset_seed, const double* keypoints, int m,
+                                           double max_distance, double confidence, int max_trials, uint64_t seed,
+                                           int want_lists, aps_image_matches** out) {
+  return aps_pairwise_image_matching_sets(c, 1, &n, desc, counts, D, dtype, layout, match_threshold, max_ratio, method,
+                                          subset, subset_seed, keypoints, m, max_distance, confidence, max_trials,
+                                          seed, want_lists, out);
 }
 
 extern "C" int aps_image_matches_nsets(const aps_image_matches* r) { return r ? r->nsets : 0; }

@@ -402,8 +402,8 @@ def featureMatchingPairwiseSets(input, allDescriptorsSets, numImgs, ctx=None, re
     ratio = float(_field(input, "Ratiothreshold", required=True))
 
     def empty_cells(n):   # featureMatchingPairwise on a set without descriptors: cell(numImg), no device touched
-        m = [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)]
-        return (m, [[None] * n for _ in range(n)]) if return_metric else m
+        m, metrics = _empty_pairwise_cells(n)
+        return (m, metrics) if return_metric else m
 
     B = len(ns)
     if kind is None:
@@ -421,13 +421,24 @@ def featureMatchingPairwiseSets(input, allDescriptorsSets, numImgs, ctx=None, re
             if empty[b]:
                 result.append(empty_cells(ns[b]))
                 continue
-            matches, metrics, _, _ = _cells_from_matchlist(outs[b], ns[b], want_metric=True)
-            _fill_upper_cells(matches, ns[b])
+            matches, metrics = _pairwise_cells(outs[b], ns[b])
             result.append((matches, metrics) if return_metric else matches)
     finally:
         for b in range(B):
             lib().aps_matchlist_free(outs[b])
     return result
+
+
+def _empty_pairwise_cells(n):
+    """featureMatchingPairwise's (matches, metrics) of a set without descriptors: cell(numImg)"""
+    return [[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)], [[None] * n for _ in range(n)]
+
+
+def _pairwise_cells(h, n):
+    """(matches, metrics) of a pairwise match list as featureMatchingPairwise returns them"""
+    matches, metrics, _, _ = _cells_from_matchlist(h, n, want_metric=True)
+    _fill_upper_cells(matches, n)
+    return matches, metrics
 
 
 def _fill_upper_cells(matches, n):
@@ -916,22 +927,7 @@ def _global_image_matching(input, allDescriptorsSets, numImgs, keypointsSets, se
         raise ValueError("input.apsGPUs is not supported by globalImageMatching[Sets]; match the sets on one GPU")
     _check_ransac_projective(input)
     ns, _, all_mats, all_counts, kind, D = _pool_descriptor_sets(allDescriptorsSets, numImgs)
-    kps_sets = list(keypointsSets)
-    if len(kps_sets) != len(ns):
-        raise ValueError("keypointsSets must hold one keypoint set per descriptor set")
-    kps = []
-    for b, (n, ks) in enumerate(zip(ns, kps_sets)):
-        if len(ks) != n:
-            raise ValueError(f"keypointsSets[{b}] must contain n elements (one per image).")
-        kps += list(ks)
-    pooled = []
-    for g, (kp, cnt) in enumerate(zip(kps, all_counts)):
-        if cnt:  # images without descriptors take part in no match
-            kp = np.asarray(kp, np.float64).reshape(-1, 2)
-            if kp.shape[0] != cnt:
-                raise ValueError(f"image {g + 1}: the keypoints must have one row per descriptor row")
-            pooled.append(kp)
-    kp = np.ascontiguousarray(np.vstack(pooled)) if pooled else np.zeros((0, 2))
+    kp = _pool_set_keypoints(keypointsSets, ns, all_counts)
     k = int(_field(input, "k", required=True))
     ratio = float(_field(input, "Ratiothreshold", required=True))
     use_bf = bool(_field(input, "BFMatch", 0))
@@ -957,7 +953,30 @@ def _global_image_matching(input, allDescriptorsSets, numImgs, keypointsSets, se
         lib().aps_image_matches_free(h)
 
 
-def _image_matches_result(h, ns, want_lists):
+def _pool_set_keypoints(keypointsSets, ns, all_counts):
+    """the keypoints of every set's images, pooled [F x 2] row-major as the descriptors are (image g: all_counts[g]
+    rows; images without descriptors take part in no match and contribute none)"""
+    kps_sets = list(keypointsSets)
+    if len(kps_sets) != len(ns):
+        raise ValueError("keypointsSets must hold one keypoint set per descriptor set")
+    kps = []
+    for b, (n, ks) in enumerate(zip(ns, kps_sets)):
+        if len(ks) != n:
+            raise ValueError(f"keypointsSets[{b}] must contain n elements (one per image).")
+        kps += list(ks)
+    pooled = []
+    for g, (kp, cnt) in enumerate(zip(kps, all_counts)):
+        if cnt:
+            kp = np.asarray(kp, np.float64).reshape(-1, 2)
+            if kp.shape[0] != cnt:
+                raise ValueError(f"image {g + 1}: the keypoints must have one row per descriptor row")
+            pooled.append(kp)
+    return np.ascontiguousarray(np.vstack(pooled)) if pooled else np.zeros((0, 2))
+
+
+def _image_matches_result(h, ns, want_lists, list_of=lambda lh, b, n: _cells_from_matchlist(lh, n)[0]):
+    """the aps_image_matches result h of ns sets -> (per set (allMatches, numMatches, tforms), per set `last`, per set
+    list_of(list handle, b, n) or None)"""
     L = lib()
     P = L.aps_image_matches_pairs(h)
 
@@ -989,7 +1008,7 @@ def _image_matches_result(h, ns, want_lists):
         results.append((allMatches, numMatches, tforms))
         lasts.append(dict(pairs_lin=lin[p0:p1], pt_ptr=pt[p0:p1 + 1] - pt[p0], n_inliers=ni[p0:p1],
                           accepted=acc[p0:p1], draws_used=du[p0:p1], models=models[p0:p1], models_inv=minv[p0:p1]))
-    lists = [_cells_from_matchlist(L.aps_image_matches_list(h, b), n)[0] for b, n in enumerate(ns)] if want_lists else None
+    lists = [list_of(L.aps_image_matches_list(h, b), b, n) for b, n in enumerate(ns)] if want_lists else None
     return results, lasts, lists
 
 
@@ -1026,6 +1045,81 @@ def globalImageMatching(input, allDescriptors, numImg, keypoints, seed=0, return
 
 
 RECORD_PAD = 16384  # APS_RECORD_PAD of include/apsmatch.h: rows the record buffer holds beyond F
+
+
+def _pairwise_image_matching(input, allDescriptorsSets, numImgs, keypointsSets, seed, return_matches, ctx, one_set):
+    """featureMatchingPairwise + imageMatching of every set in one call (aps_pairwise_image_matching[_sets]) ->
+    (per set (allMatches, numMatches, tforms), per set `last`, per set (matches, metrics) or None)"""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by pairwiseImageMatching[Sets]; match the sets on one GPU")
+    _check_ransac_projective(input)
+    ns, empty, all_mats, all_counts, kind, D = _pool_descriptor_sets(allDescriptorsSets, numImgs)
+    kp = _pool_set_keypoints(keypointsSets, ns, all_counts)
+    method = str(_field(input, "Matchingmethod", "Exhaustive")).lower()
+    if method not in ("exhaustive", "approximate"):
+        raise ValueError(f"Unknown Method: {method}")  # matchFeaturesScratch.m:164-165
+    aps_method = _resolve_method(input, method)
+    thr = float(_field(input, "Matchingthreshold", required=True))
+    ratio = float(_field(input, "Ratiothreshold", required=True))
+    subset, subset_seed = int(_field(input, "apsSubset", 12000)), int(_field(input, "apsSeed", 0))
+    m = int(_field(input, "mBrownLowe", 6))
+    md, conf, mt = _ransac_params(input)
+    ptrs, cnt, layout, keep = _desc_args(all_mats, all_counts)
+    dtype = APS_U8 if kind else APS_F32
+    B = len(ns)
+    ctx = ctx or default_context()
+    h = C.c_void_p()
+    tail = (thr, ratio, aps_method, subset, subset_seed, _ptr(kp), m, md, conf, mt, int(seed), int(return_matches),
+            C.byref(h))
+    if one_set:
+        check(lib().aps_pairwise_image_matching(ctx.handle, ptrs, cnt, ns[0], int(D or 0), dtype, layout, *tail))
+    else:
+        check(lib().aps_pairwise_image_matching_sets(ctx.handle, B, (C.c_int * max(B, 1))(*ns), ptrs, cnt, int(D or 0),
+                                                     dtype, layout, *tail))
+
+    def list_of(lh, b, n):   # what featureMatchingPairwiseSets(..., return_metric=True) returns for set b
+        return _empty_pairwise_cells(n) if empty[b] else _pairwise_cells(lh, n)
+
+    try:
+        return _image_matches_result(h, ns, return_matches, list_of)
+    finally:
+        lib().aps_image_matches_free(h)
+
+
+def pairwiseImageMatchingSets(input, allDescriptorsSets, numImgs, keypointsSets, seed=0, return_matches=False,
+                              ctx=None):
+    """[allMatchesSets, numMatchesSets, tformsSets] = pairwiseImageMatchingSets(input, allDescriptorsSets, numImgs,
+    keypointsSets)
+
+    featureMatchingPairwiseSets followed by imageMatchingSets in one call (aps_pairwise_image_matching_sets): the match
+    lists stay on the device between the two stages.  Reads the fields featureMatchingPairwiseSets reads
+    (Matchingmethod, ApproxFloatNNMethod, Matchingthreshold, Ratiothreshold, apsSubset, apsSeed; the same warning for
+    useMATLABFeatureMatch=1) and those imageMatchingSets reads (mBrownLowe, maxDistance, inliersConfidence, maxIter).
+    Returns a list of B tuples, element b exactly what
+    imageMatchingSets(input, numImgs, keypointsSets, featureMatchingPairwiseSets(input, ...), seed=seed)[b] returns.
+    return_matches=True also returns the putative lists with their metric, exactly
+    featureMatchingPairwiseSets(input, ..., return_metric=True): (results, matchesSets).
+    pairwiseImageMatchingSets.last: per set what imageMatchingSets.last holds, without the per-correspondence
+    `inliers`.  Device groups (input.apsGPUs) are not supported."""
+    results, pairwiseImageMatchingSets.last, lists = _pairwise_image_matching(
+        input, allDescriptorsSets, numImgs, keypointsSets, seed, return_matches, ctx, one_set=False)
+    return (results, lists) if return_matches else results
+
+
+def pairwiseImageMatching(input, allDescriptors, numImg, keypoints, seed=0, return_matches=False, ctx=None):
+    """[allMatches, numMatches, tforms] = pairwiseImageMatching(input, allDescriptors, numImg, keypoints)
+
+    featureMatchingPairwise followed by imageMatching in one call (aps_pairwise_image_matching, the one-set case of
+    pairwiseImageMatchingSets): the same results as imageMatching(input, numImg, keypoints,
+    featureMatchingPairwise(input, allDescriptors, numImg), seed=seed).  return_matches=True returns
+    ((allMatches, numMatches, tforms), (matches, metrics)).  pairwiseImageMatching.last as
+    pairwiseImageMatchingSets.last[0]."""
+    if not (np.isscalar(numImg) and np.isfinite(numImg) and numImg > 0):
+        raise ValueError("numImg must be a positive finite scalar")
+    results, lasts, lists = _pairwise_image_matching(input, [allDescriptors], [numImg], [keypoints], seed,
+                                                     return_matches, ctx, one_set=True)
+    pairwiseImageMatching.last = lasts[0]
+    return (results[0], lists[0]) if return_matches else results[0]
 
 
 def _csr_from_matchlist(h, n):

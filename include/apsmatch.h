@@ -351,6 +351,40 @@ const int32_t* aps_image_matches_draws_used(const aps_image_matches* r);
 const aps_matchlist* aps_image_matches_list(const aps_image_matches* r, int b);
 void aps_image_matches_free(aps_image_matches* r);
 
+/* ---- featureMatchingPairwise followed by imageMatching, in one call -----------------------------------------------
+ * With input.matchFeaturesPairwise = 1 the reference calls featureMatchingPairwise (PP/main.m:95-99) and then
+ * imageMatching (imageMatchingPanoramaConComps.m:40) on each image set.  This entry is the pair
+ * aps_feature_matching_pairwise_sets + aps_image_matching_sets with the match lists kept on the device in between: the
+ * pairwise pass keeps each batch's compacted rows and metric on the device (only each batch's per-pair match counts
+ * are downloaded, they size the compaction), the lists are laid out in cells on the device, and from there the call
+ * runs as aps_global_image_matching_sets does: partner selection on the putative counts, the candidate pairs'
+ * correspondences packed on the device, RANSAC, allMatches compacted on the device, one download at the end.
+ *
+ * Arguments: those of aps_feature_matching_pairwise_sets (sets, descriptors, match_threshold = input.Matchingthreshold,
+ * max_ratio = input.Ratiothreshold, method / subset / subset_seed as there), then keypoints, m, max_distance,
+ * confidence, max_trials, seed and want_lists as for aps_global_image_matching_sets.  Argument errors come before the
+ * context: first the statuses of aps_feature_matching_pairwise_sets (APS_ERR_TYPE, APS_ERR_METHOD, APS_ERR_ARGS for
+ * nsets < 0, a negative count, subset < 1 or pooled rows reaching 2^31 - 512, APS_ERR_DIM), then APS_ERR_ARGS for bad
+ * RANSAC parameters (max_trials <= 0, confidence outside (0, 100)), for keypoints == NULL with rows and for out == NULL.
+ *
+ * *out receives an aps_image_matches result as described above, every value BIT-IDENTICAL to
+ * aps_feature_matching_pairwise_sets followed by aps_select_partners_sets and aps_image_matching_sets with the same
+ * seeds.  With want_lists != 0, aps_image_matches_list(r, b) is set b's putative list with its metric, equal to what
+ * aps_feature_matching_pairwise_sets returns for set b.
+ * Launches do not depend on nsets (more than 65535 candidate pairs add RANSAC chunks).  Synchronisations: those of the
+ * pairwise pass (its per-batch match counts among them), one in the middle (the number of candidate pairs and of
+ * correspondences) and the final download.  aps_pairwise_image_matching is the one-set case. */
+int aps_pairwise_image_matching_sets(aps_ctx* ctx, int nsets, const int* set_images, const void* const* desc,
+                                     const int64_t* counts, int D, int dtype, int layout, double match_threshold,
+                                     double max_ratio, int method, int64_t subset, uint64_t subset_seed,
+                                     const double* keypoints, int m, double max_distance, double confidence,
+                                     int max_trials, uint64_t seed, int want_lists, aps_image_matches** out);
+int aps_pairwise_image_matching(aps_ctx* ctx, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
+                                int layout, double match_threshold, double max_ratio, int method, int64_t subset,
+                                uint64_t subset_seed, const double* keypoints, int m, double max_distance,
+                                double confidence, int max_trials, uint64_t seed, int want_lists,
+                                aps_image_matches** out);
+
 /* ---- staged global pipeline (building block of the multi-GPU host; bench.py times these) -----
  * The stages of PP/featureMatching/featureMatchingGlobal.m as separate calls: pooling + normalisation :70-97
  * (create / upload), global kNN :106-120 (knn), per-feature filter loop :123-161 (filter, then compact after the

@@ -26,27 +26,7 @@ function matchesSets = featureMatchingPairwiseSets(input, allDescriptorsSets, nu
         allDescriptorsSets cell
         numImgs (1, :) {mustBeNumeric, mustBeFinite, mustBePositive, mustBeInteger}
     end
-    % Nothing may change the match lists silently: input.apsAcceptScratchSemantics = 1 acknowledges.
-    accept = isfield(input, 'apsAcceptScratchSemantics') && input.apsAcceptScratchSemantics;
-    if ~accept && isfield(input, 'useMATLABFeatureMatch') && input.useMATLABFeatureMatch == 1
-        warning('apsmatch:semantics', ['input.useMATLABFeatureMatch = 1 selects MathWorks matchFeatures in the ' ...
-            'reference; this GPU path runs the matchFeaturesScratch semantics (featureMatchingPairwise.m:108-117).']);
-    end
-    method = 0;                                          % aps_method: 0 exhaustive, 1 subsetpdist2, 2 kdtree, 3 pca2nn
-    if isfield(input, 'Matchingmethod') && strcmpi(input.Matchingmethod, 'Approximate')
-        nn = 'pca2nn';                                   % parser default, matchFeaturesScratch.m:75
-        if isfield(input, 'ApproxFloatNNMethod'); nn = lower(char(input.ApproxFloatNNMethod)); end
-        switch nn
-            case 'subsetpdist2'
-                method = 1;
-            case 'kdtree'
-                method = 2;
-            case 'pca2nn'
-                method = 3;
-            otherwise
-                error('Select a approximate method');
-        end
-    end
+    method = apsPairwiseMethod(input);                  % aps_method, with the semantics warning
     matchesSets = aps_featureMatching_mex('pairwisesets', allDescriptorsSets, numImgs, input.Matchingthreshold, ...
         input.Ratiothreshold, method);
 end

@@ -140,6 +140,118 @@ static inline mxArray* aps_mex_cells(const aps_matchlist* ml, int n, bool fill_u
     }
   return out;
 }
+// The sets of the gateways that match and verify in one call (aps_globalImageMatching_mex, aps_pairwiseImageMatching_mex):
+// descSets{b} (1 x n_b cell of descriptor matrices or binaryFeatures), numImgs(b) and keypointsSets{b} (1 x n_b cell of
+// [Ni x 2] double, one row per descriptor row), checked before any device is touched.  Every image of every set one
+// after another in ptrs / counts, their keypoints pooled row-major in kp; dtype < 0 when every set is empty, and
+// empty[b] marks a set without descriptors.
+struct aps_mex_image_sets {
+  std::vector<int> ns;
+  std::vector<bool> empty;
+  std::vector<const void*> ptrs;
+  std::vector<int64_t> counts;
+  std::vector<double> kp;
+  std::vector<std::vector<float>> converted;
+  int dtype = -1, D = 0;
+};
+static inline void aps_mex_collect_image_sets(const mxArray* sets, const mxArray* nums, const mxArray* kps,
+                                              aps_mex_image_sets& S) {
+  if (!mxIsCell(sets) || !mxIsCell(kps))
+    mexErrMsgIdAndTxt("apsmatch:args", "descSets and keypointsSets must be cell arrays");
+  const int B = (int)mxGetNumberOfElements(sets);
+  if (!mxIsDouble(nums) || (int)mxGetNumberOfElements(nums) != B || (int)mxGetNumberOfElements(kps) != B)
+    mexErrMsgIdAndTxt("apsmatch:args", "numImgs and keypointsSets must hold one element per descriptor set");
+  S.ns.assign((size_t)B, 0);
+  S.empty.assign((size_t)B, true);
+  for (int b = 0; b < B; ++b) {
+    const double nb = mxGetPr(nums)[b];
+    const mxArray *db = mxGetCell(sets, b), *kb = mxGetCell(kps, b);
+    if (!(nb >= 1 && nb == (double)(int)nb)) mexErrMsgIdAndTxt("apsmatch:args", "numImgs must hold positive integers");
+    const int n = (int)nb;
+    if (!db || !kb || !mxIsCell(db) || !mxIsCell(kb))
+      mexErrMsgIdAndTxt("apsmatch:args", "set %d: descriptors and keypoints must be cell arrays", b + 1);
+    if ((int)mxGetNumberOfElements(kb) != n)
+      mexErrMsgIdAndTxt("apsmatch:args", "set %d: keypoints must contain n elements (one per image).", b + 1);
+    S.ns[b] = n;
+    std::vector<const void*> p;
+    std::vector<int64_t> c;
+    int dt = -1, Db = 0;
+    aps_mex_collect(db, n, p, c, dt, Db, S.converted);
+    if (dt >= 0) {
+      if (S.dtype >= 0 && dt != S.dtype)
+        mexErrMsgIdAndTxt("flann_knn:type", "all descriptor sets must have the same class");
+      if (S.dtype >= 0 && Db != S.D) mexErrMsgIdAndTxt("flann_knn:dim", "all descriptor sets must have the same width");
+      S.dtype = dt;
+      S.D = Db;
+      S.empty[b] = false;
+    }
+    for (int i = 0; i < n; ++i) {
+      if (c[i] == 0) continue;  // an image without descriptors takes part in no match
+      const mxArray* k = mxGetCell(kb, i);
+      if (!k || !mxIsDouble(k) || mxGetN(k) != 2 || (int64_t)mxGetM(k) != c[i])
+        mexErrMsgIdAndTxt("apsmatch:args", "set %d: keypoints{%d} must be [Ni x 2] double with one row per descriptor",
+                          b + 1, i + 1);
+      const double* d = mxGetPr(k);
+      for (int64_t r = 0; r < c[i]; ++r) {
+        S.kp.push_back(d[r]);
+        S.kp.push_back(d[r + c[i]]);
+      }
+    }
+    S.ptrs.insert(S.ptrs.end(), p.begin(), p.end());
+    S.counts.insert(S.counts.end(), c.begin(), c.end());
+  }
+}
+// The 1 x B outputs allMatchesSets, numMatchesSets, tformsSets (imageMatching.m:148-166) of an aps_image_matches
+// result r (NULL: no set) for the sets ns: allMatches{c} = the accepted pair's inlier rows, numMatches(c) = n_inliers,
+// tforms{i,j} = model (maps image j to image i), tforms{j,i} = its inverse.
+static inline void aps_mex_image_matches_outputs(int nlhs, mxArray* plhs[], const std::vector<int>& ns,
+                                                 const aps_image_matches* r) {
+  const int B = (int)ns.size();
+  mxArray* allM = mxCreateCellMatrix(1, (mwSize)B);
+  mxArray* numM = mxCreateCellMatrix(1, (mwSize)B);
+  mxArray* tfs = mxCreateCellMatrix(1, (mwSize)B);
+  for (int b = 0; b < B; ++b) {
+    mxSetCell(allM, b, mxCreateCellMatrix((mwSize)ns[b], (mwSize)ns[b]));
+    mxSetCell(numM, b, mxCreateDoubleMatrix((mwSize)ns[b], (mwSize)ns[b], mxREAL));
+    mxSetCell(tfs, b, mxCreateCellMatrix((mwSize)ns[b], (mwSize)ns[b]));
+  }
+  plhs[0] = allM;
+  if (nlhs > 1) plhs[1] = numM;
+  if (nlhs > 2) plhs[2] = tfs;
+  if (!r) return;
+  const int64_t* spp = aps_image_matches_set_pair_ptr(r);
+  const int64_t* lin = aps_image_matches_pairs_lin(r);
+  const int64_t* mp = aps_image_matches_match_ptr(r);
+  const uint32_t* rows = aps_image_matches_match_rows(r);
+  const double* models = aps_image_matches_models(r);
+  const double* minv = aps_image_matches_models_inv(r);
+  const int32_t* ni = aps_image_matches_n_inliers(r);
+  const uint8_t* acc = aps_image_matches_accepted(r);
+  for (int b = 0; b < B; ++b) {
+    const int64_t n = ns[b];
+    mxArray *am = mxGetCell(allM, b), *tf = mxGetCell(tfs, b);
+    double* nm = mxGetPr(mxGetCell(numM, b));
+    for (int64_t p = spp[b]; p < spp[b + 1]; ++p) {  // imageMatching.m:148-166
+      if (!acc[p]) continue;
+      const int64_t c = lin[p], i = c % n, j = c / n, m = mp[p + 1] - mp[p];
+      mxArray* a = mxCreateDoubleMatrix((mwSize)m, 2, mxREAL);
+      for (int64_t q = 0; q < m; ++q) {
+        mxGetPr(a)[q] = (double)rows[2 * (mp[p] + q)];
+        mxGetPr(a)[q + m] = (double)rows[2 * (mp[p] + q) + 1];
+      }
+      mxSetCell(am, (mwIndex)c, a);
+      nm[c] = (double)ni[p];
+      mxArray *t1 = mxCreateDoubleMatrix(3, 3, mxREAL), *t2 = mxCreateDoubleMatrix(3, 3, mxREAL);
+      for (int rr = 0; rr < 3; ++rr)
+        for (int cc = 0; cc < 3; ++cc) {  // row-major -> MATLAB column-major
+          mxGetPr(t1)[rr + 3 * cc] = models[9 * p + 3 * rr + cc];
+          mxGetPr(t2)[rr + 3 * cc] = minv[9 * p + 3 * rr + cc];
+        }
+      mxSetCell(tf, (mwIndex)(i + j * n), t1);
+      mxSetCell(tf, (mwIndex)(j + i * n), t2);
+    }
+  }
+}
 // "" or " (set b)" after a gateway message: the sets gateway names the set (1-based), the single-set one does not
 static inline std::string aps_mex_in_set(int set) {
   return set > 0 ? " (set " + std::to_string(set) + ")" : std::string();

@@ -179,6 +179,30 @@ static int file_mode(const char* in_path, const char* out_path) {
       outs.push_back(mxGetCell(out[1], (mwIndex)b));
       for (int c = 0; c < n * n; ++c) outs.push_back(mxGetCell(mxGetCell(out[2], (mwIndex)b), (mwIndex)c));
     }
+#elif defined(GATE_PIMATCH)  // scalars: B, numImgs(1..B), matchThreshold, maxRatio, method, m, maxDistance, confidence,
+    // maxIter, seed ; matrices and outputs as GATE_GIMATCH
+    const int B = (int)sc[0];
+    mxArray *ds = mxCreateCellMatrix(1, (mwSize)B), *kps = mxCreateCellMatrix(1, (mwSize)B);
+    mxArray* nums = mxCreateDoubleMatrix(1, (mwSize)B, mxREAL);
+    for (int b = 0, m0 = 0; b < B; ++b) {
+      const int n = (int)sc[1 + b];
+      mxGetPr(nums)[b] = n;
+      mxArray *dc = mxCreateCellMatrix(1, (mwSize)n), *kc = mxCreateCellMatrix(1, (mwSize)n);
+      for (int i = 0; i < n; ++i) mxSetCell(dc, (mwIndex)i, mats[m0++]);
+      for (int i = 0; i < n; ++i) mxSetCell(kc, (mwIndex)i, mats[m0++]);
+      mxSetCell(ds, (mwIndex)b, dc);
+      mxSetCell(kps, (mwIndex)b, kc);
+    }
+    const double* t = sc.data() + 1 + B;  // matchThreshold, maxRatio, method, m, maxDistance, confidence, maxIter, seed
+    std::vector<const mxArray*> in = {ds, nums, kps};
+    for (int i = 0; i < 8; ++i) in.push_back(mxCreateDoubleScalar(t[i]));
+    mexFunction(3, out, (int)in.size(), in.data());
+    for (int b = 0; b < B; ++b) {
+      const int n = (int)sc[1 + b];
+      for (int c = 0; c < n * n; ++c) outs.push_back(mxGetCell(mxGetCell(out[0], (mwIndex)b), (mwIndex)c));
+      outs.push_back(mxGetCell(out[1], (mwIndex)b));
+      for (int c = 0; c < n * n; ++c) outs.push_back(mxGetCell(mxGetCell(out[2], (mwIndex)b), (mwIndex)c));
+    }
 #else
     (void)out;
     return 3;
@@ -515,6 +539,69 @@ int main(int argc, char** argv) {
     bad += !(mxGetM(mxGetCell(out[0], 1)) == 1 && mxGetCell(mxGetCell(out[0], 1), 0) == nullptr);
   } else {
     const mxArray* in[] = {ds, nums, kps, k, ratio, bf, six, md, cf, it};
+    bad += expect_error("apsmatch:nogpu", 3, 10, in);  // no CPU fallback
+  }
+#elif defined(GATE_PIMATCH)
+  // the sets of GATE_GIMATCH: set 1 = two images, the second a copy of the first with keypoints shifted by (10, -5);
+  // set 2 = one image.  Arguments: matchThreshold, maxRatio, method (exhaustive), m, maxDistance, confidence, maxIter
+  const int N = 40, Dd = 16;
+  mxArray *d1 = mxCreateNumericMatrix(N, Dd, mxSINGLE_CLASS, mxREAL), *d2 = mxCreateNumericMatrix(N, Dd, mxSINGLE_CLASS, mxREAL);
+  mxArray *k1 = mxCreateDoubleMatrix(N, 2, mxREAL), *k2 = mxCreateDoubleMatrix(N, 2, mxREAL);
+  for (int r = 0; r < N; ++r) {
+    for (int c = 0; c < Dd; ++c)
+      ((float*)mxGetData(d1))[r + c * N] = ((float*)mxGetData(d2))[r + c * N] = (float)(((r + 3) * (c + 7) * 31) % 97);
+    const double x = (double)((r * 37) % 101) * 7.0, y = (double)((r * 53) % 89) * 9.0;
+    mxGetPr(k1)[r] = x; mxGetPr(k1)[r + N] = y;
+    mxGetPr(k2)[r] = x - 10.0; mxGetPr(k2)[r + N] = y + 5.0;
+  }
+  auto cell_of = [](int m, int n, std::vector<mxArray*> e) {
+    mxArray* c = mxCreateCellMatrix((mwSize)m, (mwSize)n);
+    for (size_t i = 0; i < e.size(); ++i) mxSetCell(c, (mwIndex)i, e[i]);
+    return c;
+  };
+  mxArray* ds = cell_of(1, 2, {cell_of(1, 2, {d1, d2}), cell_of(1, 1, {d1})});
+  mxArray* kps = cell_of(1, 2, {cell_of(1, 2, {k1, k2}), cell_of(1, 1, {k1})});
+  mxArray* nums = mxCreateDoubleMatrix(1, 2, mxREAL);
+  mxGetPr(nums)[0] = 2; mxGetPr(nums)[1] = 1;
+  mxArray *thr = mxCreateDoubleScalar(1.5), *ratio = mxCreateDoubleScalar(0.8), *meth = mxCreateDoubleScalar(0),
+          *six = mxCreateDoubleScalar(6), *md = mxCreateDoubleScalar(5.5), *cf = mxCreateDoubleScalar(99.9),
+          *it = mxCreateDoubleScalar(500);
+  { const mxArray* in[] = {ds, nums, kps, thr, ratio, meth}; bad += expect_error("apsmatch:args", 3, 6, in); }
+  { const mxArray* in[] = {ds, six, kps, thr, ratio, meth, six, md, cf, it}; bad += expect_error("apsmatch:args", 3, 10, in); }
+  { const mxArray* in[] = {six, nums, kps, thr, ratio, meth, six, md, cf, it}; bad += expect_error("apsmatch:args", 3, 10, in); }
+  { const mxArray* in[] = {ds, nums, kps, thr, ratio, mxCreateString("x"), six, md, cf, it};
+    bad += expect_error("apsmatch:args", 3, 10, in); }                                    // scalars only
+  { const mxArray* in[] = {ds, nums, cell_of(1, 2, {cell_of(1, 1, {k1}), cell_of(1, 1, {k1})}), thr, ratio, meth, six,
+                           md, cf, it};
+    bad += expect_error("apsmatch:args", 3, 10, in); }                                    // keypoints != n
+  { const mxArray* in[] = {ds, nums, cell_of(1, 2, {cell_of(1, 2, {k1, mxCreateDoubleMatrix(N - 1, 2, mxREAL)}),
+                                                    cell_of(1, 1, {k1})}), thr, ratio, meth, six, md, cf, it};
+    bad += expect_error("apsmatch:args", 3, 10, in); }                                    // a row per descriptor
+  { const mxArray* in[] = {cell_of(1, 2, {cell_of(1, 2, {d1, mxCreateDoubleMatrix(N, Dd + 1, mxREAL)}),
+                                          cell_of(1, 1, {d1})}), nums, kps, thr, ratio, meth, six, md, cf, it};
+    bad += expect_error("flann_knn:dim", 3, 10, in); }
+  if (gpu) {  // the library's own checks (the gateway creates its context first)
+    { const mxArray* in[] = {ds, nums, kps, thr, ratio, mxCreateDoubleScalar(7), six, md, cf, it};
+      bad += expect_error("apsmatch:args", 3, 10, in); }                                  // method 7
+    { const mxArray* in[] = {ds, nums, kps, thr, ratio, meth, six, md, cf, mxCreateDoubleScalar(0)};
+      bad += expect_error("apsmatch:args", 3, 10, in); }                                  // maxIter <= 0
+    mxArray* out[4] = {nullptr, nullptr, nullptr, nullptr};
+    const mxArray* in[] = {ds, nums, kps, thr, ratio, meth, six, md, cf, it};
+    mexFunction(4, out, 10, in);
+    const mxArray* a12 = mxGetCell(mxGetCell(out[0], 0), 2);
+    const mxArray* t12 = mxGetCell(mxGetCell(out[2], 0), 2);
+    const mxArray* m12 = mxGetCell(mxGetCell(out[3], 0), 2);
+    bad += !(mxGetN(out[0]) == 2 && a12 && mxGetM(a12) >= 4 && mxGetPr(mxGetCell(out[1], 0))[2] == (double)mxGetM(a12));
+    bad += !(m12 && mxGetM(m12) >= mxGetM(a12) && mxGetM(m12) <= (size_t)N);  // one row per query row at most
+    if (t12) {  // model maps image 2 keypoints to image 1: translation (+10, -5); column-major 3x3
+      const double* t = mxGetPr(t12);
+      bad += !(std::fabs(t[6] / t[8] - 10.0) < 1e-6 && std::fabs(t[7] / t[8] + 5.0) < 1e-6);
+    } else {
+      ++bad;
+    }
+    bad += !(mxGetM(mxGetCell(out[0], 1)) == 1 && mxGetCell(mxGetCell(out[0], 1), 0) == nullptr);
+  } else {
+    const mxArray* in[] = {ds, nums, kps, thr, ratio, meth, six, md, cf, it};
     bad += expect_error("apsmatch:nogpu", 3, 10, in);  // no CPU fallback
   }
 #elif defined(GATE_MATCHF)
