@@ -17,16 +17,23 @@ from .host import (  # noqa: F401
     featureMatchingGlobal,
     featureMatchingGlobalDevice,
     featureMatchingGlobalSets,
+    featureMatchingGlobalSetsDevice,
     featureMatchingPairwiseSets,
+    featureMatchingPairwiseSetsDevice,
+    featureMatchingPairwiseDevice,
     estimateTransformationRANSAC,
     featureMatchingPairwise,
     imageMatching,
     globalImageMatching,
+    globalImageMatchingDevice,
     globalImageMatchingSets,
+    globalImageMatchingSetsDevice,
     imageMatchingBatch,
     imageMatchingSets,
     pairwiseImageMatching,
+    pairwiseImageMatchingDevice,
     pairwiseImageMatchingSets,
+    pairwiseImageMatchingSetsDevice,
     ransacSampleTable,
     flann_knn_win,
     matchFeaturesScratch,

@@ -14,6 +14,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
 
 APS_COL_MAJOR, APS_ROW_MAJOR = 0, 1
 APS_F32, APS_U8 = 0, 1
+APS_KP_F64, APS_KP_F32 = 0, 1
 
 ERR_NAMES = {1: "APS_ERR_ARGS", 2: "APS_ERR_TYPE", 3: "APS_ERR_K", 4: "APS_ERR_DIM", 5: "APS_ERR_BF",
              6: "APS_ERR_NOGPU", 7: "APS_ERR_CUDA", 8: "APS_ERR_ALLOC", 9: "APS_ERR_METHOD"}
@@ -130,6 +131,15 @@ def lib():
                                                    i32, i64, C.c_uint64, vp, i32, dbl, dbl, i32, C.c_uint64, i32, pp]),
         "aps_pairwise_image_matching": (i32, [vp, pp, C.POINTER(i64), i32, i32, i32, i32, dbl, dbl, i32, i64, C.c_uint64,
                                               vp, i32, dbl, dbl, i32, C.c_uint64, i32, pp]),
+        "aps_feature_matching_global_sets_dev": (i32, [vp, i32, C.POINTER(i32), vp, C.POINTER(i64), i32, i32, i32, dbl,
+                                                       i32, i32, vp, pp]),
+        "aps_feature_matching_pairwise_sets_dev": (i32, [vp, i32, C.POINTER(i32), vp, C.POINTER(i64), i32, i32, dbl, dbl,
+                                                         i32, i64, C.c_uint64, vp, pp]),
+        "aps_global_image_matching_sets_dev": (i32, [vp, i32, C.POINTER(i32), vp, C.POINTER(i64), i32, i32, i32, dbl, i32,
+                                                     i32, vp, i32, i32, dbl, dbl, i32, C.c_uint64, i32, vp, pp]),
+        "aps_pairwise_image_matching_sets_dev": (i32, [vp, i32, C.POINTER(i32), vp, C.POINTER(i64), i32, i32, dbl, dbl,
+                                                       i32, i64, C.c_uint64, vp, i32, i32, dbl, dbl, i32, C.c_uint64, i32,
+                                                       vp, pp]),
         "aps_image_matches_nsets": (i32, [vp]),
         "aps_image_matches_pairs": (i64, [vp]),
         "aps_image_matches_set_pair_ptr": (C.POINTER(i64), [vp]),

@@ -916,21 +916,25 @@ extern "C" int aps_feature_matching_global(aps_ctx* c, const void* const* desc, 
 // the single-context pipeline behind aps_feature_matching_global (and a one-member aps_group); mutual != 0 adds the
 // opt-in cross-check of aps_gplan_filter_mutual
 int feature_matching_global_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
-                                 int layout, int k, double ratio, int mutual, aps_matchlist** out) {
+                                 int layout, int k, double ratio, int mutual, aps_matchlist** out, bool dev) {
   APS_CTX(c);
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
   *out = nullptr;
   aps_gplan* p = nullptr;
   APS_TRY(aps_gplan_create(c, counts, n, D, dtype, k, &p));
   int rc = APS_OK;
-  if (p->F > 0) rc = gplan_run(p, desc, layout, ratio, mutual);  // featureMatchingGlobal.m:49-52,65-67: all empty -> cell(numImg)
+  if (p->F > 0) rc = gplan_run(p, desc, layout, ratio, mutual, dev);  // featureMatchingGlobal.m:49-52,65-67: all empty -> cell(numImg)
   if (rc == APS_OK) rc = aps_gplan_download(p, out);
   aps_gplan_destroy(p);
   return rc;
 }
 
-int gplan_run(aps_gplan* p, const void* const* desc, int layout, double ratio, int mutual) {
-  APS_TRY(aps_gplan_upload(p, desc, layout));
+int gplan_run(aps_gplan* p, const void* const* desc, int layout, double ratio, int mutual, bool dev) {
+  if (dev)  // the pooled device matrix of the set: one copy into the plan
+    APS_CUDA(cudaMemcpyAsync(aps_gplan_desc_device(p), desc[0], (size_t)p->F * p->D * (p->dtype == APS_F32 ? 4 : 1),
+                             cudaMemcpyDeviceToDevice, p->c->stream));
+  else
+    APS_TRY(aps_gplan_upload(p, desc, layout));
   APS_TRY(aps_gplan_prepare(p));
   APS_TRY(aps_gplan_knn(p, 0, p->F));
   APS_TRY(aps_gplan_filter(p, 0, p->F, ratio));
@@ -949,39 +953,13 @@ void gplan_lists(aps_gplan* p, GlobalLists& L) {
   L.Ft = p->dtype == APS_F32 && p->tensor ? p->F : 0;
 }
 
-// Same with the pooled descriptors ALREADY ON THE DEVICE (a GPU extractor's output, or a previous stage's buffer):
-// no host staging; the pooled row-major [F x D] matrix is copied device-to-device into the plan.
+// Same with the pooled descriptors ALREADY ON THE DEVICE (a GPU extractor's output, or a previous stage's buffer): the
+// one-set case of aps_feature_matching_global_sets_dev, the context checked first as it always was.
 extern "C" int aps_feature_matching_global_dev(aps_ctx* c, const void* d_pooled, const int64_t* counts, int n, int D,
                                                int dtype, int k, double ratio, int mutual, aps_matchlist** out) {
   APS_CTX(c);
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
-  *out = nullptr;
-  aps_gplan* p = nullptr;
-  APS_TRY(aps_gplan_create(c, counts, n, D, dtype, k, &p));
-  int rc = APS_OK;
-  if (p->F > 0) {
-    if (!d_pooled) {
-      aps_gplan_destroy(p);
-      APS_FAIL(APS_ERR_ARGS, "", "device descriptor pointer is NULL");
-    }
-    cudaPointerAttributes attr;
-    if (cudaPointerGetAttributes(&attr, d_pooled) != cudaSuccess || (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged)) {
-      cudaGetLastError();
-      aps_gplan_destroy(p);
-      APS_FAIL(APS_ERR_ARGS, "", "aps_feature_matching_global_dev expects a device pointer");
-    }
-    const size_t bytes = (size_t)p->F * D * (dtype == APS_F32 ? 4 : 1);
-    if (cudaMemcpyAsync(aps_gplan_desc_device(p), d_pooled, bytes, cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess)
-      rc = APS_ERR_CUDA;
-    if (rc == APS_OK) rc = aps_gplan_prepare(p);
-    if (rc == APS_OK) rc = aps_gplan_knn(p, 0, p->F);
-    if (rc == APS_OK) rc = aps_gplan_filter(p, 0, p->F, ratio);
-    if (rc == APS_OK && mutual) rc = aps_gplan_filter_mutual(p);
-    if (rc == APS_OK) rc = aps_gplan_compact(p);
-  }
-  if (rc == APS_OK) rc = aps_gplan_download(p, out);
-  aps_gplan_destroy(p);
-  return rc;
+  return aps_feature_matching_global_sets_dev(c, 1, &n, d_pooled, counts, D, dtype, k, ratio, 0, mutual, nullptr, out);
 }
 
 // ------------------------------------------------------------------------------------------------

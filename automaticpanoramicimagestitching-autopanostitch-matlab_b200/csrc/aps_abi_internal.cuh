@@ -92,11 +92,14 @@ int ssd2_device(aps_ctx* c, const FloatSide& Q, int64_t q0, int64_t N1, const Fl
 
 // ---- one-call pipelines over the staged plans (aps_abi.cu / aps_abi_pairwise.cu; aps_abi_group.cu runs them per member)
 int gplan_upload_images(aps_gplan* p, const void* const* desc, int layout, int i0, int i1);
+// dev (here and below): desc[i] are device pointers into one pooled row-major matrix (pooled_image_ptrs), not host
+// matrices in `layout`
 int feature_matching_global_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
-                                 int layout, int k, double ratio, int mutual, aps_matchlist** out);
+                                 int layout, int k, double ratio, int mutual, aps_matchlist** out, bool dev = false);
 int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
                                    int layout, double match_threshold, double max_ratio, int method, int64_t subset,
-                                   uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out);
+                                   uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out,
+                                   bool dev = false);
 
 // ---- lists of image sets and pooled upload of many images (aps_abi_sets.cu; the sets entries) ---------------------
 // Checks the set list of a sets entry (nsets >= 0, set_images[b] >= 0, at most INT_MAX images in all) and returns
@@ -111,9 +114,19 @@ int sets_split_lists(int nsets, const std::vector<int64_t>& pair_ptr, const std:
 // img[r] = image of pooled row r (d_off: [nimg + 1] row offsets on the device)
 int sets_img_of_row(cudaStream_t s, const int64_t* d_off, int nimg, int64_t F, int32_t* img);
 // H2D of image i (host ptrs[i], off[i + 1] - off[i] rows) to rows [off[i], off[i + 1]) of the pooled row-major matrix
-// `raw`: one copy per image; column-major input is staged and transposed in ONE launch (needs img_of_row)
+// `raw`: one copy per image; column-major input is staged and transposed in ONE launch (needs img_of_row).
+// dev: ptrs[i] point into one pooled row-major device matrix; images whose rows follow each other there and in `raw`
+// go in ONE device-to-device copy (one copy in all when the pass keeps the caller's image order)
 int sets_upload(aps_ctx* c, const void* const* ptrs, const std::vector<int64_t>& off, const int64_t* d_off,
-                const int32_t* img_of_row, int D, int esz, int layout, void* raw);
+                const int32_t* img_of_row, int D, int esz, int layout, void* raw, bool dev = false);
+
+// ---- device input (the *_dev entries) ------------------------------------------------------------------------------
+// Per-image pointers into the pooled row-major device matrix d_pooled: image g starts at row sum(counts[0..g)).
+std::vector<const void*> pooled_image_ptrs(const void* d_pooled, const int64_t* counts, int64_t nimg, int D, int esz);
+// The checks and the hand-off of a *_dev entry once the host entry's statuses passed: d_pooled non-NULL when F > 0, the
+// context, d_pooled (and d_kp when not NULL) device or managed memory; then the context's stream waits for an event
+// recorded on producer_stream (when not NULL).
+int dev_inputs(aps_ctx* c, int64_t F, const void* d_pooled, const void* d_kp, void* producer_stream);
 
 // ---- global match lists kept on the device (aps_abi.cu, aps_abi_sets.cu; aps_global_image_matching_sets) ----------
 // The compaction outputs of one global pass over nsets sets, in PASS order: pass position j is the caller's set
@@ -145,10 +158,11 @@ int global_sets_args(int nsets, const int* set_images, const int64_t* counts, in
 // Nothing is synchronised; global_lists_stats sets the context's statistics once the stream has been synchronised.
 int global_lists_device(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
                         const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D,
-                        int dtype, int layout, int k, double ratio, int mutual, GlobalLists& L);
+                        int dtype, int layout, int k, double ratio, int mutual, GlobalLists& L, bool dev = false);
 void global_lists_stats(aps_ctx* c, int dtype, const GlobalLists& L);
-// The one-set pass (aps_abi.cu): the staged plan from upload to compaction, and its lists handed to L.
-int gplan_run(aps_gplan* p, const void* const* desc, int layout, double ratio, int mutual);
+// The one-set pass (aps_abi.cu): the staged plan from upload to compaction, and its lists handed to L.  dev: the
+// plan's rows are one device-to-device copy from desc[0].
+int gplan_run(aps_gplan* p, const void* const* desc, int layout, double ratio, int mutual, bool dev = false);
 void gplan_lists(aps_gplan* p, GlobalLists& L);
 
 // ---- pairwise match lists kept on the device (aps_abi_pairwise.cu; aps_pairwise_image_matching_sets) -------------
@@ -171,7 +185,7 @@ int pairwise_sets_args(int nsets, const int* set_images, const int64_t* counts, 
 // are those of the pass (the per-batch match counts among them); the pass's own buffers are released on return.
 int pairwise_rows_device(aps_ctx* c, int nsets, const int* set_images, const void* const* desc, const int64_t* counts,
                          int nimg, int D, int dtype, int layout, double match_threshold, double max_ratio, int method,
-                         int64_t subset, uint64_t seed, PairwiseRows& R);
+                         int64_t subset, uint64_t seed, PairwiseRows& R, bool dev = false);
 
 // ---- RANSAC over candidate pairs whose tables are on the device (aps_ransac.cu) ------------------------------------
 // The gather and the RANSAC chain of aps_image_matching_sets over n_pairs pairs: pair p's correspondences are

@@ -1082,7 +1082,7 @@ extern "C" int aps_pplan_match(aps_pplan* p, double match_threshold, double max_
 
 int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const int64_t* counts, int n, int D, int dtype,
                                    int layout, double match_threshold, double max_ratio, int method, int64_t subset,
-                                   uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out) {
+                                   uint64_t seed, int pair_first, int pair_stride, aps_matchlist** out, bool dev) {
   APS_CTX(c);
   if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
   *out = nullptr;
@@ -1092,7 +1092,16 @@ int feature_matching_pairwise_impl(aps_ctx* c, const void* const* desc, const in
   APS_TRY(aps_pplan_create(c, counts, n, D, dtype, &p));
   int rc = aps_pplan_set_method(p, method, subset, seed);
   if (rc == APS_OK && p->F > 0 && n >= 2) {
-    rc = aps_pplan_upload(p, desc, layout);
+    if (dev) {  // the pooled device matrix of the set: one copy into the plan
+      const cudaError_t e = cudaMemcpyAsync(aps_pplan_desc_device(p), desc[0],
+                                            (size_t)p->F * D * (dtype == APS_F32 ? 4 : 1), cudaMemcpyDeviceToDevice,
+                                            c->stream);
+      if (e != cudaSuccess) {
+        aps_set_error(APS_ERR_CUDA, "", "descriptor copy failed: %s", cudaGetErrorString(e));
+        rc = APS_ERR_CUDA;
+      }
+    } else
+      rc = aps_pplan_upload(p, desc, layout);
     if (rc == APS_OK) rc = aps_pplan_prepare(p);  // an error here must not reach the pair classification (ps.big)
   }
   if (rc == APS_OK) rc = aps_pplan_match(p, match_threshold, max_ratio, pair_first, pair_stride, out);
@@ -1120,11 +1129,12 @@ extern "C" int aps_feature_matching_pairwise_shard(aps_ctx* c, const void* const
 // dataset folder and once more per connected component; here all sets share ONE pooled plan (one upload, one K1, one
 // train view), one pair list that never crosses a set, and one pass of pairwise_match_pairs -- no host loop over sets
 // issues device work, so launches and synchronisations do not depend on nsets.
-// dev != NULL: the lists stay on the device in *dev (pairwise_rows_device) and out is not used.
+// dev != NULL: the lists stay on the device in *dev (pairwise_rows_device) and out is not used.  dev_src: desc[i] point
+// into one pooled row-major device matrix (pooled_image_ptrs), uploaded with one device-to-device copy.
 static int pairwise_sets_pass(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
                               const int64_t* counts, int nimg, int D, int dtype, int layout, double match_threshold,
                               double max_ratio, int method, int64_t subset, uint64_t seed, aps_matchlist** out,
-                              PairwiseRows* dev = nullptr) {
+                              PairwiseRows* dev = nullptr, bool dev_src = false) {
   // per image: its index in its own set (the key of its 'subsetpdist2' subset); per set: its first cell.  Set b's
   // pairs: its own column-major strict-upper-triangle list, on the engine its single-set call chooses (aps_pplan_create)
   std::vector<int32_t> local((size_t)nimg);
@@ -1168,7 +1178,7 @@ static int pairwise_sets_pass(aps_ctx* c, int nsets, const int* set_images, cons
       APS_TRY(sets_img_of_row(c->stream, d_off.p, nimg, F, img_of_row.p));
     }
     APS_TRY(sets_upload(c, desc, ps.off, d_off.p, img_of_row.p, D, dtype == APS_F32 ? 4 : 1, layout,
-                        dtype == APS_F32 ? (void*)ps.rawset.raw.p : (void*)ps.u8raw.p));
+                        dtype == APS_F32 ? (void*)ps.rawset.raw.p : (void*)ps.u8raw.p, dev_src));
     APS_TRY(pairwise_finish(c, ps, counts, nimg, D, dtype, any_tensor));
     if (dtype == APS_F32)
       APS_TRY(pairwise_build_train_view(c, ps, counts, nimg, D, any_tensor,
@@ -1183,6 +1193,24 @@ static int pairwise_sets_pass(aps_ctx* c, int nsets, const int* set_images, cons
   }
   // one list per set: cells [cell_off[b], cell_off[b + 1]], rows from pair_ptr[cell_off[b]]
   return sets_split_lists(nsets, pooled.pair_ptr, pooled.rows, &pooled.metric, cell_off, set_images, nullptr, out);
+}
+
+// the sets pass with its lists split into out[0 .. nsets), statistics of the call (none on failure)
+static int pairwise_sets_lists(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
+                               const int64_t* counts, int nimg, int D, int dtype, int layout, double match_threshold,
+                               double max_ratio, int method, int64_t subset, uint64_t seed, bool dev_src,
+                               aps_matchlist** out) {
+  c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
+  c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
+  c->h_flags[32] = 0;   // fallback rows of the call's tensor batches (aps_ctx_last_stats)
+  const int rc = pairwise_sets_pass(c, nsets, set_images, desc, counts, nimg, D, dtype, layout, match_threshold,
+                                    max_ratio, method, subset, seed, out, nullptr, dev_src);
+  if (rc != APS_OK)
+    for (int b = 0; b < nsets; ++b) {
+      aps_matchlist_free(out[b]);
+      out[b] = nullptr;
+    }
+  return rc;
 }
 
 extern "C" int aps_feature_matching_pairwise_sets(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
@@ -1200,17 +1228,33 @@ extern "C" int aps_feature_matching_pairwise_sets(aps_ctx* c, int nsets, const i
   if (nsets == 1)  // one set: the single-set call itself
     return feature_matching_pairwise_impl(c, desc, counts, set_images[0], D, dtype, layout, match_threshold, max_ratio,
                                           method, subset, seed, 0, 1, out);
-  c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
-  c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
-  c->h_flags[32] = 0;   // fallback rows of the call's tensor batches (aps_ctx_last_stats)
-  const int rc = pairwise_sets_pass(c, nsets, set_images, desc, counts, (int)nimg, D, dtype, layout, match_threshold,
-                                    max_ratio, method, subset, seed, out);
-  if (rc != APS_OK)
-    for (int b = 0; b < nsets; ++b) {
-      aps_matchlist_free(out[b]);
-      out[b] = nullptr;
-    }
-  return rc;
+  return pairwise_sets_lists(c, nsets, set_images, desc, counts, (int)nimg, D, dtype, layout, match_threshold,
+                             max_ratio, method, subset, seed, false, out);
+}
+
+// Device input: the host entry's two paths (one set: the single-set plan; several: the sets pass), each fed from the
+// pooled device matrix
+extern "C" int aps_feature_matching_pairwise_sets_dev(aps_ctx* c, int nsets, const int* set_images,
+                                                      const void* d_pooled, const int64_t* counts, int D, int dtype,
+                                                      double match_threshold, double max_ratio, int method,
+                                                      int64_t subset, uint64_t seed, void* producer_stream,
+                                                      aps_matchlist** out) {
+  // the host entry's arguments, then the device pointer, the context and the hand-off
+  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
+  for (int b = 0; b < nsets; ++b) out[b] = nullptr;
+  std::vector<int64_t> img_first;
+  APS_TRY(pairwise_sets_args(nsets, set_images, counts, D, dtype, method, subset, img_first));
+  const int64_t nimg = img_first[nsets];
+  int64_t F = 0;
+  for (int64_t g = 0; g < nimg; ++g) F += counts[g];
+  APS_TRY(dev_inputs(c, F, d_pooled, nullptr, producer_stream));
+  if (nsets == 0) return APS_OK;
+  const std::vector<const void*> ptrs = pooled_image_ptrs(d_pooled, counts, nimg, D, dtype == APS_F32 ? 4 : 1);
+  if (nsets == 1)  // one set: the single-set call itself
+    return feature_matching_pairwise_impl(c, ptrs.data(), counts, set_images[0], D, dtype, APS_ROW_MAJOR,
+                                          match_threshold, max_ratio, method, subset, seed, 0, 1, out, true);
+  return pairwise_sets_lists(c, nsets, set_images, ptrs.data(), counts, (int)nimg, D, dtype, APS_ROW_MAJOR,
+                             match_threshold, max_ratio, method, subset, seed, true, out);
 }
 
 int pairwise_sets_args(int nsets, const int* set_images, const int64_t* counts, int D, int dtype, int method,
@@ -1238,10 +1282,10 @@ int pairwise_sets_args(int nsets, const int* set_images, const int64_t* counts, 
 
 int pairwise_rows_device(aps_ctx* c, int nsets, const int* set_images, const void* const* desc, const int64_t* counts,
                          int nimg, int D, int dtype, int layout, double match_threshold, double max_ratio, int method,
-                         int64_t subset, uint64_t seed, PairwiseRows& R) {
+                         int64_t subset, uint64_t seed, PairwiseRows& R, bool dev) {
   c->stats[0] = c->stats[1] = c->stats[2] = c->stats[3] = 0;
   c->pair_stats[0] = c->pair_stats[1] = c->pair_stats[2] = c->pair_stats[3] = 0;
   c->h_flags[32] = 0;
   return pairwise_sets_pass(c, nsets, set_images, desc, counts, nimg, D, dtype, layout, match_threshold, max_ratio,
-                            method, subset, seed, nullptr, &R);
+                            method, subset, seed, nullptr, &R, dev);
 }

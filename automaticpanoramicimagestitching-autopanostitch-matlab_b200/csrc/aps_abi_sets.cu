@@ -1,5 +1,6 @@
 // aps_abi_sets.cu -- featureMatchingGlobal over many independent image sets in one call
-// (aps_feature_matching_global_sets, include/apsmatch.h).
+// (aps_feature_matching_global_sets, and aps_feature_matching_global_sets_dev for descriptors already on the device,
+// include/apsmatch.h).
 //
 // The reference runs the whole global pipeline once per dataset folder, and once per connected component; a Python user
 // matching a directory of panoramas makes one call per panorama.  Every such call pays fixed costs (allocations, a dozen
@@ -61,11 +62,27 @@ int sets_img_of_row(cudaStream_t s, const int64_t* d_off, int nimg, int64_t F, i
 }
 
 int sets_upload(aps_ctx* c, const void* const* ptrs, const std::vector<int64_t>& off, const int64_t* d_off,
-                const int32_t* img_of_row, int D, int esz, int layout, void* raw) {
+                const int32_t* img_of_row, int D, int esz, int layout, void* raw, bool dev) {
   cudaStream_t s = c->stream;
   const int nimg = (int)off.size() - 1;
   const int64_t F = off.back();
   if (F == 0) return APS_OK;
+  if (dev) {  // runs of images that are contiguous in the source as in `raw`: one device-to-device copy each
+    const size_t row = (size_t)D * esz;
+    for (int i = 0; i < nimg;) {
+      if (off[i + 1] == off[i]) {
+        ++i;
+        continue;
+      }
+      const char* src = (const char*)ptrs[i];
+      int j = i + 1;
+      while (j < nimg && (off[j + 1] == off[j] || (const char*)ptrs[j] == src + (size_t)(off[j] - off[i]) * row)) ++j;
+      APS_CUDA(cudaMemcpyAsync((char*)raw + (size_t)off[i] * row, src, (size_t)(off[j] - off[i]) * row,
+                               cudaMemcpyDeviceToDevice, s));
+      i = j;
+    }
+    return APS_OK;
+  }
   // row-major images land in place; column-major ones are staged and transposed in one launch
   DevBuf<uint8_t> stage;
   uint8_t* dst = (uint8_t*)raw;
@@ -97,6 +114,42 @@ int sets_image_offsets(int nsets, const int* set_images, std::vector<int64_t>& i
     img0[b + 1] = img0[b] + set_images[b];
   }
   if (img0[nsets] > INT_MAX) APS_FAIL(APS_ERR_ARGS, "", "more than 2^31 - 1 images");
+  return APS_OK;
+}
+
+std::vector<const void*> pooled_image_ptrs(const void* d_pooled, const int64_t* counts, int64_t nimg, int D, int esz) {
+  std::vector<const void*> ptrs((size_t)nimg);
+  int64_t r = 0;
+  for (int64_t g = 0; g < nimg; ++g) {
+    ptrs[(size_t)g] = (const char*)d_pooled + (size_t)r * D * esz;
+    r += counts[g];
+  }
+  return ptrs;
+}
+
+static bool device_memory(const void* p) {
+  cudaPointerAttributes attr;
+  if (cudaPointerGetAttributes(&attr, p) != cudaSuccess) {
+    cudaGetLastError();
+    return false;
+  }
+  return attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged;
+}
+
+int dev_inputs(aps_ctx* c, int64_t F, const void* d_pooled, const void* d_kp, void* producer_stream) {
+  if (F > 0 && !d_pooled) APS_FAIL(APS_ERR_ARGS, "", "device descriptor pointer is NULL");
+  APS_CTX(c);
+  // a host pointer is refused, never dereferenced on the device
+  if (F > 0 && !device_memory(d_pooled)) APS_FAIL(APS_ERR_ARGS, "", "d_pooled is not device or managed memory");
+  if (F > 0 && d_kp && !device_memory(d_kp)) APS_FAIL(APS_ERR_ARGS, "", "d_keypoints is not device or managed memory");
+  if (producer_stream) {  // the producer's work so far comes first, without a host synchronisation
+    cudaEvent_t ev;
+    APS_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    cudaError_t e = cudaEventRecord(ev, (cudaStream_t)producer_stream);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(c->stream, ev, 0);
+    cudaEventDestroy(ev);  // released once the wait is resolved
+    APS_CUDA(e);
+  }
   return APS_OK;
 }
 
@@ -138,7 +191,7 @@ __global__ void k_sets_fallback_groups(const int32_t* __restrict__ fb, const int
 // sets the single-set call would search on the tensor path: they occupy rows [0, Ft) of the pooled matrix.
 int pooled_pass_device(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std::vector<int64_t>& img_first,
                        const int* set_images, const void* const* desc, const int64_t* counts, int D, int dtype,
-                       int layout, int k, double ratio, int mutual, GlobalLists& L) {
+                       int layout, int k, double ratio, int mutual, GlobalLists& L, bool dev) {
   cudaStream_t s = c->stream;
   const int nsets = (int)sets.size();
   // pooled images, offsets and set tables
@@ -233,7 +286,7 @@ int pooled_pass_device(aps_ctx* c, const std::vector<int>& sets, int ntensor, co
     if (!units.empty())
       APS_CUDA(cudaMemcpyAsync(d_units.p, units.data(), units.size() * sizeof(aps_tc_unit), cudaMemcpyHostToDevice, s));
     APS_TRY(sets_img_of_row(s, d_off.p, nimg, F, img_of_row.p));
-    APS_TRY(sets_upload(c, ptrs.data(), off, d_off.p, img_of_row.p, D, esz, layout, raw.p));
+    APS_TRY(sets_upload(c, ptrs.data(), off, d_off.p, img_of_row.p, D, esz, layout, raw.p, dev));
     APS_TRY(knn_idx.alloc((size_t)F * k, s));
     APS_TRY(knn_dist.alloc((size_t)F * k, s));
     if (dtype == APS_F32) {
@@ -335,12 +388,12 @@ int pooled_pass_device(aps_ctx* c, const std::vector<int>& sets, int ntensor, co
 // pooled_pass_device, then one download split into the nsets lists
 int pooled_pass(aps_ctx* c, const std::vector<int>& sets, int ntensor, const std::vector<int64_t>& img_first,
                 const int* set_images, const void* const* desc, const int64_t* counts, int D, int dtype, int layout,
-                int k, double ratio, int mutual, aps_matchlist** out) {
+                int k, double ratio, int mutual, aps_matchlist** out, bool dev) {
   cudaStream_t s = c->stream;
   const int nsets = (int)sets.size();
   GlobalLists L;
   APS_TRY(pooled_pass_device(c, sets, ntensor, img_first, set_images, desc, counts, D, dtype, layout, k, ratio, mutual,
-                             L));
+                             L, dev));
   const int64_t cells = L.cell_off.back();
   std::vector<int64_t> pp((size_t)cells + 1, 0);
   std::vector<uint32_t> rows_h;
@@ -418,17 +471,38 @@ static int pass_order(aps_ctx* c, int nsets, const std::vector<int64_t>& set_row
 
 int global_lists_device(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
                         const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D,
-                        int dtype, int layout, int k, double ratio, int mutual, GlobalLists& L) {
+                        int dtype, int layout, int k, double ratio, int mutual, GlobalLists& L, bool dev) {
   if (nsets == 1) {  // one set: the single-set call's plan
     aps_gplan* p = nullptr;
     APS_TRY(aps_gplan_create(c, counts, set_images[0], D, dtype, k, &p));
     gplan_lists(p, L);  // L owns the plan from here
-    return gplan_run(p, desc, layout, ratio, mutual);
+    return gplan_run(p, desc, layout, ratio, mutual, dev);
   }
   std::vector<int> order;
   const int ntensor = pass_order(c, nsets, set_rows, D, dtype, k, order);
   return pooled_pass_device(c, order, ntensor, img_first, set_images, desc, counts, D, dtype, layout, k, ratio, mutual,
-                            L);
+                            L, dev);
+}
+
+// the sets entries once their arguments and the context passed
+static int global_sets_run(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
+                           const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D,
+                           int dtype, int layout, int k, double ratio, int mutual, bool dev, aps_matchlist** out) {
+  if (nsets == 0) return APS_OK;
+  if (nsets == 1)  // one set: the single-set call itself
+    return feature_matching_global_impl(c, desc, counts, set_images[0], D, dtype, layout, k, ratio, mutual, out, dev);
+
+  // one pass for every set
+  std::vector<int> order;
+  const int ntensor = pass_order(c, nsets, set_rows, D, dtype, k, order);
+  const int rc = pooled_pass(c, order, ntensor, img_first, set_images, desc, counts, D, dtype, layout, k, ratio, mutual,
+                             out, dev);
+  if (rc != APS_OK)
+    for (int b = 0; b < nsets; ++b) {
+      aps_matchlist_free(out[b]);
+      out[b] = nullptr;
+    }
+  return rc;
 }
 
 extern "C" int aps_feature_matching_global_sets(aps_ctx* c, int nsets, const int* set_images, const void* const* desc,
@@ -441,19 +515,25 @@ extern "C" int aps_feature_matching_global_sets(aps_ctx* c, int nsets, const int
   std::vector<int64_t> img_first, set_rows;
   APS_TRY(global_sets_args(nsets, set_images, counts, D, dtype, k, img_first, set_rows));
   APS_CTX(c);
-  if (nsets == 0) return APS_OK;
-  if (nsets == 1)  // one set: the single-set call itself
-    return feature_matching_global_impl(c, desc, counts, set_images[0], D, dtype, layout, k, ratio, mutual, out);
+  return global_sets_run(c, nsets, set_images, img_first, set_rows, desc, counts, D, dtype, layout, k, ratio, mutual,
+                         false, out);
+}
 
-  // one pass for every set
-  std::vector<int> order;
-  const int ntensor = pass_order(c, nsets, set_rows, D, dtype, k, order);
-  const int rc = pooled_pass(c, order, ntensor, img_first, set_images, desc, counts, D, dtype, layout, k, ratio, mutual,
-                             out);
-  if (rc != APS_OK)
-    for (int b = 0; b < nsets; ++b) {
-      aps_matchlist_free(out[b]);
-      out[b] = nullptr;
-    }
-  return rc;
+extern "C" int aps_feature_matching_global_sets_dev(aps_ctx* c, int nsets, const int* set_images, const void* d_pooled,
+                                                    const int64_t* counts, int D, int dtype, int k, double ratio,
+                                                    int use_bf, int mutual, void* producer_stream,
+                                                    aps_matchlist** out) {
+  (void)use_bf;
+  // the host entry's arguments, then the device pointer, the context and the hand-off
+  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
+  for (int b = 0; b < nsets; ++b) out[b] = nullptr;
+  std::vector<int64_t> img_first, set_rows;
+  APS_TRY(global_sets_args(nsets, set_images, counts, D, dtype, k, img_first, set_rows));
+  int64_t F = 0;
+  for (int64_t F_b : set_rows) F += F_b;
+  APS_TRY(dev_inputs(c, F, d_pooled, nullptr, producer_stream));
+  const std::vector<const void*> ptrs =
+      pooled_image_ptrs(d_pooled, counts, img_first[nsets], D, dtype == APS_F32 ? 4 : 1);
+  return global_sets_run(c, nsets, set_images, img_first, set_rows, ptrs.data(), counts, D, dtype, APS_ROW_MAJOR, k,
+                         ratio, mutual, true, out);
 }

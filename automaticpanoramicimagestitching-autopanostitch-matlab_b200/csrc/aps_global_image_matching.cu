@@ -14,7 +14,9 @@
 //   k_all_matches (rows with the inlier flag set, accepted pairs only) -> one download, reordered into the caller's set
 //   order on the host.
 // A set's candidate pairs are keyed by their index in that set's own list, so pass order changes nothing: every output
-// is the two-call chain's, bit for bit.
+// is the two-call chain's, bit for bit.  The *_dev entries take the descriptors and keypoints from device memory: the
+// passes copy the pooled descriptors device-to-device where they upload, and match_lists copies float64 keypoints or
+// widens float32 ones on the device (k_widen_keypoints) where it uploads; the rest is the same code.
 #include <climits>
 #include <new>
 #include <vector>
@@ -184,6 +186,21 @@ __global__ void __launch_bounds__(128) k_place_rows(const int64_t* __restrict__ 
   }
 }
 
+// float32 keypoints -> double2, exactly (every float is a double): one thread per keypoint, two scalar loads, so the
+// caller's pointer needs no more than float alignment
+__global__ void k_widen_keypoints(const float* __restrict__ src, int64_t n, double2* __restrict__ dst) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) dst[i] = make_double2((double)src[2 * i], (double)src[2 * i + 1]);
+}
+
+// Where the pooled [F x 2] keypoints come from: host float64 (the host entries), or device memory (the *_dev entries)
+// of aps_kp_dtype `dtype`
+struct KeypointSource {
+  const void* p;
+  bool dev;
+  int dtype;
+};
+
 // candidate pairs a set can have at most: every image marks at most min(m, n - 1) partners (imageMatching.m:86-91)
 int64_t pair_bound(const std::vector<int>& ns, int m) {
   int64_t cap = 0;
@@ -235,7 +252,7 @@ void reorder(const std::vector<int>& order, const std::vector<int64_t>& spp, con
 // packed rows, RANSAC, allMatches and the download into r.  F: pooled keypoint rows; row_bound: a bound on the rows of
 // L's lists (sizes the packed correspondences).  With want_lists, r->lists are L's lists (with L.metric when set).
 int match_lists(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
-                const int64_t* counts, int64_t F, const double* keypoints, const GlobalLists& L, int64_t row_bound,
+                const int64_t* counts, int64_t F, const KeypointSource& keypoints, const GlobalLists& L, int64_t row_bound,
                 int m, double max_distance, double confidence, int max_trials, uint64_t seed, int want_lists,
                 aps_image_matches* r) {
   cudaStream_t s = c->stream;
@@ -268,7 +285,14 @@ int match_lists(aps_ctx* c, int nsets, const int* set_images, const std::vector<
   const int64_t* d_img_off = dtab.p + 2 * nt + 2 * nsets;
   if (F > 0) {
     APS_TRY(kp.alloc((size_t)F, s));
-    APS_CUDA(cudaMemcpyAsync(kp.p, keypoints, (size_t)F * 16, cudaMemcpyHostToDevice, s));
+    if (!keypoints.dev) {
+      APS_CUDA(cudaMemcpyAsync(kp.p, keypoints.p, (size_t)F * 16, cudaMemcpyHostToDevice, s));
+    } else if (keypoints.dtype == APS_KP_F64) {
+      APS_CUDA(cudaMemcpyAsync(kp.p, keypoints.p, (size_t)F * 16, cudaMemcpyDeviceToDevice, s));
+    } else {
+      k_widen_keypoints<<<(unsigned)aps_ceil_div(F, 256), 256, 0, s>>>((const float*)keypoints.p, F, kp.p);
+      APS_LAUNCHED();
+    }
   }
   // K6 on the device counts, find() per set: sel = [set_pair_ptr (nsets + 1) | correspondences], pairs_lin in lin
   APS_TRY(sel.alloc(nt + 1, s));
@@ -375,15 +399,15 @@ int match_lists(aps_ctx* c, int nsets, const int* set_images, const std::vector<
 
 int run_global(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
                const std::vector<int64_t>& set_rows, const void* const* desc, const int64_t* counts, int D, int dtype,
-               int layout, int k, double ratio, int mutual, const double* keypoints, int m, double max_distance,
-               double confidence, int max_trials, uint64_t seed, int want_lists, aps_image_matches* r) {
+               int layout, int k, double ratio, int mutual, const KeypointSource& keypoints, int m, double max_distance,
+               double confidence, int max_trials, uint64_t seed, int want_lists, bool dev, aps_image_matches* r) {
   cudaStream_t s = c->stream;
   int64_t F = 0;
   for (int64_t F_b : set_rows) F += F_b;
   GlobalLists L;
   if (F > 0) {
     APS_TRY(global_lists_device(c, nsets, set_images, img_first, set_rows, desc, counts, D, dtype, layout, k, ratio,
-                                mutual, L));
+                                mutual, L, dev));
   } else {  // no descriptor anywhere: every putative count is 0 (partner selection still runs, imageMatching.m:75-100)
     for (int b = 0; b < nsets; ++b) L.order.push_back(b);
     L.cell_off.assign(1, 0);
@@ -402,8 +426,8 @@ int run_global(aps_ctx* c, int nsets, const int* set_images, const std::vector<i
 
 int run_pairwise(aps_ctx* c, int nsets, const int* set_images, const std::vector<int64_t>& img_first,
                  const void* const* desc, const int64_t* counts, int D, int dtype, int layout, double match_threshold,
-                 double max_ratio, int method, int64_t subset, uint64_t subset_seed, const double* keypoints, int m,
-                 double max_distance, double confidence, int max_trials, uint64_t seed, int want_lists,
+                 double max_ratio, int method, int64_t subset, uint64_t subset_seed, const KeypointSource& keypoints,
+                 int m, double max_distance, double confidence, int max_trials, uint64_t seed, int want_lists, bool dev,
                  aps_image_matches* r) {
   cudaStream_t s = c->stream;
   const int nimg = (int)img_first[nsets];
@@ -415,7 +439,7 @@ int run_pairwise(aps_ctx* c, int nsets, const int* set_images, const std::vector
   {
     PairwiseRows R;
     APS_TRY(pairwise_rows_device(c, nsets, set_images, desc, counts, nimg, D, dtype, layout, match_threshold,
-                                 max_ratio, method, subset, subset_seed, R));
+                                 max_ratio, method, subset, subset_seed, R, dev));
     // the lists in cell order, as GlobalLists: counts scattered into zeroed cells, offsets scanned, rows placed
     L.cell_off = R.cell_off;
     const int64_t cells = L.cell_off.back(), np = R.npairs;
@@ -447,6 +471,12 @@ int run_pairwise(aps_ctx* c, int nsets, const int* set_images, const std::vector
   // a query row can match once in every pair of its image: the pass's M rows bound the lists
   return match_lists(c, nsets, set_images, img_first, counts, F, keypoints, L, M, m, max_distance, confidence,
                      max_trials, seed, want_lists, r);
+}
+
+int keypoint_dtype(int kp_dtype) {
+  if (kp_dtype != APS_KP_F64 && kp_dtype != APS_KP_F32)
+    APS_FAIL(APS_ERR_TYPE, "", "kp_dtype must be APS_KP_F64 or APS_KP_F32 (got %d)", kp_dtype);
+  return APS_OK;
 }
 
 // a result for nsets sets, filled by fill(r) when nsets > 0; *out set only on success
@@ -487,7 +517,35 @@ extern "C" int aps_global_image_matching_sets(aps_ctx* c, int nsets, const int* 
   APS_CTX(c);
   return new_result(nsets, out, [&](aps_image_matches* r) {
     return run_global(c, nsets, set_images, img_first, set_rows, desc, counts, D, dtype, layout, k, ratio, mutual,
-                      keypoints, m, max_distance, confidence, max_trials, seed, want_lists, r);
+                      {keypoints, false, APS_KP_F64}, m, max_distance, confidence, max_trials, seed, want_lists, false,
+                      r);
+  });
+}
+
+extern "C" int aps_global_image_matching_sets_dev(aps_ctx* c, int nsets, const int* set_images, const void* d_pooled,
+                                                  const int64_t* counts, int D, int dtype, int k, double ratio,
+                                                  int use_bf, int mutual, const void* d_keypoints, int kp_dtype, int m,
+                                                  double max_distance, double confidence, int max_trials,
+                                                  uint64_t seed, int want_lists, void* producer_stream,
+                                                  aps_image_matches** out) {
+  (void)use_bf;
+  // the host entry's arguments, then the keypoint type, the device pointers, the context and the hand-off
+  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
+  *out = nullptr;
+  std::vector<int64_t> img_first, set_rows;
+  APS_TRY(global_sets_args(nsets, set_images, counts, D, dtype, k, img_first, set_rows));
+  APS_TRY(ransac_params(2 * (int64_t)max_trials, max_trials, confidence));
+  int64_t F = 0;
+  for (int64_t F_b : set_rows) F += F_b;
+  if (F > 0 && !d_keypoints) APS_FAIL(APS_ERR_ARGS, "", "keypoints is NULL");
+  APS_TRY(keypoint_dtype(kp_dtype));
+  APS_TRY(dev_inputs(c, F, d_pooled, d_keypoints, producer_stream));
+  const std::vector<const void*> ptrs =
+      pooled_image_ptrs(d_pooled, counts, img_first[nsets], D, dtype == APS_F32 ? 4 : 1);
+  return new_result(nsets, out, [&](aps_image_matches* r) {
+    return run_global(c, nsets, set_images, img_first, set_rows, ptrs.data(), counts, D, dtype, APS_ROW_MAJOR, k, ratio,
+                      mutual, {d_keypoints, true, kp_dtype}, m, max_distance, confidence, max_trials, seed,
+                      want_lists, true, r);
   });
 }
 
@@ -517,8 +575,34 @@ extern "C" int aps_pairwise_image_matching_sets(aps_ctx* c, int nsets, const int
   APS_CTX(c);
   return new_result(nsets, out, [&](aps_image_matches* r) {
     return run_pairwise(c, nsets, set_images, img_first, desc, counts, D, dtype, layout, match_threshold, max_ratio,
-                        method, subset, subset_seed, keypoints, m, max_distance, confidence, max_trials, seed,
-                        want_lists, r);
+                        method, subset, subset_seed, {keypoints, false, APS_KP_F64}, m, max_distance, confidence,
+                        max_trials, seed, want_lists, false, r);
+  });
+}
+
+extern "C" int aps_pairwise_image_matching_sets_dev(aps_ctx* c, int nsets, const int* set_images, const void* d_pooled,
+                                                    const int64_t* counts, int D, int dtype, double match_threshold,
+                                                    double max_ratio, int method, int64_t subset, uint64_t subset_seed,
+                                                    const void* d_keypoints, int kp_dtype, int m, double max_distance,
+                                                    double confidence, int max_trials, uint64_t seed, int want_lists,
+                                                    void* producer_stream, aps_image_matches** out) {
+  // the host entry's arguments, then the keypoint type, the device pointers, the context and the hand-off
+  std::vector<int64_t> img_first;
+  APS_TRY(pairwise_sets_args(nsets, set_images, counts, D, dtype, method, subset, img_first));
+  APS_TRY(ransac_params(2 * (int64_t)max_trials, max_trials, confidence));
+  int64_t F = 0;
+  for (int64_t g = 0; g < img_first[nsets]; ++g) F += counts[g];
+  if (F > 0 && !d_keypoints) APS_FAIL(APS_ERR_ARGS, "", "keypoints is NULL");
+  if (!out) APS_FAIL(APS_ERR_ARGS, "", "out is NULL");
+  *out = nullptr;
+  APS_TRY(keypoint_dtype(kp_dtype));
+  APS_TRY(dev_inputs(c, F, d_pooled, d_keypoints, producer_stream));
+  const std::vector<const void*> ptrs =
+      pooled_image_ptrs(d_pooled, counts, img_first[nsets], D, dtype == APS_F32 ? 4 : 1);
+  return new_result(nsets, out, [&](aps_image_matches* r) {
+    return run_pairwise(c, nsets, set_images, img_first, ptrs.data(), counts, D, dtype, APS_ROW_MAJOR, match_threshold,
+                        max_ratio, method, subset, subset_seed, {d_keypoints, true, kp_dtype}, m, max_distance,
+                        confidence, max_trials, seed, want_lists, true, r);
   });
 }
 

@@ -1122,6 +1122,281 @@ def pairwiseImageMatching(input, allDescriptors, numImg, keypoints, seed=0, retu
     return (results[0], lists[0]) if return_matches else results[0]
 
 
+# ---- device input: descriptors and keypoints already in CUDA tensors (the *_dev entries of include/apsmatch.h) -------
+# Each function takes the arguments of its host counterpart, with per-image CUDA tensors where that one takes arrays,
+# and returns exactly what it returns.  Binary descriptors are named by isBinary=True (uint8 rows, binaryFeatures on the
+# host): a uint8 tensor alone is not binary, since vl_SIFT's uint8 descriptors are float descriptors, cast to float32 on
+# the device as single(allDesc) does (featureMatchingGlobal.m:81).  The tensors of a set are pooled with torch.cat on
+# their device and handed over on torch's current stream (producer_stream): no host copy, no host synchronisation.
+
+
+def _pool_device_sets(allDescriptorsSets, numImgs, isBinary):
+    """the per-image CUDA tensors of a sets call, pooled -> (ns, empty, counts, D, pooled, device): image counts, which
+    sets have no descriptors, rows per image, the one width, the pooled ROW-major [F x D] tensor (float32, or uint8 for
+    binary; None when no set has descriptors) and its device"""
+    import torch
+
+    sets = list(allDescriptorsSets) if allDescriptorsSets is not None else []
+    nums = list(np.atleast_1d(np.asarray(numImgs, dtype=np.float64)).ravel()) if np.size(numImgs) else []
+    if len(nums) != len(sets):
+        raise ValueError("numImgs must give one image count per descriptor set")
+    for v in nums:
+        if not (np.isfinite(v) and v > 0 and v == np.round(v)):
+            raise ValueError("every numImgs entry must be a positive integer")  # featureMatchingGlobal.m:35-39
+    want = torch.uint8 if isBinary else torch.float32
+    ns, empty, counts, parts = [], [], [], []
+    D = device = None
+    for cells, num in zip(sets, nums):
+        n = int(num)
+        cells = list(cells) if cells is not None else []
+        cells = (cells + [None] * n)[:n]
+        rows0 = len(parts)
+        for x in cells:
+            if x is not None and (not isinstance(x, torch.Tensor) or not x.is_cuda):
+                raise TypeError("device-input descriptors must be CUDA tensors (use the host functions for arrays)")
+            if x is None or x.numel() == 0:
+                counts.append(0)
+                continue
+            if x.dim() != 2:
+                raise ApsError(2, "flann_knn:type", "descriptors must be 2D")
+            if isBinary and x.dtype != torch.uint8:
+                raise ApsError(2, "flann_knn:type", "binary descriptors must be uint8")
+            if not isBinary and x.dtype not in (torch.float32, torch.float64, torch.uint8, torch.int8, torch.int16,
+                                                torch.int32, torch.int64):
+                raise ApsError(2, "flann_knn:type", "Descriptors must be single (float) or uint8 (binary)")
+            if D is not None and x.shape[1] != D:
+                raise ApsError(4, "flann_knn:dim", "all descriptor matrices must have the same number of columns")
+            if device is not None and x.device != device:
+                raise ValueError("all descriptor tensors must be on one CUDA device")
+            D, device = int(x.shape[1]), x.device
+            parts.append(x.to(want))        # single(allDesc), on the device
+            counts.append(int(x.shape[0]))
+        ns.append(n)
+        empty.append(len(parts) == rows0)
+    pooled = torch.cat(parts).contiguous() if parts else None
+    return ns, empty, counts, D, pooled, device
+
+
+def _device_ctx(ctx, device):
+    if ctx is None:
+        return default_context(device.index if device is not None and device.index is not None else 0)
+    if device is not None and device.index is not None and ctx.device != device.index:
+        raise ValueError(f"the tensors are on {device} but the context is on cuda:{ctx.device}")
+    return ctx
+
+
+CUDA_STREAM_LEGACY = 1   # cudaStreamLegacy: the legacy default stream, as a handle an event can be recorded on
+
+
+def _producer_stream(device):
+    """torch's current stream on `device`, for the call's stream to wait on.  torch reports its default stream as handle
+    0, which the C ABI reads as 'no producer' (a NULL producer_stream): it is passed as cudaStreamLegacy instead, since
+    the context's stream is non-blocking and would not otherwise wait for the work queued there."""
+    import torch
+
+    if device is None:
+        return C.c_void_p(0)
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream or CUDA_STREAM_LEGACY)
+
+
+def _pool_device_keypoints(keypointsSets, ns, counts, device):
+    """the keypoints of every set's images as CUDA tensors, pooled [F x 2] row-major like the descriptors ->
+    (tensor or None, APS_KP_F32 when every part is float32, else APS_KP_F64 with the parts converted to float64)"""
+    import torch
+
+    kps_sets = list(keypointsSets)
+    if len(kps_sets) != len(ns):
+        raise ValueError("keypointsSets must hold one keypoint set per descriptor set")
+    kps = []
+    for b, (n, ks) in enumerate(zip(ns, kps_sets)):
+        if len(ks) != n:
+            raise ValueError(f"keypointsSets[{b}] must contain n elements (one per image).")
+        kps += list(ks)
+    parts = []
+    for g, (kp, cnt) in enumerate(zip(kps, counts)):
+        if cnt:
+            if not isinstance(kp, torch.Tensor) or kp.device != device:
+                raise TypeError(f"image {g + 1}: the keypoints must be a CUDA tensor on the descriptors' device")
+            kp = kp.reshape(-1, 2)
+            if kp.shape[0] != cnt:
+                raise ValueError(f"image {g + 1}: the keypoints must have one row per descriptor row")
+            parts.append(kp)
+    if not parts:
+        return None, _lib.APS_KP_F64
+    if all(p.dtype == torch.float32 for p in parts):
+        return torch.cat(parts).contiguous(), _lib.APS_KP_F32
+    return torch.cat([p.to(torch.float64) for p in parts]).contiguous(), _lib.APS_KP_F64
+
+
+def featureMatchingGlobalSetsDevice(input, allDescriptorsSets, numImgs, ctx=None, *, isBinary=False):
+    """featureMatchingGlobalSets for descriptors in CUDA tensors (aps_feature_matching_global_sets_dev):
+    allDescriptorsSets[b][i] = image i's [N x D] tensor of set b (None or empty for an image without descriptors).
+    Returns exactly what featureMatchingGlobalSets returns for the same data on the host."""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by featureMatchingGlobalSetsDevice; match the sets on one GPU")
+    ns, _, counts, D, pooled, device = _pool_device_sets(allDescriptorsSets, numImgs, isBinary)
+    k = int(_field(input, "k", required=True))
+    ratio = float(_field(input, "Ratiothreshold", required=True))
+    use_bf = bool(_field(input, "BFMatch", 0))
+    mutual = bool(int(_field(input, "apsMutual", 0)))
+    B = len(ns)
+    if pooled is None:  # every set empty: cell(numImg) each, no device touched (featureMatchingGlobal.m:49-52)
+        return [[[np.zeros((0, 0)) for _ in range(n)] for _ in range(n)] for n in ns]
+    ctx = _device_ctx(ctx, device)
+    cnt = (C.c_int64 * len(counts))(*counts)
+    outs = (C.c_void_p * max(B, 1))()
+    check(lib().aps_feature_matching_global_sets_dev(ctx.handle, B, (C.c_int * max(B, 1))(*ns),
+                                                     C.c_void_p(pooled.data_ptr()), cnt, int(D),
+                                                     APS_U8 if isBinary else APS_F32, k, ratio, int(use_bf),
+                                                     int(mutual), _producer_stream(device), outs))
+    result = []
+    try:
+        for b in range(B):
+            result.append(_cells_from_matchlist(outs[b], ns[b])[0])
+    finally:
+        for b in range(B):
+            lib().aps_matchlist_free(outs[b])
+    return result
+
+
+def featureMatchingPairwiseSetsDevice(input, allDescriptorsSets, numImgs, ctx=None, return_metric=False, *,
+                                      isBinary=False):
+    """featureMatchingPairwiseSets for descriptors in CUDA tensors (aps_feature_matching_pairwise_sets_dev): reads the
+    same fields and returns exactly what featureMatchingPairwiseSets returns for the same data on the host."""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError("input.apsGPUs is not supported by featureMatchingPairwiseSetsDevice; match the sets on one GPU")
+    ns, empty, counts, D, pooled, device = _pool_device_sets(allDescriptorsSets, numImgs, isBinary)
+    method = str(_field(input, "Matchingmethod", "Exhaustive")).lower()
+    if method not in ("exhaustive", "approximate"):
+        raise ValueError(f"Unknown Method: {method}")  # matchFeaturesScratch.m:164-165
+    aps_method = _resolve_method(input, method)
+    thr = float(_field(input, "Matchingthreshold", required=True))
+    ratio = float(_field(input, "Ratiothreshold", required=True))
+
+    def empty_cells(n):
+        m, metrics = _empty_pairwise_cells(n)
+        return (m, metrics) if return_metric else m
+
+    B = len(ns)
+    if pooled is None:
+        return [empty_cells(n) for n in ns]
+    ctx = _device_ctx(ctx, device)
+    cnt = (C.c_int64 * len(counts))(*counts)
+    outs = (C.c_void_p * max(B, 1))()
+    check(lib().aps_feature_matching_pairwise_sets_dev(ctx.handle, B, (C.c_int * max(B, 1))(*ns),
+                                                       C.c_void_p(pooled.data_ptr()), cnt, int(D),
+                                                       APS_U8 if isBinary else APS_F32, thr, ratio, aps_method,
+                                                       int(_field(input, "apsSubset", 12000)),
+                                                       int(_field(input, "apsSeed", 0)), _producer_stream(device), outs))
+    result = []
+    try:
+        for b in range(B):
+            if empty[b]:
+                result.append(empty_cells(ns[b]))
+                continue
+            matches, metrics = _pairwise_cells(outs[b], ns[b])
+            result.append((matches, metrics) if return_metric else matches)
+    finally:
+        for b in range(B):
+            lib().aps_matchlist_free(outs[b])
+    return result
+
+
+def featureMatchingPairwiseDevice(input, allDescriptors, numImg, ctx=None, return_metric=False, *, isBinary=False):
+    """featureMatchingPairwise for descriptors in CUDA tensors: the one-set case of featureMatchingPairwiseSetsDevice,
+    exactly what featureMatchingPairwise(input, allDescriptors, numImg, return_metric=return_metric) returns for the same
+    data on the host (no shard= / csr= / input.apsGPUs)."""
+    if not (np.isscalar(numImg) and np.isfinite(numImg) and numImg > 0):
+        raise ValueError("numImg must be a positive finite scalar")
+    return featureMatchingPairwiseSetsDevice(input, [allDescriptors], [numImg], ctx=ctx, return_metric=return_metric,
+                                             isBinary=isBinary)[0]
+
+
+def _device_image_matching(verb, input, allDescriptorsSets, numImgs, keypointsSets, seed, return_matches, ctx,
+                           isBinary):
+    """globalImageMatching / pairwiseImageMatching of every set in one call on CUDA tensors
+    (aps_{global,pairwise}_image_matching_sets_dev) -> what _global_image_matching / _pairwise_image_matching return"""
+    if _field(input, "apsGPUs", None) is not None:
+        raise ValueError(f"input.apsGPUs is not supported by {verb}ImageMatching[Sets]Device; match the sets on one GPU")
+    _check_ransac_projective(input)
+    ns, empty, counts, D, pooled, device = _pool_device_sets(allDescriptorsSets, numImgs, isBinary)
+    kp, kp_dtype = _pool_device_keypoints(keypointsSets, ns, counts, device)
+    m = int(_field(input, "mBrownLowe", 6))
+    md, conf, mt = _ransac_params(input)
+    dtype = APS_U8 if isBinary else APS_F32
+    B = len(ns)
+    ctx = _device_ctx(ctx, device)
+    h = C.c_void_p()
+    head = (ctx.handle, B, (C.c_int * max(B, 1))(*ns), C.c_void_p(pooled.data_ptr() if pooled is not None else 0),
+            (C.c_int64 * max(len(counts), 1))(*counts), int(D or 0), dtype)
+    tail = (C.c_void_p(kp.data_ptr() if kp is not None else 0), kp_dtype, m, md, conf, mt, int(seed),
+            int(return_matches), _producer_stream(device), C.byref(h))
+    list_of = lambda lh, b, n: _cells_from_matchlist(lh, n)[0]   # noqa: E731
+    if verb == "global":
+        k = int(_field(input, "k", required=True))
+        ratio = float(_field(input, "Ratiothreshold", required=True))
+        use_bf = bool(_field(input, "BFMatch", 0))
+        mutual = bool(int(_field(input, "apsMutual", 0)))
+        check(lib().aps_global_image_matching_sets_dev(*head, k, ratio, int(use_bf), int(mutual), *tail))
+    else:
+        method = str(_field(input, "Matchingmethod", "Exhaustive")).lower()
+        if method not in ("exhaustive", "approximate"):
+            raise ValueError(f"Unknown Method: {method}")  # matchFeaturesScratch.m:164-165
+        aps_method = _resolve_method(input, method)
+        thr = float(_field(input, "Matchingthreshold", required=True))
+        ratio = float(_field(input, "Ratiothreshold", required=True))
+        subset, subset_seed = int(_field(input, "apsSubset", 12000)), int(_field(input, "apsSeed", 0))
+        check(lib().aps_pairwise_image_matching_sets_dev(*head, thr, ratio, aps_method, subset, subset_seed, *tail))
+
+        def list_of(lh, b, n):   # what featureMatchingPairwiseSets(..., return_metric=True) returns for set b
+            return _empty_pairwise_cells(n) if empty[b] else _pairwise_cells(lh, n)
+    try:
+        return _image_matches_result(h, ns, return_matches, list_of)
+    finally:
+        lib().aps_image_matches_free(h)
+
+
+def globalImageMatchingSetsDevice(input, allDescriptorsSets, numImgs, keypointsSets, seed=0, return_matches=False,
+                                  ctx=None, *, isBinary=False):
+    """globalImageMatchingSets for descriptors and keypoints in CUDA tensors (aps_global_image_matching_sets_dev):
+    keypointsSets[b][i] = image i's [N x 2] float64 or float32 tensor.  Returns exactly what globalImageMatchingSets
+    returns for the same data on the host, and sets globalImageMatchingSetsDevice.last the same way."""
+    results, globalImageMatchingSetsDevice.last, lists = _device_image_matching(
+        "global", input, allDescriptorsSets, numImgs, keypointsSets, seed, return_matches, ctx, isBinary)
+    return (results, lists) if return_matches else results
+
+
+def globalImageMatchingDevice(input, allDescriptors, numImg, keypoints, seed=0, return_matches=False, ctx=None, *,
+                              isBinary=False):
+    """globalImageMatching for CUDA tensors: the one-set case of globalImageMatchingSetsDevice."""
+    if not (np.isscalar(numImg) and np.isfinite(numImg) and numImg > 0):
+        raise ValueError("numImg must be a positive finite scalar")  # featureMatchingGlobal.m:35-39
+    results, lasts, lists = _device_image_matching("global", input, [allDescriptors], [numImg], [keypoints], seed,
+                                                   return_matches, ctx, isBinary)
+    globalImageMatchingDevice.last = lasts[0]
+    return (results[0], lists[0]) if return_matches else results[0]
+
+
+def pairwiseImageMatchingSetsDevice(input, allDescriptorsSets, numImgs, keypointsSets, seed=0, return_matches=False,
+                                    ctx=None, *, isBinary=False):
+    """pairwiseImageMatchingSets for descriptors and keypoints in CUDA tensors (aps_pairwise_image_matching_sets_dev):
+    exactly what pairwiseImageMatchingSets returns for the same data on the host; .last as there."""
+    results, pairwiseImageMatchingSetsDevice.last, lists = _device_image_matching(
+        "pairwise", input, allDescriptorsSets, numImgs, keypointsSets, seed, return_matches, ctx, isBinary)
+    return (results, lists) if return_matches else results
+
+
+def pairwiseImageMatchingDevice(input, allDescriptors, numImg, keypoints, seed=0, return_matches=False, ctx=None, *,
+                                isBinary=False):
+    """pairwiseImageMatching for CUDA tensors: the one-set case of pairwiseImageMatchingSetsDevice."""
+    if not (np.isscalar(numImg) and np.isfinite(numImg) and numImg > 0):
+        raise ValueError("numImg must be a positive finite scalar")
+    results, lasts, lists = _device_image_matching("pairwise", input, [allDescriptors], [numImg], [keypoints], seed,
+                                                   return_matches, ctx, isBinary)
+    pairwiseImageMatchingDevice.last = lasts[0]
+    return (results[0], lists[0]) if return_matches else results[0]
+
+
 def _csr_from_matchlist(h, n):
     L = lib()
     total = L.aps_matchlist_total(h)

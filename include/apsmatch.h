@@ -16,7 +16,8 @@
  *     r + c*N); APS_ROW_MAJOR is a C / NumPy [N][D] array.  Outputs that are matrices use the same
  *     layout as the inputs of the call.
  *   - indices returned are 1-based, exactly as the reference returns them.
- *   - host entry points (aps_*) take HOST pointers and are synchronous.  The staged plan API
+ *   - host entry points (aps_*) take HOST pointers and are synchronous; the *_dev entries take their descriptors and
+ *     keypoints as DEVICE pointers and are synchronous too (outputs on the host).  The staged plan API
  *     (aps_gplan_*) exposes the same pipeline step by step on the context's stream, with DEVICE
  *     buffers reachable for collectives (NCCL broadcast / all-gather between ranks).
  */
@@ -157,7 +158,9 @@ int aps_feature_matching_global(aps_ctx* ctx, const void* const* desc, const int
 /* Same stage for descriptors that already live on the device (the step before the path, PP/featureMatching/
  * getFeaturePoints.m:32-74 -> allDescriptors, when the extractor runs on the GPU): d_pooled = pooled ROW-major [F x D]
  * device matrix (image i = rows sum(counts[0..i)) ...), float32 or uint8.  mutual != 0 adds the opt-in cross-check
- * (aps_gplan_filter_mutual).  The match list comes back on the host like aps_feature_matching_global's. */
+ * (aps_gplan_filter_mutual).  The match list comes back on the host like aps_feature_matching_global's.
+ * The one-set case of aps_feature_matching_global_sets_dev (no producer stream), except that the context is checked
+ * first. */
 int aps_feature_matching_global_dev(aps_ctx* ctx, const void* d_pooled, const int64_t* counts, int n, int D, int dtype,
                                     int k, double ratio, int mutual, aps_matchlist** out);
 
@@ -384,6 +387,47 @@ int aps_pairwise_image_matching(aps_ctx* ctx, const void* const* desc, const int
                                 uint64_t subset_seed, const double* keypoints, int m, double max_distance,
                                 double confidence, int max_trials, uint64_t seed, int want_lists,
                                 aps_image_matches** out);
+
+/* ---- device input: the sets entries for descriptors and keypoints already on the GPU ------------------------------
+ * When the extractor runs on the GPU (PP/featureMatching/getFeaturePoints.m:32-74 -> allDescriptors, keypoints), these
+ * take its output where it is instead of host copies.  Each takes the arguments of its host counterpart, except:
+ *   d_pooled     replaces desc / layout: ONE pooled ROW-major [F x D] device matrix, float32 (APS_F32) or uint8 (APS_U8),
+ *                holding the images of all sets one after another in `counts` order (image g = the counts[g] rows
+ *                after those of images 0 .. g-1), as the sets entries pool them;
+ *   d_keypoints  (fused entries) replaces keypoints: ONE pooled ROW-major [F x 2] device array in the same image order,
+ *   kp_dtype     float64 (APS_KP_F64) or float32 (APS_KP_F32, widened exactly to double on the device);
+ *   producer_stream  a cudaStream_t, or NULL.  Non-NULL: the call records an event on it and the context's stream waits
+ *                for that event, so a producer on another stream hands over without a host synchronisation.  NULL: the
+ *                caller guarantees the data is ready.  NULL is not the default stream here: a producer on the legacy
+ *                default stream passes cudaStreamLegacy (per-thread default stream: cudaStreamPerThread), since the
+ *                context's own stream is non-blocking and does not wait for it.
+ * The descriptors enter the pass with one device-to-device copy where the host entry uploads per image; from there the
+ * call runs the host entry's pass, so every output is BIT-IDENTICAL to the host entry given the same data on the host.
+ * Outputs are on the host, as the host entries return them.  The device data are only read, and only until the call
+ * returns.  Argument checks, all before any device work: the host entry's statuses first (a NULL d_keypoints with rows
+ * is its NULL keypoints); then APS_ERR_TYPE for a kp_dtype other than the two; then APS_ERR_ARGS for a NULL d_pooled
+ * with rows; then the context (APS_ERR_NOGPU); then APS_ERR_ARGS for a d_pooled or d_keypoints that is neither device
+ * nor managed memory (cudaPointerGetAttributes).  nsets == 1 is the one-set call, run by the host entry's one-set path
+ * (same launches and context statistics); there are no separate one-set entries. */
+enum aps_kp_dtype { APS_KP_F64 = 0, APS_KP_F32 = 1 };
+int aps_feature_matching_global_sets_dev(aps_ctx* ctx, int nsets, const int* set_images, const void* d_pooled,
+                                         const int64_t* counts, int D, int dtype, int k, double ratio, int use_bf,
+                                         int mutual, void* producer_stream, aps_matchlist** out);
+int aps_feature_matching_pairwise_sets_dev(aps_ctx* ctx, int nsets, const int* set_images, const void* d_pooled,
+                                           const int64_t* counts, int D, int dtype, double match_threshold,
+                                           double max_ratio, int method, int64_t subset, uint64_t seed,
+                                           void* producer_stream, aps_matchlist** out);
+int aps_global_image_matching_sets_dev(aps_ctx* ctx, int nsets, const int* set_images, const void* d_pooled,
+                                       const int64_t* counts, int D, int dtype, int k, double ratio, int use_bf,
+                                       int mutual, const void* d_keypoints, int kp_dtype, int m, double max_distance,
+                                       double confidence, int max_trials, uint64_t seed, int want_lists,
+                                       void* producer_stream, aps_image_matches** out);
+int aps_pairwise_image_matching_sets_dev(aps_ctx* ctx, int nsets, const int* set_images, const void* d_pooled,
+                                         const int64_t* counts, int D, int dtype, double match_threshold,
+                                         double max_ratio, int method, int64_t subset, uint64_t subset_seed,
+                                         const void* d_keypoints, int kp_dtype, int m, double max_distance,
+                                         double confidence, int max_trials, uint64_t seed, int want_lists,
+                                         void* producer_stream, aps_image_matches** out);
 
 /* ---- staged global pipeline (building block of the multi-GPU host; bench.py times these) -----
  * The stages of PP/featureMatching/featureMatchingGlobal.m as separate calls: pooling + normalisation :70-97
